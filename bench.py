@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - headline measurement of the hot path (BASELINE.json: env-steps/sec; TD3 updates/sec rides along).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 Workload at every N (weak scaling, per GPU): BASELINE.json configs[1] - a batched dynamics rollout of 4096 envs,
 random actions U(-7.5, 7.5), 1000 steps.  One bench "step" = LAUNCHES_PER_STEP such rollouts back to back (one launch of the
@@ -41,6 +41,22 @@ def make_workload(rank, n, T, buffers):
     starts = rs.uniform(0, 98.9999, (n, 2)).astype(np.float32)
     acts = [rs.uniform(-ACTION_RANGE, ACTION_RANGE, (T, 2, n)).astype(np.float32) for _ in range(buffers)]
     return starts, acts
+
+
+DUMP_BYTES = 60 * 10 ** 6   # --dump-outputs stays under 64 MB, .npy headers included
+
+
+def dump_outputs(out_dir, state, traj):
+    """What a caller of rtd3_env_rollout receives from the last launch of the last timed step: the final state `[2,n]` and the
+    trajectory `[T,2,n]` (float32).  A trajectory over the budget keeps a fixed, seeded sample of env columns."""
+    T, _, n = traj.shape
+    keep = min(n, (DUMP_BYTES - state.numel() * 4) // (T * 2 * 4))
+    traj = traj.cpu().numpy()
+    if keep < n:
+        traj = traj[:, :, np.sort(np.random.RandomState(0).choice(n, keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "final_state.npy"), state.cpu().numpy())
+    np.save(os.path.join(out_dir, "trajectory.npy"), np.ascontiguousarray(traj))
 
 
 def load_peaks():
@@ -571,6 +587,9 @@ def run_b200(args):
     e1.record(stream)
     barrier()
     launches = rt._lib.launch_count()
+    if args.dump_outputs and rank == 0:
+        last = ((args.warmup + args.steps) * LPS - 1) % R            # trajectory buffer of the last launch of the last step
+        dump_outputs(args.dump_outputs, env._state, trajs[last])
     ms = e0.elapsed_time(e1)
     if world > 1:
         t = torch.tensor([ms], device=dev, dtype=torch.float64)
@@ -582,7 +601,7 @@ def run_b200(args):
     # ---- e2e: host action buffers -> public API -> host trajectory, copies inside the timed region
     h_act = [torch.from_numpy(acts_np[j % R].copy()).pin_memory() for j in range(2)]      # the workload's actions, in pinned host memory
     h_traj = [torch.empty((T, 2, n), dtype=torch.float32).pin_memory() for _ in range(2)]
-    e2e_steps = max(3, min(args.steps, 20))
+    e2e_steps = args.steps
     EPS = E2E_CALLS_PER_STEP
 
     def e2e_step(k):
@@ -736,7 +755,11 @@ def main():
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--no-td3", action="store_true")
     ap.add_argument("--no-loop", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the final state and trajectory of the last rollout as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version banner to stdout on the
     # first communicator): point fd 1 at stderr for the whole run and keep the real stdout for the result line only.
     global _RESULT_FD

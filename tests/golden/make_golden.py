@@ -594,3 +594,34 @@ def make_demo():
 
 if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "demo":
     make_demo()
+
+
+def make_adam():
+    """torch.optim.Adam (the reference's optimiser, robot.py:237-239) on CPU: five steps on 100003 parameters from
+    torch.manual_seed(0), recorded on an x86 CPU with torch's AVX-512 kernels (the operation order oracle/td3_oracle.py adam_step
+    restates).  The step is elementwise, so a seeded sample of 2048 elements is stored: inputs, exp_avg, exp_avg_sq and parameters
+    after every step."""
+    import torch
+    torch.manual_seed(0)
+    n, steps = 100003, 5
+    p0 = torch.randn(n)
+    par = torch.nn.Parameter(p0.clone())
+    opt = torch.optim.Adam([par], lr=1e-3)
+    grads, m, v, p = [], [], [], []
+    for _ in range(steps):
+        g = (torch.randn(n) * 0.05 * torch.rand(n)).numpy().astype(np.float32)
+        par.grad = torch.from_numpy(g.copy())
+        opt.step()
+        grads.append(g)
+        m.append(opt.state[par]["exp_avg"].numpy().copy())
+        v.append(opt.state[par]["exp_avg_sq"].numpy().copy())
+        p.append(par.detach().numpy().copy())
+    idx = np.sort(np.random.RandomState(0).choice(n, 2048, replace=False))
+    out = {"cpu_capability": np.array(torch.backends.cpu.get_cpu_capability()), "p0": p0.numpy()[idx],
+           "grad": np.stack(grads)[:, idx], "exp_avg": np.stack(m)[:, idx], "exp_avg_sq": np.stack(v)[:, idx], "param": np.stack(p)[:, idx]}
+    np.savez_compressed(os.path.join(HERE, "adam_golden.npz"), **out)
+    print("adam_golden.npz written:", {k: v.shape for k, v in out.items()})
+
+
+if __name__ == "__main__" and len(sys.argv) > 1 and sys.argv[1] == "adam":
+    make_adam()

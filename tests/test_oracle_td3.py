@@ -4,6 +4,8 @@ Tolerance (BASELINE.json north_star): losses and Q-values within 1e-3 relative a
 Parameters: after one Adam step every element has moved by lr * m_hat / (sqrt(v_hat) + eps) ~ +-1e-5, so they are compared
 on the update itself.
 """
+import os
+
 import numpy as np
 
 from oracle import td3_oracle as to
@@ -112,22 +114,19 @@ def test_td3_update_six_epochs(td3_golden):
 def test_adam_step_bit_exact_vs_torch():
     """oracle adam_step == torch.optim.Adam on CPU, element for element over five steps (exp_avg, exp_avg_sq bit-exact; parameters
     bit-exact but for the rare element where torch's vectorised division rounds the other way: >= 99.99 %).  The CUDA kernels apply
-    the same operation order (csrc/rtd3_td3.cuh: adam_element)."""
-    import torch
-    torch.manual_seed(0)
-    n = 100003
-    p0 = torch.randn(n)
-    par = torch.nn.Parameter(p0.clone())
-    opt = torch.optim.Adam([par], lr=1e-3)
-    st = to.AdamState(n)
-    p = p0.numpy().copy()
-    for step in range(5):
-        g = (torch.randn(n) * 0.05 * torch.rand(n)).numpy().astype(np.float32)
-        par.grad = torch.from_numpy(g.copy())
-        opt.step()
-        to.adam_step(p, g, st, lr=1e-3)
-        assert (st.m == opt.state[par]["exp_avg"].numpy()).all()
-        assert (st.v == opt.state[par]["exp_avg_sq"].numpy()).all()
-        tp = par.detach().numpy()
-        assert (p == tp).mean() >= 0.9999 and np.abs(p - tp).max() <= 2.4e-7 * max(1.0, float(np.abs(tp).max()))
+    the same operation order (csrc/rtd3_td3.cuh: adam_element).  torch's results are the stored ones (tests/golden/make_golden.py
+    adam): which kernels torch runs, and so how it rounds, depends on the CPU it runs on.  They are a sample of 2048 elements, too
+    few for a rate of 1 in 10^4 in one step, so the rate is taken over the five steps together."""
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "adam_golden.npz"))
+    st = to.AdamState(g["p0"].size)
+    p = g["p0"].copy()
+    equal = []
+    for step in range(g["grad"].shape[0]):
+        to.adam_step(p, g["grad"][step], st, lr=1e-3)
+        assert (st.m == g["exp_avg"][step]).all()
+        assert (st.v == g["exp_avg_sq"][step]).all()
+        tp = g["param"][step]
+        equal.append(p == tp)
+        assert np.abs(p - tp).max() <= 2.4e-7 * max(1.0, float(np.abs(tp).max()))
         p[...] = tp                                      # continue from torch's parameters: the next step is again element-exact
+    assert np.mean(equal) >= 0.9999
