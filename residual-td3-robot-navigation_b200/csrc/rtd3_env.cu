@@ -31,8 +31,41 @@ __global__ void build_table_kernel(const float* __restrict__ speed, const float*
 }
 
 
-// Stage the 80 KB table into shared memory with bulk-async copies signalled on one mbarrier.
-// All threads of the CTA call this; returns once the table is readable.
+// ---- halo table of the warp-pair rollout -----------------------------------------------------------------------------
+// The pair kernel's chain warp takes the table address of step t+1 from the UNCLIPPED next state of step t, which keeps the
+// clip to [0, 98.9999] off its dependent chain.  On a map that fits (every cell moves a state by at most kHaloReach < 8 per
+// step under actions clipped to +-kMaxAction) an unclipped coordinate v of a state that was in [0, 98.9999] lies in
+// [-8, 107), and the halo table is laid out so that halo[floor(v) + 8] == table[floor(clip(v))] there: indices 0..7 repeat
+// cell 0, 8..106 are cells 0..98 and 107..114 repeat cell 98.  Cell 99 is reachable only from a state in [99, 100) (a start
+// state, or one kept through NaN actions); it sits at index 115, and an address taken from a state maps 107 to it.
+constexpr int kHalo = 8;
+constexpr int kHaloDim = kWorld + 2 * kHalo;                                   // 116
+constexpr uint32_t kHaloBytes = kHaloDim * kHaloDim * sizeof(float2);          // 107 648 B
+constexpr uint32_t kHaloRowBytes = kHaloDim * sizeof(float2);
+constexpr float kHaloReach = 7.99f;   // < 8 with room for the two roundings of the step
+static_assert(kHaloBytes % (16 * kTableChunks) == 0, "bulk copy sizes must be multiples of 16 B");
+
+__device__ __forceinline__ int halo_cell(int i) {
+  return i < kHalo ? 0 : i < kWorld - 1 + kHalo ? i - kHalo : i < kHaloDim - 1 ? kWorld - 2 : kWorld - 1;
+}
+
+// One CTA: copies the finished table into the halo layout and writes whether the map fits, in device memory so that
+// rtd3_env_set_map stays asynchronous (and capturable).  Non-finite cells were zeroed by build_table_kernel and fit.
+__global__ void __launch_bounds__(1024) build_halo_kernel(const float2* __restrict__ table, float2* __restrict__ halo, int* __restrict__ fits) {
+  bool ok = true;
+  for (int i = threadIdx.x; i < kCells; i += blockDim.x) {
+    const float2 cs = table[i];
+    ok = ok && kMaxAction * (fabsf(cs.x) + fabsf(cs.y)) <= kHaloReach;
+  }
+  for (int i = threadIdx.x; i < kHaloDim * kHaloDim; i += blockDim.x)
+    halo[i] = table[halo_cell(i / kHaloDim) * kWorld + halo_cell(i % kHaloDim)];
+  ok = __syncthreads_and(ok);
+  if (threadIdx.x == 0) *fits = ok ? 1 : 0;
+}
+
+// Stage a table (kBytes: the 80 KB plain one or the 105 KB halo one) into shared memory with bulk-async copies signalled
+// on one mbarrier.  All threads of the CTA call this; returns once the copies are issued, mbar_wait(bar, 0) waits for them.
+template <uint32_t kBytes = kTableBytes>
 __device__ __forceinline__ void stage_table(float2* s_table, uint64_t* bar, const float2* __restrict__ g_table) {
   if (threadIdx.x == 0) {
     mbar_init(bar, 1);
@@ -40,8 +73,8 @@ __device__ __forceinline__ void stage_table(float2* s_table, uint64_t* bar, cons
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    mbar_arrive_expect_tx(bar, kTableBytes);
-    constexpr uint32_t chunk = kTableBytes / kTableChunks;
+    mbar_arrive_expect_tx(bar, kBytes);
+    constexpr uint32_t chunk = kBytes / kTableChunks;
 #pragma unroll
     for (int c = 0; c < kTableChunks; ++c)
       bulk_g2s(reinterpret_cast<char*>(s_table) + c * chunk, reinterpret_cast<const char*>(g_table) + c * chunk, chunk,
@@ -112,6 +145,12 @@ constexpr int kU = 16;
 constexpr int kDeep = 8;      // chunks in flight per thread, latency-bound launches (128 steps of lead)
 constexpr int kShallow = 2;   // chunks in flight per thread, occupancy-bound launches
 
+__device__ __forceinline__ float2 lds_f2(uint32_t addr) {
+  float2 v;
+  asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(v.x), "=f"(v.y) : "r"(addr));
+  return v;
+}
+
 // The dependent chain of one rollout step.  trunc(x) comes from a round-toward-zero add of 2^23 (the low mantissa
 // bits of x + 2^23 are floor(x) for 0 <= x < 2^23), so the shared-memory byte address is two IMADs away from the state:
 //   addr = bits(x+2^23)*800 + bits(y+2^23)*8 + (table_base - 0x4B000000*808)
@@ -119,9 +158,25 @@ __device__ __forceinline__ void rollout_step(uint32_t addr_bias, const StepIn& i
   const uint32_t bx = __float_as_uint(__fadd_rz(x, 8388608.0f));
   const uint32_t by = __float_as_uint(__fadd_rz(y, 8388608.0f));
   const uint32_t addr = bx * 800u + (by * 8u + addr_bias);
-  float2 cs;
-  asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(cs.x), "=f"(cs.y) : "r"(addr));
-  advance(cs, in, x, y);
+  advance(lds_f2(addr), in, x, y);
+}
+
+// Halo-table addresses (addr_bias = table base - 0x4B000000 * (kHaloRowBytes + 8)).  With 2^23 + 8 every v in [-8, 107)
+// stays in the binade whose grid is 1, so the low bits of v + 2^23 + 8, rounded toward zero, are exactly floor(v) + 8
+// (with 2^23 a v in (-1, 0) would fall to the 0.5 grid below 2^23 and floor wrongly).
+__device__ __forceinline__ uint32_t halo_addr(uint32_t addr_bias, float x, float y) {
+  const uint32_t bx = __float_as_uint(__fadd_rz(x, 8388616.0f));
+  const uint32_t by = __float_as_uint(__fadd_rz(y, 8388616.0f));
+  return bx * kHaloRowBytes + (by * 8u + addr_bias);
+}
+// the address of table[floor(x)][floor(y)] for a state in [0, 100): index 107 (floor 99) is cell 99, stored at 115
+__device__ __forceinline__ uint32_t halo_addr_state(uint32_t addr_bias, float x, float y) {
+  constexpr uint32_t k99 = 0x4B000000u + kHalo + kWorld - 1;
+  uint32_t bx = __float_as_uint(__fadd_rz(x, 8388616.0f));
+  uint32_t by = __float_as_uint(__fadd_rz(y, 8388616.0f));
+  bx = bx == k99 ? bx + kHalo : bx;
+  by = by == k99 ? by + kHalo : by;
+  return bx * kHaloRowBytes + (by * 8u + addr_bias);
 }
 
 // Actions reach the SM through a per-thread cp.async ring in shared memory: kStages chunks of kU steps are in
@@ -323,32 +378,35 @@ env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x
 // ---- T-step rollout, warp-pair variant: chain warp + helper warp per 32 envs -------------------------------------------
 // At 4096 envs every SM gets one warp, and that warp's issue slots - not memory - bound the TMA kernel above (31
 // instr/step, of which only 13 are the state recurrence; ncu r1: 42 % fixed-latency waits).  Here the recurrence runs
-// alone on the CHAIN warp (per step: one LDS.64 of the pre-clipped action, the 13-instruction chain, two STS of the new
-// state); a HELPER warp on another scheduler of the same SM waits for the TMA action tiles, clips them (or flags the
-// chunk for the careful NaN path), re-arms the loads and issues the trajectory tile stores.  The two meet on mbarriers
-// over double-buffered shared-memory tiles.
+// alone on the CHAIN warp (per step: one LDS.64 of the pre-clipped action, the chain, two STS of the new state); a
+// HELPER warp on another scheduler of the same SM waits for the TMA action tiles, clips them (or flags the chunk for the
+// careful NaN path), re-arms the loads and issues the trajectory tile stores.  The two meet on mbarriers over
+// double-buffered shared-memory tiles.  The table is the halo table (see kHalo), so that on a map that fits, the chain
+// of a step is FFMA, FFMA -> FADD.RZ -> IMAD, IMAD -> LDS.64: the clip, the action load and the trajectory stores are
+// issued while the table load is in flight.
 constexpr int kPairU = 32;        // steps per tile of the pair kernel
-constexpr int kPairStages = 4;    // action tiles in flight (128 steps of lead, as kDeep x kU)
+constexpr int kPairStages = 4;    // action tiles in flight (128 steps of lead, as kDeep x kU), one pair per CTA
+constexpr int kPairStages2 = 3;   // two pairs per CTA: 4 stages do not fit next to the halo table
 struct PairSmem {
   static constexpr int kBars = 16;   // full[8] | prepped[2] | consumed[2] | outfull[2] | outfree[2]
 };
 
 template <bool kTraj, int kStages, int kUp>
 __global__ void __launch_bounds__(256)
-env_rollout_pair_kernel(const float2* __restrict__ g_table, float* __restrict__ x, float* __restrict__ y,
+env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict__ g_fits, float* __restrict__ x, float* __restrict__ y,
                         const __grid_constant__ CUtensorMap tm_act, const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int kU = kUp;                            // steps per action / trajectory tile of this kernel (shadows the file-wide kU)
   constexpr int kTileFloats = kU * 2 * 32;
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
-  uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);
+  uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kHaloBytes);
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, npairs = blockDim.x >> 6;
   const int pair = warp >> 1;
   const bool is_chain = (warp & 1) == 0;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes + 16) + pair * PairSmem::kBars;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + kHaloBytes + 16) + pair * PairSmem::kBars;
   uint64_t* full = bars, *prepped = bars + 8, *consumed = bars + 10, *outfull = bars + 12, *outfree = bars + 14;
   // per pair: kStages raw tiles | 2 prepped tiles (float2 per step and env = 2 tiles' worth each... [kU][32] float2 = 4 KB) | 2 out tiles
-  float* tiles = reinterpret_cast<float*>(smem_raw + ((kTableBytes + 16 + npairs * PairSmem::kBars * 8 + 127) & ~127u));
+  float* tiles = reinterpret_cast<float*>(smem_raw + ((kHaloBytes + 16 + npairs * PairSmem::kBars * 8 + 127) & ~127u));
   float* my = tiles + (size_t)pair * (kStages + 4) * kTileFloats;
   float* raw = my;                                   // [kStages][kU*2][32]
   float2* prep = reinterpret_cast<float2*>(my + kStages * kTileFloats);                 // [2][kU][32]
@@ -360,7 +418,7 @@ env_rollout_pair_kernel(const float2* __restrict__ g_table, float* __restrict__ 
     for (int b = 0; b < 2; ++b) { mbar_init(prepped + b, 32); mbar_init(consumed + b, 32); mbar_init(outfull + b, 32); mbar_init(outfree + b, 1); }
     fence_mbar_init();
   }
-  stage_table(s_table, bar, g_table);   // contains the __syncthreads that publishes the barrier inits
+  stage_table<kHaloBytes>(s_table, bar, g_halo);   // contains the __syncthreads that publishes the barrier inits
 
   const int64_t i0 = ((int64_t)blockIdx.x * npairs + pair) * 32;
   if (i0 >= n) return;
@@ -430,36 +488,53 @@ env_rollout_pair_kernel(const float2* __restrict__ g_table, float* __restrict__ 
   // ================================= chain warp =================================
   const int64_t i = i0 + lane;
   const bool live = i < n;
+  const bool fits = *g_fits != 0;                    // lands while the table is staging
   float sx = live ? fminf(fmaxf(x[i], 0.0f), 99.99999f) : 0.0f;
   float sy = live ? fminf(fmaxf(y[i], 0.0f), 99.99999f) : 0.0f;
-  const uint32_t addr_bias = smem_u32(s_table) - 0x4B000000u * 808u;
+  const uint32_t addr_bias = smem_u32(s_table) - 0x4B000000u * (kHaloRowBytes + 8u);
   mbar_wait(bar, 0);
   for (int64_t c = 0; c < chunks; ++c) {
     const int b = (int)(c & 1);
     mbar_wait(prepped + b, (uint32_t)((c >> 1) & 1));
     if (kTraj && c >= 2) mbar_wait(outfree + b, (uint32_t)(((c >> 1) - 1) & 1));   // out tile b has been stored (chunk c-2)
     const bool careful = s_flag[pair][b] != 0;
-    const float2* tp = prep + b * (kU * 32) + lane;
-    float* tout = outt + b * kTileFloats + lane;
-    if (!careful) {
+    const uint32_t tp = smem_u32(prep + b * (kU * 32) + lane);
+    const uint32_t tout = smem_u32(outt + b * kTileFloats + lane);
+    auto store_state = [&](int u) {                  // the state after step u into the trajectory tile
+      asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u) * 128u), "f"(sx) : "memory");
+      asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u + 1) * 128u), "f"(sy) : "memory");
+    };
+    if (!careful && fits) {
+      // Step 0 is addressed from the state (which may be in [99, 100) after NaN actions) and step 1 from its clipped
+      // successor; every later step from the unclipped successor of the step before.  The previous step's trajectory
+      // stores follow the table load in program order: issued before it, ptxas put them between the address IMAD and the
+      // load (a store may not move past a load that could alias it).  The next step's action is loaded one step ahead.
+      float2 a = lds_f2(tp);
+      uint32_t addr = halo_addr_state(addr_bias, sx, sy);
 #pragma unroll
       for (int u = 0; u < kU; ++u) {
-        const float2 a = tp[u * 32];
-        StepIn in;
-        in.ax = a.x; in.ay = a.y; in.lo = 0.0f; in.hi = kClipHi; in.bad = false;
-        rollout_step(addr_bias, in, sx, sy);
-        if (kTraj) { tout[(2 * u) * 32] = sx; tout[(2 * u + 1) * 32] = sy; }
+        const float2 cs = lds_f2(addr);
+        if (kTraj && u > 0) store_state(u - 1);
+        const float2 an = u + 1 < kU ? lds_f2(tp + (u + 1) * 256u) : a;
+        const float nx = fmaf(a.x, cs.x, fmaf(-a.y, cs.y, sx));
+        const float ny = fmaf(a.x, cs.y, fmaf(a.y, cs.x, sy));
+        sx = fminf(fmaxf(nx, 0.0f), kClipHi);
+        sy = fminf(fmaxf(ny, 0.0f), kClipHi);
+        addr = u == 0 ? halo_addr(addr_bias, sx, sy) : halo_addr(addr_bias, nx, ny);
+        a = an;
       }
+      if (kTraj) store_state(kU - 1);
     } else {
+      // NaN / inf actions, the ragged last chunk, or a map that does not fit: every step addressed from the state
       const int steps = (int)min((int64_t)kU, T - c * kU);
 #pragma unroll
       for (int u = 0; u < kU; ++u) {
         if (u < steps) {
-          const float2 a = tp[u * 32];
+          const float2 a = lds_f2(tp + u * 256u);
           const StepIn in = prep_action(a.x, a.y);
-          rollout_step(addr_bias, in, sx, sy);
+          advance(lds_f2(halo_addr_state(addr_bias, sx, sy)), in, sx, sy);
         }
-        if (kTraj) { tout[(2 * u) * 32] = sx; tout[(2 * u + 1) * 32] = sy; }
+        if (kTraj) store_state(u);
       }
     }
     mbar_arrive(consumed + b);
@@ -629,9 +704,13 @@ int32_t rtd3_env_create(rtd3_env** out, int32_t device) {
   h->device = device;
   h->has_map = false;
   h->table = nullptr;
+  h->halo = nullptr;
+  h->halo_fits = nullptr;
   h->host_pipe = nullptr;
   RTD3_CUDA(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, device));
   RTD3_CUDA(cudaMalloc(&h->table, kTableBytes));
+  RTD3_CUDA(cudaMalloc(&h->halo, kHaloBytes));
+  RTD3_CUDA(cudaMalloc(&h->halo_fits, sizeof(int)));
   if (!g_encode_tiled) load_encode_tiled();
   const int smem = kTableBytes + 16;
   RTD3_CUDA(cudaFuncSetAttribute(env_step_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -643,6 +722,8 @@ int32_t rtd3_env_create(rtd3_env** out, int32_t device) {
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<false, kShallow>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<true, kPairStages, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<false, kPairStages, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
+  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<true, kPairStages2, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
+  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<false, kPairStages2, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_tma_kernel<true, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_tma_kernel<false, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_tma_kernel<true, kShallow>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
@@ -656,6 +737,8 @@ int32_t rtd3_env_destroy(rtd3_env* h) {
   if (!h) return 0;
   rtd3::host_pipe_destroy(h);
   if (h->table) cudaFree(h->table);
+  if (h->halo) cudaFree(h->halo);
+  if (h->halo_fits) cudaFree(h->halo_fits);
   delete h;
   return 0;
 }
@@ -663,6 +746,8 @@ int32_t rtd3_env_destroy(rtd3_env* h) {
 int32_t rtd3_env_set_map(rtd3_env* h, const float* speed, const float* angle, void* stream) {
   RTD3_CHECK_ARG(h && speed && angle, "null argument");
   build_table_kernel<<<(int)ceil_div(kCells, 256), 256, 0, (cudaStream_t)stream>>>(speed, angle, h->table);
+  RTD3_LAUNCHED();
+  build_halo_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(h->table, h->halo, h->halo_fits);
   RTD3_LAUNCHED();
   h->has_map = true;
   return 0;
@@ -736,10 +821,12 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
       // (the per-tile hand-over - two barrier waits, the flag read, two arrives - was ~20 % of the chain warp's samples at 16)
       const int ppc = (int)std::max<int64_t>(1, std::min<int64_t>(2, ceil_div(warps_total, (int64_t)h->num_sms)));
       const int pgrid = (int)ceil_div(warps_total, ppc);
-      const int psmem = ((kTableBytes + 16 + ppc * PairSmem::kBars * 8 + 127) & ~127) + ppc * (kPairStages + 4) * (kPairU * 2 * 32) * 4;
+      const int pstages = ppc == 1 ? kPairStages : kPairStages2;
+      const int psmem = ((kHaloBytes + 16 + ppc * PairSmem::kBars * 8 + 127) & ~127) + ppc * (pstages + 4) * (kPairU * 2 * 32) * 4;
       if (make_plane_map(&tm_act, actions, n, T, kPairU) != 0 || make_plane_map(&tm_traj, traj ? traj : actions, n, T, kPairU) != 0) return RTD3_ERR_STATE;
-      if (traj) env_rollout_pair_kernel<true, kPairStages, kPairU><<<pgrid, ppc * 64, psmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);
-      else env_rollout_pair_kernel<false, kPairStages, kPairU><<<pgrid, ppc * 64, psmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);
+      auto kern = ppc == 1 ? (traj ? env_rollout_pair_kernel<true, kPairStages, kPairU> : env_rollout_pair_kernel<false, kPairStages, kPairU>)
+                           : (traj ? env_rollout_pair_kernel<true, kPairStages2, kPairU> : env_rollout_pair_kernel<false, kPairStages2, kPairU>);
+      kern<<<pgrid, ppc * 64, psmem, st>>>(h->halo, h->halo_fits, x, y, tm_act, tm_traj, n, T);
     } else if (deep) {
       if (traj) env_rollout_tma_kernel<true, kDeep><<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);
       else env_rollout_tma_kernel<false, kDeep><<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);

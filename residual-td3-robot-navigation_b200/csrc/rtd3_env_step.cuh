@@ -8,6 +8,8 @@ struct rtd3_env {
   int device;
   int num_sms;
   float2* table;   // [100*100] (speed*cos(rot), speed*sin(rot)), indexed x*100+y
+  float2* halo;    // [116*116] the same table with an 8-cell border, read by the warp-pair rollout (rtd3_env.cu: build_halo_kernel)
+  int* halo_fits;  // 1 when every cell moves a state by less than the border per step (kMaxAction*(|c|+|s|) <= kHaloReach)
   bool has_map;
   void* host_pipe;   // rtd3::HostPipe of rtd3_env_rollout_host (rtd3_env_host.cu), created on first use
 };
