@@ -58,8 +58,34 @@ int32_t rtd3_env_destroy(rtd3_env* h);
 /* Replaces assigning Environment.dynamics_speed / dynamics_angle (environment.py:20-21, 84, 95).
  * speed, angle: DEVICE float32 [100*100], row-major [x][y].  Builds the packed table on `stream`:
  * rot = float32(angle*2*pi) (float32 as numpy>=2 evaluates environment.py:107), then
- * (speed*cos(rot), speed*sin(rot)) evaluated in float64 and rounded once to float32. */
+ * (speed*cos(rot), speed*sin(rot)) evaluated in float64 and rounded once to float32.
+ * The same as rtd3_env_set_maps with K = 1 followed by clearing the map index: every env steps on this map. */
 int32_t rtd3_env_set_map(rtd3_env* h, const float* speed, const float* angle, void* stream);
+
+/* Map bank: a handle holds K maps and, optionally, a map index of length m.  Env v of ANY launch (step, dynamics, rollout,
+ * rollout_host, tick, the planner's P*n virtual envs v = p*n + i) steps on map index[v % m]; with no index every env steps on
+ * map 0 and every launch runs the single-map kernels.  Kernels clamp an index entry to [0, K), so a bad entry never reads
+ * outside the bank (validating it is the caller's job).  A bank costs about 188 KB of HBM per map.
+ *
+ * rtd3_env_set_maps: speed, angle DEVICE float32 [K][100*100]; builds the K tables on `stream`.  Asynchronous while K does not
+ * exceed the number of maps already allocated (the handle starts with one); a larger K reallocates the bank, which synchronises
+ * the device and drops the graphs cached by rtd3_env_rollout_host.  The index is kept as it is.
+ *
+ * rtd3_env_set_map_index: copies `index` (DEVICE int32 [m]) into the handle with a device-to-device cudaMemcpyAsync on `stream`
+ * (asynchronous and capturable while m does not exceed the largest m set before; a captured launch reads the handle's copy, so
+ * a graph replayed after an index change of the same length sees the new contents).  index == NULL or m == 0 clears the index.
+ *
+ * Kernels with an index: rtd3_env_step / rtd3_env_dynamics read the tables through the read-only path whatever the variant
+ * (RTD3_STEP_SMEM falls back to RTD3_STEP_LDG: a CTA covers envs of many maps, there is no one table to stage); the rollout
+ * kernels stage the map of a CTA's first env, and a warp whose envs all use that map runs the single-map loop, while any other
+ * warp reads every lane's table from global memory, which is several times slower (DESIGN.md section 3).  Keep the envs of one
+ * map in contiguous blocks that cover whole CTAs to stay on the fast path: 32 envs up to 4 736 envs per launch, 64 up to 9 472,
+ * 256 above. */
+int32_t rtd3_env_set_maps(rtd3_env* h, const float* speed, const float* angle, int32_t K, void* stream);
+int32_t rtd3_env_set_map_index(rtd3_env* h, const int32_t* index, int64_t m, void* stream);
+/* The map configuration launches capture as kernel arguments: bank address, index address (NULL without an index), K, m.
+ * A caller that captures launches into a CUDA graph compares these to decide whether to recapture.  Any output may be NULL. */
+int32_t rtd3_env_map_config(const rtd3_env* h, const void** tables, const void** index, int32_t* num_maps, int64_t* index_len);
 
 /* Variant selector for rtd3_env_step (evidence for each lives in profiles/). */
 #define RTD3_STEP_AUTO 0

@@ -15,10 +15,11 @@ static_assert(kTableBytes % (16 * kTableChunks) == 0, "bulk copy sizes must be m
 
 // rot = float32(angle*2*pi): numpy >= 2 keeps float32*int*pyfloat in float32 (environment.py:107).
 // cos/sin are taken in float64 like the reference does for (action_angle + rotation).
+// Runs over the cells of all `cells / kCells` maps of a bank: map k's table is table[k * kCells ...].
 __global__ void build_table_kernel(const float* __restrict__ speed, const float* __restrict__ angle,
-                                   float2* __restrict__ table) {
-  int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= kCells) return;
+                                   float2* __restrict__ table, int64_t cells) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= cells) return;
   float rot = __fmul_rn(__fmul_rn(angle[i], 2.0f), 3.14159274101257324f);
   double s, c;
   sincos((double)rot, &s, &c);
@@ -49,9 +50,12 @@ __device__ __forceinline__ int halo_cell(int i) {
   return i < kHalo ? 0 : i < kWorld - 1 + kHalo ? i - kHalo : i < kHaloDim - 1 ? kWorld - 2 : kWorld - 1;
 }
 
-// One CTA: copies the finished table into the halo layout and writes whether the map fits, in device memory so that
-// rtd3_env_set_map stays asynchronous (and capturable).  Non-finite cells were zeroed by build_table_kernel and fit.
+// One CTA per map of the bank: copies the finished table into the halo layout and writes whether the map fits, in device memory so
+// that rtd3_env_set_map(s) stays asynchronous (and capturable).  Non-finite cells were zeroed by build_table_kernel and fit.
 __global__ void __launch_bounds__(1024) build_halo_kernel(const float2* __restrict__ table, float2* __restrict__ halo, int* __restrict__ fits) {
+  table += (size_t)blockIdx.x * kCells;
+  halo += (size_t)blockIdx.x * (kHaloDim * kHaloDim);
+  fits += blockIdx.x;
   bool ok = true;
   for (int i = threadIdx.x; i < kCells; i += blockDim.x) {
     const float2 cs = table[i];
@@ -85,11 +89,14 @@ __device__ __forceinline__ void stage_table(float2* s_table, uint64_t* bar, cons
 // ---- single step over n envs ------------------------------------------------------------------
 // Each thread owns 4 consecutive envs per iteration: four 16 B loads (x,y,ax,ay) and two 16 B stores,
 // all coalesced (a warp covers 512 B contiguous per plane).  kKeepOnNan=false gives pure dynamics().
-template <bool kSmem, bool kKeepOnNan>
+// kBank: env j steps on its own map, bank.table_of(j), read through the read-only path (a CTA covers envs of many maps, so
+// there is no one table to stage: kBank goes with kSmem == false).
+template <bool kSmem, bool kKeepOnNan, bool kBank = false>
 __global__ void __launch_bounds__(kSmem ? 512 : 256, kSmem ? 2 : 4)
 env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x, const float* __restrict__ y,
                 const float* __restrict__ ax, const float* __restrict__ ay, float* __restrict__ ox,
-                float* __restrict__ oy, int64_t n, int vec_ok) {
+                float* __restrict__ oy, int64_t n, int vec_ok, MapBank bank) {
+  static_assert(!(kBank && kSmem), "a bank step reads its tables from global memory");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);
@@ -122,10 +129,17 @@ env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x,
     float4 px, py, pax, pay;
     if (have_next) { px = __ldcs(x4 + inext); py = __ldcs(y4 + inext); pax = __ldcs(ax4 + inext); pay = __ldcs(ay4 + inext); }
     float4 rx, ry;
-    step_one<kKeepOnNan>(table, vx.x, vy.x, vax.x, vay.x, rx.x, ry.x);
-    step_one<kKeepOnNan>(table, vx.y, vy.y, vax.y, vay.y, rx.y, ry.y);
-    step_one<kKeepOnNan>(table, vx.z, vy.z, vax.z, vay.z, rx.z, ry.z);
-    step_one<kKeepOnNan>(table, vx.w, vy.w, vax.w, vay.w, rx.w, ry.w);
+    if constexpr (kBank) {
+      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i)}, vx.x, vy.x, vax.x, vay.x, rx.x, ry.x);
+      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i + 1)}, vx.y, vy.y, vax.y, vay.y, rx.y, ry.y);
+      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i + 2)}, vx.z, vy.z, vax.z, vay.z, rx.z, ry.z);
+      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i + 3)}, vx.w, vy.w, vax.w, vay.w, rx.w, ry.w);
+    } else {
+      step_one<kKeepOnNan>(table, vx.x, vy.x, vax.x, vay.x, rx.x, ry.x);
+      step_one<kKeepOnNan>(table, vx.y, vy.y, vax.y, vay.y, rx.y, ry.y);
+      step_one<kKeepOnNan>(table, vx.z, vy.z, vax.z, vay.z, rx.z, ry.z);
+      step_one<kKeepOnNan>(table, vx.w, vy.w, vax.w, vay.w, rx.w, ry.w);
+    }
     __stcs(reinterpret_cast<float4*>(ox) + i, rx);
     __stcs(reinterpret_cast<float4*>(oy) + i, ry);
     i = inext; have = have_next;
@@ -135,7 +149,8 @@ env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x,
   // ragged tail (n % 4 envs), handled by the first threads of the grid
   for (int64_t j = (n4 << 2) + tid; j < n; j += nthreads) {
     float rx, ry;
-    step_one<kKeepOnNan>(table, x[j], y[j], ax[j], ay[j], rx, ry);
+    if constexpr (kBank) step_one<kKeepOnNan>(LdgTable{bank.table_of(j)}, x[j], y[j], ax[j], ay[j], rx, ry);
+    else step_one<kKeepOnNan>(table, x[j], y[j], ax[j], ay[j], rx, ry);
     ox[j] = rx; oy[j] = ry;
   }
 }
@@ -179,6 +194,27 @@ __device__ __forceinline__ uint32_t halo_addr_state(uint32_t addr_bias, float x,
   return bx * kHaloRowBytes + (by * 8u + addr_bias);
 }
 
+// Rollout kernels with a map bank (kBank): the CTA stages the map of its first env.  A warp whose live envs all step on that map
+// runs the shared-memory loop unchanged; a warp that mixes maps (mixed) steps every lane from its own map's plain table in global
+// memory, addressed from the state like the careful path - the same cell, the same values, so the same bits.
+struct BankLanes {
+  int staged;      // map staged in shared memory (the CTA's first env's)
+  bool mixed;      // warp-uniform
+  const float2* table;   // this lane's plain table
+};
+__device__ __forceinline__ BankLanes bank_lanes(const MapBank& b, int64_t cta_first, int64_t i, bool live) {
+  BankLanes r;
+  r.staged = b.map_of(cta_first);
+  const int mine = live ? b.map_of(i) : r.staged;
+  r.mixed = !__all_sync(0xffffffffu, mine == r.staged);
+  r.table = b.tables + (size_t)mine * kCells;
+  return r;
+}
+// one state-addressed step from the lane's own table (the mixed-warp path)
+__device__ __forceinline__ void ldg_step(const float2* __restrict__ table, const StepIn& in, float& x, float& y) {
+  advance(__ldg(table + cell_index(x, y)), in, x, y);
+}
+
 // Actions reach the SM through a per-thread cp.async ring in shared memory: kStages chunks of kU steps are in
 // flight, so the HBM latency (~1 us) is hidden even when a CTA is a single warp (4096 envs on 148 SMs); every
 // thread reads back only the words it copied itself, so cp.async.wait_group is the only synchronisation.
@@ -189,14 +225,20 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int kN>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(kN) : "memory"); }
 
-template <bool kTraj, int kStages>
+template <bool kTraj, int kStages, bool kBank = false>
 __global__ void __launch_bounds__(256)
 env_rollout_kernel(const float2* __restrict__ g_table, float* __restrict__ x, float* __restrict__ y,
-                   const float* __restrict__ actions, float* __restrict__ traj, int64_t n, int64_t T) {
+                   const float* __restrict__ actions, float* __restrict__ traj, int64_t n, int64_t T, MapBank bank) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);
   float* ring = reinterpret_cast<float*>(smem_raw + kTableBytes + 16);   // [kStages][kU][2][blockDim]
+  BankLanes bl{};
+  if constexpr (kBank) {
+    const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    bl = bank_lanes(bank, (int64_t)blockIdx.x * blockDim.x, env, env < n);
+    g_table = bank.tables + (size_t)bl.staged * kCells;
+  }
   stage_table(s_table, bar, g_table);   // contains the only __syncthreads of the kernel
 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -242,17 +284,26 @@ env_rollout_kernel(const float2* __restrict__ g_table, float* __restrict__ x, fl
       in[u] = prep_action(ax, ay);
     }
     issue_chunk(c + kStages);           // refill the slot just drained (its values are in registers now)
+    if (kBank && bl.mixed) {
 #pragma unroll
-    for (int u = 0; u < kU; ++u) {
-      rollout_step(addr_bias, in[u], sx, sy);
-      if (kTraj) { __stcs(pt, sx); __stcs(pt + n, sy); pt += n2; }
+      for (int u = 0; u < kU; ++u) {
+        ldg_step(bl.table, in[u], sx, sy);
+        if (kTraj) { __stcs(pt, sx); __stcs(pt + n, sy); pt += n2; }
+      }
+    } else {
+#pragma unroll
+      for (int u = 0; u < kU; ++u) {
+        rollout_step(addr_bias, in[u], sx, sy);
+        if (kTraj) { __stcs(pt, sx); __stcs(pt + n, sy); pt += n2; }
+      }
     }
   }
   pa += full * (kU * n2);
   for (int64_t t = full * kU; t < T; ++t) {   // ragged tail, T % kU steps
     const StepIn in = prep_action(__ldcs(pa), __ldcs(pa + n));
     pa += n2;
-    rollout_step(addr_bias, in, sx, sy);
+    if (kBank && bl.mixed) ldg_step(bl.table, in, sx, sy);
+    else rollout_step(addr_bias, in, sx, sy);
     if (kTraj) { __stcs(pt, sx); __stcs(pt + n, sy); pt += n2; }
   }
   cp_async_wait<0>();
@@ -282,10 +333,11 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, int c0, int 
                : "memory");
 }
 
-template <bool kTraj, int kStages>
+template <bool kTraj, int kStages, bool kBank = false>
 __global__ void __launch_bounds__(256)
 env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x, float* __restrict__ y,
-                       const __grid_constant__ CUtensorMap tm_act, const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T) {
+                       const __grid_constant__ CUtensorMap tm_act, const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T,
+                       MapBank bank) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);            // table barrier
@@ -299,6 +351,12 @@ env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x
 #pragma unroll
     for (int s = 0; s < kStages; ++s) mbar_init(full + s, 1);
     fence_mbar_init();
+  }
+  BankLanes bl{};
+  if constexpr (kBank) {
+    const int64_t env = ((int64_t)blockIdx.x * nwarps + warp) * 32 + lane;
+    bl = bank_lanes(bank, (int64_t)blockIdx.x * nwarps * 32, env, env < n);
+    g_table = bank.tables + (size_t)bl.staged * kCells;
   }
   stage_table(s_table, bar, g_table);   // init + fence + __syncthreads, then the table's bulk copies
 
@@ -342,7 +400,7 @@ env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x
     __syncwarp();
     const int steps = (int)min((int64_t)kU, T - c * kU);
     const bool careful = __any_sync(0xffffffffu, nanacc != 0.0f) || steps < kU;
-    if (!careful) {
+    if (!careful && !(kBank && bl.mixed)) {
 #pragma unroll
       for (int u = 0; u < kU; ++u) {
         StepIn in;
@@ -350,6 +408,12 @@ env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x
         in.ay = fminf(fmaxf(cay[u], -kMaxAction), kMaxAction);
         in.lo = 0.0f; in.hi = kClipHi; in.bad = false;
         rollout_step(addr_bias, in, sx, sy);
+        if (kTraj) { tout[(2 * u) * 32] = sx; tout[(2 * u + 1) * 32] = sy; }
+      }
+    } else if (kBank && bl.mixed) {
+#pragma unroll
+      for (int u = 0; u < kU; ++u) {
+        if (u < steps) ldg_step(bl.table, prep_action(cax[u], cay[u]), sx, sy);
         if (kTraj) { tout[(2 * u) * 32] = sx; tout[(2 * u + 1) * 32] = sy; }
       }
     } else {
@@ -391,10 +455,11 @@ struct PairSmem {
   static constexpr int kBars = 16;   // full[8] | prepped[2] | consumed[2] | outfull[2] | outfree[2]
 };
 
-template <bool kTraj, int kStages, int kUp>
+template <bool kTraj, int kStages, int kUp, bool kBank = false>
 __global__ void __launch_bounds__(256)
 env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict__ g_fits, float* __restrict__ x, float* __restrict__ y,
-                        const __grid_constant__ CUtensorMap tm_act, const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T) {
+                        const __grid_constant__ CUtensorMap tm_act, const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T,
+                        MapBank bank) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int kU = kUp;                            // steps per action / trajectory tile of this kernel (shadows the file-wide kU)
   constexpr int kTileFloats = kU * 2 * 32;
@@ -417,6 +482,13 @@ env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict
     for (int s = 0; s < kStages; ++s) mbar_init(full + s, 1);
     for (int b = 0; b < 2; ++b) { mbar_init(prepped + b, 32); mbar_init(consumed + b, 32); mbar_init(outfull + b, 32); mbar_init(outfree + b, 1); }
     fence_mbar_init();
+  }
+  BankLanes bl{};
+  if constexpr (kBank) {                             // the CTA stages the halo table of its first env's map
+    const int64_t env = ((int64_t)blockIdx.x * npairs + pair) * 32 + lane;
+    bl = bank_lanes(bank, (int64_t)blockIdx.x * npairs * 32, env, env < n);
+    g_halo = bank.halos + (size_t)bl.staged * (kHaloDim * kHaloDim);
+    g_fits = bank.fits + bl.staged;
   }
   stage_table<kHaloBytes>(s_table, bar, g_halo);   // contains the __syncthreads that publishes the barrier inits
 
@@ -504,7 +576,7 @@ env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict
       asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u) * 128u), "f"(sx) : "memory");
       asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u + 1) * 128u), "f"(sy) : "memory");
     };
-    if (!careful && fits) {
+    if (!careful && fits && !(kBank && bl.mixed)) {
       // Step 0 is addressed from the state (which may be in [99, 100) after NaN actions) and step 1 from its clipped
       // successor; every later step from the unclipped successor of the step before.  The previous step's trajectory
       // stores follow the table load in program order: issued before it, ptxas put them between the address IMAD and the
@@ -524,6 +596,17 @@ env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict
         a = an;
       }
       if (kTraj) store_state(kU - 1);
+    } else if (kBank && bl.mixed) {
+      // lanes on different maps: each steps from its own map's plain table, addressed from the state as below
+      const int steps = (int)min((int64_t)kU, T - c * kU);
+#pragma unroll
+      for (int u = 0; u < kU; ++u) {
+        if (u < steps) {
+          const float2 a = lds_f2(tp + u * 256u);
+          ldg_step(bl.table, prep_action(a.x, a.y), sx, sy);
+        }
+        if (kTraj) store_state(u);
+      }
     } else {
       // NaN / inf actions, the ragged last chunk, or a map that does not fit: every step addressed from the state
       const int steps = (int)min((int64_t)kU, T - c * kU);
@@ -659,6 +742,7 @@ static int32_t check_bank(const rtd3_mt_bank* b) {
 
 using namespace rtd3;
 
+constexpr int kMaxMaps = 65536;
 static bool g_force_plain_rollout = false;
 static int g_rollout_variant = 0;            // test hook: 1 = single-warp TMA kernel instead of the warp-pair kernel
 
@@ -691,6 +775,46 @@ static int32_t make_plane_map(CUtensorMap* tm, const float* base, int64_t n, int
   return 0;
 }   // test hook: exercise the cp.async variant on aligned sizes too
 
+// (Re)allocates the bank for `cap` maps (synchronous: kernels in flight may read the old bank).  The contents are not kept.
+static int32_t alloc_bank(rtd3_env* h, int cap) {
+  if (h->tables) {
+    rtd3::host_pipe_drop_graphs(h);   // they hold the old bank addresses
+    cudaDeviceSynchronize();
+    cudaFree(h->tables);
+    cudaFree(h->halos);
+    cudaFree(h->fits);
+  }
+  h->tables = h->halos = h->table = h->halo = nullptr;
+  h->fits = h->halo_fits = nullptr;
+  h->map_cap = h->num_maps = 0;
+  h->has_map = false;
+  RTD3_CUDA(cudaMalloc(&h->tables, (size_t)cap * kTableBytes));
+  RTD3_CUDA(cudaMalloc(&h->halos, (size_t)cap * kHaloBytes));
+  RTD3_CUDA(cudaMalloc(&h->fits, (size_t)cap * sizeof(int)));
+  h->table = h->tables;
+  h->halo = h->halos;
+  h->halo_fits = h->fits;
+  h->map_cap = cap;
+  return 0;
+}
+
+// the bank instantiations of the rollout kernels need the same shared memory as the single-map ones
+static int32_t set_bank_smem(int smem_roll) {
+  const void* full[] = {(const void*)env_rollout_kernel<true, kDeep, true>, (const void*)env_rollout_kernel<false, kDeep, true>,
+                        (const void*)env_rollout_kernel<true, kShallow, true>, (const void*)env_rollout_kernel<false, kShallow, true>,
+                        (const void*)env_rollout_tma_kernel<true, kDeep, true>, (const void*)env_rollout_tma_kernel<false, kDeep, true>,
+                        (const void*)env_rollout_tma_kernel<true, kShallow, true>, (const void*)env_rollout_tma_kernel<false, kShallow, true>};
+  const void* pair[] = {(const void*)env_rollout_pair_kernel<true, kPairStages, kPairU, true>, (const void*)env_rollout_pair_kernel<false, kPairStages, kPairU, true>,
+                        (const void*)env_rollout_pair_kernel<true, kPairStages2, kPairU, true>, (const void*)env_rollout_pair_kernel<false, kPairStages2, kPairU, true>};
+  for (const void* f : full) RTD3_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
+  for (const void* f : pair) RTD3_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
+  return 0;
+}
+
+static MapBank map_bank(const rtd3_env* h) {
+  return MapBank{h->tables, h->halos, h->fits, h->index_len ? h->index : nullptr, h->index_len, h->num_maps};
+}
+
 extern "C" {
 
 void rtd3_env_force_plain_rollout(int32_t on) { g_force_plain_rollout = on == 1; g_rollout_variant = on == 2 ? 1 : 0; }
@@ -707,15 +831,19 @@ int32_t rtd3_env_create(rtd3_env** out, int32_t device) {
   h->halo = nullptr;
   h->halo_fits = nullptr;
   h->host_pipe = nullptr;
+  h->tables = h->halos = nullptr;
+  h->fits = nullptr;
+  h->num_maps = h->map_cap = 0;
+  h->index = nullptr;
+  h->index_len = h->index_cap = 0;
   RTD3_CUDA(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, device));
-  RTD3_CUDA(cudaMalloc(&h->table, kTableBytes));
-  RTD3_CUDA(cudaMalloc(&h->halo, kHaloBytes));
-  RTD3_CUDA(cudaMalloc(&h->halo_fits, sizeof(int)));
+  if (int32_t e = alloc_bank(h, 1)) return e;
   if (!g_encode_tiled) load_encode_tiled();
   const int smem = kTableBytes + 16;
   RTD3_CUDA(cudaFuncSetAttribute(env_step_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   RTD3_CUDA(cudaFuncSetAttribute(env_step_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
   const int smem_roll = 227 * 1024;
+  if (int32_t e = set_bank_smem(smem_roll)) return e;
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<true, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<false, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
   RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<true, kShallow>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
@@ -736,20 +864,75 @@ int32_t rtd3_env_create(rtd3_env** out, int32_t device) {
 int32_t rtd3_env_destroy(rtd3_env* h) {
   if (!h) return 0;
   rtd3::host_pipe_destroy(h);
-  if (h->table) cudaFree(h->table);
-  if (h->halo) cudaFree(h->halo);
-  if (h->halo_fits) cudaFree(h->halo_fits);
+  if (h->tables) cudaFree(h->tables);
+  if (h->halos) cudaFree(h->halos);
+  if (h->fits) cudaFree(h->fits);
+  if (h->index) cudaFree(h->index);
   delete h;
   return 0;
 }
 
-int32_t rtd3_env_set_map(rtd3_env* h, const float* speed, const float* angle, void* stream) {
+int32_t rtd3_env_set_maps(rtd3_env* h, const float* speed, const float* angle, int32_t K, void* stream) {
   RTD3_CHECK_ARG(h && speed && angle, "null argument");
-  build_table_kernel<<<(int)ceil_div(kCells, 256), 256, 0, (cudaStream_t)stream>>>(speed, angle, h->table);
+  RTD3_CHECK_ARG(K >= 1 && K <= kMaxMaps, "map count K must be in [1, 65536]");
+  if (K > h->map_cap) {
+    int prev = 0;
+    RTD3_CUDA(cudaGetDevice(&prev));
+    RTD3_CUDA(cudaSetDevice(h->device));
+    const int32_t e = alloc_bank(h, K);
+    cudaSetDevice(prev);
+    if (e) return e;
+  }
+  const int64_t cells = (int64_t)K * kCells;
+  build_table_kernel<<<(int)ceil_div(cells, 256), 256, 0, (cudaStream_t)stream>>>(speed, angle, h->tables, cells);
   RTD3_LAUNCHED();
-  build_halo_kernel<<<1, 1024, 0, (cudaStream_t)stream>>>(h->table, h->halo, h->halo_fits);
+  build_halo_kernel<<<K, 1024, 0, (cudaStream_t)stream>>>(h->tables, h->halos, h->fits);
   RTD3_LAUNCHED();
+  h->num_maps = K;
   h->has_map = true;
+  return 0;
+}
+
+int32_t rtd3_env_set_map(rtd3_env* h, const float* speed, const float* angle, void* stream) {
+  if (int32_t e = rtd3_env_set_maps(h, speed, angle, 1, stream)) return e;
+  return rtd3_env_set_map_index(h, nullptr, 0, stream);
+}
+
+int32_t rtd3_env_set_map_index(rtd3_env* h, const int32_t* index, int64_t m, void* stream) {
+  RTD3_CHECK_ARG(h, "null handle");
+  RTD3_CHECK_ARG(m >= 0, "negative index length");
+  if (!index || m == 0) {
+    h->index_len = 0;
+    return 0;
+  }
+  if (m > h->index_cap) {
+    int prev = 0;
+    RTD3_CUDA(cudaGetDevice(&prev));
+    RTD3_CUDA(cudaSetDevice(h->device));
+    rtd3::host_pipe_drop_graphs(h);   // they hold the old index address
+    cudaDeviceSynchronize();          // kernels in flight may still read the old index
+    if (h->index) cudaFree(h->index);
+    h->index = nullptr;
+    h->index_len = h->index_cap = 0;
+    const cudaError_t ce = cudaMalloc(&h->index, (size_t)m * sizeof(int32_t));
+    cudaSetDevice(prev);
+    if (ce != cudaSuccess) {
+      rtd3::set_error("cudaMalloc of a %lld-entry map index -> %s", (long long)m, cudaGetErrorString(ce));
+      return (int32_t)ce;
+    }
+    h->index_cap = m;
+  }
+  RTD3_CUDA(cudaMemcpyAsync(h->index, index, (size_t)m * sizeof(int32_t), cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
+  h->index_len = m;
+  return 0;
+}
+
+int32_t rtd3_env_map_config(const rtd3_env* h, const void** tables, const void** index, int32_t* num_maps, int64_t* index_len) {
+  RTD3_CHECK_ARG(h, "null handle");
+  if (tables) *tables = h->tables;
+  if (index) *index = h->index_len ? h->index : nullptr;
+  if (num_maps) *num_maps = h->num_maps;
+  if (index_len) *index_len = h->index_len;
   return 0;
 }
 
@@ -764,17 +947,23 @@ static int32_t launch_step(rtd3_env* h, const float* x, const float* y, const fl
   RTD3_CHECK_ARG(variant >= RTD3_STEP_AUTO && variant <= RTD3_STEP_LDG, "unknown step variant");
   const int64_t n4 = vec_ok ? (n + 3) / 4 : n;
   if (variant == RTD3_STEP_AUTO) variant = (n >= 262144) ? RTD3_STEP_SMEM : RTD3_STEP_LDG;
-  if (variant == RTD3_STEP_SMEM) {
+  const MapBank bank = map_bank(h);
+  if (bank.index) {                  // one table per env: no table to stage, every variant reads through the read-only path
+    const int block = 256;
+    const int grid = (int)std::min<int64_t>(ceil_div(n4, block), (int64_t)h->num_sms * 4);
+    if (keep_on_nan) env_step_kernel<false, true, true><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
+    else env_step_kernel<false, false, true><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
+  } else if (variant == RTD3_STEP_SMEM) {
     const int block = 512;
     const int grid = (int)std::min<int64_t>(ceil_div(n4, block), (int64_t)h->num_sms * 2);
     const int smem = kTableBytes + 16;
-    if (keep_on_nan) env_step_kernel<true, true><<<grid, block, smem, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok);
-    else env_step_kernel<true, false><<<grid, block, smem, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok);
+    if (keep_on_nan) env_step_kernel<true, true><<<grid, block, smem, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
+    else env_step_kernel<true, false><<<grid, block, smem, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
   } else {
     const int block = 256;
     const int grid = (int)std::min<int64_t>(ceil_div(n4, block), (int64_t)h->num_sms * 4);
-    if (keep_on_nan) env_step_kernel<false, true><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok);
-    else env_step_kernel<false, false><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok);
+    if (keep_on_nan) env_step_kernel<false, true><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
+    else env_step_kernel<false, false><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
   }
   RTD3_LAUNCHED();
   return 0;
@@ -806,6 +995,7 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
   const int stages = deep ? kDeep : kShallow;
   const int smem = kTableBytes + 16 + stages * kU * 2 * block * 4;
   cudaStream_t st = (cudaStream_t)stream;
+  const MapBank bank = map_bank(h);   // bank.index == nullptr: the single-map kernels
   const bool tma_ok = (n % 4 == 0) && (n < (1ll << 31)) && (2 * T < (1ll << 31)) && ((uintptr_t)actions % 16 == 0) &&
                       (!traj || (uintptr_t)traj % 16 == 0) && !g_force_plain_rollout && g_encode_tiled;
   CUtensorMap tm_act, tm_traj;
@@ -824,26 +1014,29 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
       const int pstages = ppc == 1 ? kPairStages : kPairStages2;
       const int psmem = ((kHaloBytes + 16 + ppc * PairSmem::kBars * 8 + 127) & ~127) + ppc * (pstages + 4) * (kPairU * 2 * 32) * 4;
       if (make_plane_map(&tm_act, actions, n, T, kPairU) != 0 || make_plane_map(&tm_traj, traj ? traj : actions, n, T, kPairU) != 0) return RTD3_ERR_STATE;
-      auto kern = ppc == 1 ? (traj ? env_rollout_pair_kernel<true, kPairStages, kPairU> : env_rollout_pair_kernel<false, kPairStages, kPairU>)
+      decltype(&env_rollout_pair_kernel<true, kPairStages, kPairU>) kern;
+      if (bank.index) kern = ppc == 1 ? (traj ? env_rollout_pair_kernel<true, kPairStages, kPairU, true> : env_rollout_pair_kernel<false, kPairStages, kPairU, true>)
+                                      : (traj ? env_rollout_pair_kernel<true, kPairStages2, kPairU, true> : env_rollout_pair_kernel<false, kPairStages2, kPairU, true>);
+      else kern = ppc == 1 ? (traj ? env_rollout_pair_kernel<true, kPairStages, kPairU> : env_rollout_pair_kernel<false, kPairStages, kPairU>)
                            : (traj ? env_rollout_pair_kernel<true, kPairStages2, kPairU> : env_rollout_pair_kernel<false, kPairStages2, kPairU>);
-      kern<<<pgrid, ppc * 64, psmem, st>>>(h->halo, h->halo_fits, x, y, tm_act, tm_traj, n, T);
-    } else if (deep) {
-      if (traj) env_rollout_tma_kernel<true, kDeep><<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);
-      else env_rollout_tma_kernel<false, kDeep><<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);
+      kern<<<pgrid, ppc * 64, psmem, st>>>(h->halo, h->halo_fits, x, y, tm_act, tm_traj, n, T, bank);
     } else {
-      if (traj) env_rollout_tma_kernel<true, kShallow><<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);
-      else env_rollout_tma_kernel<false, kShallow><<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T);
+      decltype(&env_rollout_tma_kernel<true, kDeep>) kern;
+      if (bank.index) kern = deep ? (traj ? env_rollout_tma_kernel<true, kDeep, true> : env_rollout_tma_kernel<false, kDeep, true>)
+                                  : (traj ? env_rollout_tma_kernel<true, kShallow, true> : env_rollout_tma_kernel<false, kShallow, true>);
+      else kern = deep ? (traj ? env_rollout_tma_kernel<true, kDeep> : env_rollout_tma_kernel<false, kDeep>)
+                       : (traj ? env_rollout_tma_kernel<true, kShallow> : env_rollout_tma_kernel<false, kShallow>);
+      kern<<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T, bank);
     }
     RTD3_LAUNCHED();
     return 0;
   }
-  if (deep) {
-    if (traj) env_rollout_kernel<true, kDeep><<<grid, block, smem, st>>>(h->table, x, y, actions, traj, n, T);
-    else env_rollout_kernel<false, kDeep><<<grid, block, smem, st>>>(h->table, x, y, actions, nullptr, n, T);
-  } else {
-    if (traj) env_rollout_kernel<true, kShallow><<<grid, block, smem, st>>>(h->table, x, y, actions, traj, n, T);
-    else env_rollout_kernel<false, kShallow><<<grid, block, smem, st>>>(h->table, x, y, actions, nullptr, n, T);
-  }
+  decltype(&env_rollout_kernel<true, kDeep>) kern;
+  if (bank.index) kern = deep ? (traj ? env_rollout_kernel<true, kDeep, true> : env_rollout_kernel<false, kDeep, true>)
+                              : (traj ? env_rollout_kernel<true, kShallow, true> : env_rollout_kernel<false, kShallow, true>);
+  else kern = deep ? (traj ? env_rollout_kernel<true, kDeep> : env_rollout_kernel<false, kDeep>)
+                   : (traj ? env_rollout_kernel<true, kShallow> : env_rollout_kernel<false, kShallow>);
+  kern<<<grid, block, smem, st>>>(h->table, x, y, actions, traj, n, T, bank);
   RTD3_LAUNCHED();
   return 0;
 }

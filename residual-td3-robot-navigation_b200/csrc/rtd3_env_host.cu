@@ -12,10 +12,21 @@
 
 namespace rtd3 {
 
+// The map configuration a captured rollout kernel holds as arguments (and whether it is the single-map or the bank kernel).
+// Reallocating the bank or the index drops the cached graphs; a change of K or m without one makes them miss here.
+struct MapKey {
+  const void *tables, *index;
+  int64_t m;
+  int32_t K;
+  bool operator==(const MapKey& o) const { return tables == o.tables && index == o.index && m == o.m && K == o.K; }
+};
+static MapKey map_key(const rtd3_env* h) { return MapKey{h->tables, h->index_len ? h->index : nullptr, h->index_len, h->num_maps}; }
+
 struct HostGraph {
   const void *x, *y, *act, *traj;
   int64_t n, T;
   int32_t chunks, mode;
+  MapKey map;
   cudaGraphExec_t exec;
 };
 
@@ -36,6 +47,10 @@ static void drop_graphs(HostPipe* p) {
   cudaDeviceSynchronize();           // a cached graph may still be running on the caller's stream
   for (auto& g : p->graphs) cudaGraphExecDestroy(g.exec);
   p->graphs.clear();
+}
+
+void host_pipe_drop_graphs(rtd3_env* h) {
+  if (h->host_pipe) drop_graphs((HostPipe*)h->host_pipe);
 }
 
 void host_pipe_destroy(rtd3_env* h) {
@@ -159,9 +174,11 @@ extern "C" int32_t rtd3_env_rollout_host(rtd3_env* h, float* x, float* y, const 
   HostPipe* p = nullptr;
   int32_t rc = pipe_prepare(h, &p, (size_t)(2 * n * T), 2 * chunks + 2);
   cudaGraphExec_t exec = nullptr;
+  const MapKey mk = map_key(h);
   if (rc == 0) {
     for (auto& g : p->graphs)
-      if (g.x == x && g.y == y && g.act == actions_host && g.traj == traj_host && g.n == n && g.T == T && g.chunks == chunks && g.mode == mode)
+      if (g.x == x && g.y == y && g.act == actions_host && g.traj == traj_host && g.n == n && g.T == T && g.chunks == chunks && g.mode == mode &&
+          g.map == mk)
         exec = g.exec;
     if (!exec) {
       if (p->graphs.size() >= kMaxHostGraphs) {
@@ -192,7 +209,7 @@ extern "C" int32_t rtd3_env_rollout_host(rtd3_env* h, float* x, float* y, const 
         if (graph) cudaGraphDestroy(graph);
         if (rc != 0) cudaGetLastError();
       }
-      if (rc == 0) p->graphs.push_back(HostGraph{x, y, actions_host, traj_host, n, T, chunks, mode, exec});
+      if (rc == 0) p->graphs.push_back(HostGraph{x, y, actions_host, traj_host, n, T, chunks, mode, mk, exec});
     }
     if (rc == 0) {
       cudaError_t ce = cudaGraphLaunch(exec, (cudaStream_t)stream);

@@ -7,16 +7,42 @@
 struct rtd3_env {
   int device;
   int num_sms;
-  float2* table;   // [100*100] (speed*cos(rot), speed*sin(rot)), indexed x*100+y
+  float2* table;   // [100*100] (speed*cos(rot), speed*sin(rot)), indexed x*100+y: map 0 of the bank
   float2* halo;    // [116*116] the same table with an 8-cell border, read by the warp-pair rollout (rtd3_env.cu: build_halo_kernel)
   int* halo_fits;  // 1 when every cell moves a state by less than the border per step (kMaxAction*(|c|+|s|) <= kHaloReach)
   bool has_map;
   void* host_pipe;   // rtd3::HostPipe of rtd3_env_rollout_host (rtd3_env_host.cu), created on first use
+  // Map bank (rtd3_env_set_maps / rtd3_env_set_map_index): map_cap maps allocated, num_maps of them set.  tables / halos / fits
+  // are [map_cap][...] and table / halo / halo_fits point at map 0.  Env v of a launch steps on map index[v % index_len]; with
+  // index_len == 0 there is no index and every launch runs the single-map kernels on map 0.
+  float2* tables;
+  float2* halos;
+  int* fits;
+  int num_maps, map_cap;
+  int32_t* index;
+  int64_t index_len, index_cap;
 };
 
 namespace rtd3 {
 
 void host_pipe_destroy(rtd3_env* h);   // rtd3_env_host.cu: streams, staging buffers and cached graphs of the host-buffer rollout
+void host_pipe_drop_graphs(rtd3_env* h);   // rtd3_env_host.cu: the cached graphs only (they hold the bank / index addresses)
+
+// What a kernel needs to step env v on its own map.  Passed by value; index == nullptr (single map) in the launches without a bank.
+struct MapBank {
+  const float2* tables;   // [K][kCells]
+  const float2* halos;    // [K][116*116]
+  const int* fits;        // [K]
+  const int32_t* index;   // [m]
+  int64_t m;
+  int K;
+  // the map of env v, clamped to [0, K) so that a bad index can never read outside the bank
+  __device__ __forceinline__ int map_of(int64_t v) const {
+    const int k = __ldg(index + (v < m ? v : v % m));
+    return min(max(k, 0), K - 1);
+  }
+  __device__ __forceinline__ const float2* table_of(int64_t v) const { return tables + (size_t)map_of(v) * kCells; }
+};
 
 // One env-step, the rotation form of environment.py:100-117 (no atan2):
 //   s' = clip(s + speed*(ax*cos(rot) - ay*sin(rot), ax*sin(rot) + ay*cos(rot)), 0, 98.9999)

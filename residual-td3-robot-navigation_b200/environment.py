@@ -8,6 +8,9 @@ With `num_envs == 1` (the default) calls take / return numpy `[2]` float64 array
 seed is given, draw from numpy's *global* legacy MT19937 stream exactly as the reference does.  With
 `num_envs > 1` they take / return CUDA tensors `[N,2]` (views of plane-major `[2,N]` storage, so no copies).
 
+Beyond the reference, the envs of one `Environment` can step on different maps (domain randomisation): `maps` / `set_maps` take a
+bank of K maps `[K,100,100]` and `map_index` / `set_map_index` say which map each env uses (`num_maps`, `map_index`).
+
 All arithmetic happens in csrc/librtd3.so (hand-written sm_100a kernels); there is no CPU path.
 """
 import numpy as np
@@ -117,7 +120,9 @@ def _planes(t, n, name):
 
 
 class Environment:
-    def __init__(self, num_envs=1, device=None, seed=None, maps=None):
+    def __init__(self, num_envs=1, device=None, seed=None, maps=None, map_index=None):
+        """`maps`: (speed, angle), each `[100,100]` or a bank `[K,100,100]`; None builds the reference's Perlin maps.
+        `map_index`: int `[num_envs]`, the map of every env (see `set_maps`)."""
         if not torch.cuda.is_available():
             raise RuntimeError("Environment needs a CUDA device (B200); there is no CPU path")
         self.num_envs = int(num_envs)
@@ -138,11 +143,15 @@ class Environment:
         self.step_variant = STEP_AUTO
         self._pipe = None
         self._pipe_buf = None
+        self._map_index = None
+        self.num_maps = 1
         self.set_init_and_goal()
         if maps is None:
             self.set_dynamics()
+            if map_index is not None:
+                self.set_map_index(map_index)
         else:
-            self.set_maps(*maps)
+            self.set_maps(*maps, index=map_index)
 
     def __del__(self):
         try:
@@ -203,21 +212,76 @@ class Environment:
     def set_dynamics(self):
         self.set_maps(*perlin_maps(configuration.RANDOM_SEED))
 
-    def set_maps(self, speed, angle):
+    def set_maps(self, speed, angle, index=None):
+        """Set the dynamics maps: `[100,100]` speed and angle (every env on that map), or a bank of K maps `[K,100,100]`.
+        With a bank, env i steps on map `index[i]` (int `[num_envs]`, values in [0, K)); the default index for K > 1 is
+        contiguous blocks, `index[i] = i*K // num_envs`: the rollout kernels stage one map per CTA (32 to 256 consecutive envs),
+        and warps on their CTA's map run at the single-map speed; other warps read their tables from global memory, several times
+        slower.  `dynamics_speed` / `dynamics_angle` are `[K,100,100]` for K > 1 and `[100,100]` otherwise."""
         W = constants.WORLD_SIZE
         speed = torch.as_tensor(np.asarray(speed.cpu() if isinstance(speed, torch.Tensor) else speed, dtype=np.float32))
         angle = torch.as_tensor(np.asarray(angle.cpu() if isinstance(angle, torch.Tensor) else angle, dtype=np.float32))
-        if speed.shape != (W, W) or angle.shape != (W, W):
-            raise ValueError("maps must be [%d,%d]" % (W, W))
-        self.dynamics_speed = speed.numpy().copy()
-        self.dynamics_angle = angle.numpy().copy()
+        if speed.shape != angle.shape or speed.dim() not in (2, 3) or tuple(speed.shape[-2:]) != (W, W) or speed.numel() == 0:
+            raise ValueError("maps must be [%d,%d] or [K,%d,%d], speed and angle alike" % (W, W, W, W))
+        K = 1 if speed.dim() == 2 else int(speed.shape[0])
+        if speed.dim() == 3 and index is None and K > 1:
+            n = self.num_envs
+            index = torch.arange(n, dtype=torch.int64) * K // n
+        idx = None if index is None else self._checked_index(index, K)
+        self.dynamics_speed = (speed[0] if K == 1 and speed.dim() == 3 else speed).numpy().copy()
+        self.dynamics_angle = (angle[0] if K == 1 and angle.dim() == 3 else angle).numpy().copy()
         self._speed_dev = speed.contiguous().to(self.device)
         self._angle_dev = angle.contiguous().to(self.device)
-        _lib.check(_lib.lib().rtd3_env_set_map(self._handle, _lib.ptr(self._speed_dev), _lib.ptr(self._angle_dev),
-                                               _lib.stream_ptr(self.device)), "env_set_map")
+        if speed.dim() == 2:
+            _lib.check(_lib.lib().rtd3_env_set_map(self._handle, _lib.ptr(self._speed_dev), _lib.ptr(self._angle_dev),
+                                                   _lib.stream_ptr(self.device)), "env_set_map")
+        else:
+            _lib.check(_lib.lib().rtd3_env_set_maps(self._handle, _lib.ptr(self._speed_dev), _lib.ptr(self._angle_dev), K,
+                                                    _lib.stream_ptr(self.device)), "env_set_maps")
+        self.num_maps = K
+        self._set_index(idx)
+
+    def set_map_index(self, index):
+        """Which map of the bank each env steps on: int `[num_envs]` with values in [0, num_maps) (None: every env on map 0).
+        Raises ValueError for a non-integer dtype, a wrong length or a value out of range; the range check reads the index's
+        minimum and maximum back to the host (one synchronisation per call).  The handle keeps its own copy, written
+        asynchronously in place, so a captured CUDA graph replayed afterwards sees the new index.  Rule of every kernel: with
+        an index of length m, env (or row) v of a launch steps on map `index[v % m]`."""
+        self._set_index(None if index is None else self._checked_index(index, self.num_maps))
+
+    @property
+    def map_index(self):
+        """int32 `[num_envs]` CUDA tensor (a copy), or None when every env steps on map 0 without an index."""
+        return None if self._map_index is None else self._map_index.clone()
+
+    def _checked_index(self, index, K):
+        n = self.num_envs
+        t = index if isinstance(index, torch.Tensor) else torch.as_tensor(np.asarray(index))
+        if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+            raise ValueError("map index must have an integer dtype, got %s" % t.dtype)
+        if t.dim() != 1 or t.shape[0] != n:
+            raise ValueError("map index must have shape [%d], got %s" % (n, list(t.shape)))
+        t = t.to(self.device)
+        lo, hi = torch.stack(torch.aminmax(t)).tolist()   # the one host synchronisation of a set
+        if lo < 0 or hi >= K:
+            raise ValueError("map index values must lie in [0, %d), got [%d, %d]" % (K, lo, hi))
+        return t.to(dtype=torch.int32, copy=True).contiguous()   # our own copy: the caller may reuse theirs
+
+    def _set_index(self, idx):
+        self._map_index = idx                              # kept alive: the library copies it asynchronously
+        _lib.check(_lib.lib().rtd3_env_set_map_index(self._handle, _lib.ptr(idx), 0 if idx is None else idx.numel(),
+                                                     _lib.stream_ptr(self.device)), "env_set_map_index")
+
+    def _map_config(self):
+        """(bank address, index address, K, m) as the library's launches capture them (rtd3_env_map_config)."""
+        tables, index, K, m = _lib.c_void_p(), _lib.c_void_p(), _lib.c_int32(), _lib.c_int64()
+        _lib.check(_lib.lib().rtd3_env_map_config(self._handle, _lib.ctypes.byref(tables), _lib.ctypes.byref(index),
+                                                  _lib.ctypes.byref(K), _lib.ctypes.byref(m)), "env_map_config")
+        return tables.value, index.value, K.value, m.value
 
     # ---- environment.py:98-119 ----------------------------------------------------------------------
     def dynamics(self, state, action):
+        """Pure next state of n rows; with a map bank row j uses env `j % num_envs`'s map."""
         single = not isinstance(state, torch.Tensor)
         if single:
             s = torch.as_tensor(np.asarray(state, dtype=np.float32).reshape(1, 2)).to(self.device)

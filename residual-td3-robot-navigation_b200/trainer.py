@@ -408,8 +408,9 @@ class BatchedTrainer:
         return self.robot.maybe_update_async() if self.async_check else self.robot.maybe_update()
 
     def _check_graphs(self):
-        """A captured tick holds the device pointers of the demonstration set and the choice of forward kernel: drop the graphs
-        when either has changed since the capture (`set_demonstration_states`, `process_demonstration`, `precision`)."""
+        """A captured tick holds the device pointers of the demonstration set, the env's map configuration (bank and index
+        addresses, K, index length) and the choice of forward kernel: drop the graphs when any has changed since the capture
+        (`set_demonstration_states`, `process_demonstration`, `set_maps` / `set_map_index`, `precision`)."""
         robot, agent = self.robot, self.robot.td3_agent
         p = lambda t: None if t is None else t.data_ptr()
         # of the operand copies only the one this precision's forward reads (the learner allocates `params_u` at its first
@@ -418,7 +419,7 @@ class BatchedTrainer:
         fwd = p(agent.params_h) if agent._f16_ok(self.n) else (p(agent.params_u) if agent._tc_ok(self.n) else None)
         ed = robot._env_demo
         sig = (p(robot._demo_dev), p(robot._demo_cells), p(robot._demo_list), agent.precision, fwd,
-               None if ed is None else (p(ed["sorted"]), p(ed["cells"]), ed["cap"]))
+               None if ed is None else (p(ed["sorted"]), p(ed["cells"]), ed["cap"]), self.env._map_config())
         if sig != getattr(self, "_graph_sig", None):
             self._graph = self._graph_k = None
             self._graph_sig = sig
