@@ -43,6 +43,28 @@ cudaError_t current_num_sms(int* out);                           // multiprocess
     RTD3_CUDA(cudaGetLastError());          \
   } while (0)
 
+// Makes a device current until the end of the scope and then restores the caller's, on every return path.
+class DeviceGuard {
+ public:
+  DeviceGuard() = default;
+  DeviceGuard(const DeviceGuard&) = delete;
+  DeviceGuard& operator=(const DeviceGuard&) = delete;
+  ~DeviceGuard() {
+    if (prev_ >= 0) cudaSetDevice(prev_);
+  }
+  cudaError_t enter(int device) {
+    int cur = 0;
+    if (cudaError_t e = cudaGetDevice(&cur)) return e;
+    if (cur == device) return cudaSuccess;
+    if (cudaError_t e = cudaSetDevice(device)) return e;
+    prev_ = cur;
+    return cudaSuccess;
+  }
+
+ private:
+  int prev_ = -1;   // the device to restore, -1 when the guard did not switch
+};
+
 constexpr float kMaxAction = 5.0f;                 // constants.py:34
 constexpr float kClipHi = 98.9999f;                // float32(WORLD_SIZE - 1.0001), environment.py:117
 constexpr int kWorld = RTD3_WORLD_SIZE;

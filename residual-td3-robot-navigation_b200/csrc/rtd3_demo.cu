@@ -277,7 +277,7 @@ extern "C" {
 int32_t rtd3_env_get_demonstration(rtd3_env* h, const rtd3_mt_bank* bank, const double* region, const double* goal, const rtd3_cem_workspace* w,
                                    int32_t iterations, int32_t paths, int32_t steps, int32_t elites, int32_t it_begin, int32_t it_end,
                                    int32_t finish, float* demo_states, float* demo_actions, void* stream) {
-  RTD3_CHECK_ARG(h && h->has_map, "environment has no dynamics map (call rtd3_env_set_map)");
+  RTD3_CHECK_ARG(h && h->num_maps > 0, "environment has no dynamics map (call rtd3_env_set_map)");
   RTD3_CHECK_ARG(bank && bank->mt && bank->pos && bank->has_gauss && bank->gauss && bank->n >= 0, "bad MT19937 bank");
   RTD3_CHECK_ARG(region && goal && w, "null argument");
   RTD3_CHECK_ARG(w->actions && w->x && w->y && w->start_x && w->start_y && w->rewards && w->elite && w->best && w->mean && w->std &&

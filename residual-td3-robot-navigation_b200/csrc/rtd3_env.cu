@@ -2,6 +2,9 @@
 // Reference behaviour: /root/reference/environment.py:28-56, 98-137 (see include/rtd3.h per entry point).
 #include <cuda.h>
 
+#include <memory>
+#include <utility>
+
 #include "rtd3_common.cuh"
 #include "rtd3_env_step.cuh"
 #include "rtd3_mt.cuh"
@@ -89,13 +92,14 @@ __device__ __forceinline__ void stage_table(float2* s_table, uint64_t* bar, cons
 // ---- single step over n envs ------------------------------------------------------------------
 // Each thread owns 4 consecutive envs per iteration: four 16 B loads (x,y,ax,ay) and two 16 B stores,
 // all coalesced (a warp covers 512 B contiguous per plane).  kKeepOnNan=false gives pure dynamics().
-// kBank: env j steps on its own map, bank.table_of(j), read through the read-only path (a CTA covers envs of many maps, so
-// there is no one table to stage: kBank goes with kSmem == false).
+// kBank: env j steps on its own map, bank.table<true>(j), read through the read-only path (a CTA covers envs of many maps, so
+// there is no one table to stage: kBank goes with kSmem == false).  Without it every env steps on map 0.
+// Parameter order: the scalar first puts the six pointers at 8 mod 16 in the constant bank, where ptxas pairs their loads
+// into the schedule this kernel was measured with (62 registers for dynamics()).
 template <bool kSmem, bool kKeepOnNan, bool kBank = false>
 __global__ void __launch_bounds__(kSmem ? 512 : 256, kSmem ? 2 : 4)
-env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x, const float* __restrict__ y,
-                const float* __restrict__ ax, const float* __restrict__ ay, float* __restrict__ ox,
-                float* __restrict__ oy, int64_t n, int vec_ok, MapBank bank) {
+env_step_kernel(int vec_ok, const float* __restrict__ x, const float* __restrict__ y, const float* __restrict__ ax, const float* __restrict__ ay,
+                float* __restrict__ ox, float* __restrict__ oy, int64_t n, MapBank bank) {
   static_assert(!(kBank && kSmem), "a bank step reads its tables from global memory");
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
@@ -109,7 +113,7 @@ env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x,
   const float4* ax4 = reinterpret_cast<const float4*>(ax);
   const float4* ay4 = reinterpret_cast<const float4*>(ay);
 
-  if constexpr (kSmem) stage_table(s_table, bar, g_table);
+  if constexpr (kSmem) stage_table(s_table, bar, bank.tables);
 
   // issue the first iteration's streaming loads before waiting for the table
   int64_t i = tid;
@@ -118,10 +122,16 @@ env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x,
   if (have) { vx = __ldcs(x4 + i); vy = __ldcs(y4 + i); vax = __ldcs(ax4 + i); vay = __ldcs(ay4 + i); }
   if constexpr (kSmem) mbar_wait(bar, 0);
 
-  auto table = [&]() {
+  // env j's table: env j's own map with the bank, else the one table of every env, built once (a table object built per call
+  // reorders ptxas's schedule of the loop)
+  const auto one_table = [&]() {
     if constexpr (kSmem) return SmemTable{s_table};
-    else return LdgTable{g_table};
+    else return LdgTable{bank.tables};
   }();
+  auto table = [&](int64_t j) -> decltype(auto) {
+    if constexpr (kBank) return LdgTable{bank.table<kBank>(j)};
+    else return std::as_const(one_table);
+  };
 
   while (have) {
     const int64_t inext = i + nthreads;
@@ -129,17 +139,10 @@ env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x,
     float4 px, py, pax, pay;
     if (have_next) { px = __ldcs(x4 + inext); py = __ldcs(y4 + inext); pax = __ldcs(ax4 + inext); pay = __ldcs(ay4 + inext); }
     float4 rx, ry;
-    if constexpr (kBank) {
-      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i)}, vx.x, vy.x, vax.x, vay.x, rx.x, ry.x);
-      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i + 1)}, vx.y, vy.y, vax.y, vay.y, rx.y, ry.y);
-      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i + 2)}, vx.z, vy.z, vax.z, vay.z, rx.z, ry.z);
-      step_one<kKeepOnNan>(LdgTable{bank.table_of(4 * i + 3)}, vx.w, vy.w, vax.w, vay.w, rx.w, ry.w);
-    } else {
-      step_one<kKeepOnNan>(table, vx.x, vy.x, vax.x, vay.x, rx.x, ry.x);
-      step_one<kKeepOnNan>(table, vx.y, vy.y, vax.y, vay.y, rx.y, ry.y);
-      step_one<kKeepOnNan>(table, vx.z, vy.z, vax.z, vay.z, rx.z, ry.z);
-      step_one<kKeepOnNan>(table, vx.w, vy.w, vax.w, vay.w, rx.w, ry.w);
-    }
+    step_one<kKeepOnNan>(table(4 * i), vx.x, vy.x, vax.x, vay.x, rx.x, ry.x);
+    step_one<kKeepOnNan>(table(4 * i + 1), vx.y, vy.y, vax.y, vay.y, rx.y, ry.y);
+    step_one<kKeepOnNan>(table(4 * i + 2), vx.z, vy.z, vax.z, vay.z, rx.z, ry.z);
+    step_one<kKeepOnNan>(table(4 * i + 3), vx.w, vy.w, vax.w, vay.w, rx.w, ry.w);
     __stcs(reinterpret_cast<float4*>(ox) + i, rx);
     __stcs(reinterpret_cast<float4*>(oy) + i, ry);
     i = inext; have = have_next;
@@ -149,8 +152,7 @@ env_step_kernel(const float2* __restrict__ g_table, const float* __restrict__ x,
   // ragged tail (n % 4 envs), handled by the first threads of the grid
   for (int64_t j = (n4 << 2) + tid; j < n; j += nthreads) {
     float rx, ry;
-    if constexpr (kBank) step_one<kKeepOnNan>(LdgTable{bank.table_of(j)}, x[j], y[j], ax[j], ay[j], rx, ry);
-    else step_one<kKeepOnNan>(table, x[j], y[j], ax[j], ay[j], rx, ry);
+    step_one<kKeepOnNan>(table(j), x[j], y[j], ax[j], ay[j], rx, ry);
     ox[j] = rx; oy[j] = ry;
   }
 }
@@ -194,19 +196,17 @@ __device__ __forceinline__ uint32_t halo_addr_state(uint32_t addr_bias, float x,
   return bx * kHaloRowBytes + (by * 8u + addr_bias);
 }
 
-// Rollout kernels with a map bank (kBank): the CTA stages the map of its first env.  A warp whose live envs all step on that map
-// runs the shared-memory loop unchanged; a warp that mixes maps (mixed) steps every lane from its own map's plain table in global
-// memory, addressed from the state like the careful path - the same cell, the same values, so the same bits.
+// Rollout kernels with a map bank (kBank): the CTA stages the map of its first env (map 0 without the bank).  A warp whose live envs
+// all step on that map runs the shared-memory loop unchanged; a warp that mixes maps (mixed) steps every lane from its own map's
+// plain table in global memory, addressed from the state like the careful path - the same cell, the same values, so the same bits.
 struct BankLanes {
-  int staged;      // map staged in shared memory (the CTA's first env's)
   bool mixed;      // warp-uniform
   const float2* table;   // this lane's plain table
 };
-__device__ __forceinline__ BankLanes bank_lanes(const MapBank& b, int64_t cta_first, int64_t i, bool live) {
+__device__ __forceinline__ BankLanes bank_lanes(const MapBank& b, int staged, int64_t i, bool live) {
   BankLanes r;
-  r.staged = b.map_of(cta_first);
-  const int mine = live ? b.map_of(i) : r.staged;
-  r.mixed = !__all_sync(0xffffffffu, mine == r.staged);
+  const int mine = live ? b.map_of(i) : staged;
+  r.mixed = !__all_sync(0xffffffffu, mine == staged);
   r.table = b.tables + (size_t)mine * kCells;
   return r;
 }
@@ -225,21 +225,22 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int kN>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(kN) : "memory"); }
 
+// Parameter order: n first for the same reason as env_step_kernel's vec_ok.
 template <bool kTraj, int kStages, bool kBank = false>
 __global__ void __launch_bounds__(256)
-env_rollout_kernel(const float2* __restrict__ g_table, float* __restrict__ x, float* __restrict__ y,
-                   const float* __restrict__ actions, float* __restrict__ traj, int64_t n, int64_t T, MapBank bank) {
+env_rollout_kernel(int64_t n, float* __restrict__ x, float* __restrict__ y, const float* __restrict__ actions, float* __restrict__ traj,
+                   int64_t T, MapBank bank) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);
   float* ring = reinterpret_cast<float*>(smem_raw + kTableBytes + 16);   // [kStages][kU][2][blockDim]
+  const int staged = bank.map<kBank>((int64_t)blockIdx.x * blockDim.x);
   BankLanes bl{};
   if constexpr (kBank) {
     const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    bl = bank_lanes(bank, (int64_t)blockIdx.x * blockDim.x, env, env < n);
-    g_table = bank.tables + (size_t)bl.staged * kCells;
+    bl = bank_lanes(bank, staged, env, env < n);
   }
-  stage_table(s_table, bar, g_table);   // contains the only __syncthreads of the kernel
+  stage_table(s_table, bar, bank.tables + (size_t)staged * kCells);   // contains the only __syncthreads of the kernel
 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;                   // thread 0 of every launched CTA is live, so the bulk copy always has an owner
@@ -333,11 +334,11 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, int c0, int 
                : "memory");
 }
 
+// Parameter order: n first for the same reason as env_step_kernel's vec_ok.
 template <bool kTraj, int kStages, bool kBank = false>
 __global__ void __launch_bounds__(256)
-env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x, float* __restrict__ y,
-                       const __grid_constant__ CUtensorMap tm_act, const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T,
-                       MapBank bank) {
+env_rollout_tma_kernel(int64_t n, float* __restrict__ x, float* __restrict__ y, const __grid_constant__ CUtensorMap tm_act,
+                       const __grid_constant__ CUtensorMap tm_traj, int64_t T, MapBank bank) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);            // table barrier
@@ -352,13 +353,13 @@ env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x
     for (int s = 0; s < kStages; ++s) mbar_init(full + s, 1);
     fence_mbar_init();
   }
+  const int staged = bank.map<kBank>((int64_t)blockIdx.x * nwarps * 32);
   BankLanes bl{};
   if constexpr (kBank) {
     const int64_t env = ((int64_t)blockIdx.x * nwarps + warp) * 32 + lane;
-    bl = bank_lanes(bank, (int64_t)blockIdx.x * nwarps * 32, env, env < n);
-    g_table = bank.tables + (size_t)bl.staged * kCells;
+    bl = bank_lanes(bank, staged, env, env < n);
   }
-  stage_table(s_table, bar, g_table);   // init + fence + __syncthreads, then the table's bulk copies
+  stage_table(s_table, bar, bank.tables + (size_t)staged * kCells);   // init + fence + __syncthreads, then the table's bulk copies
 
   const int64_t i0 = ((int64_t)blockIdx.x * nwarps + warp) * 32;                  // first env of this warp
   if (i0 >= n) return;
@@ -411,6 +412,8 @@ env_rollout_tma_kernel(const float2* __restrict__ g_table, float* __restrict__ x
         if (kTraj) { tout[(2 * u) * 32] = sx; tout[(2 * u + 1) * 32] = sy; }
       }
     } else if (kBank && bl.mixed) {
+      // A loop of its own: folded into the loop below (the table read chosen per step), it made the mixed-warp launches
+      // ~2 % slower.
 #pragma unroll
       for (int u = 0; u < kU; ++u) {
         if (u < steps) ldg_step(bl.table, prep_action(cax[u], cay[u]), sx, sy);
@@ -457,9 +460,8 @@ struct PairSmem {
 
 template <bool kTraj, int kStages, int kUp, bool kBank = false>
 __global__ void __launch_bounds__(256)
-env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict__ g_fits, float* __restrict__ x, float* __restrict__ y,
-                        const __grid_constant__ CUtensorMap tm_act, const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T,
-                        MapBank bank) {
+env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __grid_constant__ CUtensorMap tm_act,
+                        const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T, MapBank bank) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   constexpr int kU = kUp;                            // steps per action / trajectory tile of this kernel (shadows the file-wide kU)
   constexpr int kTileFloats = kU * 2 * 32;
@@ -483,14 +485,14 @@ env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict
     for (int b = 0; b < 2; ++b) { mbar_init(prepped + b, 32); mbar_init(consumed + b, 32); mbar_init(outfull + b, 32); mbar_init(outfree + b, 1); }
     fence_mbar_init();
   }
+  const int staged = bank.map<kBank>((int64_t)blockIdx.x * npairs * 32);   // the CTA stages the halo table of its first env's map
   BankLanes bl{};
-  if constexpr (kBank) {                             // the CTA stages the halo table of its first env's map
+  if constexpr (kBank) {
     const int64_t env = ((int64_t)blockIdx.x * npairs + pair) * 32 + lane;
-    bl = bank_lanes(bank, (int64_t)blockIdx.x * npairs * 32, env, env < n);
-    g_halo = bank.halos + (size_t)bl.staged * (kHaloDim * kHaloDim);
-    g_fits = bank.fits + bl.staged;
+    bl = bank_lanes(bank, staged, env, env < n);
   }
-  stage_table<kHaloBytes>(s_table, bar, g_halo);   // contains the __syncthreads that publishes the barrier inits
+  // contains the __syncthreads that publishes the barrier inits
+  stage_table<kHaloBytes>(s_table, bar, bank.halos + (size_t)staged * (kHaloDim * kHaloDim));
 
   const int64_t i0 = ((int64_t)blockIdx.x * npairs + pair) * 32;
   if (i0 >= n) return;
@@ -560,7 +562,7 @@ env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict
   // ================================= chain warp =================================
   const int64_t i = i0 + lane;
   const bool live = i < n;
-  const bool fits = *g_fits != 0;                    // lands while the table is staging
+  const bool fits = __ldg(bank.fits + staged) != 0;  // lands while the table is staging
   float sx = live ? fminf(fmaxf(x[i], 0.0f), 99.99999f) : 0.0f;
   float sy = live ? fminf(fmaxf(y[i], 0.0f), 99.99999f) : 0.0f;
   const uint32_t addr_bias = smem_u32(s_table) - 0x4B000000u * (kHaloRowBytes + 8u);
@@ -597,7 +599,8 @@ env_rollout_pair_kernel(const float2* __restrict__ g_halo, const int* __restrict
       }
       if (kTraj) store_state(kU - 1);
     } else if (kBank && bl.mixed) {
-      // lanes on different maps: each steps from its own map's plain table, addressed from the state as below
+      // lanes on different maps: each steps from its own map's plain table, addressed from the state as below (a loop of its
+      // own for the same reason as in env_rollout_tma_kernel)
       const int steps = (int)min((int64_t)kU, T - c * kU);
 #pragma unroll
       for (int u = 0; u < kU; ++u) {
@@ -743,8 +746,46 @@ static int32_t check_bank(const rtd3_mt_bank* b) {
 using namespace rtd3;
 
 constexpr int kMaxMaps = 65536;
-static bool g_force_plain_rollout = false;
-static int g_rollout_variant = 0;            // test hook: 1 = single-warp TMA kernel instead of the warp-pair kernel
+static int g_rollout_hook = 0;   // rtd3_env_force_plain_rollout: 1 = the cp.async kernel, 2 = the single-warp TMA kernel for every size
+
+// Every kernel instantiation a launch can pick.  The launches index these tables, and rtd3_env_create sets the shared-memory
+// limit of every entry.
+// env_step_kernel, [table][keep_on_nan]; table 0: read-only path, 1: staged in shared memory, 2: each env's own map of the bank
+using StepKernel = decltype(&env_step_kernel<false, false>);
+static const StepKernel kStepKernels[3][2] = {{env_step_kernel<false, false>, env_step_kernel<false, true>},
+                                              {env_step_kernel<true, false>, env_step_kernel<true, true>},
+                                              {env_step_kernel<false, false, true>, env_step_kernel<false, true, true>}};
+// rollout kernels, [bank][traj][stages]; stages 1: kDeep (latency-bound batches), 0: kShallow
+using RolloutKernel = decltype(&env_rollout_kernel<false, kDeep>);
+static const RolloutKernel kRolloutKernels[2][2][2] = {
+    {{env_rollout_kernel<false, kShallow>, env_rollout_kernel<false, kDeep>},
+     {env_rollout_kernel<true, kShallow>, env_rollout_kernel<true, kDeep>}},
+    {{env_rollout_kernel<false, kShallow, true>, env_rollout_kernel<false, kDeep, true>},
+     {env_rollout_kernel<true, kShallow, true>, env_rollout_kernel<true, kDeep, true>}}};
+using TmaKernel = decltype(&env_rollout_tma_kernel<false, kDeep>);
+static const TmaKernel kTmaKernels[2][2][2] = {
+    {{env_rollout_tma_kernel<false, kShallow>, env_rollout_tma_kernel<false, kDeep>},
+     {env_rollout_tma_kernel<true, kShallow>, env_rollout_tma_kernel<true, kDeep>}},
+    {{env_rollout_tma_kernel<false, kShallow, true>, env_rollout_tma_kernel<false, kDeep, true>},
+     {env_rollout_tma_kernel<true, kShallow, true>, env_rollout_tma_kernel<true, kDeep, true>}}};
+// pair kernel, [bank][traj][two pairs per CTA]
+using PairKernel = decltype(&env_rollout_pair_kernel<false, kPairStages, kPairU>);
+static const PairKernel kPairKernels[2][2][2] = {
+    {{env_rollout_pair_kernel<false, kPairStages, kPairU>, env_rollout_pair_kernel<false, kPairStages2, kPairU>},
+     {env_rollout_pair_kernel<true, kPairStages, kPairU>, env_rollout_pair_kernel<true, kPairStages2, kPairU>}},
+    {{env_rollout_pair_kernel<false, kPairStages, kPairU, true>, env_rollout_pair_kernel<false, kPairStages2, kPairU, true>},
+     {env_rollout_pair_kernel<true, kPairStages, kPairU, true>, env_rollout_pair_kernel<true, kPairStages2, kPairU, true>}}};
+
+template <typename... Args>
+static cudaError_t set_max_smem(void (*kernel)(Args...), int bytes) {
+  return cudaFuncSetAttribute((const void*)kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+}
+template <typename T, size_t N>
+static cudaError_t set_max_smem(const T (&kernels)[N], int bytes) {
+  for (const T& k : kernels)
+    if (cudaError_t e = set_max_smem(k, bytes)) return e;
+  return cudaSuccess;
+}
 
 // cuTensorMapEncodeTiled comes from the driver (libcuda); it is looked up at run time so that librtd3.so links against
 // the runtime only.  If the lookup fails the rollout falls back to the cp.async kernel.
@@ -760,8 +801,8 @@ static void load_encode_tiled() {
     g_encode_tiled = (EncodeTiledFn)fn;
 }
 
-// [T][2][n] float32 planes as a 2-D tensor: inner dim n, outer dim 2T, box = 32 envs x 2*kU rows
-static int32_t make_plane_map(CUtensorMap* tm, const float* base, int64_t n, int64_t T, int steps_per_tile = kU) {
+// [T][2][n] float32 planes as a 2-D tensor: inner dim n, outer dim 2T, box = 32 envs x 2*steps_per_tile rows
+static int32_t make_plane_map(CUtensorMap* tm, const float* base, int64_t n, int64_t T, int steps_per_tile) {
   const cuuint64_t dims[2] = {(cuuint64_t)n, (cuuint64_t)(2 * T)};
   const cuuint64_t strides[1] = {(cuuint64_t)n * 4};
   const cuuint32_t box[2] = {32, (cuuint32_t)(2 * steps_per_tile)};
@@ -773,7 +814,7 @@ static int32_t make_plane_map(CUtensorMap* tm, const float* base, int64_t n, int
     return RTD3_ERR_STATE;
   }
   return 0;
-}   // test hook: exercise the cp.async variant on aligned sizes too
+}
 
 // (Re)allocates the bank for `cap` maps (synchronous: kernels in flight may read the old bank).  The contents are not kept.
 static int32_t alloc_bank(rtd3_env* h, int cap) {
@@ -784,80 +825,35 @@ static int32_t alloc_bank(rtd3_env* h, int cap) {
     cudaFree(h->halos);
     cudaFree(h->fits);
   }
-  h->tables = h->halos = h->table = h->halo = nullptr;
-  h->fits = h->halo_fits = nullptr;
+  h->tables = h->halos = nullptr;
+  h->fits = nullptr;
   h->map_cap = h->num_maps = 0;
-  h->has_map = false;
   RTD3_CUDA(cudaMalloc(&h->tables, (size_t)cap * kTableBytes));
   RTD3_CUDA(cudaMalloc(&h->halos, (size_t)cap * kHaloBytes));
   RTD3_CUDA(cudaMalloc(&h->fits, (size_t)cap * sizeof(int)));
-  h->table = h->tables;
-  h->halo = h->halos;
-  h->halo_fits = h->fits;
   h->map_cap = cap;
   return 0;
 }
 
-// the bank instantiations of the rollout kernels need the same shared memory as the single-map ones
-static int32_t set_bank_smem(int smem_roll) {
-  const void* full[] = {(const void*)env_rollout_kernel<true, kDeep, true>, (const void*)env_rollout_kernel<false, kDeep, true>,
-                        (const void*)env_rollout_kernel<true, kShallow, true>, (const void*)env_rollout_kernel<false, kShallow, true>,
-                        (const void*)env_rollout_tma_kernel<true, kDeep, true>, (const void*)env_rollout_tma_kernel<false, kDeep, true>,
-                        (const void*)env_rollout_tma_kernel<true, kShallow, true>, (const void*)env_rollout_tma_kernel<false, kShallow, true>};
-  const void* pair[] = {(const void*)env_rollout_pair_kernel<true, kPairStages, kPairU, true>, (const void*)env_rollout_pair_kernel<false, kPairStages, kPairU, true>,
-                        (const void*)env_rollout_pair_kernel<true, kPairStages2, kPairU, true>, (const void*)env_rollout_pair_kernel<false, kPairStages2, kPairU, true>};
-  for (const void* f : full) RTD3_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  for (const void* f : pair) RTD3_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
-  return 0;
-}
-
-static MapBank map_bank(const rtd3_env* h) {
-  return MapBank{h->tables, h->halos, h->fits, h->index_len ? h->index : nullptr, h->index_len, h->num_maps};
-}
-
 extern "C" {
 
-void rtd3_env_force_plain_rollout(int32_t on) { g_force_plain_rollout = on == 1; g_rollout_variant = on == 2 ? 1 : 0; }
+void rtd3_env_force_plain_rollout(int32_t on) { g_rollout_hook = on == 1 || on == 2 ? on : 0; }
 
 int32_t rtd3_env_create(rtd3_env** out, int32_t device) {
   RTD3_CHECK_ARG(out, "out is null");
-  int prev = 0;
-  RTD3_CUDA(cudaGetDevice(&prev));
-  RTD3_CUDA(cudaSetDevice(device));
-  rtd3_env* h = new rtd3_env();
+  DeviceGuard guard;
+  RTD3_CUDA(guard.enter(device));
+  std::unique_ptr<rtd3_env, int32_t (*)(rtd3_env*)> h(new rtd3_env(), rtd3_env_destroy);   // freed on every error return
   h->device = device;
-  h->has_map = false;
-  h->table = nullptr;
-  h->halo = nullptr;
-  h->halo_fits = nullptr;
-  h->host_pipe = nullptr;
-  h->tables = h->halos = nullptr;
-  h->fits = nullptr;
-  h->num_maps = h->map_cap = 0;
-  h->index = nullptr;
-  h->index_len = h->index_cap = 0;
   RTD3_CUDA(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, device));
-  if (int32_t e = alloc_bank(h, 1)) return e;
+  if (int32_t e = alloc_bank(h.get(), 1)) return e;
   if (!g_encode_tiled) load_encode_tiled();
-  const int smem = kTableBytes + 16;
-  RTD3_CUDA(cudaFuncSetAttribute(env_step_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  RTD3_CUDA(cudaFuncSetAttribute(env_step_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+  RTD3_CUDA(set_max_smem(kStepKernels[1], kTableBytes + 16));
   const int smem_roll = 227 * 1024;
-  if (int32_t e = set_bank_smem(smem_roll)) return e;
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<true, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<false, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<true, kShallow>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_kernel<false, kShallow>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<true, kPairStages, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<false, kPairStages, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<true, kPairStages2, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_pair_kernel<false, kPairStages2, kPairU>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll - 1024));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_tma_kernel<true, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_tma_kernel<false, kDeep>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_tma_kernel<true, kShallow>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaFuncSetAttribute(env_rollout_tma_kernel<false, kShallow>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_roll));
-  RTD3_CUDA(cudaSetDevice(prev));
-  *out = h;
+  RTD3_CUDA(set_max_smem(kRolloutKernels, smem_roll));
+  RTD3_CUDA(set_max_smem(kTmaKernels, smem_roll));
+  RTD3_CUDA(set_max_smem(kPairKernels, smem_roll - 1024));
+  *out = h.release();
   return 0;
 }
 
@@ -876,12 +872,9 @@ int32_t rtd3_env_set_maps(rtd3_env* h, const float* speed, const float* angle, i
   RTD3_CHECK_ARG(h && speed && angle, "null argument");
   RTD3_CHECK_ARG(K >= 1 && K <= kMaxMaps, "map count K must be in [1, 65536]");
   if (K > h->map_cap) {
-    int prev = 0;
-    RTD3_CUDA(cudaGetDevice(&prev));
-    RTD3_CUDA(cudaSetDevice(h->device));
-    const int32_t e = alloc_bank(h, K);
-    cudaSetDevice(prev);
-    if (e) return e;
+    DeviceGuard guard;
+    RTD3_CUDA(guard.enter(h->device));
+    if (int32_t e = alloc_bank(h, K)) return e;
   }
   const int64_t cells = (int64_t)K * kCells;
   build_table_kernel<<<(int)ceil_div(cells, 256), 256, 0, (cudaStream_t)stream>>>(speed, angle, h->tables, cells);
@@ -889,7 +882,6 @@ int32_t rtd3_env_set_maps(rtd3_env* h, const float* speed, const float* angle, i
   build_halo_kernel<<<K, 1024, 0, (cudaStream_t)stream>>>(h->tables, h->halos, h->fits);
   RTD3_LAUNCHED();
   h->num_maps = K;
-  h->has_map = true;
   return 0;
 }
 
@@ -906,16 +898,14 @@ int32_t rtd3_env_set_map_index(rtd3_env* h, const int32_t* index, int64_t m, voi
     return 0;
   }
   if (m > h->index_cap) {
-    int prev = 0;
-    RTD3_CUDA(cudaGetDevice(&prev));
-    RTD3_CUDA(cudaSetDevice(h->device));
+    DeviceGuard guard;
+    RTD3_CUDA(guard.enter(h->device));
     rtd3::host_pipe_drop_graphs(h);   // they hold the old index address
     cudaDeviceSynchronize();          // kernels in flight may still read the old index
     if (h->index) cudaFree(h->index);
     h->index = nullptr;
     h->index_len = h->index_cap = 0;
     const cudaError_t ce = cudaMalloc(&h->index, (size_t)m * sizeof(int32_t));
-    cudaSetDevice(prev);
     if (ce != cudaSuccess) {
       rtd3::set_error("cudaMalloc of a %lld-entry map index -> %s", (long long)m, cudaGetErrorString(ce));
       return (int32_t)ce;
@@ -929,16 +919,17 @@ int32_t rtd3_env_set_map_index(rtd3_env* h, const int32_t* index, int64_t m, voi
 
 int32_t rtd3_env_map_config(const rtd3_env* h, const void** tables, const void** index, int32_t* num_maps, int64_t* index_len) {
   RTD3_CHECK_ARG(h, "null handle");
-  if (tables) *tables = h->tables;
-  if (index) *index = h->index_len ? h->index : nullptr;
-  if (num_maps) *num_maps = h->num_maps;
-  if (index_len) *index_len = h->index_len;
+  const MapBank b = map_bank(h);
+  if (tables) *tables = b.tables;
+  if (index) *index = b.index;
+  if (num_maps) *num_maps = b.K;
+  if (index_len) *index_len = b.m;
   return 0;
 }
 
 static int32_t launch_step(rtd3_env* h, const float* x, const float* y, const float* ax, const float* ay, float* ox,
                            float* oy, int64_t n, int32_t variant, bool keep_on_nan, cudaStream_t st) {
-  RTD3_CHECK_ARG(h && h->has_map, "environment has no dynamics map (call rtd3_env_set_map)");
+  RTD3_CHECK_ARG(h && h->num_maps > 0, "environment has no dynamics map (call rtd3_env_set_map)");
   RTD3_CHECK_ARG(n >= 0, "negative n");
   if (n == 0) return 0;
   RTD3_CHECK_ARG(x && y && ax && ay && ox && oy, "null state/action pointer");
@@ -948,23 +939,12 @@ static int32_t launch_step(rtd3_env* h, const float* x, const float* y, const fl
   const int64_t n4 = vec_ok ? (n + 3) / 4 : n;
   if (variant == RTD3_STEP_AUTO) variant = (n >= 262144) ? RTD3_STEP_SMEM : RTD3_STEP_LDG;
   const MapBank bank = map_bank(h);
-  if (bank.index) {                  // one table per env: no table to stage, every variant reads through the read-only path
-    const int block = 256;
-    const int grid = (int)std::min<int64_t>(ceil_div(n4, block), (int64_t)h->num_sms * 4);
-    if (keep_on_nan) env_step_kernel<false, true, true><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
-    else env_step_kernel<false, false, true><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
-  } else if (variant == RTD3_STEP_SMEM) {
-    const int block = 512;
-    const int grid = (int)std::min<int64_t>(ceil_div(n4, block), (int64_t)h->num_sms * 2);
-    const int smem = kTableBytes + 16;
-    if (keep_on_nan) env_step_kernel<true, true><<<grid, block, smem, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
-    else env_step_kernel<true, false><<<grid, block, smem, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
-  } else {
-    const int block = 256;
-    const int grid = (int)std::min<int64_t>(ceil_div(n4, block), (int64_t)h->num_sms * 4);
-    if (keep_on_nan) env_step_kernel<false, true><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
-    else env_step_kernel<false, false><<<grid, block, 0, st>>>(h->table, x, y, ax, ay, ox, oy, n, vec_ok, bank);
-  }
+  // with an index there is one table per env and none to stage: every variant reads through the read-only path
+  const bool smem = !bank.index && variant == RTD3_STEP_SMEM;
+  const int block = smem ? 512 : 256;
+  const int grid = (int)std::min<int64_t>(ceil_div(n4, block), (int64_t)h->num_sms * (smem ? 2 : 4));
+  const StepKernel kern = kStepKernels[bank.index ? 2 : smem ? 1 : 0][keep_on_nan];
+  kern<<<grid, block, smem ? kTableBytes + 16 : 0, st>>>(vec_ok, x, y, ax, ay, ox, oy, n, bank);
   RTD3_LAUNCHED();
   return 0;
 }
@@ -981,7 +961,7 @@ int32_t rtd3_env_dynamics(rtd3_env* h, const float* x, const float* y, const flo
 
 int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, float* traj, int64_t n, int64_t T,
                          void* stream) {
-  RTD3_CHECK_ARG(h && h->has_map, "environment has no dynamics map (call rtd3_env_set_map)");
+  RTD3_CHECK_ARG(h && h->num_maps > 0, "environment has no dynamics map (call rtd3_env_set_map)");
   RTD3_CHECK_ARG(n >= 0 && T >= 0, "negative n or T");
   if (n == 0 || T == 0) return 0;
   RTD3_CHECK_ARG(x && y && actions, "null state/action pointer");
@@ -990,53 +970,42 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
   // 128-thread CTAs, kShallow chunks in flight, up to 2 CTAs per SM next to the 80 KB table.
   const int64_t per_sm = ceil_div(n, (int64_t)h->num_sms);
   const bool deep = per_sm <= 64;
-  const int block = deep ? (int)std::max<int64_t>(32, ceil_div(per_sm, 32) * 32) : 128;
-  const int grid = (int)ceil_div(n, block);
   const int stages = deep ? kDeep : kShallow;
-  const int smem = kTableBytes + 16 + stages * kU * 2 * block * 4;
   cudaStream_t st = (cudaStream_t)stream;
   const MapBank bank = map_bank(h);   // bank.index == nullptr: the single-map kernels
+  const bool with_bank = bank.index != nullptr, with_traj = traj != nullptr;
+  // latency-bound batches run the warp-pair kernel, with tiles of kPairU steps (the per-tile hand-over - two barrier waits, the
+  // flag read, two arrives - was ~20 % of the chain warp's samples at 16)
+  const bool pair = deep && g_rollout_hook != 2;
   const bool tma_ok = (n % 4 == 0) && (n < (1ll << 31)) && (2 * T < (1ll << 31)) && ((uintptr_t)actions % 16 == 0) &&
-                      (!traj || (uintptr_t)traj % 16 == 0) && !g_force_plain_rollout && g_encode_tiled;
+                      (!traj || (uintptr_t)traj % 16 == 0) && g_rollout_hook != 1 && g_encode_tiled;
   CUtensorMap tm_act, tm_traj;
+  const int tile_steps = pair ? kPairU : kU;
   // an encode failure (unexpected shape limits) is not an error: the cp.async kernel below handles every shape
-  if (tma_ok && make_plane_map(&tm_act, actions, n, T) == 0 && make_plane_map(&tm_traj, traj ? traj : actions, n, T) == 0) {
-    // one warp per 32 envs; few warps per CTA while the batch cannot fill the SMs, 8 once it can
+  if (tma_ok && make_plane_map(&tm_act, actions, n, T, tile_steps) == 0 &&
+      make_plane_map(&tm_traj, traj ? traj : actions, n, T, tile_steps) == 0) {
     const int64_t warps_total = ceil_div(n, 32);
-    const int wpc = deep ? (int)std::max<int64_t>(1, std::min<int64_t>(8, ceil_div(warps_total, (int64_t)h->num_sms))) : 8;
-    const int bgrid = (int)ceil_div(warps_total, wpc);
-    const int bsmem = ((kTableBytes + 16 + wpc * stages * 8 + 127) & ~127) + wpc * (stages + 2) * kTileFloats * 4;
-    if (deep && g_rollout_variant != 1) {
-      // latency-bound batches: one chain warp + one helper warp per 32 envs, up to 2 pairs per CTA; tiles of kPairU steps
-      // (the per-tile hand-over - two barrier waits, the flag read, two arrives - was ~20 % of the chain warp's samples at 16)
+    if (pair) {
+      // one chain warp + one helper warp per 32 envs, up to 2 pairs per CTA
       const int ppc = (int)std::max<int64_t>(1, std::min<int64_t>(2, ceil_div(warps_total, (int64_t)h->num_sms)));
-      const int pgrid = (int)ceil_div(warps_total, ppc);
       const int pstages = ppc == 1 ? kPairStages : kPairStages2;
       const int psmem = ((kHaloBytes + 16 + ppc * PairSmem::kBars * 8 + 127) & ~127) + ppc * (pstages + 4) * (kPairU * 2 * 32) * 4;
-      if (make_plane_map(&tm_act, actions, n, T, kPairU) != 0 || make_plane_map(&tm_traj, traj ? traj : actions, n, T, kPairU) != 0) return RTD3_ERR_STATE;
-      decltype(&env_rollout_pair_kernel<true, kPairStages, kPairU>) kern;
-      if (bank.index) kern = ppc == 1 ? (traj ? env_rollout_pair_kernel<true, kPairStages, kPairU, true> : env_rollout_pair_kernel<false, kPairStages, kPairU, true>)
-                                      : (traj ? env_rollout_pair_kernel<true, kPairStages2, kPairU, true> : env_rollout_pair_kernel<false, kPairStages2, kPairU, true>);
-      else kern = ppc == 1 ? (traj ? env_rollout_pair_kernel<true, kPairStages, kPairU> : env_rollout_pair_kernel<false, kPairStages, kPairU>)
-                           : (traj ? env_rollout_pair_kernel<true, kPairStages2, kPairU> : env_rollout_pair_kernel<false, kPairStages2, kPairU>);
-      kern<<<pgrid, ppc * 64, psmem, st>>>(h->halo, h->halo_fits, x, y, tm_act, tm_traj, n, T, bank);
+      const PairKernel kern = kPairKernels[with_bank][with_traj][ppc == 2];
+      kern<<<(int)ceil_div(warps_total, ppc), ppc * 64, psmem, st>>>(x, y, tm_act, tm_traj, n, T, bank);
     } else {
-      decltype(&env_rollout_tma_kernel<true, kDeep>) kern;
-      if (bank.index) kern = deep ? (traj ? env_rollout_tma_kernel<true, kDeep, true> : env_rollout_tma_kernel<false, kDeep, true>)
-                                  : (traj ? env_rollout_tma_kernel<true, kShallow, true> : env_rollout_tma_kernel<false, kShallow, true>);
-      else kern = deep ? (traj ? env_rollout_tma_kernel<true, kDeep> : env_rollout_tma_kernel<false, kDeep>)
-                       : (traj ? env_rollout_tma_kernel<true, kShallow> : env_rollout_tma_kernel<false, kShallow>);
-      kern<<<bgrid, wpc * 32, bsmem, st>>>(h->table, x, y, tm_act, tm_traj, n, T, bank);
+      // one warp per 32 envs; few warps per CTA while the batch cannot fill the SMs, 8 once it can
+      const int wpc = deep ? (int)std::max<int64_t>(1, std::min<int64_t>(8, ceil_div(warps_total, (int64_t)h->num_sms))) : 8;
+      const int bsmem = ((kTableBytes + 16 + wpc * stages * 8 + 127) & ~127) + wpc * (stages + 2) * kTileFloats * 4;
+      const TmaKernel kern = kTmaKernels[with_bank][with_traj][deep];
+      kern<<<(int)ceil_div(warps_total, wpc), wpc * 32, bsmem, st>>>(n, x, y, tm_act, tm_traj, T, bank);
     }
     RTD3_LAUNCHED();
     return 0;
   }
-  decltype(&env_rollout_kernel<true, kDeep>) kern;
-  if (bank.index) kern = deep ? (traj ? env_rollout_kernel<true, kDeep, true> : env_rollout_kernel<false, kDeep, true>)
-                              : (traj ? env_rollout_kernel<true, kShallow, true> : env_rollout_kernel<false, kShallow, true>);
-  else kern = deep ? (traj ? env_rollout_kernel<true, kDeep> : env_rollout_kernel<false, kDeep>)
-                   : (traj ? env_rollout_kernel<true, kShallow> : env_rollout_kernel<false, kShallow>);
-  kern<<<grid, block, smem, st>>>(h->table, x, y, actions, traj, n, T, bank);
+  const int block = deep ? (int)std::max<int64_t>(32, ceil_div(per_sm, 32) * 32) : 128;
+  const int smem = kTableBytes + 16 + stages * kU * 2 * block * 4;
+  const RolloutKernel kern = kRolloutKernels[with_bank][with_traj][deep];
+  kern<<<(int)ceil_div(n, block), block, smem, st>>>(n, x, y, actions, traj, T, bank);
   RTD3_LAUNCHED();
   return 0;
 }

@@ -12,21 +12,13 @@
 
 namespace rtd3 {
 
-// The map configuration a captured rollout kernel holds as arguments (and whether it is the single-map or the bank kernel).
-// Reallocating the bank or the index drops the cached graphs; a change of K or m without one makes them miss here.
-struct MapKey {
-  const void *tables, *index;
-  int64_t m;
-  int32_t K;
-  bool operator==(const MapKey& o) const { return tables == o.tables && index == o.index && m == o.m && K == o.K; }
-};
-static MapKey map_key(const rtd3_env* h) { return MapKey{h->tables, h->index_len ? h->index : nullptr, h->index_len, h->num_maps}; }
-
 struct HostGraph {
   const void *x, *y, *act, *traj;
   int64_t n, T;
   int32_t chunks, mode;
-  MapKey map;
+  // The map configuration the captured rollout kernels hold as arguments (and whether they are the single-map or the bank
+  // kernels).  Reallocating the bank or the index drops the cached graphs; a change of K or m without one makes them miss.
+  MapBank map;
   cudaGraphExec_t exec;
 };
 
@@ -56,9 +48,8 @@ void host_pipe_drop_graphs(rtd3_env* h) {
 void host_pipe_destroy(rtd3_env* h) {
   HostPipe* p = (HostPipe*)h->host_pipe;
   if (!p) return;
-  int prev = 0;
-  cudaGetDevice(&prev);
-  cudaSetDevice(h->device);
+  DeviceGuard guard;
+  guard.enter(h->device);
   drop_graphs(p);
   for (cudaEvent_t e : p->events) cudaEventDestroy(e);
   if (p->d_act) cudaFree(p->d_act);
@@ -66,7 +57,6 @@ void host_pipe_destroy(rtd3_env* h) {
   if (p->cap) cudaStreamDestroy(p->cap);
   if (p->s_in) cudaStreamDestroy(p->s_in);
   if (p->s_out) cudaStreamDestroy(p->s_out);
-  cudaSetDevice(prev);
   delete p;
   h->host_pipe = nullptr;
 }
@@ -157,7 +147,7 @@ using namespace rtd3;
 
 extern "C" int32_t rtd3_env_rollout_host(rtd3_env* h, float* x, float* y, const float* actions_host, float* traj_host, int64_t n,
                                          int64_t T, int32_t chunks, int32_t mode, void* stream) {
-  RTD3_CHECK_ARG(h && h->has_map, "environment has no dynamics map (call rtd3_env_set_map)");
+  RTD3_CHECK_ARG(h && h->num_maps > 0, "environment has no dynamics map (call rtd3_env_set_map)");
   RTD3_CHECK_ARG(n >= 0 && T >= 0, "negative n or T");
   RTD3_CHECK_ARG(mode >= 0 && mode <= 3, "mode is a bit set: 1 = stage the actions, 2 = stage the trajectory");
   if (n == 0 || T == 0) return 0;
@@ -167,14 +157,13 @@ extern "C" int32_t rtd3_env_rollout_host(rtd3_env* h, float* x, float* y, const 
     return rtd3_env_rollout(h, x, y, actions_host, traj_host, n, T, stream);
   chunks = (int32_t)std::max<int64_t>(1, std::min<int64_t>(chunks, std::min<int64_t>(T, 256)));
   const bool stage_in = mode & 1, stage_out = mode & 2;
-  int prev = 0;
-  RTD3_CUDA(cudaGetDevice(&prev));
-  if (prev != h->device) RTD3_CUDA(cudaSetDevice(h->device));
+  DeviceGuard guard;
+  RTD3_CUDA(guard.enter(h->device));
   std::lock_guard<std::mutex> lock(g_pipe_mu);
   HostPipe* p = nullptr;
   int32_t rc = pipe_prepare(h, &p, (size_t)(2 * n * T), 2 * chunks + 2);
   cudaGraphExec_t exec = nullptr;
-  const MapKey mk = map_key(h);
+  const MapBank mk = map_bank(h);
   if (rc == 0) {
     for (auto& g : p->graphs)
       if (g.x == x && g.y == y && g.act == actions_host && g.traj == traj_host && g.n == n && g.T == T && g.chunks == chunks && g.mode == mode &&
@@ -221,6 +210,5 @@ extern "C" int32_t rtd3_env_rollout_host(rtd3_env* h, float* x, float* y, const 
       }
     }
   }
-  if (prev != h->device) cudaSetDevice(prev);
   return rc;
 }

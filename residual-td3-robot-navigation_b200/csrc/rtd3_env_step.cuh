@@ -5,22 +5,18 @@
 #include "rtd3_mt.cuh"
 
 struct rtd3_env {
-  int device;
-  int num_sms;
-  float2* table;   // [100*100] (speed*cos(rot), speed*sin(rot)), indexed x*100+y: map 0 of the bank
-  float2* halo;    // [116*116] the same table with an 8-cell border, read by the warp-pair rollout (rtd3_env.cu: build_halo_kernel)
-  int* halo_fits;  // 1 when every cell moves a state by less than the border per step (kMaxAction*(|c|+|s|) <= kHaloReach)
-  bool has_map;
-  void* host_pipe;   // rtd3::HostPipe of rtd3_env_rollout_host (rtd3_env_host.cu), created on first use
-  // Map bank (rtd3_env_set_maps / rtd3_env_set_map_index): map_cap maps allocated, num_maps of them set.  tables / halos / fits
-  // are [map_cap][...] and table / halo / halo_fits point at map 0.  Env v of a launch steps on map index[v % index_len]; with
-  // index_len == 0 there is no index and every launch runs the single-map kernels on map 0.
-  float2* tables;
-  float2* halos;
-  int* fits;
-  int num_maps, map_cap;
-  int32_t* index;
-  int64_t index_len, index_cap;
+  int device = 0;
+  int num_sms = 0;
+  void* host_pipe = nullptr;   // rtd3::HostPipe of rtd3_env_rollout_host (rtd3_env_host.cu), created on first use
+  // Map bank (rtd3_env_set_maps / rtd3_env_set_map_index): map_cap maps allocated, num_maps of them set (none before the first
+  // rtd3_env_set_map(s)).  Env v of a launch steps on map index[v % index_len]; with index_len == 0 there is no index and every
+  // launch runs the single-map kernels on map 0.
+  float2* tables = nullptr;   // [map_cap][100*100] (speed*cos(rot), speed*sin(rot)), indexed x*100+y
+  float2* halos = nullptr;    // [map_cap][116*116] the same tables with an 8-cell border, read by the warp-pair rollout (rtd3_env.cu: build_halo_kernel)
+  int* fits = nullptr;        // [map_cap] 1 when every cell moves a state by less than the border per step (kMaxAction*(|c|+|s|) <= kHaloReach)
+  int num_maps = 0, map_cap = 0;
+  int32_t* index = nullptr;
+  int64_t index_len = 0, index_cap = 0;
 };
 
 namespace rtd3 {
@@ -41,8 +37,21 @@ struct MapBank {
     const int k = __ldg(index + (v < m ? v : v % m));
     return min(max(k, 0), K - 1);
   }
-  __device__ __forceinline__ const float2* table_of(int64_t v) const { return tables + (size_t)map_of(v) * kCells; }
+  // the map env v steps on in a kernel instantiated with or without the bank: its own, or map 0 (the launches without an index)
+  template <bool kBank>
+  __device__ __forceinline__ int map(int64_t v) const { return kBank ? map_of(v) : 0; }
+  template <bool kBank>
+  __device__ __forceinline__ const float2* table(int64_t v) const { return tables + (size_t)map<kBank>(v) * kCells; }
+  // the same launch arguments: a launch captured with one is a launch with the other
+  bool operator==(const MapBank& o) const {
+    return tables == o.tables && halos == o.halos && fits == o.fits && index == o.index && m == o.m && K == o.K;
+  }
 };
+
+// The only place a MapBank is built: what every step, rollout and tick launch of `h` passes.
+inline MapBank map_bank(const rtd3_env* h) {
+  return MapBank{h->tables, h->halos, h->fits, h->index_len ? h->index : nullptr, h->index_len, h->num_maps};
+}
 
 // One env-step, the rotation form of environment.py:100-117 (no atan2):
 //   s' = clip(s + speed*(ax*cos(rot) - ay*sin(rot), ax*sin(rot) + ay*cos(rot)), 0, 98.9999)

@@ -142,19 +142,18 @@ __device__ __forceinline__ void tick_post_env(const rtd3_tick_state& t, const fl
   reset_finish_warp(t.env_bank, resets, i, rl, t.x, t.y, t.state64);
 }
 
-// kBank: env i steps on its own map of the bank (`table` is map 0, the table of the single-map launches)
+// kBank: env i steps on its own map of the bank, else on map 0
 template <bool kBank = false>
-__global__ void __launch_bounds__(256, 2) tick_post_kernel(rtd3_tick_state t, const float2* __restrict__ table,
-                                                           const float* __restrict__ residual /*[n][2]*/,
+__global__ void __launch_bounds__(256, 2) tick_post_kernel(rtd3_tick_state t, const float* __restrict__ residual /*[n][2]*/,
                                                            const double* __restrict__ unit_noise /*[2][n], mode 1*/, int noise_mode,
                                                            MapBank bank) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const bool in = i < t.n;
   const int64_t ii = in ? i : 0;
-  if constexpr (kBank) table = bank.table_of(ii);
   // the Philox noise of a tick is keyed by the number of ticks run including this one (word 1 of the counter, see tick_pre_kernel)
   const uint64_t tick_index = t.tick_counter ? t.tick_counter[1] : 0ull;
-  tick_post_env<true>(t, table, i, in, in ? (int)t.type[ii] : 1, reinterpret_cast<const float2*>(residual)[ii], unit_noise, noise_mode, tick_index);
+  tick_post_env<true>(t, bank.table<kBank>(ii), i, in, in ? (int)t.type[ii] : 1, reinterpret_cast<const float2*>(residual)[ii], unit_noise,
+                      noise_mode, tick_index);
   if (i == 0 && t.tick_counter) t.tick_counter[0] = tick_index;
 }
 
@@ -168,8 +167,8 @@ __global__ void __launch_bounds__(256, 2) tick_post_kernel(rtd3_tick_state t, co
 // (tests/test_tick_gpu.py).  Needs candidate lists or no demonstration states (no block-wide sweep here) and Philox or no noise.
 template <bool kBank = false>
 __global__ void __launch_bounds__(kHfThreads, 1)
-tick_f16_kernel(rtd3_tick_state t, const float2* __restrict__ table, NetShape s, const float* __restrict__ P, const uint16_t* __restrict__ Wh,
-                int noise_mode, int K, uint64_t tick_base, uint32_t tmem_cols, MapBank bank) {
+tick_f16_kernel(rtd3_tick_state t, NetShape s, const float* __restrict__ P, const uint16_t* __restrict__ Wh, int noise_mode, int K,
+                uint64_t tick_base, uint32_t tmem_cols, MapBank bank) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
   const int H = s.hid;
   const HfSmem m = hf_carve(smem_raw, H);
@@ -229,7 +228,7 @@ tick_f16_kernel(rtd3_tick_state t, const float2* __restrict__ table, NetShape s,
         bar_sync(1, kHfRowThreads);
         // the other twelve warps go on to wait for the next tick's actor input; sbase / part are rewritten only after barriers the
         // owners reach after they are done reading them
-        if (owner) tick_post_env<false>(t, kBank ? bank.table_of(in ? i : 0) : table, i, in, type, hf_output(m, rt, 0), nullptr, noise_mode,
+        if (owner) tick_post_env<false>(t, bank.table<kBank>(in ? i : 0), i, in, type, hf_output(m, rt, 0), nullptr, noise_mode,
                                         tick_base + (uint64_t)k + 1ull);
       }
     }
@@ -281,7 +280,7 @@ int32_t rtd3_tick_pre(const rtd3_tick_state* t, void* stream) {
 int32_t rtd3_tick_post(rtd3_env* h, const rtd3_tick_state* t, const float* residual, const double* unit_noise, int32_t noise_mode,
                        void* stream) {
   if (int32_t e = check_state(t)) return e;
-  RTD3_CHECK_ARG(h && h->has_map, "environment has no dynamics map (call rtd3_env_set_map)");
+  RTD3_CHECK_ARG(h && h->num_maps > 0, "environment has no dynamics map (call rtd3_env_set_map)");
   RTD3_CHECK_ARG(residual, "null residual");
   RTD3_CHECK_ARG(noise_mode >= RTD3_TICK_NOISE_NONE && noise_mode <= RTD3_TICK_NOISE_PHILOX, "unknown noise mode");
   RTD3_CHECK_ARG(noise_mode != RTD3_TICK_NOISE_GIVEN || unit_noise, "noise mode 'given' needs unit_noise");
@@ -290,9 +289,9 @@ int32_t rtd3_tick_post(rtd3_env* h, const rtd3_tick_state* t, const float* resid
   cudaStream_t st = (cudaStream_t)stream;
   // elementwise work plus a few candidate demo states per env: small CTAs spread a small batch over more SMs
   const int block = t->n <= (int64_t)h->num_sms * 256 ? 128 : 256;
-  const MapBank bank{h->tables, h->halos, h->fits, h->index_len ? h->index : nullptr, h->index_len, h->num_maps};
-  if (bank.index) tick_post_kernel<true><<<(int)ceil_div(t->n, block), block, 0, st>>>(*t, h->table, residual, unit_noise, noise_mode, bank);
-  else tick_post_kernel<false><<<(int)ceil_div(t->n, block), block, 0, st>>>(*t, h->table, residual, unit_noise, noise_mode, bank);
+  const MapBank bank = map_bank(h);
+  const auto kern = bank.index ? tick_post_kernel<true> : tick_post_kernel<false>;
+  kern<<<(int)ceil_div(t->n, block), block, 0, st>>>(*t, residual, unit_noise, noise_mode, bank);
   RTD3_LAUNCHED();
   return 0;
 }
@@ -300,7 +299,7 @@ int32_t rtd3_tick_post(rtd3_env* h, const rtd3_tick_state* t, const float* resid
 int32_t rtd3_tick_run_f16(rtd3_env* h, const rtd3_tick_state* t, int32_t hidden, int32_t layers, const float* params,
                           const uint16_t* params_h, int32_t noise_mode, int64_t ticks, uint64_t tick_base, void* stream) {
   if (int32_t e = check_state(t)) return e;
-  RTD3_CHECK_ARG(h && h->has_map, "environment has no dynamics map (call rtd3_env_set_map)");
+  RTD3_CHECK_ARG(h && h->num_maps > 0, "environment has no dynamics map (call rtd3_env_set_map)");
   RTD3_CHECK_ARG(params && params_h, "null parameters");
   RTD3_CHECK_ARG(hidden % 32 == 0 && hidden >= 64 && hidden <= 256 && layers == 2, "needs layers == 2 and hidden in {64..256} divisible by 32");
   RTD3_CHECK_ARG(noise_mode == RTD3_TICK_NOISE_NONE || noise_mode == RTD3_TICK_NOISE_PHILOX, "noise must be none or philox");
@@ -312,14 +311,14 @@ int32_t rtd3_tick_run_f16(rtd3_env* h, const rtd3_tick_state* t, int32_t hidden,
   if (t->n == 0 || ticks == 0) return 0;
   const NetShape s{2, hidden, layers, 2};
   const size_t smem = hf_smem_bytes(hidden) + kHfRows * sizeof(float2);
-  const MapBank bank{h->tables, h->halos, h->fits, h->index_len ? h->index : nullptr, h->index_len, h->num_maps};
+  const MapBank bank = map_bank(h);
   const auto kern = bank.index ? tick_f16_kernel<true> : tick_f16_kernel<false>;
   RTD3_CUDA(ensure_dyn_smem((const void*)kern, smem));
   uint32_t cols = 32;
   while (cols < (uint32_t)hidden) cols <<= 1;
   const int64_t tiles = ceil_div(t->n, kHfRows);
   const int grid = (int)(tiles < h->num_sms ? tiles : h->num_sms);
-  kern<<<grid, kHfThreads, smem, (cudaStream_t)stream>>>(*t, h->table, s, params, params_h, noise_mode, (int)ticks, tick_base, cols, bank);
+  kern<<<grid, kHfThreads, smem, (cudaStream_t)stream>>>(*t, s, params, params_h, noise_mode, (int)ticks, tick_base, cols, bank);
   RTD3_LAUNCHED();
   return 0;
 }
