@@ -233,7 +233,7 @@ int32_t rtd3_td3_actor_step(rtd3_td3* h, const float* params, const float* param
  * on the target nets selected by `polyak` (same bit layout) with the freshly updated online parameters.
  * params_uv (nullable): the tensor-core operand copies of the arena (see rtd3_tc_sync_weights), kept in step too. */
 int32_t rtd3_td3_adam_polyak(rtd3_td3* h, float* params, float* params_t, float* params_uv, float* grads, float* adam_m, float* adam_v,
-                             const double* beta_pows, int32_t nets, float lr_actor, float lr_critic, float grad_scale, int32_t polyak,
+                             const double* beta_pows, int32_t nets, double lr_actor, double lr_critic, float grad_scale, int32_t polyak,
                              float tau, void* stream);
 
 /* Forward of one network of the arena (robot.py:153-159 / 193-200): x [batch][in] -> y [batch][out]. */
@@ -426,7 +426,9 @@ typedef struct rtd3_td3_update_args {
   const float* noise;
   uint64_t noise_seed;
   uint64_t* noise_counter;       /* DEVICE uint64 [1] */
-  float gamma, policy_noise, noise_clip, max_action, lr_actor, lr_critic, tau;
+  float gamma, policy_noise, noise_clip, max_action;
+  double lr_actor, lr_critic;     /* double, like torch's lr: the step size lr / (1 - 0.9^t) is rounded to float32 once */
+  float tau;
   /* outputs: the values the reference collects at robot.py:274-280 */
   float* critic_losses;          /* [epochs][2] */
   float* actor_losses;           /* [ceil(epochs / policy_update_delay)] */

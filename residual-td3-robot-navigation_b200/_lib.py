@@ -61,7 +61,8 @@ class Td3UpdateArgs(Structure):
                                          "rp_s", "rp_a", "rp_r", "rp_s2", "rp_notdone", "idx")]
                 + [("batch", c_int32), ("epochs", c_int32), ("policy_update_delay", c_int32)]
                 + [("noise", c_void_p), ("noise_seed", c_uint64), ("noise_counter", c_void_p)]
-                + [(k, c_float) for k in ("gamma", "policy_noise", "noise_clip", "max_action", "lr_actor", "lr_critic", "tau")]
+                + [(k, c_float) for k in ("gamma", "policy_noise", "noise_clip", "max_action")]
+                + [("lr_actor", c_double), ("lr_critic", c_double), ("tau", c_float)]
                 + [("critic_losses", c_void_p), ("actor_losses", c_void_p), ("world", c_int32), ("tf32", c_int32), ("comm", c_void_p),
                    ("p2p", POINTER(P2pStateStruct))])
 
@@ -103,7 +104,7 @@ _SIGNATURES = {
     "rtd3_td3_sync_transposed": (c_int32, [_P, _P, _P, _P]),
     "rtd3_td3_critic_step": (c_int32, [_P] * 12 + [c_int32, c_float, c_float, c_float, c_float] + [_P] * 6),
     "rtd3_td3_actor_step": (c_int32, [_P] * 7 + [c_int32, _P, _P, _P, _P]),
-    "rtd3_td3_adam_polyak": (c_int32, [_P] * 8 + [c_int32, c_float, c_float, c_float, c_int32, c_float, _P]),
+    "rtd3_td3_adam_polyak": (c_int32, [_P] * 8 + [c_int32, c_double, c_double, c_float, c_int32, c_float, _P]),
     "rtd3_mlp_forward": (c_int32, [_P, c_int32, _P, _P, _P, _P, c_int64, _P]),
     "rtd3_tc_sync_weights": (c_int32, [c_int32, c_int32, _P, _P, _P]),
     "rtd3_mlp_forward_tf32": (c_int32, [c_int32, c_int32, c_int32, c_int64, _P, _P, _P, _P, c_int64, _P]),

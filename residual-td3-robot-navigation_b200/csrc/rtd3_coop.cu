@@ -110,7 +110,8 @@ struct CoopArgs {
   const int32_t* idx;
   const float* noise;        // nullable [E][B][2]
   Td3Hyper hp;
-  float lr_actor, lr_critic, tau;
+  double lr_actor, lr_critic;
+  float tau;
   int B, E, delay;
   float* critic_losses;      // [E][2]
   float* actor_losses;       // [ceil(E/delay)]
@@ -619,7 +620,7 @@ __device__ __noinline__ void adam_stage(const CoopArgs& a, int nets, int polyak,
   __shared__ float s_step[2], s_bc2[2];
   if (threadIdx.x < 2) {
     const double bc1 = 1.0 - a.beta_pows[2 * threadIdx.x], bc2 = 1.0 - a.beta_pows[2 * threadIdx.x + 1];
-    const double lr = threadIdx.x == 0 ? (double)a.lr_actor : (double)a.lr_critic;
+    const double lr = threadIdx.x == 0 ? a.lr_actor : a.lr_critic;
     s_step[threadIdx.x] = (float)(lr / bc1);
     s_bc2[threadIdx.x] = (float)sqrt(bc2);
   }

@@ -102,7 +102,7 @@ __global__ void __launch_bounds__(256) p2p_allreduce_adam_kernel(P2pPeers peers,
   const int tid = threadIdx.x;
   if (tid < 2) {                                                      // 0: actor optimiser, 1: both critic optimisers
     const double bc1 = 1.0 - o.beta_pows[2 * tid], bc2 = 1.0 - o.beta_pows[2 * tid + 1];
-    const double lr = tid == 0 ? (double)o.lr_actor : (double)o.lr_critic;
+    const double lr = tid == 0 ? o.lr_actor : o.lr_critic;
     s_step[tid] = (float)(lr / bc1);
     s_bc2[tid] = (float)sqrt(bc2);
   }

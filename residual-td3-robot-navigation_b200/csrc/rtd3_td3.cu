@@ -163,7 +163,7 @@ struct AdamFuse {
   float* m;
   float* v;
   const double* beta_pows;
-  float lr;
+  double lr;
   int opt;                  // 0 actor optimiser, 1 critic optimisers (index into beta_pows)
   int polyak;               // blend the target copy of every updated parameter
   float tau;
@@ -417,7 +417,7 @@ wgrad_kernel(NetShape s, const float* __restrict__ scratch, float* __restrict__ 
   if (fz.params) { bp1 = fz.beta_pows[2 * fz.opt]; bp2 = fz.beta_pows[2 * fz.opt + 1]; }
   float s_step = 0.f, s_bc2 = 1.f;
   auto bias_corrections = [&]() {
-    s_step = (float)((double)fz.lr / (1.0 - bp1));
+    s_step = (float)(fz.lr / (1.0 - bp1));
     s_bc2 = (float)sqrt(1.0 - bp2);
   };
   // the optimiser's operands of one element, fetched BEFORE the batch reduction (the small jobs' five emits were five dependent
@@ -689,12 +689,12 @@ __global__ void td3_sync_transposed_kernel(Arena ar, const float* __restrict__ p
 }
 
 __global__ void td3_adam_polyak_kernel(Arena ar, float* __restrict__ params, float* __restrict__ params_t, float* __restrict__ params_uv, float* __restrict__ grads, float* __restrict__ m,
-                                       float* __restrict__ v, const double* __restrict__ beta_pows, int nets, float lr_actor,
-                                       float lr_critic, float grad_scale, int polyak, float tau) {
+                                       float* __restrict__ v, const double* __restrict__ beta_pows, int nets, double lr_actor,
+                                       double lr_critic, float grad_scale, int polyak, float tau) {
   __shared__ float s_step[2], s_bc2[2];
   if (threadIdx.x < 2) {                                              // 0: actor optimiser, 1: both critic optimisers
     const double bc1 = 1.0 - beta_pows[2 * threadIdx.x], bc2 = 1.0 - beta_pows[2 * threadIdx.x + 1];
-    const double lr = threadIdx.x == 0 ? (double)lr_actor : (double)lr_critic;
+    const double lr = threadIdx.x == 0 ? lr_actor : lr_critic;
     s_step[threadIdx.x] = (float)(lr / bc1);
     s_bc2[threadIdx.x] = (float)sqrt(bc2);
   }
@@ -973,7 +973,7 @@ static int32_t actor_step_fused(rtd3_td3* h, const float* params, const float* p
 extern "C" {
 
 int32_t rtd3_td3_adam_polyak(rtd3_td3* h, float* params, float* params_t, float* params_uv, float* grads, float* adam_m, float* adam_v, const double* beta_pows, int32_t nets,
-                             float lr_actor, float lr_critic, float grad_scale, int32_t polyak, float tau, void* stream) {
+                             double lr_actor, double lr_critic, float grad_scale, int32_t polyak, float tau, void* stream) {
   RTD3_CHECK_ARG(h && params && params_t && grads && adam_m && adam_v && beta_pows, "null argument");
   const int64_t n = h->ar.online_total();
   const int block = 256;

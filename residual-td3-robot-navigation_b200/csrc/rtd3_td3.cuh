@@ -206,7 +206,8 @@ struct P2pAdamArgs {
   Arena ar;
   float* params; float* params_t; float* params_uv; float* m; float* v;
   const double* beta_pows;
-  float lr_actor, lr_critic, grad_scale, tau;
+  double lr_actor, lr_critic;
+  float grad_scale, tau;
   int nets, polyak;
   int64_t off;
 };
