@@ -98,20 +98,13 @@ struct CoopPeers {
 
 struct CoopArgs {
   long long* prof;           // nullable (development): block 0 stamps %globaltimer at every stage boundary of the last epoch
-  Arena ar;
-  float* params;
-  float* params_t;
+  AdamState adam;            // adam.params_uv is not used: this kernel keeps no tensor-core copies
   float* grads;
-  float* adam_m;
-  float* adam_v;
   int32_t* steps;
-  double* beta_pows;
   ReplayView rp;
   const int32_t* idx;
   const float* noise;        // nullable [E][B][2]
   Td3Hyper hp;
-  double lr_actor, lr_critic;
-  float tau;
   int B, E, delay;
   float* critic_losses;      // [E][2]
   float* actor_losses;       // [ceil(E/delay)]
@@ -375,10 +368,10 @@ struct NetRef {
 
 __device__ __forceinline__ NetRef net_ref(const CoopArgs& a, int net, int slot) {
   NetRef r;
-  r.s = (net == 0 || net == 3) ? a.ar.actor : a.ar.critic;
-  r.P = a.params + a.ar.off(net);
-  r.Pt = a.params_t + a.ar.off(net);
-  r.G = net < 3 ? a.grads + a.ar.off(net) : nullptr;
+  r.s = (net == 0 || net == 3) ? a.adam.ar.actor : a.adam.ar.critic;
+  r.P = a.adam.params + a.adam.ar.off(net);
+  r.Pt = a.adam.params_t + a.adam.ar.off(net);
+  r.G = net < 3 ? a.grads + a.adam.ar.off(net) : nullptr;
   r.slot = slot;
   return r;
 }
@@ -558,17 +551,6 @@ __device__ __noinline__ void small_grads(const CoopArgs& a, const Scratch& sc, c
 
 // The one-hidden-layer case has no dZ_0 array (the top gradient is generated): L >= 2 is required by the launcher.
 
-// index of parameter o (offset inside its net's slot) in the transposed arena
-__device__ __forceinline__ int transposed_off(const NetShape& s, int o) {
-  const int first = s.in * s.hid + s.hid, blk = s.hid * s.hid + s.hid;
-  if (o < first) return o;
-  const unsigned o2 = (unsigned)(o - first);
-  const unsigned l = o2 / (unsigned)blk, rem = o2 - l * (unsigned)blk;
-  if ((int)l >= s.layers - 1 || rem >= (unsigned)(s.hid * s.hid)) return o;
-  const unsigned n = rem / (unsigned)s.hid, k = rem - n * (unsigned)s.hid;
-  return first + (int)l * blk + (int)(k * s.hid + n);
-}
-
 __device__ __forceinline__ unsigned long long ld_acquire_sys_u64(const unsigned long long* p) {
   unsigned long long v;
   asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
@@ -587,8 +569,10 @@ __device__ __forceinline__ float ld_volatile_f32(const float* p) {
 // World > 1: the gradients are first pushed to every rank's receive slot, one flag per rank is raised after a grid barrier, and the
 // optimiser sums the `world` slots of this rank's area in rank order (bit-identical replicas).
 __device__ __noinline__ void adam_stage(const CoopArgs& a, int nets, int polyak, unsigned long long seq) {
-  const int n_online = (int)a.ar.online_total();
-  const int off1 = (int)a.ar.off(1), off2 = (int)a.ar.off(2);
+  AdamState os = a.adam;
+  os.params_uv = nullptr;            // the tensor-core copies are not kept (learner.py marks them stale after a cooperative update)
+  const int n_online = (int)os.ar.online_total();
+  const int off1 = (int)os.ar.off(1), off2 = (int)os.ar.off(2);
   const int lo = (nets & 1) ? 0 : off1, hi = (nets & 6) ? n_online : off1;      // range of gradients this step produced
   const int gtid = (int)blockIdx.x * kCT + (int)threadIdx.x, gthreads = (int)gridDim.x * kCT;
   const float* slots = nullptr;
@@ -619,10 +603,9 @@ __device__ __noinline__ void adam_stage(const CoopArgs& a, int nets, int polyak,
   }
   __shared__ float s_step[2], s_bc2[2];
   if (threadIdx.x < 2) {
-    const double bc1 = 1.0 - a.beta_pows[2 * threadIdx.x], bc2 = 1.0 - a.beta_pows[2 * threadIdx.x + 1];
-    const double lr = threadIdx.x == 0 ? a.lr_actor : a.lr_critic;
-    s_step[threadIdx.x] = (float)(lr / bc1);
-    s_bc2[threadIdx.x] = (float)sqrt(bc2);
+    const AdamStep k = adam_step(threadIdx.x == 0 ? os.lr[0] : os.lr[1], os.beta_pows[2 * threadIdx.x], os.beta_pows[2 * threadIdx.x + 1]);
+    s_step[threadIdx.x] = k.step;
+    s_bc2[threadIdx.x] = k.sqrt_bc2;
   }
   __syncthreads();
   const float scale = 1.0f / (float)a.world;
@@ -631,33 +614,24 @@ __device__ __noinline__ void adam_stage(const CoopArgs& a, int nets, int polyak,
     const bool do_adam = (nets >> net) & 1, do_polyak = (polyak >> net) & 1;
     if (!do_adam && !do_polyak) continue;
     const int noff = net == 0 ? 0 : (net == 1 ? off1 : off2);
-    const NetShape s = net == 0 ? a.ar.actor : a.ar.critic;
+    const NetShape s = net == 0 ? os.ar.actor : os.ar.critic;
     if (i - noff >= (int)net_param_count(s)) continue;                        // slot padding
-    const int ti = transposed_off(s, i - noff);
-    float p = ldcg(a.params + i);
+    const float p = ldcg(os.params + i);
+    float g = 0.f, m = 0.f, v = 0.f, t = 0.f;
     if (do_adam) {
-      float g;
       if (a.world > 1) {
-        g = 0.f;
         for (int r = 0; r < a.world; ++r) g += ld_volatile_f32(slots + (long long)r * a.slot_floats + i);
       } else {
         g = ldcg(a.grads + i);
       }
       g *= scale;
-      const int o = net == 0 ? 0 : 1;
-      float mi = a.adam_m[i], vi = a.adam_v[i];
-      adam_element(g, mi, vi, p, s_step[o], s_bc2[o]);
-      a.adam_m[i] = mi;
-      a.adam_v[i] = vi;
-      a.params[i] = p;
-      a.params_t[noff + ti] = p;
+      m = os.m[i];
+      v = os.v[i];
     }
-    if (do_polyak) {
-      const int t_i = n_online + i;
-      const float tv = __fadd_rn(__fmul_rn(ldcg(a.params + t_i), 1.0f - a.tau), __fmul_rn(p, a.tau));   // robot.py:309, three roundings
-      a.params[t_i] = tv;
-      a.params_t[n_online + noff + ti] = tv;
-    }
+    if (do_polyak) t = ldcg(os.params + n_online + i);
+    const int o = net == 0 ? 0 : 1;
+    adam_polyak1(os, i, noff, copy_index(s, i - noff), g, m, v, p, t, AdamStep{s_step[o], s_bc2[o]}, do_adam, do_polyak, n_online,
+                 (int)os.ar.total());
   }
 }
 
@@ -680,8 +654,8 @@ __shared__ NetRef s_nets[2];
 
 __global__ void __launch_bounds__(kCT, 1) td3_update_coop_kernel(CoopArgs a) {
   extern __shared__ __align__(16) float coop_smem[];
-  const Scratch sc{a.scratch, (a.B + 31) / 32 * 32, a.ar.critic.hid, a.ar.critic.layers};
-  const int L = a.ar.critic.layers, B = a.B;
+  const Scratch sc{a.scratch, (a.B + 31) / 32 * 32, a.adam.ar.critic.hid, a.adam.ar.critic.layers};
+  const int L = a.adam.ar.critic.layers, B = a.B;
   const int lane = threadIdx.x & 31;
   unsigned long long seq = a.world > 1 ? *reinterpret_cast<volatile unsigned long long*>(a.seq_counter) : 0ull;
   int k_idx = 0, ka = 0;
@@ -695,7 +669,7 @@ __global__ void __launch_bounds__(kCT, 1) td3_update_coop_kernel(CoopArgs a) {
       const int32_t* idx = a.idx + (int64_t)k_idx * B;
       ++k_idx;
       const NetRef ta = net_ref(a, 3, 0), tc1 = net_ref(a, 4, 1), tc2 = net_ref(a, 5, 2), c1 = net_ref(a, 1, 3), c2 = net_ref(a, 2, 4);
-      if (blockIdx.x == 0 && threadIdx.x == 0) advance_adam_clock(a.steps, a.beta_pows, 1);
+      if (blockIdx.x == 0 && threadIdx.x == 0) advance_adam_clock(a.steps, a.adam.beta_pows, 1);
       // gather: net inputs of the target actor (s2) and of both critics (s, a)
       for (int b = (int)blockIdx.x * kCT + (int)threadIdx.x; b < B; b += (int)gridDim.x * kCT) {
         const int j = idx[b];
@@ -783,7 +757,7 @@ __global__ void __launch_bounds__(kCT, 1) td3_update_coop_kernel(CoopArgs a) {
       const int32_t* idx = a.idx + (int64_t)k_idx * B;
       ++k_idx;
       const NetRef ac = net_ref(a, 0, 0), c1 = net_ref(a, 1, 1);
-      if (blockIdx.x == 0 && threadIdx.x == 0) advance_adam_clock(a.steps, a.beta_pows, 0);
+      if (blockIdx.x == 0 && threadIdx.x == 0) advance_adam_clock(a.steps, a.adam.beta_pows, 0);
       for (int b = (int)blockIdx.x * kCT + (int)threadIdx.x; b < B; b += (int)gridDim.x * kCT) {
         const float2 s = a.rp.s[idx[b]];
         *reinterpret_cast<float4*>(sc.in4(0) + 4 * b) = make_float4(s.x, s.y, 0.f, 0.f);   // the actor is fed the raw state, robot.py:386
@@ -902,14 +876,12 @@ int32_t rtd3_td3_update_coop(rtd3_td3* h, const rtd3_td3_update_args* a, float* 
   cudaStream_t st = (cudaStream_t)stream;
   CoopArgs c{};
   c.prof = g_coop_prof;
-  c.ar = h->ar;
-  c.params = a->params; c.params_t = a->params_t; c.grads = a->grads; c.adam_m = a->adam_m; c.adam_v = a->adam_v;
-  c.steps = a->steps; c.beta_pows = a->beta_pows;
+  c.adam = adam_state(h, a);
+  c.grads = a->grads; c.steps = a->steps;
   c.rp = ReplayView{(const float2*)a->rp_s, (const float2*)a->rp_a, a->rp_r, (const float2*)a->rp_s2, a->rp_notdone};
   c.idx = a->idx; c.noise = a->noise;
   c.hp = Td3Hyper{a->gamma, a->policy_noise, a->noise_clip, a->max_action, (unsigned long long)a->noise_seed,
                   (const unsigned long long*)a->noise_counter, 0ull};
-  c.lr_actor = a->lr_actor; c.lr_critic = a->lr_critic; c.tau = a->tau;
   c.B = a->batch; c.E = a->epochs; c.delay = a->policy_update_delay;
   c.critic_losses = a->critic_losses; c.actor_losses = a->actor_losses;
   // the first kBarWords floats of the scratch hold the barrier words (zero-initialised by the caller once; the barrier leaves them zero /

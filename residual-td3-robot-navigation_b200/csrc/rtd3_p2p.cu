@@ -101,15 +101,14 @@ __global__ void __launch_bounds__(256) p2p_allreduce_adam_kernel(P2pPeers peers,
   __shared__ unsigned long long s_seq;
   const int tid = threadIdx.x;
   if (tid < 2) {                                                      // 0: actor optimiser, 1: both critic optimisers
-    const double bc1 = 1.0 - o.beta_pows[2 * tid], bc2 = 1.0 - o.beta_pows[2 * tid + 1];
-    const double lr = tid == 0 ? o.lr_actor : o.lr_critic;
-    s_step[tid] = (float)(lr / bc1);
-    s_bc2[tid] = (float)sqrt(bc2);
+    const AdamStep k = adam_step(tid == 0 ? o.adam.lr[0] : o.adam.lr[1], o.adam.beta_pows[2 * tid], o.adam.beta_pows[2 * tid + 1]);
+    s_step[tid] = k.step;
+    s_bc2[tid] = k.sqrt_bc2;
   }
   if (tid == 0) s_seq = *reinterpret_cast<volatile unsigned long long*>(seq_counter) + 1ull;
   __syncthreads();
   const unsigned long long seq = s_seq;
-  const int n4 = (int)(o.ar.online_total() >> 2), off4 = (int)(o.off >> 2), end4 = off4 + (int)count4;
+  const int n4 = (int)(o.adam.ar.online_total() >> 2), off4 = (int)(o.off >> 2), end4 = off4 + (int)count4;
   const int gstride = gridDim.x * blockDim.x;
   const int64_t slot = ((int64_t)(seq & 1ull) * kWorld + rank) * stride4;
   // (1) push this block's elements of the slice into slot [step parity][rank] of every rank, clear them locally
@@ -136,7 +135,7 @@ __global__ void __launch_bounds__(256) p2p_allreduce_adam_kernel(P2pPeers peers,
   if (tid < kWorld) wait_flag(peers.flags[rank] + kP2pBlockFlagBase + tid * kP2pBlockFlags + blockIdx.x, seq);
   __syncthreads();
   const float4* mine = reinterpret_cast<const float4*>(peers.recv[rank]) + (int64_t)(seq & 1ull) * kWorld * stride4;
-  const int off1 = (int)o.ar.off(1), off2 = (int)o.ar.off(2);
+  const int off1 = (int)o.adam.ar.off(1), off2 = (int)o.adam.ar.off(2);
   for (int i4 = blockIdx.x * blockDim.x + tid; i4 < n4; i4 += gstride) {
     const int i = i4 * 4;
     const int net = i < off1 ? 0 : (i < off2 ? 1 : 2);               // slots are multiples of 4 floats: a group never straddles two
@@ -146,7 +145,7 @@ __global__ void __launch_bounds__(256) p2p_allreduce_adam_kernel(P2pPeers peers,
     if (do_adam) g = p2p_sum_slots<kWorld>(mine, stride4, (int64_t)(i4 - off4));
     const float gg[4] = {g.x * o.grad_scale, g.y * o.grad_scale, g.z * o.grad_scale, g.w * o.grad_scale};
     const int k = net == 0 ? 0 : 1;
-    adam_polyak_apply4(o.ar, i, net, gg, do_adam, do_polyak, o.params, o.params_t, o.params_uv, o.m, o.v, s_step[k], s_bc2[k], o.tau);
+    adam_polyak_apply4(o.adam, i, net, gg, AdamStep{s_step[k], s_bc2[k]}, do_adam, do_polyak);
   }
 }
 
@@ -208,7 +207,7 @@ int32_t rtd3::p2p_allreduce_adam_launch(const rtd3_p2p_state* ps, float* local_g
   int64_t count4 = count / 4, stride4 = ps->slot_floats / 4;
   int num_sms = 0;
   RTD3_CUDA(current_num_sms(&num_sms));
-  const int grid = (int)std::min<int64_t>(std::min<int64_t>((int64_t)num_sms, kP2pBlockFlags), ceil_div(opt.ar.online_total() / 4, 256));
+  const int grid = (int)std::min<int64_t>(std::min<int64_t>((int64_t)num_sms, kP2pBlockFlags), ceil_div(opt.adam.ar.online_total() / 4, 256));
   unsigned long long* sc = (unsigned long long*)ps->seq_counter;
   int rk = rank;
   unsigned int* bc = ps->block_counter;

@@ -291,12 +291,9 @@ __global__ void sync_half_kernel(Arena ar, const float* __restrict__ params, uin
     int net = 5;
     while (net > 0 && i < ar.off(net)) --net;
     const NetShape& s = (net % 3 == 0) ? ar.actor : ar.critic;
-    const int64_t off = ar.off(net);
-    if (!is_hidden_weight(s, off, i)) continue;
-    const int64_t first = (int64_t)s.in * s.hid + s.hid, blk = (int64_t)s.hid * s.hid + s.hid, hh = (int64_t)s.hid * s.hid;
-    const int64_t o2 = i - off - first;
-    const int64_t l = o2 / blk, rem = o2 - l * blk;
-    const int64_t n = rem / s.hid, k = rem - n * s.hid;
+    const SlotPos q = slot_pos(s, (int)(i - ar.off(net)));
+    if (!q.hidden) continue;
+    const int64_t hh = (int64_t)s.hid * s.hid, l = q.l, n = q.n, k = q.k;
     params_h[((int64_t)net * (s.layers - 1) + l) * hh + ((k >> 3) * s.hid + n) * 8 + (k & 7)] =
         __half_as_ushort(__float2half_rn(fminf(fmaxf(params[i], -65504.f), 65504.f)));
   }
@@ -310,11 +307,10 @@ __global__ void sync_chunk_major_kernel(NetShape actor, NetShape critic, int64_t
     const int64_t j = i < n_online ? i : i - n_online;
     const int net = j < sa ? 0 : (j < sa + sc ? 1 : 2);
     const int64_t off = (i < n_online ? 0 : n_online) + (net == 0 ? 0 : (net == 1 ? sa : sa + sc));
-    const NetShape& s = net == 0 ? actor : critic;
-    const bool hidden = is_hidden_weight(s, off, i);
-    const float p = params[i];
-    params_uv[chunk_major_index(s, off, i)] = hidden ? tf32_rn(p) : p;
-    params_uv[total + chunk_major_index_v(s, off, i)] = hidden ? tf32_rn(p) : p;
+    const CopyIndex c = copy_index(net == 0 ? actor : critic, (int)(i - off));
+    const float p = c.hidden ? tf32_rn(params[i]) : params[i];
+    params_uv[off + c.u] = p;
+    params_uv[total + off + c.v] = p;
   }
 }
 
@@ -326,7 +322,7 @@ extern "C" {
 
 /* Rebuild the chunk-major (UMMA operand order) copy of all hidden-layer weights from the torch-layout arena. */
 int32_t rtd3_tc_sync_weights(int32_t hidden, int32_t layers, const float* params, float* params_uv, void* stream) {
-  RTD3_CHECK_ARG(params && params_uv && hidden >= 4 && layers >= 1, "bad argument");
+  RTD3_CHECK_ARG(params && params_uv && hidden >= 4 && hidden <= kMaxHidden && layers >= 1 && layers <= kMaxLayers, "bad argument");
   const NetShape a{2, hidden, layers, 2}, c{4, hidden, layers, 1};
   sync_chunk_major_kernel<<<296, 256, 0, (cudaStream_t)stream>>>(a, c, net_stride(a), net_stride(c), params, params_uv);
   RTD3_LAUNCHED();
@@ -358,7 +354,7 @@ int32_t rtd3_mlp_forward_tf32(int32_t hidden, int32_t layers, int32_t is_actor, 
 
 /* fp16 chunk-major copies of the hidden-to-hidden weights of all six networks (see mlp_forward_f16_kernel). */
 int32_t rtd3_tc_sync_weights_f16(int32_t hidden, int32_t layers, const float* params, uint16_t* params_h, void* stream) {
-  RTD3_CHECK_ARG(params && params_h && hidden >= 4 && layers >= 1, "bad argument");
+  RTD3_CHECK_ARG(params && params_h && hidden >= 4 && hidden <= kMaxHidden && layers >= 1 && layers <= kMaxLayers, "bad argument");
   const Arena ar{NetShape{2, hidden, layers, 2}, NetShape{4, hidden, layers, 1}};
   sync_half_kernel<<<296, 256, 0, (cudaStream_t)stream>>>(ar, params, params_h);
   RTD3_LAUNCHED();

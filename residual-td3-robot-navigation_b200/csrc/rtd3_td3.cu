@@ -154,21 +154,13 @@ td3_actor_kernel(Arena ar, const float* __restrict__ params, const float* __rest
 }
 
 // Optional optimiser fused into the weight-gradient pass (single GPU, batch <= 512: every gradient element is final when its job
-// writes it): torch.optim.Adam on the element (the arithmetic of td3_adam_polyak_kernel, bit for bit) and, on request, the Polyak
-// blend of the matching target parameter - the two separate optimiser launches of an epoch (13 us at B = 256) disappear.
+// writes it): torch.optim.Adam on the element and, on request, the Polyak blend of the matching target parameter (adam_polyak4 /
+// adam_polyak1) - the two separate optimiser launches of an epoch (13 us at B = 256) disappear.
 struct AdamFuse {
-  float* params;            // nullptr: not fused, gradients are stored
-  float* params_t;
-  float* params_uv;         // nullable
-  float* m;
-  float* v;
-  const double* beta_pows;
-  double lr;
-  int opt;                  // 0 actor optimiser, 1 critic optimisers (index into beta_pows)
+  AdamState adam;           // adam.params == nullptr: not fused, gradients are stored
+  int opt;                  // 0 actor optimiser, 1 critic optimisers (index into lr and beta_pows)
   int polyak;               // blend the target copy of every updated parameter
-  float tau;
-  int n_online, total;
-  NetShape shape;
+  int n_online, total;      // adam.ar.online_total() / total(): derived at every use, they made the kernel 8 % longer, B = 256 0.6 % slower
 };
 
 // Optional peer-memory exchange fused into the same pass (data parallel, world > 1, with AdamFuse): a job PUSHES the gradient elements
@@ -412,52 +404,31 @@ wgrad_kernel(NetShape s, const float* __restrict__ scratch, float* __restrict__ 
     __syncthreads();                                                 // every thread of the block has read the step number
     if (threadIdx.x == 32) p2p_step_done(px, seq64, ncta);
   }
-  // fused optimiser: bias corrections from the Adam clocks (loaded now, used after the batch reduction)
+  // fused optimiser: the Adam clocks are loaded now, the step size is formed after the batch reduction
+  const AdamState& os = fz.adam;
   double bp1 = 0.0, bp2 = 0.0;
-  if (fz.params) { bp1 = fz.beta_pows[2 * fz.opt]; bp2 = fz.beta_pows[2 * fz.opt + 1]; }
-  float s_step = 0.f, s_bc2 = 1.f;
-  auto bias_corrections = [&]() {
-    s_step = (float)(fz.lr / (1.0 - bp1));
-    s_bc2 = (float)sqrt(1.0 - bp2);
-  };
+  if (os.params) { bp1 = os.beta_pows[2 * fz.opt]; bp2 = os.beta_pows[2 * fz.opt + 1]; }
+  const double lr = fz.opt ? os.lr[1] : os.lr[0];   // selected before the reduction: selected after it, it sent the whole AdamFuse to the stack (256 B, spills)
+  auto step_size = [&]() { return adam_step(lr, bp1, bp2); };
   // the optimiser's operands of one element, fetched BEFORE the batch reduction (the small jobs' five emits were five dependent
   // chains of two L2 round trips each - the longest blocks of the launch)
   struct OptPre { float m, v, p, t; };
   auto pre_load = [&](int64_t net_off, int64_t o) {
     OptPre q{0.f, 0.f, 0.f, 0.f};
-    if (fz.params) {
+    if (os.params) {
       const int64_t i = net_off + o;
-      q.m = fz.m[i]; q.v = fz.v[i]; q.p = fz.params[i];
-      if (fz.polyak) q.t = fz.params[fz.n_online + i];
+      q.m = os.m[i]; q.v = os.v[i]; q.p = os.params[i];
+      if (fz.polyak) q.t = os.params[fz.n_online + i];
     }
     return q;
   };
   auto emit_pre = [&](int64_t net_off, int64_t o, float g, bool atomic_acc, const OptPre& q) {
-    if (!fz.params) {
+    if (!os.params) {
       float* dst = grads + net_off + o;
       if (atomic_acc) atomicAdd(dst, g); else *dst = g;
       return;
     }
-    const int64_t i = net_off + o;
-    const CopyIndex ci = copy_index(fz.shape, (int)o);
-    float mi = q.m, vi = q.v, p = q.p;
-    adam_element(g, mi, vi, p, s_step, s_bc2);
-    fz.m[i] = mi;
-    fz.v[i] = vi;
-    fz.params[i] = p;
-    fz.params_t[net_off + ci.t] = p;
-    if (fz.params_uv) {
-      const float pr = ci.hidden ? tf32_rn(p) : p;
-      fz.params_uv[net_off + ci.u] = pr;
-      fz.params_uv[fz.total + net_off + ci.v] = pr;
-    }
-    if (fz.polyak) {
-      const int64_t ti = fz.n_online + i;
-      const float tv = __fadd_rn(__fmul_rn(q.t, 1.0f - fz.tau), __fmul_rn(p, fz.tau));   // robot.py:309, three roundings
-      fz.params[ti] = tv;
-      fz.params_t[fz.n_online + net_off + ci.t] = tv;
-      if (fz.params_uv) fz.params_uv[fz.n_online + net_off + ci.u] = ci.hidden ? tf32_rn(tv) : tv;
-    }
+    adam_polyak1(os, (int)(net_off + o), (int)net_off, copy_index(s, (int)o), g, q.m, q.v, q.p, q.t, step_size(), true, fz.polyak, fz.n_online, fz.total);
   };
   const int H = s.hid, L = s.layers;
   const int nch = (H + 31) / 32;
@@ -487,11 +458,11 @@ wgrad_kernel(NetShape s, const float* __restrict__ scratch, float* __restrict__ 
     const bool out_ok = gn < H && gk < H;
     const int64_t off = net_w_off(s, l) + (int64_t)gn * H + gk;
     float4 m4 = make_float4(0.f, 0.f, 0.f, 0.f), v4 = m4, p4 = m4, t4 = m4;
-    if (fz.params && out_ok) {
-      m4 = *reinterpret_cast<const float4*>(fz.m + G0 + off);
-      v4 = *reinterpret_cast<const float4*>(fz.v + G0 + off);
-      p4 = *reinterpret_cast<const float4*>(fz.params + G0 + off);
-      if (fz.polyak) t4 = *reinterpret_cast<const float4*>(fz.params + fz.n_online + G0 + off);
+    if (os.params && out_ok) {
+      m4 = *reinterpret_cast<const float4*>(os.m + G0 + off);
+      v4 = *reinterpret_cast<const float4*>(os.v + G0 + off);
+      p4 = *reinterpret_cast<const float4*>(os.params + G0 + off);
+      if (fz.polyak) t4 = *reinterpret_cast<const float4*>(os.params + fz.n_online + G0 + off);
     }
     float acc[4][8];
 #pragma unroll
@@ -544,45 +515,12 @@ wgrad_kernel(NetShape s, const float* __restrict__ scratch, float* __restrict__ 
       p2p_stamp(px, cta, 5);
     }
     if (out_ok) {
-      if (!fz.params) {
+      if (!os.params) {
         if (!atomic) *reinterpret_cast<float4*>(grads + G0 + off) = v;
         else { atomicAdd(grads + G0 + off, v.x); atomicAdd(grads + G0 + off + 1, v.y); atomicAdd(grads + G0 + off + 2, v.z); atomicAdd(grads + G0 + off + 3, v.w); }
-      } else {
-        // torch.optim.Adam on 4 consecutive elements of a hidden weight W_l[gn][gk..gk+3] (the arithmetic of emit_pre(), element by element)
-        bias_corrections();
+      } else {                                // W_l[gn][gk..gk+3]
         const float g4[4] = {v.x, v.y, v.z, v.w};
-        const float mo[4] = {m4.x, m4.y, m4.z, m4.w}, vo[4] = {v4.x, v4.y, v4.z, v4.w}, po[4] = {p4.x, p4.y, p4.z, p4.w};
-        const float to[4] = {t4.x, t4.y, t4.z, t4.w};
-        float mn[4], vn[4], pn[4], tn[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          mn[e] = mo[e]; vn[e] = vo[e]; pn[e] = po[e];
-          adam_element(g4[e], mn[e], vn[e], pn[e], s_step, s_bc2);
-          tn[e] = __fadd_rn(__fmul_rn(to[e], 1.0f - fz.tau), __fmul_rn(pn[e], fz.tau));
-        }
-        const int64_t i0 = G0 + off;
-        *reinterpret_cast<float4*>(fz.m + i0) = make_float4(mn[0], mn[1], mn[2], mn[3]);
-        *reinterpret_cast<float4*>(fz.v + i0) = make_float4(vn[0], vn[1], vn[2], vn[3]);
-        *reinterpret_cast<float4*>(fz.params + i0) = make_float4(pn[0], pn[1], pn[2], pn[3]);
-        const int64_t wb = G0 + net_w_off(s, l);                                   // this weight matrix in the derived copies
-        const int64_t it = wb + (int64_t)gk * H + gn;                             // transposed copy: Wt[k][n]
-        const int64_t iu = wb + ((int64_t)(gk >> 2) * H + gn) * 4;                // chunk-major forward copy, k % 4 = 0..3 contiguous
-        const int64_t iv = wb + ((int64_t)(gn >> 2) * H + gk) * 4 + (gn & 3);     // chunk-major input-gradient copy, stride 4
-#pragma unroll
-        for (int e = 0; e < 4; ++e) fz.params_t[it + (int64_t)e * H] = pn[e];
-        if (fz.params_uv) {
-          const float4 pr = make_float4(tf32_rn(pn[0]), tf32_rn(pn[1]), tf32_rn(pn[2]), tf32_rn(pn[3]));
-          *reinterpret_cast<float4*>(fz.params_uv + iu) = pr;
-          fz.params_uv[fz.total + iv] = pr.x; fz.params_uv[fz.total + iv + 4] = pr.y;
-          fz.params_uv[fz.total + iv + 8] = pr.z; fz.params_uv[fz.total + iv + 12] = pr.w;
-        }
-        if (fz.polyak) {
-          *reinterpret_cast<float4*>(fz.params + fz.n_online + i0) = make_float4(tn[0], tn[1], tn[2], tn[3]);
-#pragma unroll
-          for (int e = 0; e < 4; ++e) fz.params_t[fz.n_online + it + (int64_t)e * H] = tn[e];
-          if (fz.params_uv)
-            *reinterpret_cast<float4*>(fz.params_uv + fz.n_online + iu) = make_float4(tf32_rn(tn[0]), tf32_rn(tn[1]), tf32_rn(tn[2]), tf32_rn(tn[3]));
-        }
+        adam_polyak4(os, (int)(G0 + off), (int)G0, copy_index(s, l - 1, gn, gk), H, g4, m4, v4, p4, t4, step_size(), true, fz.polyak, fz.n_online, fz.total);
       }
     }
     p2p_stamp(px, cta, 6);
@@ -620,10 +558,7 @@ wgrad_kernel(NetShape s, const float* __restrict__ scratch, float* __restrict__ 
       const bool lv[1] = {own};
       p2p_exchange_n<1>(px, seq, cta % px.world, ix, lv, v);
     }
-    if (own) {
-      if (fz.params) bias_corrections();
-      emit_pre(G0, o, v[0], atomic, pre);
-    }
+    if (own) emit_pre(G0, o, v[0], atomic, pre);
   } else {
     // output layer: warp o < 2 finishes W_L[o][k] for k = lane of this chunk, warp 2 of chunk 0 the biases
     const int chunk = job - nT - nS, k = chunk * 32 + lane;
@@ -653,28 +588,8 @@ wgrad_kernel(NetShape s, const float* __restrict__ scratch, float* __restrict__ 
       const bool lv[1] = {own};
       p2p_exchange_n<1>(px, seq, cta % px.world, ix, lv, v);
     }
-    if (own) {
-      if (fz.params) bias_corrections();
-      emit_pre(G0, o, v[0], atomic, pre);
-    }
+    if (own) emit_pre(G0, o, v[0], atomic, pre);
   }
-}
-
-// ---- Adam (torch.optim.Adam defaults, robot.py:237-239) + optional Polyak (robot.py:293-310), one pass --------------
-// nets: bit 0 actor, bit 1 critic1, bit 2 critic2 get an Adam step from `grads` (then the gradients are zeroed);
-// polyak: same bit layout; afterwards the selected target slots are blended with their (updated) online net:
-// t = t*(1-tau) + p*tau.
-// Index of parameter i (arena index inside slot `net_off`) in the transposed arena: hidden-layer weights W_l [H][H]
-// (l = 1..L-1) are stored as Wt_l [in][out] at the same offset; everything else keeps its place.
-__device__ __forceinline__ int64_t transposed_index(const NetShape& s, int64_t net_off, int64_t i) {
-  const int64_t o = i - net_off;
-  const int64_t first = (int64_t)s.in * s.hid + s.hid, blk = (int64_t)s.hid * s.hid + s.hid;
-  if (o < first) return i;
-  const int64_t o2 = o - first;
-  const int64_t l = o2 / blk, rem = o2 - l * blk;
-  if (l >= s.layers - 1 || rem >= (int64_t)s.hid * s.hid) return i;
-  const int64_t n = rem / s.hid, k = rem - n * s.hid;
-  return net_off + first + l * blk + k * s.hid + n;
 }
 
 // Rebuild the whole transposed arena from the parameters (after weights were written from outside the optimiser).
@@ -684,25 +599,26 @@ __global__ void td3_sync_transposed_kernel(Arena ar, const float* __restrict__ p
     const int64_t j = i < n_online ? i : i - n_online;
     const int net = j < ar.off(1) ? 0 : (j < ar.off(2) ? 1 : 2);
     const int64_t base = (i < n_online ? 0 : n_online) + ar.off(net);
-    params_t[transposed_index(net == 0 ? ar.actor : ar.critic, base, i)] = params[i];
+    params_t[base + copy_index(net == 0 ? ar.actor : ar.critic, (int)(i - base)).t] = params[i];
   }
 }
 
-__global__ void td3_adam_polyak_kernel(Arena ar, float* __restrict__ params, float* __restrict__ params_t, float* __restrict__ params_uv, float* __restrict__ grads, float* __restrict__ m,
-                                       float* __restrict__ v, const double* __restrict__ beta_pows, int nets, double lr_actor,
-                                       double lr_critic, float grad_scale, int polyak, float tau) {
+// ---- Adam (torch.optim.Adam defaults, robot.py:237-239) + optional Polyak (robot.py:293-310), one pass --------------
+// nets: bit 0 actor, bit 1 critic1, bit 2 critic2 get an Adam step from `grads` (then the gradients are zeroed);
+// polyak: same bit layout; afterwards the selected target slots are blended with their (updated) online net:
+// t = t*(1-tau) + p*tau.
+__global__ void td3_adam_polyak_kernel(AdamState st, float* __restrict__ grads, int nets, float grad_scale, int polyak) {
   __shared__ float s_step[2], s_bc2[2];
   if (threadIdx.x < 2) {                                              // 0: actor optimiser, 1: both critic optimisers
-    const double bc1 = 1.0 - beta_pows[2 * threadIdx.x], bc2 = 1.0 - beta_pows[2 * threadIdx.x + 1];
-    const double lr = threadIdx.x == 0 ? lr_actor : lr_critic;
-    s_step[threadIdx.x] = (float)(lr / bc1);
-    s_bc2[threadIdx.x] = (float)sqrt(bc2);
+    const AdamStep k = adam_step(threadIdx.x == 0 ? st.lr[0] : st.lr[1], st.beta_pows[2 * threadIdx.x], st.beta_pows[2 * threadIdx.x + 1]);
+    s_step[threadIdx.x] = k.step;
+    s_bc2[threadIdx.x] = k.sqrt_bc2;
   }
   __syncthreads();
-  const int n4 = (int)(ar.online_total() >> 2);                     // slots are multiples of 4 floats: a group of 4 never straddles two networks
+  const int n4 = (int)(st.ar.online_total() >> 2);                  // slots are multiples of 4 floats: a group of 4 never straddles two networks
   for (int i4 = blockIdx.x * blockDim.x + threadIdx.x; i4 < n4; i4 += gridDim.x * blockDim.x) {
     const int i = i4 * 4;
-    const int net = i < (int)ar.off(1) ? 0 : (i < (int)ar.off(2) ? 1 : 2);
+    const int net = i < (int)st.ar.off(1) ? 0 : (i < (int)st.ar.off(2) ? 1 : 2);
     const bool do_adam = (nets >> net) & 1, do_polyak = (polyak >> net) & 1;
     if (!do_adam && !do_polyak) continue;
     float g[4] = {0.f, 0.f, 0.f, 0.f};
@@ -711,7 +627,8 @@ __global__ void td3_adam_polyak_kernel(Arena ar, float* __restrict__ params, flo
       g[0] = g4.x * grad_scale; g[1] = g4.y * grad_scale; g[2] = g4.z * grad_scale; g[3] = g4.w * grad_scale;
       *reinterpret_cast<float4*>(grads + i) = make_float4(0.f, 0.f, 0.f, 0.f);
     }
-    adam_polyak_apply4(ar, i, net, g, do_adam, do_polyak, params, params_t, params_uv, m, v, s_step[net == 0 ? 0 : 1], s_bc2[net == 0 ? 0 : 1], tau);
+    const int o = net == 0 ? 0 : 1;
+    adam_polyak_apply4(st, i, net, g, AdamStep{s_step[o], s_bc2[o]}, do_adam, do_polyak);
   }
 }
 
@@ -788,6 +705,15 @@ static cudaError_t set_smem(K kernel, size_t bytes) {
   return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
 }
 
+// Every row-tile instantiation a launch can pick, [pick_tile]; rtd3_td3_create sets the shared-memory limit of every entry.
+static_assert(kNumTiles == 4 && kRowTiles[0] == 2 && kRowTiles[1] == 4 && kRowTiles[2] == 8 && kRowTiles[3] == 16, "tables follow kRowTiles");
+using CriticKernel = decltype(&td3_critic_kernel<2>);
+static const CriticKernel kCriticKernels[kNumTiles] = {td3_critic_kernel<2>, td3_critic_kernel<4>, td3_critic_kernel<8>, td3_critic_kernel<16>};
+using ActorKernel = decltype(&td3_actor_kernel<2>);
+static const ActorKernel kActorKernels[kNumTiles] = {td3_actor_kernel<2>, td3_actor_kernel<4>, td3_actor_kernel<8>, td3_actor_kernel<16>};
+using FwdKernel = decltype(&mlp_forward_kernel<2>);
+static const FwdKernel kFwdKernels[kNumTiles] = {mlp_forward_kernel<2>, mlp_forward_kernel<4>, mlp_forward_kernel<8>, mlp_forward_kernel<16>};
+
 static unsigned long long* g_p2p_prof = nullptr;   // development: stage stamps of the last fused weight-gradient launch
 
 static int wgrad_jobs(const NetShape& s) {
@@ -800,8 +726,8 @@ static int32_t launch_wgrad(rtd3_td3* h, const NetShape& s, const float* scratch
   const int jobs = wgrad_jobs(s);
   const int rows_per_split = 512;
   const int bsplit = (B + rows_per_split - 1) / rows_per_split;
-  RTD3_CHECK_ARG(!fz.params || bsplit == 1, "the fused optimiser needs batch <= 512");
-  RTD3_CHECK_ARG(!px.world || (fz.params && jobs * nslots <= kP2pBlockFlags), "the fused peer exchange needs the fused optimiser and at most 256 blocks");
+  RTD3_CHECK_ARG(!fz.adam.params || bsplit == 1, "the fused optimiser needs batch <= 512");
+  RTD3_CHECK_ARG(!px.world || (fz.adam.params && jobs * nslots <= kP2pBlockFlags), "the fused peer exchange needs the fused optimiser and at most 256 blocks");
   RTD3_CUDA(ensure_dyn_smem((const void*)wgrad_kernel, kWgradSmem));
   static const bool coop_env = !(getenv("RTD3_P2P_COOP") && atoi(getenv("RTD3_P2P_COOP")) == 0);
   if (px.world && coop_env) {
@@ -815,6 +741,51 @@ static int32_t launch_wgrad(rtd3_td3* h, const NetShape& s, const float* scratch
   }
   RTD3_LAUNCHED();
   return 0;
+}
+
+// One critic / actor step of the fp32 kernels: the row tiles or the cluster kernels, then the weight-gradient pass (with the optimiser
+// and the peer exchange fused into it on request).
+static int32_t critic_step(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const ReplayView& rp,
+                           const int32_t* idx, const float* noise, int32_t batch, const Td3Hyper& hp, float* loss2, float* q_out, float* y_out,
+                           int32_t* steps, double* beta_pows, cudaStream_t st, const AdamFuse& fz = AdamFuse{}, const P2pFuse& px = P2pFuse{}) {
+  if (cluster_path_ok(h, batch)) {
+    const int32_t rc = critic_cluster_launch(h, params, params_t, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows, st);
+    if (rc) return rc;
+  } else {
+    const int ti = pick_tile(batch, h->num_sms);
+    const int R = kRowTiles[ti];
+    kCriticKernels[ti]<<<(batch + R - 1) / R, kThreads, h->smem_critic[ti], st>>>(h->ar, params, params_t, scratch, rp, idx, noise, batch, hp, loss2,
+                                                                                   q_out, y_out, steps, beta_pows);
+    RTD3_LAUNCHED();
+  }
+  WgradSlots slots;
+  const int64_t per = RowScratch::floats(batch, h->ar.critic.hid, h->ar.critic.layers);
+  slots.grad_off[0] = h->ar.off(1); slots.grad_off[1] = h->ar.off(2);
+  slots.scratch_off[0] = 0; slots.scratch_off[1] = per;
+  return launch_wgrad(h, h->ar.critic, scratch, grads, slots, 2, batch, st, fz, px);
+}
+
+static int32_t actor_step(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const float* rp_s,
+                          const int32_t* idx, int32_t batch, float* loss1, int32_t* steps, double* beta_pows, void* stream,
+                          const AdamFuse& fz = AdamFuse{}, const P2pFuse& px = P2pFuse{}) {
+  RTD3_CHECK_ARG(h && params && params_t && grads && scratch && rp_s && idx && loss1 && steps && beta_pows, "null argument");
+  RTD3_CHECK_ARG(batch > 0, "batch must be positive");
+  ReplayView rp{(const float2*)rp_s, nullptr, nullptr, nullptr, nullptr};
+  cudaStream_t st = (cudaStream_t)stream;
+  if (cluster_path_ok(h, batch)) {
+    const int32_t rc = actor_cluster_launch(h, params, params_t, scratch, rp, idx, batch, loss1, steps, beta_pows, st);
+    if (rc) return rc;
+  } else {
+    const int ti = pick_tile(batch, h->num_sms);
+    const int R = kRowTiles[ti];
+    kActorKernels[ti]<<<(batch + R - 1) / R, kThreads, h->smem_actor[ti], st>>>(h->ar, params, params_t, scratch, rp, idx, batch, loss1, steps,
+                                                                                 beta_pows);
+    RTD3_LAUNCHED();
+  }
+  WgradSlots slots;
+  slots.grad_off[0] = h->ar.off(0); slots.grad_off[1] = 0;
+  slots.scratch_off[0] = 0; slots.scratch_off[1] = 0;
+  return launch_wgrad(h, h->ar.actor, scratch, grads, slots, 1, batch, st, fz, px);
 }
 
 extern "C" {
@@ -839,19 +810,10 @@ int32_t rtd3_td3_create(rtd3_td3** out, int32_t device, int32_t hidden, int32_t 
     h->smem_critic[i] = mlp_smem_bytes(R, hidden, layers);
     h->smem_actor[i] = actor_phase_smem(h->ar, R);
     h->smem_fwd[i] = mlp_smem_bytes(R, hidden, 0);
+    RTD3_CUDA(set_smem(kCriticKernels[i], h->smem_critic[i]));
+    RTD3_CUDA(set_smem(kActorKernels[i], h->smem_actor[i]));
+    RTD3_CUDA(set_smem(kFwdKernels[i], h->smem_fwd[i]));
   }
-  RTD3_CUDA(set_smem(td3_critic_kernel<2>, h->smem_critic[0]));
-  RTD3_CUDA(set_smem(td3_critic_kernel<4>, h->smem_critic[1]));
-  RTD3_CUDA(set_smem(td3_critic_kernel<8>, h->smem_critic[2]));
-  RTD3_CUDA(set_smem(td3_critic_kernel<16>, h->smem_critic[3]));
-  RTD3_CUDA(set_smem(td3_actor_kernel<2>, h->smem_actor[0]));
-  RTD3_CUDA(set_smem(td3_actor_kernel<4>, h->smem_actor[1]));
-  RTD3_CUDA(set_smem(td3_actor_kernel<8>, h->smem_actor[2]));
-  RTD3_CUDA(set_smem(td3_actor_kernel<16>, h->smem_actor[3]));
-  RTD3_CUDA(set_smem(mlp_forward_kernel<2>, h->smem_fwd[0]));
-  RTD3_CUDA(set_smem(mlp_forward_kernel<4>, h->smem_fwd[1]));
-  RTD3_CUDA(set_smem(mlp_forward_kernel<8>, h->smem_fwd[2]));
-  RTD3_CUDA(set_smem(mlp_forward_kernel<16>, h->smem_fwd[3]));
   if (const char* e = getenv("RTD3_TILE")) g_tile_override = atoi(e);
   h->cluster_cap = std::max(0, rtd3_td3_cluster_occupancy(h, 256));     // (queried here, never inside a stream capture)
   RTD3_CUDA(cudaSetDevice(prev));
@@ -894,83 +856,13 @@ int32_t rtd3_td3_critic_step(rtd3_td3* h, const float* params, const float* para
   RTD3_CHECK_ARG(batch > 0, "batch must be positive");
   ReplayView rp{(const float2*)rp_s, (const float2*)rp_a, rp_r, (const float2*)rp_s2, rp_notdone};
   Td3Hyper hp{gamma, policy_noise, noise_clip, max_action, 0ull, nullptr, 0ull};
-  return critic_step_launch(h, params, params_t, grads, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows, (cudaStream_t)stream);
+  return critic_step(h, params, params_t, grads, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows, (cudaStream_t)stream);
 }
-
-}  // extern "C"
-
-static int32_t critic_step_fused(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const ReplayView& rp,
-                                 const int32_t* idx, const float* noise, int32_t batch, const Td3Hyper& hp, float* loss2, float* q_out, float* y_out,
-                                 int32_t* steps, double* beta_pows, cudaStream_t st, const AdamFuse& fz, const P2pFuse& px = P2pFuse{});
-
-int32_t rtd3::critic_step_launch(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const ReplayView& rp,
-                                 const int32_t* idx, const float* noise, int32_t batch, const Td3Hyper& hp, float* loss2, float* q_out, float* y_out,
-                                 int32_t* steps, double* beta_pows, cudaStream_t st) {
-  return critic_step_fused(h, params, params_t, grads, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows, st, AdamFuse{});
-}
-
-static int32_t critic_step_fused(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const ReplayView& rp,
-                                 const int32_t* idx, const float* noise, int32_t batch, const Td3Hyper& hp, float* loss2, float* q_out, float* y_out,
-                                 int32_t* steps, double* beta_pows, cudaStream_t st, const AdamFuse& fz, const P2pFuse& px) {
-  if (cluster_path_ok(h, batch)) {
-    const int32_t rc = critic_cluster_launch(h, params, params_t, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows, st);
-    if (rc) return rc;
-  } else {
-    const int ti = pick_tile(batch, h->num_sms);
-    const int R = kRowTiles[ti];
-    const int grid = (batch + R - 1) / R;
-#define RTD3_CRITIC(RR) \
-  td3_critic_kernel<RR><<<grid, kThreads, h->smem_critic[ti], st>>>(h->ar, params, params_t, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows)
-    if (ti == 0) RTD3_CRITIC(2); else if (ti == 1) RTD3_CRITIC(4); else if (ti == 2) RTD3_CRITIC(8); else RTD3_CRITIC(16);
-#undef RTD3_CRITIC
-    RTD3_LAUNCHED();
-  }
-  WgradSlots slots;
-  const int64_t per = RowScratch::floats(batch, h->ar.critic.hid, h->ar.critic.layers);
-  slots.grad_off[0] = h->ar.off(1); slots.grad_off[1] = h->ar.off(2);
-  slots.scratch_off[0] = 0; slots.scratch_off[1] = per;
-  return launch_wgrad(h, h->ar.critic, scratch, grads, slots, 2, batch, st, fz, px);
-}
-
-extern "C" {
-
-static int32_t actor_step_fused(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const float* rp_s,
-                                const int32_t* idx, int32_t batch, float* loss1, int32_t* steps, double* beta_pows, void* stream, const AdamFuse& fz,
-                                const P2pFuse& px = P2pFuse{});
 
 int32_t rtd3_td3_actor_step(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const float* rp_s, const int32_t* idx,
                             int32_t batch, float* loss1, int32_t* steps, double* beta_pows, void* stream) {
-  return actor_step_fused(h, params, params_t, grads, scratch, rp_s, idx, batch, loss1, steps, beta_pows, stream, AdamFuse{});
+  return actor_step(h, params, params_t, grads, scratch, rp_s, idx, batch, loss1, steps, beta_pows, stream);
 }
-
-}  // extern "C"
-
-static int32_t actor_step_fused(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const float* rp_s,
-                                const int32_t* idx, int32_t batch, float* loss1, int32_t* steps, double* beta_pows, void* stream, const AdamFuse& fz,
-                                const P2pFuse& px) {
-  RTD3_CHECK_ARG(h && params && params_t && grads && scratch && rp_s && idx && loss1 && steps && beta_pows, "null argument");
-  RTD3_CHECK_ARG(batch > 0, "batch must be positive");
-  ReplayView rp{(const float2*)rp_s, nullptr, nullptr, nullptr, nullptr};
-  cudaStream_t st = (cudaStream_t)stream;
-  if (cluster_path_ok(h, batch)) {
-    const int32_t rc = actor_cluster_launch(h, params, params_t, scratch, rp, idx, batch, loss1, steps, beta_pows, st);
-    if (rc) return rc;
-  } else {
-    const int ti = pick_tile(batch, h->num_sms);
-    const int R = kRowTiles[ti];
-    const int grid = (batch + R - 1) / R;
-#define RTD3_ACTOR(RR) td3_actor_kernel<RR><<<grid, kThreads, h->smem_actor[ti], st>>>(h->ar, params, params_t, scratch, rp, idx, batch, loss1, steps, beta_pows)
-    if (ti == 0) RTD3_ACTOR(2); else if (ti == 1) RTD3_ACTOR(4); else if (ti == 2) RTD3_ACTOR(8); else RTD3_ACTOR(16);
-#undef RTD3_ACTOR
-    RTD3_LAUNCHED();
-  }
-  WgradSlots slots;
-  slots.grad_off[0] = h->ar.off(0); slots.grad_off[1] = 0;
-  slots.scratch_off[0] = 0; slots.scratch_off[1] = 0;
-  return launch_wgrad(h, h->ar.actor, scratch, grads, slots, 1, batch, st, fz, px);
-}
-
-extern "C" {
 
 int32_t rtd3_td3_adam_polyak(rtd3_td3* h, float* params, float* params_t, float* params_uv, float* grads, float* adam_m, float* adam_v, const double* beta_pows, int32_t nets,
                              double lr_actor, double lr_critic, float grad_scale, int32_t polyak, float tau, void* stream) {
@@ -978,8 +870,8 @@ int32_t rtd3_td3_adam_polyak(rtd3_td3* h, float* params, float* params_t, float*
   const int64_t n = h->ar.online_total();
   const int block = 256;
   const int grid = (int)std::min<int64_t>(ceil_div(n / 4, block), (int64_t)h->num_sms * 8);
-  td3_adam_polyak_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(h->ar, params, params_t, params_uv, grads, adam_m, adam_v, beta_pows, nets, lr_actor,
-                                                                    lr_critic, grad_scale, polyak, tau);
+  const AdamState opt{h->ar, params, params_t, params_uv, adam_m, adam_v, const_cast<double*>(beta_pows), {lr_actor, lr_critic}, tau};   // clocks read only
+  td3_adam_polyak_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(opt, grads, nets, grad_scale, polyak);
   RTD3_LAUNCHED();
   return 0;
 }
@@ -994,10 +886,7 @@ int32_t rtd3_mlp_forward(rtd3_td3* h, int32_t net, const float* params, const fl
   const int ti = pick_tile(batch, h->num_sms);
   const int R = kRowTiles[ti];
   const int grid = (int)((batch + R - 1) / R);
-  cudaStream_t st = (cudaStream_t)stream;
-#define RTD3_FWD(RR) mlp_forward_kernel<RR><<<grid, kThreads, h->smem_fwd[ti], st>>>(s, params + h->ar.off(net), params_t + h->ar.off(net), x, y, (int)batch)
-  if (ti == 0) RTD3_FWD(2); else if (ti == 1) RTD3_FWD(4); else if (ti == 2) RTD3_FWD(8); else RTD3_FWD(16);
-#undef RTD3_FWD
+  kFwdKernels[ti]<<<grid, kThreads, h->smem_fwd[ti], (cudaStream_t)stream>>>(s, params + h->ar.off(net), params_t + h->ar.off(net), x, y, (int)batch);
   RTD3_LAUNCHED();
   return 0;
 }
@@ -1083,7 +972,6 @@ int32_t rtd3_td3_update(rtd3_td3* h, const rtd3_td3_update_args* a, void* stream
   RTD3_CUDA(cudaMemsetAsync(a->critic_losses, 0, sizeof(float) * 2 * (size_t)E, st));
   RTD3_CUDA(cudaMemsetAsync(a->actor_losses, 0, sizeof(float) * (size_t)n_actor, st));
   const ReplayView rp{(const float2*)a->rp_s, (const float2*)a->rp_a, a->rp_r, (const float2*)a->rp_s2, a->rp_notdone};
-  const ReplayView rp_actor{(const float2*)a->rp_s, nullptr, nullptr, nullptr, nullptr};
   Td3Hyper hp{a->gamma, a->policy_noise, a->noise_clip, a->max_action, (unsigned long long)a->noise_seed,
               (const unsigned long long*)a->noise_counter, 0ull};
   float* opt_grads = (a->world > 1 && a->p2p) ? a->p2p->sum : a->grads;      // what the optimiser consumes
@@ -1114,23 +1002,12 @@ int32_t rtd3_td3_update(rtd3_td3* h, const rtd3_td3_update_args* a, void* stream
     px.mode = p2p_mode_env >= 0 ? p2p_mode_env : (a->world > 2 ? 1 : 0);
     return px;
   };
-  auto fuse_for = [&](bool actor, bool polyak) {
-    AdamFuse fz{};
-    fz.params = a->params; fz.params_t = a->params_t; fz.params_uv = a->params_uv; fz.m = a->adam_m; fz.v = a->adam_v;
-    fz.beta_pows = a->beta_pows; fz.lr = actor ? a->lr_actor : a->lr_critic; fz.opt = actor ? 0 : 1; fz.polyak = polyak ? 1 : 0;
-    fz.tau = a->tau; fz.n_online = (int)n_online; fz.total = (int)h->ar.total(); fz.shape = actor ? h->ar.actor : h->ar.critic;
-    return fz;
-  };
+  const AdamState opt = adam_state(h, a);
+  auto fuse_for = [&](bool actor, bool polyak) { return AdamFuse{opt, actor ? 0 : 1, polyak ? 1 : 0, (int)n_online, (int)h->ar.total()}; };
   // Data parallel over peer memory: the all-reduce kernel applies the optimiser to the sums it forms (one launch and one pass over the
   // arena less per optimiser step); RTD3_P2P_FUSE=0 keeps the two-kernel form (development)
   const bool fuse_p2p = a->world > 1 && a->p2p && p2p_fuse_env >= 1 && !fuse_wg;
-  auto p2p_opt = [&](int nets, int polyak, int64_t off) {
-    P2pAdamArgs o{};
-    o.ar = h->ar; o.params = a->params; o.params_t = a->params_t; o.params_uv = a->params_uv; o.m = a->adam_m; o.v = a->adam_v;
-    o.beta_pows = a->beta_pows; o.lr_actor = a->lr_actor; o.lr_critic = a->lr_critic; o.grad_scale = scale; o.tau = a->tau;
-    o.nets = nets; o.polyak = polyak; o.off = off;
-    return o;
-  };
+  auto p2p_opt = [&](int nets, int polyak, int64_t off) { return P2pAdamArgs{opt, scale, nets, polyak, off}; };
   int64_t k = 0, ka = 0;
   int32_t rc = 0;
   for (int e = 0; e < E; ++e) {
@@ -1142,8 +1019,8 @@ int32_t rtd3_td3_update(rtd3_td3* h, const rtd3_td3_update_args* a, void* stream
       rc = critic_step_tc_launch(h, a->params, a->params_uv, a->grads, rp, ix, nz, B, hp, a->critic_losses + 2 * e, nullptr, nullptr, a->steps,
                                  a->beta_pows, st);
     else
-      rc = critic_step_fused(h, a->params, a->params_t, a->grads, a->scratch, rp, ix, nz, B, hp, a->critic_losses + 2 * e, nullptr, nullptr,
-                             a->steps, a->beta_pows, st, fuse ? fuse_for(false, e % delay == 0) : AdamFuse{}, px_for(false));
+      rc = critic_step(h, a->params, a->params_t, a->grads, a->scratch, rp, ix, nz, B, hp, a->critic_losses + 2 * e, nullptr, nullptr, a->steps,
+                       a->beta_pows, st, fuse ? fuse_for(false, e % delay == 0) : AdamFuse{}, px_for(false));
     if (rc) return rc;
     if (fuse_p2p) {
       if ((rc = p2p_allreduce_adam_launch(a->p2p, a->grads, n_online - off_c, p2p_opt(0b110, 0, off_c), st))) return rc;
@@ -1159,8 +1036,8 @@ int32_t rtd3_td3_update(rtd3_td3* h, const rtd3_td3_update_args* a, void* stream
       if (tc)
         rc = rtd3_td3_actor_step_tf32(h, a->params, a->params_uv, a->grads, a->rp_s, ixa, B, a->actor_losses + ka, a->steps, a->beta_pows, st);
       else
-        rc = actor_step_fused(h, a->params, a->params_t, a->grads, a->scratch, a->rp_s, ixa, B, a->actor_losses + ka, a->steps, a->beta_pows, st,
-                              fuse ? fuse_for(true, true) : AdamFuse{}, px_for(true));
+        rc = actor_step(h, a->params, a->params_t, a->grads, a->scratch, a->rp_s, ixa, B, a->actor_losses + ka, a->steps, a->beta_pows, st,
+                        fuse ? fuse_for(true, true) : AdamFuse{}, px_for(true));
       ++ka;
       if (rc) return rc;
       if (fuse_p2p) {
@@ -1173,7 +1050,6 @@ int32_t rtd3_td3_update(rtd3_td3* h, const rtd3_td3_update_args* a, void* stream
       }
     }
   }
-  (void)rp_actor;
   if (!a->noise) return advance_noise_counter(a->noise_counter, (uint64_t)E, st);
   return 0;
 }

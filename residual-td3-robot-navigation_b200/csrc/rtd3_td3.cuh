@@ -52,34 +52,27 @@ struct Arena {
   __host__ __device__ int64_t total() const { return 2 * online_total(); }
 };
 
-// Tensor-core operand copies of the arena (params_uv = [u | v], each `total()` floats).  Hidden-to-hidden weights W_l [H][H]
-// (l = 1..L-1) are stored chunk-major at the offset of W_l and rounded to TF32 (round-to-nearest):
-//   u (forward, B operand K-major):            Wu[(k/4)*H + n][k%4] = W[n][k]
-//   v (input gradient, B operand K-major of W^T): Wv[(n/4)*H + k][n%4] = W[n][k]
-// every other parameter keeps its place and value.
-__host__ __device__ inline bool is_hidden_weight(const NetShape& s, int64_t net_off, int64_t i) {
-  const int64_t o = i - net_off;
-  const int64_t first = (int64_t)s.in * s.hid + s.hid, blk = (int64_t)s.hid * s.hid + s.hid;
-  if (o < first) return false;
-  const int64_t o2 = o - first;
-  const int64_t l = o2 / blk, rem = o2 - l * blk;
-  return l < s.layers - 1 && rem < (int64_t)s.hid * s.hid;
-}
-__host__ __device__ inline int64_t chunk_major_index(const NetShape& s, int64_t net_off, int64_t i) {
-  if (!is_hidden_weight(s, net_off, i)) return i;
-  const int64_t first = (int64_t)s.in * s.hid + s.hid, blk = (int64_t)s.hid * s.hid + s.hid;
-  const int64_t o2 = i - net_off - first;
-  const int64_t l = o2 / blk, rem = o2 - l * blk;
-  const int64_t n = rem / s.hid, k = rem - n * s.hid;
-  return net_off + first + l * blk + ((k >> 2) * s.hid + n) * 4 + (k & 3);
-}
-__host__ __device__ inline int64_t chunk_major_index_v(const NetShape& s, int64_t net_off, int64_t i) {
-  if (!is_hidden_weight(s, net_off, i)) return i;
-  const int64_t first = (int64_t)s.in * s.hid + s.hid, blk = (int64_t)s.hid * s.hid + s.hid;
-  const int64_t o2 = i - net_off - first;
-  const int64_t l = o2 / blk, rem = o2 - l * blk;
-  const int64_t n = rem / s.hid, k = rem - n * s.hid;
-  return net_off + first + l * blk + ((n >> 2) * s.hid + k) * 4 + (n & 3);
+// The optimiser's state: the parameter arena with its derived copies, torch.optim.Adam's moments and clocks (robot.py:237-239) and the
+// Polyak rate.  One per update call; every kernel that applies the optimiser takes it.
+struct AdamState {
+  Arena ar;
+  float* params;            // the arena (online | target)
+  float* params_t;          // transposed copy
+  float* params_uv;         // nullable: the tensor-core operand copies [u | v] are not kept
+  float* m;
+  float* v;
+  double* beta_pows;        // [2][2]: beta1^t, beta2^t of optimiser 0 (actor) and 1 (critics)
+  double lr[2];             // 0 actor, 1 critics
+  float tau;
+};
+
+// torch.optim.Adam's step size lr / (1 - beta1^t) and sqrt(1 - beta2^t), formed in double from the double lr and the running powers
+// (as torch forms them in Python floats) and rounded to float once each.
+struct AdamStep {
+  float step, sqrt_bc2;
+};
+__device__ __forceinline__ AdamStep adam_step(double lr, double beta1_pow, double beta2_pow) {
+  return AdamStep{(float)(lr / (1.0 - beta1_pow)), (float)sqrt(1.0 - beta2_pow)};
 }
 
 // One element of torch.optim.Adam (defaults, robot.py:237-239) in the operation order of torch's CPU kernels, measured against
@@ -87,88 +80,133 @@ __host__ __device__ inline int64_t chunk_major_index_v(const NetShape& s, int64_
 //   exp_avg.lerp_(grad, 1 - beta1)                       m = fma(g - m, 0.1f, m)
 //   exp_avg_sq.mul_(beta2).addcmul_(g, g, 1 - beta2)     v = fma(0.001f * g, g, v * 0.999f)         (both products rounded)
 //   denom = sqrt(v) / sqrt(bc2) + eps;  param.addcdiv_(exp_avg, denom, -step)      p = p + (-step * m) / denom
-// Every rounding is spelled out so that the three kernels that apply it (td3_adam_polyak_kernel, the optimiser fused into
-// wgrad_kernel, the cooperative kernel) agree bit for bit - left to the compiler, the contraction of a*b + c*d differs between them.
+// Every rounding is spelled out: its callers, adam_polyak4 and adam_polyak1, are inlined into kernels of different shapes, and left to
+// the compiler, the contraction of a*b + c*d would differ between them.
 __device__ __forceinline__ void adam_element(float g, float& m, float& v, float& p, float step, float sqrt_bc2) {
   m = __fmaf_rn(__fsub_rn(g, m), 0.1f, m);
   v = __fmaf_rn(__fmul_rn(0.001f, g), g, __fmul_rn(v, 0.999f));
   const float denom = __fadd_rn(__fdiv_rn(sqrtf(v), sqrt_bc2), 1e-8f);
   p = __fadd_rn(p, __fdiv_rn(__fmul_rn(-step, m), denom));
 }
+// robot.py:309, three roundings
+__device__ __forceinline__ float polyak_blend(float t, float p, float tau) { return __fadd_rn(__fmul_rn(t, 1.0f - tau), __fmul_rn(p, tau)); }
 
-// Where arena element o (offset inside its network's slot) sits in the derived copies, decomposed ONCE per element in 32-bit
-// arithmetic: the 64-bit divisions of transposed_index / chunk_major_index (five calls per element) made this kernel ~13 us.
-struct CopyIndex {
-  int t, u, v;          // offsets inside the slot in the transposed / forward chunk-major / input-gradient chunk-major copies
-  bool hidden;          // a hidden-to-hidden weight (the only entries that move, and that are TF32-rounded in u / v)
+// Arena element o (offset inside its network's slot) as a hidden-to-hidden weight W_{l+1}[n][k] (l = 0..L-2), or not one.  32-bit
+// arithmetic: a slot of H <= kMaxHidden, L <= kMaxLayers holds well under 2^31 elements (the 64-bit divisions of an earlier per-copy
+// index function made the optimiser kernel ~13 us).
+struct SlotPos {
+  bool hidden;
+  unsigned l, n, k;
 };
-__device__ __forceinline__ CopyIndex copy_index(const NetShape& s, int o) {
-  CopyIndex c{o, o, o, false};
+__device__ __forceinline__ SlotPos slot_pos(const NetShape& s, int o) {
   const int first = s.in * s.hid + s.hid, blk = s.hid * s.hid + s.hid;
-  if (o < first) return c;
+  if (o < first) return SlotPos{false, 0u, 0u, 0u};
   const unsigned o2 = (unsigned)(o - first);
   const unsigned l = o2 / (unsigned)blk, rem = o2 - l * (unsigned)blk;
-  if ((int)l >= s.layers - 1 || rem >= (unsigned)(s.hid * s.hid)) return c;
-  const unsigned n = rem / (unsigned)s.hid, k = rem - n * (unsigned)s.hid;
-  const int base = first + (int)l * blk;
-  c.hidden = true;
-  c.t = base + (int)(k * s.hid + n);
-  c.u = base + (int)((((k >> 2) * s.hid + n) << 2) + (k & 3u));
-  c.v = base + (int)((((n >> 2) * s.hid + k) << 2) + (n & 3u));
-  return c;
+  if ((int)l >= s.layers - 1 || rem >= (unsigned)(s.hid * s.hid)) return SlotPos{false, 0u, 0u, 0u};
+  const unsigned n = rem / (unsigned)s.hid;
+  return SlotPos{true, l, n, rem - n * (unsigned)s.hid};
 }
 
+// Where a parameter sits in the derived copies of the arena (offsets inside its network's slot).  Hidden-to-hidden weights W [H][H]
+// move; every other parameter keeps its place and value in all three:
+//   t  (transposed, forward operand of the fp32 kernels):          Wt[k][n] = W[n][k]
+//   u  (tensor cores, forward B operand K-major, TF32-rounded):     Wu[(k/4)*H + n][k%4] = W[n][k]
+//   v  (tensor cores, input-gradient B operand K-major of W^T):     Wv[(n/4)*H + k][n%4] = W[n][k]
+// params_uv = [u | v], each ar.total() floats.
+struct CopyIndex {
+  int t, u, v;
+  bool hidden;          // a hidden-to-hidden weight (the only entries that move, and that are TF32-rounded in u / v)
+};
+__device__ __forceinline__ CopyIndex copy_index(const NetShape& s, unsigned l, unsigned n, unsigned k) {   // of W_{l+1}[n][k]
+  const int base = s.in * s.hid + s.hid + (int)l * (s.hid * s.hid + s.hid);
+  return CopyIndex{base + (int)(k * s.hid + n), base + (int)((((k >> 2) * s.hid + n) << 2) + (k & 3u)),
+                   base + (int)((((n >> 2) * s.hid + k) << 2) + (n & 3u)), true};
+}
+__device__ __forceinline__ CopyIndex copy_index(const NetShape& s, int o) {
+  const SlotPos q = slot_pos(s, o);
+  return q.hidden ? copy_index(s, q.l, q.n, q.k) : CopyIndex{o, o, o, false};
+}
 
-// Four consecutive arena elements i .. i+3 of the optimiser pass (i a multiple of 4: network slots, weight matrices and bias vectors all
-// start at multiples of 4, so the four are either four neighbours of one row of a hidden weight matrix or four elements that keep
-// their place in the derived copies): Adam (when do_adam, with the already scaled gradients g) on the parameters of online network
-// `net`, then (when do_polyak) the blend of the matching target parameters, t = t*(1-tau) + p*tau; the transposed copy and the
-// tensor-core operand copies (params_uv, nullable) are kept in step.  One round of 16-byte loads per group.  Shared by
-// td3_adam_polyak_kernel and the peer-memory all-reduce that applies the optimiser to the sums it forms (rtd3_p2p.cu).
-__device__ __forceinline__ void adam_polyak_apply4(const Arena& ar, int i, int net, const float (&g)[4], bool do_adam, bool do_polyak,
-                                                   float* __restrict__ params, float* __restrict__ params_t, float* __restrict__ params_uv,
-                                                   float* __restrict__ m, float* __restrict__ v, float step, float sqrt_bc2, float tau) {
-  const int n_online = (int)ar.online_total(), total = (int)ar.total();
-  const int noff = net == 0 ? 0 : (int)ar.off(net);
-  const CopyIndex ci = copy_index(net == 0 ? ar.actor : ar.critic, i - noff);      // of element i; hidden: .t stride H, .u contiguous, .v stride 4
-  const int H = (net == 0 ? ar.actor : ar.critic).hid;
+// The optimiser on four consecutive arena elements i .. i+3 of an online network (slot offset noff, ci = copy_index of element i,
+// H its hidden width; n_online, total = s.ar.online_total(), s.ar.total()) from operands the caller has loaded: Adam (when do_adam)
+// with the already scaled gradients g on the moments m4, v4 and the parameters p4, then (when do_polyak) the blend of the target
+// parameters t4, t = t*(1-tau) + p*tau; the results are stored into the arena, the moments and every derived copy.  i is a multiple of 4 (network slots, weight matrices and bias vectors
+// all start at multiples of 4), so the four are either four neighbours of one row of a hidden weight matrix (in t a column, stride H;
+// in v stride 4) or four elements that keep their place.
+__device__ __forceinline__ void adam_polyak4(const AdamState& s, int i, int noff, const CopyIndex& ci, int H, const float (&g)[4], float4 m4,
+                                             float4 v4, float4 p4, float4 t4, AdamStep k, bool do_adam, bool do_polyak, int n_online, int total) {
   const int st = ci.hidden ? H : 1, sv = ci.hidden ? 4 : 1;
-  float4 p4 = *reinterpret_cast<const float4*>(params + i);
   float p[4] = {p4.x, p4.y, p4.z, p4.w};
-  float4 t4 = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (do_polyak) t4 = *reinterpret_cast<const float4*>(params + n_online + i);
   if (do_adam) {
-    const float4 m4 = *reinterpret_cast<const float4*>(m + i), v4 = *reinterpret_cast<const float4*>(v + i);
     float mm[4] = {m4.x, m4.y, m4.z, m4.w}, vv[4] = {v4.x, v4.y, v4.z, v4.w};
 #pragma unroll
-    for (int e = 0; e < 4; ++e) adam_element(g[e], mm[e], vv[e], p[e], step, sqrt_bc2);
-    *reinterpret_cast<float4*>(m + i) = make_float4(mm[0], mm[1], mm[2], mm[3]);
-    *reinterpret_cast<float4*>(v + i) = make_float4(vv[0], vv[1], vv[2], vv[3]);
-    *reinterpret_cast<float4*>(params + i) = make_float4(p[0], p[1], p[2], p[3]);
+    for (int e = 0; e < 4; ++e) adam_element(g[e], mm[e], vv[e], p[e], k.step, k.sqrt_bc2);
+    *reinterpret_cast<float4*>(s.m + i) = make_float4(mm[0], mm[1], mm[2], mm[3]);
+    *reinterpret_cast<float4*>(s.v + i) = make_float4(vv[0], vv[1], vv[2], vv[3]);
+    *reinterpret_cast<float4*>(s.params + i) = make_float4(p[0], p[1], p[2], p[3]);
 #pragma unroll
-    for (int e = 0; e < 4; ++e) params_t[noff + ci.t + e * st] = p[e];
-    if (params_uv) {
+    for (int e = 0; e < 4; ++e) s.params_t[noff + ci.t + e * st] = p[e];
+    if (s.params_uv) {
       float pr[4];
 #pragma unroll
       for (int e = 0; e < 4; ++e) pr[e] = ci.hidden ? tf32_rn(p[e]) : p[e];
-      *reinterpret_cast<float4*>(params_uv + noff + ci.u) = make_float4(pr[0], pr[1], pr[2], pr[3]);
+      *reinterpret_cast<float4*>(s.params_uv + noff + ci.u) = make_float4(pr[0], pr[1], pr[2], pr[3]);
 #pragma unroll
-      for (int e = 0; e < 4; ++e) params_uv[total + noff + ci.v + e * sv] = pr[e];
+      for (int e = 0; e < 4; ++e) s.params_uv[total + noff + ci.v + e * sv] = pr[e];
     }
   }
   if (do_polyak) {
     const float to[4] = {t4.x, t4.y, t4.z, t4.w};
     float tv[4];
 #pragma unroll
-    for (int e = 0; e < 4; ++e) tv[e] = __fadd_rn(__fmul_rn(to[e], 1.0f - tau), __fmul_rn(p[e], tau));   // robot.py:309, three roundings
-    *reinterpret_cast<float4*>(params + n_online + i) = make_float4(tv[0], tv[1], tv[2], tv[3]);
+    for (int e = 0; e < 4; ++e) tv[e] = polyak_blend(to[e], p[e], s.tau);
+    *reinterpret_cast<float4*>(s.params + n_online + i) = make_float4(tv[0], tv[1], tv[2], tv[3]);
 #pragma unroll
-    for (int e = 0; e < 4; ++e) params_t[n_online + noff + ci.t + e * st] = tv[e];
-    if (params_uv)
-      *reinterpret_cast<float4*>(params_uv + n_online + noff + ci.u) =
+    for (int e = 0; e < 4; ++e) s.params_t[n_online + noff + ci.t + e * st] = tv[e];
+    if (s.params_uv)   // the target networks run forward only: their v copy is not kept
+      *reinterpret_cast<float4*>(s.params_uv + n_online + noff + ci.u) =
           make_float4(ci.hidden ? tf32_rn(tv[0]) : tv[0], ci.hidden ? tf32_rn(tv[1]) : tv[1], ci.hidden ? tf32_rn(tv[2]) : tv[2],
                       ci.hidden ? tf32_rn(tv[3]) : tv[3]);
   }
+}
+// The same on one element i.
+__device__ __forceinline__ void adam_polyak1(const AdamState& s, int i, int noff, const CopyIndex& ci, float g, float m, float v, float p,
+                                             float t, AdamStep k, bool do_adam, bool do_polyak, int n_online, int total) {
+  if (do_adam) {
+    adam_element(g, m, v, p, k.step, k.sqrt_bc2);
+    s.m[i] = m;
+    s.v[i] = v;
+    s.params[i] = p;
+    s.params_t[noff + ci.t] = p;
+    if (s.params_uv) {
+      const float pr = ci.hidden ? tf32_rn(p) : p;
+      s.params_uv[noff + ci.u] = pr;
+      s.params_uv[total + noff + ci.v] = pr;
+    }
+  }
+  if (do_polyak) {
+    const float tv = polyak_blend(t, p, s.tau);
+    s.params[n_online + i] = tv;
+    s.params_t[n_online + noff + ci.t] = tv;
+    if (s.params_uv) s.params_uv[n_online + noff + ci.u] = ci.hidden ? tf32_rn(tv) : tv;
+  }
+}
+
+// Load-then-apply form of adam_polyak4 for the kernels that walk the online arena in groups of 4 (td3_adam_polyak_kernel, and the
+// peer-memory all-reduce that applies the optimiser to the sums it forms, rtd3_p2p.cu): one round of 16-byte loads per group.
+__device__ __forceinline__ void adam_polyak_apply4(const AdamState& s, int i, int net, const float (&g)[4], AdamStep k, bool do_adam, bool do_polyak) {
+  const int noff = net == 0 ? 0 : (int)s.ar.off(net);
+  const NetShape& sh = net == 0 ? s.ar.actor : s.ar.critic;
+  const CopyIndex ci = copy_index(sh, i - noff);
+  const float4 p4 = *reinterpret_cast<const float4*>(s.params + i);
+  float4 t4 = make_float4(0.f, 0.f, 0.f, 0.f), m4 = t4, v4 = t4;
+  if (do_polyak) t4 = *reinterpret_cast<const float4*>(s.params + (int)s.ar.online_total() + i);
+  if (do_adam) {
+    m4 = *reinterpret_cast<const float4*>(s.m + i);
+    v4 = *reinterpret_cast<const float4*>(s.v + i);
+  }
+  adam_polyak4(s, i, noff, ci, sh.hid, g, m4, v4, p4, t4, k, do_adam, do_polyak, (int)s.ar.online_total(), (int)s.ar.total());
 }
 
 // Adam bookkeeping advanced by the first thread of a step kernel: the step counter and the running powers
@@ -181,12 +219,9 @@ __device__ __forceinline__ void advance_adam_clock(int32_t* steps, double* beta_
 
 }  // namespace rtd3
 
-// launch helpers shared by the public step entry points and rtd3_td3_update (rtd3_td3.cu, rtd3_tc_learner.cu)
+// launch helpers shared by the learner sources
 struct rtd3_td3;
 namespace rtd3 {
-int32_t critic_step_launch(rtd3_td3* h, const float* params, const float* params_t, float* grads, float* scratch, const ReplayView& rp,
-                           const int32_t* idx, const float* noise, int32_t batch, const Td3Hyper& hp, float* loss2, float* q_out, float* y_out,
-                           int32_t* steps, double* beta_pows, cudaStream_t st);
 int32_t advance_noise_counter(uint64_t* counter, uint64_t by, cudaStream_t st);   // counter[0] += by on the stream
 int32_t critic_step_tc_launch(rtd3_td3* h, const float* params, const float* params_uv, float* grads, const ReplayView& rp, const int32_t* idx,
                               const float* noise, int32_t batch, const Td3Hyper& hp, float* loss2, float* q_out, float* y_out, int32_t* steps,
@@ -203,11 +238,8 @@ int32_t actor_cluster_launch(rtd3_td3* h, const float* params, const float* para
 // rtd3_td3_adam_polyak do in two launches and two passes over the arena.  [off, off + count) = the slice of the gradient arena this
 // optimiser step reduces; nets / polyak as in rtd3_td3_adam_polyak.
 struct P2pAdamArgs {
-  Arena ar;
-  float* params; float* params_t; float* params_uv; float* m; float* v;
-  const double* beta_pows;
-  double lr_actor, lr_critic;
-  float grad_scale, tau;
+  AdamState adam;
+  float grad_scale;
   int nets, polyak;
   int64_t off;
 };
@@ -225,4 +257,9 @@ struct rtd3_td3 {
   size_t smem_critic[kNumTiles], smem_actor[kNumTiles], smem_fwd[kNumTiles];
   int cluster_cap;      // clusters of the cluster step kernels the device holds at once (set by rtd3_td3_create; 0: path unavailable)
 };
+
+// the optimiser state of an update call (rtd3_td3_update, rtd3_td3_update_coop)
+inline rtd3::AdamState adam_state(const rtd3_td3* h, const rtd3_td3_update_args* a) {
+  return rtd3::AdamState{h->ar, a->params, a->params_t, a->params_uv, a->adam_m, a->adam_v, a->beta_pows, {a->lr_actor, a->lr_critic}, a->tau};
+}
 

@@ -25,7 +25,7 @@ M are loose by the networks' cancellation.  TF32 operands resolve only the actor
 
 Optimiser: the Adam / Polyak kernel, element for element against oracle/td3_oracle.py's adam_step / soft_update (pinned to
 torch.optim.Adam), with lr a Python float as in torch, and the Adam step of the fused, cooperative and TF32 update paths against the
-same formula on the device's own moments.
+same formula on the device's own moments; the kernels that rebuild the derived weight copies from the whole arena against their layouts.
 """
 import numpy as np
 import pytest
@@ -284,6 +284,33 @@ def derived_copies(agent, params):
             u[o:o + H * H] = Wr.T.reshape(H // 4, 4, H).transpose(0, 2, 1).reshape(-1)
             v[o:o + H * H] = Wr.reshape(H // 4, 4, H).transpose(0, 2, 1).reshape(-1)
     return pt, np.concatenate([u, v])
+
+
+@pytest.mark.parametrize("H,L", [(64, 2), (128, 3), (32, 4)])
+def test_sync_kernels_bit_exact(pkg, H, L):
+    """The kernels that rebuild the derived copies from the whole arena (after weights were written from outside the optimiser):
+    params_t, [u | v] and the fp16 hidden weights (W_l[n][k] at ((net*(L-1) + l-1)*H*H + ((k/8)*H + n)*8 + k%8) bit-equal to their
+    layouts, for parameters of every scale, zeros and subnormals included."""
+    rs = np.random.RandomState(H + L)
+    agent = make_agent(pkg, make_nets(rs, H, L), H, L, 16)
+    params = special_grads(rs, agent.params.numel())
+    agent.params.copy_(torch.from_numpy(params))
+    agent.sync_transposed()
+    agent._sync_chunk_major()
+    agent._sync_half(force=True)
+    torch.cuda.synchronize()
+    pt, puv = derived_copies(agent, params)
+    assert np.array_equal(bits(agent.params_t.cpu().numpy()), bits(pt))
+    uv = agent.params_u.cpu().numpy()
+    assert np.array_equal(bits(uv), bits(puv)), int((uv != puv).sum())
+    ph = []
+    for k in range(6):
+        i = 2 if k % 3 == 0 else 4
+        for l in range(L - 1):
+            o = agent._off[k] + i * H + H + l * (H * H + H)
+            W = np.clip(params[o:o + H * H], -65504, 65504).astype(np.float16).reshape(H, H // 8, 8)
+            ph.append(W.transpose(1, 0, 2).reshape(-1))
+    assert np.array_equal(agent.params_h.cpu().numpy().view(np.uint16), np.concatenate(ph).view(np.uint16))
 
 
 @pytest.mark.parametrize("lr", [1e-5, 3e-4, 1e-3])
