@@ -109,6 +109,11 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
 /* Test hook: 1 forces the cp.async variant of the rollout kernel, 2 the single-warp TMA variant (instead of the
  * warp-pair TMA kernel used for latency-bound batches), 0 restores the automatic choice. */
 void rtd3_env_force_plain_rollout(int32_t on);
+/* Test hook: 0 launches every rollout kernel with a full dependency on the stream's previous work; 1 (the default) lets a
+ * rollout launch start while the previous kernel of the stream drains (programmatic dependent launch: the kernel stages its
+ * table before it waits for that kernel, and reads state and actions after).  Launches while the stream is capturing, and the
+ * first rollout launch after rtd3_env_set_map(s), always take the full dependency.  Results are the same either way. */
+void rtd3_env_set_launch_overlap(int32_t on);
 
 /* rtd3_env_rollout for HOST buffers: actions_host / traj_host are page-locked host memory [T][2][n] (same loop, robot-learning.py:97-100).
  * mode is a bit set - 1: the copy engine stages the actions in HBM, 2: the trajectory goes back through the copy engine; an

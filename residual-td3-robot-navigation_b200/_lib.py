@@ -84,6 +84,7 @@ _SIGNATURES = {
     "rtd3_env_dynamics": (c_int32, [_P, _P, _P, _P, _P, _P, _P, c_int64, _P]),
     "rtd3_env_rollout": (c_int32, [_P, _P, _P, _P, _P, c_int64, c_int64, _P]),
     "rtd3_env_force_plain_rollout": (None, [c_int32]),
+    "rtd3_env_set_launch_overlap": (None, [c_int32]),
     "rtd3_env_rollout_host": (c_int32, [_P, _P, _P, _P, _P, c_int64, c_int64, c_int32, c_int32, _P]),
     "rtd3_mt_seed": (c_int32, [POINTER(MtBankStruct), _P, _P]),
     "rtd3_mt_draw_u32": (c_int32, [POINTER(MtBankStruct), _P, c_int64, _P]),

@@ -123,6 +123,13 @@ __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.w
 template <int kN>
 __device__ __forceinline__ void bulk_wait() { asm volatile("cp.async.bulk.wait_group %0;" ::"n"(kN) : "memory"); }
 
+// Programmatic dependent launch.  launch_dependents lets the next kernel of the stream (launched with
+// cudaLaunchAttributeProgrammaticStreamSerialization) start once every CTA of this grid has issued it; grid_dep_wait blocks until
+// the grids this one depends on have completed and their memory is visible.  Both are no-ops in a grid launched without the
+// attribute.
+__device__ __forceinline__ void launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+__device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+
 // Philox4x32-10 (Salmon et al. 2011), the counter-based generator used for the non-parity index draw.
 __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
 #pragma unroll

@@ -234,13 +234,19 @@ env_rollout_kernel(int64_t n, float* __restrict__ x, float* __restrict__ y, cons
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);
   float* ring = reinterpret_cast<float*>(smem_raw + kTableBytes + 16);   // [kStages][kU][2][blockDim]
-  const int staged = bank.map<kBank>((int64_t)blockIdx.x * blockDim.x);
+  launch_dependents();                  // launch overlap as in env_rollout_pair_kernel
+  int staged = 0;
   BankLanes bl{};
+  // contains the only __syncthreads of the kernel
+  const auto stage = [&] { stage_table(s_table, bar, bank.tables + (size_t)staged * kCells); };
+  if constexpr (!kBank) stage();
+  grid_dep_wait();
   if constexpr (kBank) {
+    staged = bank.map<kBank>((int64_t)blockIdx.x * blockDim.x);
     const int64_t env = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     bl = bank_lanes(bank, staged, env, env < n);
+    stage();
   }
-  stage_table(s_table, bar, bank.tables + (size_t)staged * kCells);   // contains the only __syncthreads of the kernel
 
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;                   // thread 0 of every launched CTA is live, so the bulk copy always has an owner
@@ -334,12 +340,23 @@ __device__ __forceinline__ void tma_store_2d(const CUtensorMap* tm, int c0, int 
                : "memory");
 }
 
-// Parameter order: n first for the same reason as env_step_kernel's vec_ok.
+__device__ __forceinline__ void prefetch_tensormap(const CUtensorMap* tm) {
+  asm volatile("prefetch.tensormap [%0];" ::"l"(reinterpret_cast<uint64_t>(tm)) : "memory");
+}
+// Pulls a tile into L2 only: safe before grid_dep_wait, since L2 is where writes of the previous grid become coherent.
+__device__ __forceinline__ void tma_prefetch_l2_2d(const CUtensorMap* tm, int c0, int c1) {
+  asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];" ::"l"(reinterpret_cast<uint64_t>(tm)), "r"(c0), "r"(c1)
+               : "memory");
+}
+
+// Parameter order: n first for the same reason as env_step_kernel's vec_ok.  Launch overlap and traj_host as in
+// env_rollout_pair_kernel.
 template <bool kTraj, int kStages, bool kBank = false>
 __global__ void __launch_bounds__(256)
 env_rollout_tma_kernel(int64_t n, float* __restrict__ x, float* __restrict__ y, const __grid_constant__ CUtensorMap tm_act,
-                       const __grid_constant__ CUtensorMap tm_traj, int64_t T, MapBank bank) {
+                       const __grid_constant__ CUtensorMap tm_traj, int64_t T, MapBank bank, int traj_host) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
+  launch_dependents();
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kTableBytes);            // table barrier
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nwarps = blockDim.x >> 5;
@@ -353,13 +370,22 @@ env_rollout_tma_kernel(int64_t n, float* __restrict__ x, float* __restrict__ y, 
     for (int s = 0; s < kStages; ++s) mbar_init(full + s, 1);
     fence_mbar_init();
   }
-  const int staged = bank.map<kBank>((int64_t)blockIdx.x * nwarps * 32);
+  if (threadIdx.x == 0) {
+    prefetch_tensormap(&tm_act);
+    if (kTraj) prefetch_tensormap(&tm_traj);
+  }
+  int staged = 0;
   BankLanes bl{};
+  // init + fence + __syncthreads, then the table's bulk copies
+  const auto stage = [&] { stage_table(s_table, bar, bank.tables + (size_t)staged * kCells); };
+  if constexpr (!kBank) stage();
+  grid_dep_wait();
   if constexpr (kBank) {
+    staged = bank.map<kBank>((int64_t)blockIdx.x * nwarps * 32);
     const int64_t env = ((int64_t)blockIdx.x * nwarps + warp) * 32 + lane;
     bl = bank_lanes(bank, staged, env, env < n);
+    stage();
   }
-  stage_table(s_table, bar, bank.tables + (size_t)staged * kCells);   // init + fence + __syncthreads, then the table's bulk copies
 
   const int64_t i0 = ((int64_t)blockIdx.x * nwarps + warp) * 32;                  // first env of this warp
   if (i0 >= n) return;
@@ -439,7 +465,10 @@ env_rollout_tma_kernel(int64_t n, float* __restrict__ x, float* __restrict__ y, 
     }
   }
   if (live) { x[i] = sx; y[i] = sy; }
-  if (kTraj && lane == 0) bulk_wait<0>();       // the stores must have left shared memory before the CTA exits
+  if (kTraj && lane == 0) {                     // the stores must have left shared memory before the CTA exits
+    if (traj_host) bulk_wait<0>();
+    else bulk_wait_read<0>();
+  }
 }
 
 // ---- T-step rollout, warp-pair variant: chain warp + helper warp per 32 envs -------------------------------------------
@@ -458,11 +487,65 @@ struct PairSmem {
   static constexpr int kBars = 16;   // full[8] | prepped[2] | consumed[2] | outfull[2] | outfree[2]
 };
 
+// ---- launch phase stamps (builds with -DRTD3_ROLLOUT_STAMPS only; tools/rollout_launch_stamps.py) --------------------------------
+// Every CTA of the pair kernel takes one record of kStampWords %globaltimer values in the buffer armed by rtd3_rollout_stamps_arm.
+// Records are handed out in CTA start order; the launch a record belongs to is recovered from the start stamps (every CTA of
+// launch k starts before any CTA of launch k+1, with or without programmatic dependent launch).
+enum StampPhase {
+  kStampStart,        // CTA start
+  kStampWaited,       // grid_dep_wait returned
+  kStampTable,        // the chain warp saw the table land
+  kStampPrepped0,     // the helper prepped the first tile
+  kStampChain0,       // the chain warp starts chunk 0
+  kStampChainEnd,     // the chain warp ends the last chunk
+  kStampLastStore,    // the helper issued the last trajectory store
+  kStampHelperExit,   // the helper's last instruction
+  kStampChainExit,    // the chain warp's last instruction
+  kStampMeta,         // blockIdx.x | smid << 32
+  kStampWords
+};
+#ifdef RTD3_ROLLOUT_STAMPS
+__device__ unsigned long long* g_stamps = nullptr;
+__device__ unsigned long long g_stamp_next = 0, g_stamp_cap = 0;
+__device__ __forceinline__ unsigned long long globaltimer() {
+  unsigned long long t;
+  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+  return t;
+}
+__device__ __forceinline__ void stamp(uint32_t slot, int phase) {
+  if (g_stamps && slot < g_stamp_cap) g_stamps[(size_t)slot * kStampWords + phase] = globaltimer();
+}
+#define RTD3_STAMP_SLOT_DECL __shared__ uint32_t s_stamp_slot;
+#define RTD3_STAMP_SLOT_TAKE()                                                                                             \
+  if (threadIdx.x == 0) {                                                                                                  \
+    s_stamp_slot = (uint32_t)atomicAdd(&g_stamp_next, 1ull);                                                               \
+    stamp(s_stamp_slot, kStampStart);                                                                                      \
+    uint32_t smid;                                                                                                         \
+    asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));                                                                      \
+    if (g_stamps && s_stamp_slot < g_stamp_cap) g_stamps[(size_t)s_stamp_slot * kStampWords + kStampMeta] = blockIdx.x | (unsigned long long)smid << 32; \
+  }
+#define RTD3_STAMP(cond, phase) \
+  if (cond) stamp(s_stamp_slot, phase)
+#else
+#define RTD3_STAMP_SLOT_DECL
+#define RTD3_STAMP_SLOT_TAKE()
+#define RTD3_STAMP(cond, phase)
+#endif
+
+// Launch overlap: every CTA lets the next launch of the stream start at once, and does before grid_dep_wait only what cannot depend
+// on the grid before it - barrier inits, tensor-map and L2 prefetches, and (single map) the table staging: the host launches with
+// programmatic serialization only when the tables were not rebuilt since the previous rollout launch.  State, actions and (bank)
+// the map index are read after the wait.  traj_host: the trajectory is host memory, so the helper waits for its last store to
+// complete before exiting; for device memory the completion of the grid covers it, and the helper only waits for the store to
+// have read its shared-memory tile.
 template <bool kTraj, int kStages, int kUp, bool kBank = false>
 __global__ void __launch_bounds__(256)
 env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __grid_constant__ CUtensorMap tm_act,
-                        const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T, MapBank bank) {
+                        const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T, MapBank bank, int traj_host) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
+  RTD3_STAMP_SLOT_DECL
+  RTD3_STAMP_SLOT_TAKE()
+  launch_dependents();
   constexpr int kU = kUp;                            // steps per action / trajectory tile of this kernel (shadows the file-wide kU)
   constexpr int kTileFloats = kU * 2 * 32;
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
@@ -485,18 +568,30 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
     for (int b = 0; b < 2; ++b) { mbar_init(prepped + b, 32); mbar_init(consumed + b, 32); mbar_init(outfull + b, 32); mbar_init(outfree + b, 1); }
     fence_mbar_init();
   }
-  const int staged = bank.map<kBank>((int64_t)blockIdx.x * npairs * 32);   // the CTA stages the halo table of its first env's map
+  const int64_t i0 = ((int64_t)blockIdx.x * npairs + pair) * 32;
+  const int64_t chunks = (T + kU - 1) / kU;
+  if (lane == 0 && !is_chain) {
+    prefetch_tensormap(&tm_act);
+    if (kTraj) prefetch_tensormap(&tm_traj);
+    if (i0 < n)
+      for (int s = 0; s < kStages && s < chunks; ++s) tma_prefetch_l2_2d(&tm_act, (int)i0, s * (2 * kU));
+  }
+  int staged = 0;
   BankLanes bl{};
+  const auto stage = [&] {   // contains the __syncthreads that publishes the barrier inits
+    stage_table<kHaloBytes>(s_table, bar, bank.halos + (size_t)staged * (kHaloDim * kHaloDim));
+  };
+  if constexpr (!kBank) stage();
+  grid_dep_wait();
+  RTD3_STAMP(threadIdx.x == 0, kStampWaited);
   if constexpr (kBank) {
+    staged = bank.map<kBank>((int64_t)blockIdx.x * npairs * 32);   // the CTA stages the halo table of its first env's map
     const int64_t env = ((int64_t)blockIdx.x * npairs + pair) * 32 + lane;
     bl = bank_lanes(bank, staged, env, env < n);
+    stage();
   }
-  // contains the __syncthreads that publishes the barrier inits
-  stage_table<kHaloBytes>(s_table, bar, bank.halos + (size_t)staged * (kHaloDim * kHaloDim));
 
-  const int64_t i0 = ((int64_t)blockIdx.x * npairs + pair) * 32;
   if (i0 >= n) return;
-  const int64_t chunks = (T + kU - 1) / kU;
 
   if (!is_chain) {
     // ================================= helper warp =================================
@@ -532,6 +627,7 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
       __syncwarp();
       issue_load(c + kStages);                                       // raw stage s is in registers / prepped now
       mbar_arrive(prepped + b);
+      RTD3_STAMP(lane == 0 && c == 0, kStampPrepped0);
       if (kTraj && c >= 1) {                                         // trajectory tile of the previous chunk
         const int pb = (int)((c - 1) & 1);
         mbar_wait(outfull + pb, (uint32_t)(((c - 1) >> 1) & 1));
@@ -552,10 +648,13 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
       if (lane == 0) {
         tma_store_2d(&tm_traj, (int)i0, (int)((chunks - 1) * (2 * kU)), outt + pb * kTileFloats);
         bulk_commit();
-        bulk_wait<0>();
+        RTD3_STAMP(true, kStampLastStore);
+        if (traj_host) bulk_wait<0>();
+        else bulk_wait_read<0>();
       }
       __syncwarp();
     }
+    RTD3_STAMP(lane == 0, kStampHelperExit);
     return;
   }
 
@@ -567,9 +666,11 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
   float sy = live ? fminf(fmaxf(y[i], 0.0f), 99.99999f) : 0.0f;
   const uint32_t addr_bias = smem_u32(s_table) - 0x4B000000u * (kHaloRowBytes + 8u);
   mbar_wait(bar, 0);
+  RTD3_STAMP(lane == 0, kStampTable);
   for (int64_t c = 0; c < chunks; ++c) {
     const int b = (int)(c & 1);
     mbar_wait(prepped + b, (uint32_t)((c >> 1) & 1));
+    RTD3_STAMP(lane == 0 && c == 0, kStampChain0);
     if (kTraj && c >= 2) mbar_wait(outfree + b, (uint32_t)(((c >> 1) - 1) & 1));   // out tile b has been stored (chunk c-2)
     const bool careful = s_flag[pair][b] != 0;
     const uint32_t tp = smem_u32(prep + b * (kU * 32) + lane);
@@ -626,7 +727,9 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
     mbar_arrive(consumed + b);
     if (kTraj) mbar_arrive(outfull + b);
   }
+  RTD3_STAMP(lane == 0, kStampChainEnd);
   if (live) { x[i] = sx; y[i] = sy; }
+  RTD3_STAMP(lane == 0, kStampChainExit);
 }
 
 // ---- seeded init / reset on per-env legacy MT19937 streams ------------------------------------
@@ -747,6 +850,7 @@ using namespace rtd3;
 
 constexpr int kMaxMaps = 65536;
 static int g_rollout_hook = 0;   // rtd3_env_force_plain_rollout: 1 = the cp.async kernel, 2 = the single-warp TMA kernel for every size
+static bool g_launch_overlap = true;   // rtd3_env_set_launch_overlap
 
 // Every kernel instantiation a launch can pick.  The launches index these tables, and rtd3_env_create sets the shared-memory
 // limit of every entry.
@@ -775,6 +879,23 @@ static const PairKernel kPairKernels[2][2][2] = {
      {env_rollout_pair_kernel<true, kPairStages, kPairU>, env_rollout_pair_kernel<true, kPairStages2, kPairU>}},
     {{env_rollout_pair_kernel<false, kPairStages, kPairU, true>, env_rollout_pair_kernel<false, kPairStages2, kPairU, true>},
      {env_rollout_pair_kernel<true, kPairStages, kPairU, true>, env_rollout_pair_kernel<true, kPairStages2, kPairU, true>}}};
+
+// A rollout launch; with `overlap` it may start while the stream's previous kernel drains (programmatic dependent launch, see
+// env_rollout_pair_kernel).
+template <typename... KArgs, typename... Args>
+static cudaError_t launch_rollout(void (*kernel)(KArgs...), int grid, int block, int smem, cudaStream_t st, bool overlap, Args&&... args) {
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr.val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(block);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cfg.attrs = &attr;
+  cfg.numAttrs = overlap ? 1 : 0;
+  return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
+}
 
 template <typename... Args>
 static cudaError_t set_max_smem(void (*kernel)(Args...), int bytes) {
@@ -838,6 +959,7 @@ static int32_t alloc_bank(rtd3_env* h, int cap) {
 extern "C" {
 
 void rtd3_env_force_plain_rollout(int32_t on) { g_rollout_hook = on == 1 || on == 2 ? on : 0; }
+void rtd3_env_set_launch_overlap(int32_t on) { g_launch_overlap = on != 0; }
 
 int32_t rtd3_env_create(rtd3_env** out, int32_t device) {
   RTD3_CHECK_ARG(out, "out is null");
@@ -882,6 +1004,7 @@ int32_t rtd3_env_set_maps(rtd3_env* h, const float* speed, const float* angle, i
   build_halo_kernel<<<K, 1024, 0, (cudaStream_t)stream>>>(h->tables, h->halos, h->fits);
   RTD3_LAUNCHED();
   h->num_maps = K;
+  h->maps_rebuilt = true;
   return 0;
 }
 
@@ -961,6 +1084,20 @@ int32_t rtd3_env_dynamics(rtd3_env* h, const float* x, const float* y, const flo
 
 int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, float* traj, int64_t n, int64_t T,
                          void* stream) {
+  // a trajectory in host (or managed) memory: the kernel waits for its writes to complete before exiting
+  bool traj_host = false;
+  if (traj) {
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, traj) != cudaSuccess) cudaGetLastError();
+    else traj_host = a.type != cudaMemoryTypeDevice;
+  }
+  return env_rollout(h, x, y, actions, traj, n, T, traj_host, (cudaStream_t)stream);
+}
+
+}  // extern "C"
+
+int32_t rtd3::env_rollout(rtd3_env* h, float* x, float* y, const float* actions, float* traj, int64_t n, int64_t T, bool traj_host,
+                          cudaStream_t st) {
   RTD3_CHECK_ARG(h && h->num_maps > 0, "environment has no dynamics map (call rtd3_env_set_map)");
   RTD3_CHECK_ARG(n >= 0 && T >= 0, "negative n or T");
   if (n == 0 || T == 0) return 0;
@@ -971,7 +1108,17 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
   const int64_t per_sm = ceil_div(n, (int64_t)h->num_sms);
   const bool deep = per_sm <= 64;
   const int stages = deep ? kDeep : kShallow;
-  cudaStream_t st = (cudaStream_t)stream;
+  // Launch overlap (see env_rollout_pair_kernel) needs the tables unchanged since the previous rollout launch.  A captured launch
+  // runs without it (a graph may replay a table rebuild or be launched after any work), and leaves the flag set for the next one.
+  cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &cap) != cudaSuccess) {
+    cudaGetLastError();
+    cap = cudaStreamCaptureStatusActive;
+  }
+  const bool capturing = cap != cudaStreamCaptureStatusNone;
+  const bool overlap = g_launch_overlap && !h->maps_rebuilt && !capturing;
+  h->maps_rebuilt = capturing;
+  const int th = traj_host ? 1 : 0;
   const MapBank bank = map_bank(h);   // bank.index == nullptr: the single-map kernels
   const bool with_bank = bank.index != nullptr, with_traj = traj != nullptr;
   // latency-bound batches run the warp-pair kernel, with tiles of kPairU steps (the per-tile hand-over - two barrier waits, the
@@ -991,13 +1138,13 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
       const int pstages = ppc == 1 ? kPairStages : kPairStages2;
       const int psmem = ((kHaloBytes + 16 + ppc * PairSmem::kBars * 8 + 127) & ~127) + ppc * (pstages + 4) * (kPairU * 2 * 32) * 4;
       const PairKernel kern = kPairKernels[with_bank][with_traj][ppc == 2];
-      kern<<<(int)ceil_div(warps_total, ppc), ppc * 64, psmem, st>>>(x, y, tm_act, tm_traj, n, T, bank);
+      RTD3_CUDA(launch_rollout(kern, (int)ceil_div(warps_total, ppc), ppc * 64, psmem, st, overlap, x, y, tm_act, tm_traj, n, T, bank, th));
     } else {
       // one warp per 32 envs; few warps per CTA while the batch cannot fill the SMs, 8 once it can
       const int wpc = deep ? (int)std::max<int64_t>(1, std::min<int64_t>(8, ceil_div(warps_total, (int64_t)h->num_sms))) : 8;
       const int bsmem = ((kTableBytes + 16 + wpc * stages * 8 + 127) & ~127) + wpc * (stages + 2) * kTileFloats * 4;
       const TmaKernel kern = kTmaKernels[with_bank][with_traj][deep];
-      kern<<<(int)ceil_div(warps_total, wpc), wpc * 32, bsmem, st>>>(n, x, y, tm_act, tm_traj, T, bank);
+      RTD3_CUDA(launch_rollout(kern, (int)ceil_div(warps_total, wpc), wpc * 32, bsmem, st, overlap, n, x, y, tm_act, tm_traj, T, bank, th));
     }
     RTD3_LAUNCHED();
     return 0;
@@ -1005,10 +1152,12 @@ int32_t rtd3_env_rollout(rtd3_env* h, float* x, float* y, const float* actions, 
   const int block = deep ? (int)std::max<int64_t>(32, ceil_div(per_sm, 32) * 32) : 128;
   const int smem = kTableBytes + 16 + stages * kU * 2 * block * 4;
   const RolloutKernel kern = kRolloutKernels[with_bank][with_traj][deep];
-  kern<<<(int)ceil_div(n, block), block, smem, st>>>(n, x, y, actions, traj, T, bank);
+  RTD3_CUDA(launch_rollout(kern, (int)ceil_div(n, block), block, smem, st, overlap, n, x, y, actions, traj, T, bank));
   RTD3_LAUNCHED();
   return 0;
 }
+
+extern "C" {
 
 int32_t rtd3_mt_seed(const rtd3_mt_bank* bank, const uint32_t* seeds, void* stream) {
   if (int32_t e = check_bank(bank)) return e;
@@ -1059,5 +1208,19 @@ int32_t rtd3_env_reset(const rtd3_mt_bank* bank, const double* region, const uin
   RTD3_LAUNCHED();
   return 0;
 }
+
+#ifdef RTD3_ROLLOUT_STAMPS
+// Arms the phase stamps of env_rollout_pair_kernel: records go to buf [cap][kStampWords] (device memory, zeroed by the caller) in
+// CTA start order.  Not part of the ABI: only the stamped build exports it.
+int32_t rtd3_rollout_stamps_arm(void* buf, int64_t cap) {
+  unsigned long long* p = (unsigned long long*)buf;
+  const unsigned long long zero = 0, c = (unsigned long long)cap;
+  RTD3_CUDA(cudaMemcpyToSymbol(g_stamps, &p, sizeof(p)));
+  RTD3_CUDA(cudaMemcpyToSymbol(g_stamp_next, &zero, sizeof(zero)));
+  RTD3_CUDA(cudaMemcpyToSymbol(g_stamp_cap, &c, sizeof(c)));
+  return 0;
+}
+int32_t rtd3_rollout_stamp_words() { return kStampWords; }
+#endif
 
 }  // extern "C"

@@ -116,7 +116,7 @@ static int32_t issue_pipeline(rtd3_env* h, HostPipe* p, float* x, float* y, cons
     if (stage_in) RTD3_CUDA(cudaStreamWaitEvent(p->cap, in_done[c], 0));
     const float* src = (stage_in ? p->d_act : act) + t0 * plane;
     float* dst = (stage_out ? p->d_traj : traj) + t0 * plane;
-    if (int32_t e = rtd3_env_rollout(h, x, y, src, dst, n, len, (void*)p->cap)) return e;
+    if (int32_t e = env_rollout(h, x, y, src, dst, n, len, !stage_out, p->cap)) return e;
     if (stage_out) {
       cudaEvent_t k = ev[e_next++];
       RTD3_CUDA(cudaEventRecord(k, p->cap));
@@ -154,7 +154,7 @@ extern "C" int32_t rtd3_env_rollout_host(rtd3_env* h, float* x, float* y, const 
   RTD3_CHECK_ARG(x && y && actions_host && traj_host, "null state / action / trajectory pointer");
   RTD3_CHECK_ARG(is_pinned(actions_host) && is_pinned(traj_host), "actions_host and traj_host must be page-locked host memory");
   if (mode == 0)                     // zero copy: the kernel's TMA tiles cross PCIe themselves
-    return rtd3_env_rollout(h, x, y, actions_host, traj_host, n, T, stream);
+    return env_rollout(h, x, y, actions_host, traj_host, n, T, true, (cudaStream_t)stream);
   chunks = (int32_t)std::max<int64_t>(1, std::min<int64_t>(chunks, std::min<int64_t>(T, 256)));
   const bool stage_in = mode & 1, stage_out = mode & 2;
   DeviceGuard guard;

@@ -17,12 +17,18 @@ struct rtd3_env {
   int num_maps = 0, map_cap = 0;
   int32_t* index = nullptr;
   int64_t index_len = 0, index_cap = 0;
+  // The tables were rebuilt (rtd3_env_set_maps) since the last rollout launch, or may be by a replayed graph: the next rollout
+  // launch waits for the whole previous grid, since its table staging could otherwise read the tables before they are written.
+  bool maps_rebuilt = true;
 };
 
 namespace rtd3 {
 
 void host_pipe_destroy(rtd3_env* h);   // rtd3_env_host.cu: streams, staging buffers and cached graphs of the host-buffer rollout
 void host_pipe_drop_graphs(rtd3_env* h);   // rtd3_env_host.cu: the cached graphs only (they hold the bank / index addresses)
+// rtd3_env_rollout (rtd3_env.cu) with traj_host: the trajectory is host memory, whose writes the kernel waits for before it exits
+int32_t env_rollout(rtd3_env* h, float* x, float* y, const float* actions, float* traj, int64_t n, int64_t T, bool traj_host,
+                    cudaStream_t st);
 
 // What a kernel needs to step env v on its own map.  Passed by value; index == nullptr (single map) in the launches without a bank.
 struct MapBank {
