@@ -83,6 +83,23 @@ int32_t rtd3_env_set_map(rtd3_env* h, const float* speed, const float* angle, vo
  * 256 above. */
 int32_t rtd3_env_set_maps(rtd3_env* h, const float* speed, const float* angle, int32_t K, void* stream);
 int32_t rtd3_env_set_map_index(rtd3_env* h, const int32_t* index, int64_t m, void* stream);
+
+/* Environment.set_dynamics (environment.py:59-95) for K seeds: map k of speed / angle (DEVICE float32 [K][100*100], [x][y])
+ * is perlin_maps(seeds[k]) (environment.py of this package) under the exactness rules below.  seeds: DEVICE int64 [K],
+ * each in [0, 2^63).  Asynchronous on `stream`, no allocation, no synchronisation, capturable.  K in [1, 65536].
+ * Exactness:
+ *   - the float32 fields before normalisation (n(5) + 0.5 n(10) + 0.25 n(20) for speed, n(5) for angle, each float64 sum
+ *     rounded once to float32) are bit-identical to perlin_maps's;
+ *   - angle, their float32 min-max normalisation (c - min) / (max - min), is bit-identical to perlin_maps's;
+ *   - speed = 1 / (1 + exp(-10 * (norm - 0.5))) in numpy's float32 operation order, except that exp is evaluated in float64
+ *     and rounded once to float32.  numpy's float32 exp is a SIMD routine picked by the host CPU and not correctly rounded, so
+ *     speed can differ from perlin_maps's by a few ulp (up to 4 measured); it is the same on every host.
+ * A flat field (max == min) gives NaN cells, as in numpy; rtd3_env_set_maps makes them dead cells.  Hand the maps to
+ * rtd3_env_set_maps on the same stream to install them without a host round trip. */
+int32_t rtd3_perlin_maps(const int64_t* seeds, int32_t K, float* speed, float* angle, void* stream);
+/* Test hook: 1 makes rtd3_perlin_maps write the float32 fields before normalisation instead of the maps, 0 (the default)
+ * restores the maps. */
+void rtd3_perlin_set_raw_fields(int32_t on);
 /* The map configuration launches capture as kernel arguments: bank address, index address (NULL without an index), K, m.
  * A caller that captures launches into a CUDA graph compares these to decide whether to recapture.  Any output may be NULL. */
 int32_t rtd3_env_map_config(const rtd3_env* h, const void** tables, const void** index, int32_t* num_maps, int64_t* index_len);

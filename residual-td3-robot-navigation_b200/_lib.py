@@ -79,6 +79,8 @@ _SIGNATURES = {
     "rtd3_env_set_map": (c_int32, [_P, _P, _P, _P]),
     "rtd3_env_set_maps": (c_int32, [_P, _P, _P, c_int32, _P]),
     "rtd3_env_set_map_index": (c_int32, [_P, _P, c_int64, _P]),
+    "rtd3_perlin_maps": (c_int32, [_P, c_int32, _P, _P, _P]),
+    "rtd3_perlin_set_raw_fields": (None, [c_int32]),
     "rtd3_env_map_config": (c_int32, [_P, POINTER(c_void_p), POINTER(c_void_p), POINTER(c_int32), POINTER(c_int64)]),
     "rtd3_env_step": (c_int32, [_P, _P, _P, _P, _P, c_int64, c_int32, _P]),
     "rtd3_env_dynamics": (c_int32, [_P, _P, _P, _P, _P, _P, _P, c_int64, _P]),

@@ -69,6 +69,7 @@ constexpr float kMaxAction = 5.0f;                 // constants.py:34
 constexpr float kClipHi = 98.9999f;                // float32(WORLD_SIZE - 1.0001), environment.py:117
 constexpr int kWorld = RTD3_WORLD_SIZE;
 constexpr int kCells = RTD3_MAP_CELLS;
+constexpr int kMaxMaps = 65536;                  // maps of a bank (rtd3_env_set_maps) and of one rtd3_perlin_maps call
 
 static inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 

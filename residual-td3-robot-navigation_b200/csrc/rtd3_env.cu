@@ -848,7 +848,6 @@ static int32_t check_bank(const rtd3_mt_bank* b) {
 
 using namespace rtd3;
 
-constexpr int kMaxMaps = 65536;
 static int g_rollout_hook = 0;   // rtd3_env_force_plain_rollout: 1 = the cp.async kernel, 2 = the single-warp TMA kernel for every size
 static bool g_launch_overlap = true;   // rtd3_env_set_launch_overlap
 

@@ -10,6 +10,7 @@ seed is given, draw from numpy's *global* legacy MT19937 stream exactly as the r
 
 Beyond the reference, the envs of one `Environment` can step on different maps (domain randomisation): `maps` / `set_maps` take a
 bank of K maps `[K,100,100]` and `map_index` / `set_map_index` say which map each env uses (`num_maps`, `map_index`).
+`map_seeds` / `set_perlin_maps` build such a bank of the reference's own Perlin maps, one per seed, on the device.
 
 All arithmetic happens in csrc/librtd3.so (hand-written sm_100a kernels); there is no CPU path.
 """
@@ -106,6 +107,55 @@ def perlin_maps(seed=None):
     return s.copy(), a.copy()
 
 
+def _checked_seeds(seeds):
+    """Seeds of `perlin_maps_device` / `set_perlin_maps` -> int64 CPU tensor `[K]`: a list, a numpy array or an integer tensor on any
+    device, 1-D, 1 <= K <= 65536, every value in [0, 2^63); ValueError otherwise.  A CUDA tensor is read back once."""
+    if isinstance(seeds, torch.Tensor):
+        if seeds.dtype.is_floating_point or seeds.dtype.is_complex or seeds.dtype == torch.bool:
+            raise ValueError("map seeds must have an integer dtype, got %s" % seeds.dtype)
+        t = seeds.detach().to("cpu")
+    else:
+        try:
+            a = np.asarray(seeds)
+        except (OverflowError, ValueError, TypeError) as e:
+            raise ValueError("map seeds must be integers in [0, 2^63): %s" % e)
+        if a.dtype.kind not in "iu":
+            raise ValueError("map seeds must have an integer dtype, got %s" % a.dtype)
+        if a.dtype.kind == "u" and a.size and int(a.max()) >= 2 ** 63:
+            raise ValueError("map seeds must lie in [0, 2^63)")
+        t = torch.from_numpy(a.astype(np.int64))
+    if t.dim() != 1 or not 1 <= t.shape[0] <= 65536:
+        raise ValueError("map seeds must have shape [K] with 1 <= K <= 65536, got %s" % list(t.shape))
+    t = t.to(torch.int64)
+    if int(t.min()) < 0:
+        raise ValueError("map seeds must lie in [0, 2^63), got %d" % int(t.min()))
+    return t.clone()
+
+
+def _perlin_maps_device(seeds, device):
+    """`rtd3_perlin_maps` for checked int64 CPU seeds `[K]` -> (speed, angle) float32 `[K,100,100]` on `device`."""
+    W = constants.WORLD_SIZE
+    K = seeds.shape[0]
+    with torch.cuda.device(device):
+        dev_seeds = seeds.to(device)
+        speed = torch.empty((K, W, W), dtype=torch.float32, device=device)
+        angle = torch.empty((K, W, W), dtype=torch.float32, device=device)
+        _lib.check(_lib.lib().rtd3_perlin_maps(_lib.ptr(dev_seeds), K, _lib.ptr(speed), _lib.ptr(angle), _lib.stream_ptr(device)),
+                   "perlin_maps")
+    return speed, angle
+
+
+def perlin_maps_device(seeds, device=None):
+    """`perlin_maps` for K seeds at once, on the GPU -> (speed, angle) CUDA float32 `[K,100,100]`, map k from `seeds[k]`.
+    `seeds`: a list, a numpy array or an integer tensor, 1-D, 1 <= K <= 65536, values in [0, 2^63) (ValueError otherwise).
+    `device`: the seeds' CUDA device, else the current one.  `angle` and the fields before normalisation are bit-identical to
+    `perlin_maps`; `speed` evaluates exp in float64 rounded once to float32, where numpy uses its host-dependent float32 exp, and
+    so differs from `perlin_maps` by a few ulp (include/rtd3.h, rtd3_perlin_maps)."""
+    if device is None:
+        device = seeds.device if isinstance(seeds, torch.Tensor) and seeds.is_cuda else torch.cuda.current_device()
+    return _perlin_maps_device(_checked_seeds(seeds), torch.device(device))
+
+
 def _planes(t, n, name):
     """[N,2] (any strides) or [2,N] CUDA float32 -> contiguous [2,N] planes; zero-copy when already plane-backed."""
     if t.dim() != 2:
@@ -120,9 +170,12 @@ def _planes(t, n, name):
 
 
 class Environment:
-    def __init__(self, num_envs=1, device=None, seed=None, maps=None, map_index=None):
+    def __init__(self, num_envs=1, device=None, seed=None, maps=None, map_index=None, map_seeds=None):
         """`maps`: (speed, angle), each `[100,100]` or a bank `[K,100,100]`; None builds the reference's Perlin maps.
+        `map_seeds`: instead of `maps`, a bank of the reference's Perlin maps, one per seed, built on the device (`set_perlin_maps`).
         `map_index`: int `[num_envs]`, the map of every env (see `set_maps`)."""
+        if maps is not None and map_seeds is not None:
+            raise ValueError("pass maps or map_seeds, not both")
         if not torch.cuda.is_available():
             raise RuntimeError("Environment needs a CUDA device (B200); there is no CPU path")
         self.num_envs = int(num_envs)
@@ -144,9 +197,12 @@ class Environment:
         self._pipe = None
         self._pipe_buf = None
         self._map_index = None
+        self._map_seeds = None
         self.num_maps = 1
         self.set_init_and_goal()
-        if maps is None:
+        if map_seeds is not None:
+            self.set_perlin_maps(map_seeds, index=map_index)
+        elif maps is None:
             self.set_dynamics()
             if map_index is not None:
                 self.set_map_index(map_index)
@@ -223,13 +279,35 @@ class Environment:
         angle = torch.as_tensor(np.asarray(angle.cpu() if isinstance(angle, torch.Tensor) else angle, dtype=np.float32))
         if speed.shape != angle.shape or speed.dim() not in (2, 3) or tuple(speed.shape[-2:]) != (W, W) or speed.numel() == 0:
             raise ValueError("maps must be [%d,%d] or [K,%d,%d], speed and angle alike" % (W, W, W, W))
+        self._install_maps(speed, angle, index)
+
+    def set_perlin_maps(self, seeds, index=None):
+        """`set_maps` with the bank `perlin_maps_device(seeds)`: map k is the reference's Perlin map of `seeds[k]`, generated on the
+        device and handed to the library there; only `dynamics_speed` / `dynamics_angle` take one device-to-host copy.  `seeds`: a
+        list, a numpy array or an integer tensor, 1-D, 1 <= K <= 65536, values in [0, 2^63) (ValueError otherwise); `index` as in
+        `set_maps`.  `map_seeds` holds the seeds until maps are next set another way."""
+        seeds = _checked_seeds(seeds)
+        self._install_maps(*_perlin_maps_device(seeds, self.device), index, seeds=seeds)
+
+    @property
+    def map_seeds(self):
+        """int64 `[K]` CPU tensor (a copy) of the seeds the maps were generated from, or None for maps from `maps=`, `set_maps` or
+        `set_dynamics`."""
+        return None if self._map_seeds is None else self._map_seeds.clone()
+
+    def _install_maps(self, speed, angle, index, seeds=None):
+        """Installs float32 maps `[100,100]` or `[K,100,100]` (checked by the caller): CPU tensors are uploaded, CUDA tensors on this
+        device go to the library as they are.  Nothing changes when `index` is rejected."""
         K = 1 if speed.dim() == 2 else int(speed.shape[0])
         if speed.dim() == 3 and index is None and K > 1:
             n = self.num_envs
             index = torch.arange(n, dtype=torch.int64) * K // n
         idx = None if index is None else self._checked_index(index, K)
-        self.dynamics_speed = (speed[0] if K == 1 and speed.dim() == 3 else speed).numpy().copy()
-        self.dynamics_angle = (angle[0] if K == 1 and angle.dim() == 3 else angle).numpy().copy()
+        def host(t):                                       # the numpy attribute: [100,100] for a single map
+            t = t[0] if K == 1 and t.dim() == 3 else t
+            return t.cpu().numpy() if t.is_cuda else t.numpy().copy()
+        self.dynamics_speed = host(speed)
+        self.dynamics_angle = host(angle)
         self._speed_dev = speed.contiguous().to(self.device)
         self._angle_dev = angle.contiguous().to(self.device)
         if speed.dim() == 2:
@@ -239,6 +317,7 @@ class Environment:
             _lib.check(_lib.lib().rtd3_env_set_maps(self._handle, _lib.ptr(self._speed_dev), _lib.ptr(self._angle_dev), K,
                                                     _lib.stream_ptr(self.device)), "env_set_maps")
         self.num_maps = K
+        self._map_seeds = seeds
         self._set_index(idx)
 
     def set_map_index(self, index):
