@@ -603,6 +603,31 @@ int32_t rtd3_tick_run_f16(rtd3_env* h, const rtd3_tick_state* t, int32_t hidden,
                           const uint16_t* params_h, int32_t noise_mode, int64_t ticks, uint64_t tick_base, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
+ * Batched policy evaluation: the test phase of robot-learning.py:104-117 for n envs
+ * For t = 1..T: base = state - goal, residual = actor(base), action = clip(base + residual, +-5) (get_next_action_testing,
+ * robot.py:572-595), state = Environment.step(action) on env i's map of `h` (map index[i % m]), d = |state - goal| (float64, as
+ * np.linalg.norm).  best = min(best, d); d <= 5 (constants.py:50): success, the env stops with steps = t; t == T: it stops with
+ * steps = T.  A stopped env keeps its state.  goal [2][n] float64; x, y [n] float32: the start state in, the final state out;
+ * success uint8 [n], steps int32 [n], best float64 [n].  traj: [T][2][n] float32, row t-1 = the state after step t, the rows
+ * after an env's stop repeat its final state; given exactly when `record` is set.  Both entry points check every argument
+ * before any launch, are asynchronous on `stream`, allocate nothing and can be captured.  n < 2^31, 1 <= T < 2^30.
+ * ---------------------------------------------------------------------------------------------- */
+
+/* One step for every env that has not stopped (!success[i] && steps[i] < T), given residual [n][2] = actor(base) from any forward;
+ * writes the next step's actor input to base [n][2].  Before the first step the caller sets success = 0, steps = 0, best = +inf
+ * and base = state - goal (rtd3_robot_baseline), then calls a forward and this function T times. */
+int32_t rtd3_eval_step(rtd3_env* h, const double* goal, float* x, float* y, const float* residual, float* base, uint8_t* success,
+                       int32_t* steps, double* best, float* traj, int32_t record, int64_t n, int64_t T, void* stream);
+
+/* The whole evaluation in ONE launch, the actor (network 0 of the arena, 2 -> hidden -> hidden -> 2) evaluated in the kernel by
+ * the f16 resident-weight forward (params_h from rtd3_tc_sync_weights_f16); writes success, steps and best itself.  CTAs take
+ * 128-env tiles from the device word `work` (DEVICE uint32 [1], reset on `stream` by this call) and a tile ends when all of its
+ * envs have stopped.  Bit-identical to T rounds of rtd3_mlp_forward_f16 + rtd3_eval_step.  layers == 2, hidden % 32 == 0, 64..256. */
+int32_t rtd3_eval_run_f16(rtd3_env* h, int32_t hidden, int32_t layers, const float* params, const uint16_t* params_h, const double* goal,
+                          float* x, float* y, uint8_t* success, int32_t* steps, double* best, float* traj, int32_t record, int64_t n,
+                          int64_t T, uint32_t* work, void* stream);
+
+/* ------------------------------------------------------------------------------------------------
  * Tensor-core (tcgen05 / TMEM, TF32) large-batch forward - opt-in throughput mode, not the parity path
  * ---------------------------------------------------------------------------------------------- */
 

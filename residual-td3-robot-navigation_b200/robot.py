@@ -37,6 +37,11 @@ ACTION_TYPES = ("step", "demo", "reset")
 DEMO_GRID, DEMO_CELL = 100, 1.0         # RTD3_DEMO_GRID / RTD3_DEMO_CELL of include/rtd3.h
 ENV_DEMO_CELLS = 625                    # RTD3_ENV_DEMO_CELLS
 
+EVAL_MAX_STEPS = 1 << 30                # rtd3_eval_step / rtd3_eval_run_f16 take 1 <= T < 2^30
+EVAL_BLOCK_STEPS = 64                   # test steps per captured graph of the per-step evaluation
+EVAL_CHECK_BLOCKS = True                # per-step evaluation: read "some env still runs" after each block and end early when none does
+EVAL_GRAPHS_KEPT = 4                    # captured evaluation graphs kept per Robot (one per signature)
+
 
 class PathToDraw:
     """graphics.py:22-30 (pure Python there as well); kept so that `robot.paths_to_draw` has the reference's shape."""
@@ -121,6 +126,9 @@ class Robot:
         # one.  The default N keeps the reference's rhythm (every env finishes about one episode between updates) and is
         # exactly the reference for the single-env drop-in (robot.py:480-483).
         self.episodes_per_update = self.num_envs
+        self.eval_kernel = True                                 # evaluate() may use rtd3_eval_run_f16 (False: the per-step path)
+        self._eval_graphs = {}
+        self._eval_work = None
 
     # ---- reference attributes (single-env views of the device state) --------------------------------------------
     def _scalar(self, t):
@@ -274,6 +282,98 @@ class Robot:
         x = torch.as_tensor(np.asarray(state, dtype=np.float32).reshape(-1, 2)).to(self.device) if not isinstance(state, torch.Tensor) else state
         out = self.td3_agent.forward(NET_ACTOR, x)
         return out if self.batched else out[0].cpu().numpy()
+
+    # ---- robot-learning.py:104-117: the test phase, batched ------------------------------------------------------------
+    def evaluate(self, environment, max_steps=None, record=False):
+        """The reference's test phase for every env i of `environment` (any size and map configuration), with this Robot's
+        current actor.  From env i's current state (call `environment.reset()` first for the reference's start), for
+        t = 1 .. T (T = `max_steps`, default TEST_TIMEOUT x UPDATE_RATE = 1000): action = get_next_action_testing (no noise)
+        against the ENVIRONMENT's goal, step on env i's map, d = |state - goal|; the env stops with success when d <= 5, or at
+        t == T.  Returns a dict of CUDA tensors: "success" bool `[N]`, "steps" int32 `[N]` (the step it stopped at),
+        "best_distance" float64 `[N]` (smallest d seen) and, with `record`, "trajectory" `[T,N,2]` (a view of `[T,2,N]` planes;
+        the rows after an env's stop repeat its final state).  `environment.robot_state` ends at the final states; nothing of
+        the Robot changes (only derived weight copies are refreshed, as by any forward).
+
+        With the f16 forward (`precision="f16"`, 2 x H) the whole evaluation is one launch (`rtd3_eval_run_f16`); otherwise each
+        step is the actor forward the learner's precision selects for N rows plus `rtd3_eval_step`, replayed from CUDA graphs
+        of EVAL_BLOCK_STEPS steps.  Both paths give bit-identical results for the same forward."""
+        if max_steps is None:
+            T = int(round(constants.TEST_TIMEOUT * constants.UPDATE_RATE))
+        else:
+            if isinstance(max_steps, bool) or not isinstance(max_steps, (int, np.integer)) or not 1 <= int(max_steps) < EVAL_MAX_STEPS:
+                raise ValueError("max_steps must be an integer in [1, 2^30), got %r" % (max_steps,))
+            T = int(max_steps)
+        if torch.device(environment.device) != self.device:
+            raise ValueError("environment is on %s, the robot on %s" % (environment.device, self.device))
+        n = environment.num_envs
+        agent = self.td3_agent
+        agent.prepare_forward(n)
+        dev = self.device
+        success = torch.zeros(n, dtype=torch.bool, device=dev)
+        steps = torch.zeros(n, dtype=torch.int32, device=dev)
+        best = torch.full((n,), float("inf"), dtype=torch.float64, device=dev)
+        traj = torch.empty((T, 2, n), dtype=torch.float32, device=dev) if record else None
+        if n > 0:
+            if self.eval_kernel and agent._f16_ok(n):
+                if self._eval_work is None:
+                    self._eval_work = torch.zeros(1, dtype=torch.int32, device=dev)
+                _lib.check(_lib.lib().rtd3_eval_run_f16(
+                    environment._handle, agent.hidden, agent.layers, _lib.ptr(agent.params), _lib.ptr(agent.params_h), _lib.ptr(environment._goal),
+                    _lib.ptr(environment._state[0]), _lib.ptr(environment._state[1]), _lib.ptr(success), _lib.ptr(steps), _lib.ptr(best),
+                    _lib.ptr(traj), 1 if record else 0, n, T, _lib.ptr(self._eval_work), _lib.stream_ptr(dev)), "eval_run_f16")
+            else:
+                self._evaluate_steps(environment, T, traj, success, steps, best)
+        environment._state_np = None
+        out = {"success": success, "steps": steps, "best_distance": best}
+        if record:
+            out["trajectory"] = traj.permute(0, 2, 1)
+        return out
+
+    def _evaluate_steps(self, environment, T, traj, success, steps, best):
+        """The per-step evaluation: the test steps in blocks of S, each block one replay of a captured graph of S (forward,
+        `rtd3_eval_step`) pairs.  Envs that have stopped are left alone by the kernel, so the last block may run past T; S is
+        chosen so that it runs fewer extra forwards than there are blocks."""
+        agent, n, dev = self.td3_agent, environment.num_envs, self.device
+        blocks = -(-T // EVAL_BLOCK_STEPS)
+        S = -(-T // blocks)
+        p = lambda t: None if t is None else t.data_ptr()
+        fwd = p(agent.params_h) if agent._f16_ok(n) else (p(agent.params_u) if agent._tc_ok(n) else p(agent.params_t))
+        sig = (environment._handle.value, n, S, T, agent.precision, p(agent.params), fwd, environment._map_config(), p(environment._state),
+               p(environment._goal), p(traj))
+        st = self._eval_graphs.get(sig)
+        if st is None:
+            if len(self._eval_graphs) >= EVAL_GRAPHS_KEPT:
+                self._eval_graphs.pop(next(iter(self._eval_graphs)))
+            st = {"base": torch.zeros((n, 2), dtype=torch.float32, device=dev), "success": torch.zeros(n, dtype=torch.uint8, device=dev),
+                  "steps": torch.zeros(n, dtype=torch.int32, device=dev), "best": torch.zeros(n, dtype=torch.float64, device=dev)}
+            L, x, y = _lib.lib(), environment._state[0], environment._state[1]
+
+            def step():
+                residual = agent.forward(NET_ACTOR, st["base"])
+                _lib.check(L.rtd3_eval_step(environment._handle, _lib.ptr(environment._goal), _lib.ptr(x), _lib.ptr(y), _lib.ptr(residual),
+                                            _lib.ptr(st["base"]), _lib.ptr(st["success"]), _lib.ptr(st["steps"]), _lib.ptr(st["best"]),
+                                            _lib.ptr(traj), 0 if traj is None else 1, n, T, _lib.stream_ptr(dev)), "eval_step")
+            graph = torch.cuda.CUDAGraph()
+            before = _lib.launch_count()
+            with _lib.capture(graph):
+                for _ in range(S):
+                    step()
+            st["graph"], st["launches"] = graph, _lib.launch_count() - before
+            _lib.lib().rtd3_launch_count_add(-st["launches"])
+            self._eval_graphs[sig] = st
+        st["success"].zero_()
+        st["steps"].zero_()
+        st["best"].fill_(float("inf"))
+        _lib.check(_lib.lib().rtd3_robot_baseline(_lib.ptr(environment._state[0]), _lib.ptr(environment._state[1]), _lib.ptr(environment._goal),
+                                                  _lib.ptr(st["base"]), n, _lib.stream_ptr(dev)), "robot_baseline")
+        for b in range(blocks):
+            st["graph"].replay()
+            _lib.lib().rtd3_launch_count_add(st["launches"])
+            if EVAL_CHECK_BLOCKS and b + 1 < blocks and not bool(((st["steps"] < T) & (st["success"] == 0)).any()):
+                break
+        success.copy_(st["success"])
+        steps.copy_(st["steps"])
+        best.copy_(st["best"])
 
     # ---- robot.py:645-675 ------------------------------------------------------------------------------------------
     def process_transition(self, state, action, next_state, money_remaining, push=True, types=None):
