@@ -627,6 +627,28 @@ int32_t rtd3_eval_run_f16(rtd3_env* h, int32_t hidden, int32_t layers, const flo
                           float* x, float* y, uint8_t* success, int32_t* steps, double* best, float* traj, int32_t record, int64_t n,
                           int64_t T, uint32_t* work, void* stream);
 
+/* E test episodes of every env, each from one of the env's own reset draws: bit-identical to E rounds of (rtd3_env_reset, the
+ * evaluation above).  Episode e of env i starts from the (e+1)-th draw of stream i, steps on env i's map and is tested against
+ * env i's goal.  1 <= E <= 1024, E * n < 2^31; every argument is checked before any launch.
+ *
+ * rtd3_eval_starts: the E draws of every env of `bank` (n = bank->n) in one launch.  starts [E][2][n] float32 gets the start
+ * states in draw order; the stream words and pos end where E rtd3_env_reset calls leave them (streams that wrap included), and
+ * state64 [2][n] holds the last draw.  base: nullable [E*n][2] float32, the first actor input state - goal of row e*n + i (for
+ * rtd3_eval_step_episodes); goal [2][n] is read only when base is given. */
+int32_t rtd3_eval_starts(const rtd3_mt_bank* bank, const double* region, const double* goal, int64_t E, float* starts, float* base,
+                         double* state64, void* stream);
+
+/* rtd3_eval_step for a batch of E*n rows, row e*n + i being episode e of env i: xs [E][2][n] the states (the starts in, the final
+ * states out), residual / base [E*n][2], success / steps / best [E][n], traj [E][T][2][n]. */
+int32_t rtd3_eval_step_episodes(rtd3_env* h, const double* goal, int64_t E, float* xs, const float* residual, float* base, uint8_t* success,
+                                int32_t* steps, double* best, float* traj, int32_t record, int64_t n, int64_t T, void* stream);
+
+/* rtd3_eval_run_f16 for E episodes in ONE launch: CTAs take (episode, tile) work items, E * ceil(n / 128) of them.  Episode e
+ * starts from starts [E][2][n]; success / steps / best [E][n], traj [E][T][2][n]; x, y [n] get the final states of episode E-1. */
+int32_t rtd3_eval_run_f16_episodes(rtd3_env* h, int32_t hidden, int32_t layers, const float* params, const uint16_t* params_h,
+                                   const double* goal, const float* starts, int64_t E, float* x, float* y, uint8_t* success, int32_t* steps,
+                                   double* best, float* traj, int32_t record, int64_t n, int64_t T, uint32_t* work, void* stream);
+
 /* ------------------------------------------------------------------------------------------------
  * Tensor-core (tcgen05 / TMEM, TF32) large-batch forward - opt-in throughput mode, not the parity path
  * ---------------------------------------------------------------------------------------------- */

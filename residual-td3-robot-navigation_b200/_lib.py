@@ -142,6 +142,9 @@ _SIGNATURES = {
     "rtd3_tick_run_f16": (c_int32, [_P, POINTER(TickStateStruct), c_int32, c_int32, _P, _P, c_int32, c_int64, c_uint64, _P]),
     "rtd3_eval_step": (c_int32, [_P] * 10 + [c_int32, c_int64, c_int64, _P]),
     "rtd3_eval_run_f16": (c_int32, [_P, c_int32, c_int32] + [_P] * 9 + [c_int32, c_int64, c_int64, _P, _P]),
+    "rtd3_eval_starts": (c_int32, [POINTER(MtBankStruct), _P, _P, c_int64, _P, _P, _P, _P]),
+    "rtd3_eval_step_episodes": (c_int32, [_P, _P, c_int64] + [_P] * 7 + [c_int32, c_int64, c_int64, _P]),
+    "rtd3_eval_run_f16_episodes": (c_int32, [_P, c_int32, c_int32] + [_P] * 4 + [c_int64] + [_P] * 6 + [c_int32, c_int64, c_int64, _P, _P]),
     "rtd3_robot_baseline": (c_int32, [_P, _P, _P, _P, c_int64, _P]),
     "rtd3_robot_compose_action": (c_int32, [_P] * 10 + [c_int64, _P]),
     "rtd3_demo_lists": (c_int32, [_P, c_int64, _P, _P, _P, _P]),

@@ -529,6 +529,15 @@ class Environment:
             return self._state_np
         return self.robot_state
 
+    def _episode_starts(self, starts, base=None):
+        """E calls of `reset()` in one launch (`rtd3_eval_starts`), for E evaluation episodes: the draws go to `starts`
+        `[E,2,N]` float32 instead of the state, the streams advance by E resets and `_state64` holds the last draw.  `base`:
+        optional `[E*N,2]` float32 that gets each episode's first actor input, start - goal."""
+        self._rng_in()
+        _lib.check(_lib.lib().rtd3_eval_starts(self._bank.ref, _lib.ptr(self._region), _lib.ptr(self._goal), starts.shape[0], _lib.ptr(starts),
+                                               _lib.ptr(base), _lib.ptr(self._state64), _lib.stream_ptr(self.device)), "eval_starts")
+        self._rng_out()
+
     def get_random_robot_init_state(self):
         """environment.py:135-137: a draw that does not move the robot."""
         keep, keep_np = self._state.clone(), self._state_np

@@ -532,18 +532,21 @@ class TD3:
     def flat_grad(self, net):
         return self.grads[self._off[net]:self._off[net] + self._cnt[net]]
 
-    def forward(self, net, x):
-        """Forward of arena network `net` on `x` `[B,in]` (CUDA float32) -> `[B,out]`."""
+    def forward(self, net, x, select=None):
+        """Forward of arena network `net` on `x` `[B,in]` (CUDA float32) -> `[B,out]`.  The kernel (f16, TF32 or fp32) is the one
+        the precision selects for `select` rows (default B); each kernel's output rows do not depend on B, so `select` = N on a
+        stack of E batches of N rows gives, batch by batch, what the forward of N rows gives."""
         x = x.to(device=self.device, dtype=torch.float32).contiguous()
         out_dim = 2 if net in (NET_ACTOR, NET_T_ACTOR) else 1
         y = torch.empty((x.shape[0], out_dim), dtype=torch.float32, device=self.device)
+        rows = x.shape[0] if select is None else int(select)
         self.sync_transposed(force=False)
-        if self._f16_ok(x.shape[0]):
+        if self._f16_ok(rows):
             self._sync_half()
             _lib.check(_lib.lib().rtd3_mlp_forward_f16(self.hidden, self.layers, net, _lib.ptr(self.params), _lib.ptr(self.params_h), _lib.ptr(x),
                                                        _lib.ptr(y), x.shape[0], _lib.stream_ptr(self.device)), "mlp_forward_f16")
             return y
-        if self._tc_ok(x.shape[0]):
+        if self._tc_ok(rows):
             self._sync_chunk_major()
             _lib.check(_lib.lib().rtd3_mlp_forward_tf32(self.hidden, self.layers, 1 if net in (NET_ACTOR, NET_T_ACTOR) else 0, self._off[net],
                                                         _lib.ptr(self.params), _lib.ptr(self.params_u), _lib.ptr(x), _lib.ptr(y), x.shape[0],

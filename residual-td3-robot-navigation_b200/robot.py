@@ -41,6 +41,8 @@ EVAL_MAX_STEPS = 1 << 30                # rtd3_eval_step / rtd3_eval_run_f16 tak
 EVAL_BLOCK_STEPS = 64                   # test steps per captured graph of the per-step evaluation
 EVAL_CHECK_BLOCKS = True                # per-step evaluation: read "some env still runs" after each block and end early when none does
 EVAL_GRAPHS_KEPT = 4                    # captured evaluation graphs kept per Robot (one per signature)
+EVAL_MAX_EPISODES = 1024                # evaluate(episodes=E): 1 <= E <= 1024 and E x N < 2^31 (EVAL_MAX_ROWS), as the kernels take
+EVAL_MAX_ROWS = 1 << 31
 
 
 class PathToDraw:
@@ -284,7 +286,7 @@ class Robot:
         return out if self.batched else out[0].cpu().numpy()
 
     # ---- robot-learning.py:104-117: the test phase, batched ------------------------------------------------------------
-    def evaluate(self, environment, max_steps=None, record=False):
+    def evaluate(self, environment, max_steps=None, record=False, episodes=None):
         """The reference's test phase for every env i of `environment` (any size and map configuration), with this Robot's
         current actor.  From env i's current state (call `environment.reset()` first for the reference's start), for
         t = 1 .. T (T = `max_steps`, default TEST_TIMEOUT x UPDATE_RATE = 1000): action = get_next_action_testing (no noise)
@@ -294,65 +296,102 @@ class Robot:
         the rows after an env's stop repeat its final state).  `environment.robot_state` ends at the final states; nothing of
         the Robot changes (only derived weight copies are refreshed, as by any forward).
 
-        With the f16 forward (`precision="f16"`, 2 x H) the whole evaluation is one launch (`rtd3_eval_run_f16`); otherwise each
-        step is the actor forward the learner's precision selects for N rows plus `rtd3_eval_step`, replayed from CUDA graphs
-        of EVAL_BLOCK_STEPS steps.  Both paths give bit-identical results for the same forward."""
+        `episodes` = E (1 <= E <= 1024, E x N < 2^31): E test episodes of every env in one call, bit-identical to
+        `for e in range(E): environment.reset(); r[e] = robot.evaluate(environment, max_steps, record)`.  Episode e of env i
+        starts from the (e+1)-th reset draw of env i's stream and runs on env i's map against env i's goal.  The results gain a
+        leading episode axis: "success", "steps", "best_distance" `[E,N]`, "start" float32 `[E,N,2]` (each episode's start
+        state) and, with `record`, "trajectory" `[E,T,N,2]` (a view of `[E,T,2,N]` float32 planes: E x T x 2 x N x 4 bytes).
+        The environment ends where that loop leaves it: the final states of episode E-1, its streams (numpy's global stream
+        for a single env without a seed) advanced by E resets, and the last draw as the reset's float64 state.
+
+        With the f16 forward (`precision="f16"`, 2 x H) the whole evaluation, all E episodes included, is one launch
+        (`rtd3_eval_run_f16`, `rtd3_eval_run_f16_episodes`); otherwise each step is the actor forward the learner's precision
+        selects for N rows (also on the E x N rows of E episodes) plus `rtd3_eval_step` (`rtd3_eval_step_episodes`), replayed
+        from CUDA graphs of EVAL_BLOCK_STEPS steps.  Both paths give bit-identical results for the same forward."""
         if max_steps is None:
             T = int(round(constants.TEST_TIMEOUT * constants.UPDATE_RATE))
         else:
             if isinstance(max_steps, bool) or not isinstance(max_steps, (int, np.integer)) or not 1 <= int(max_steps) < EVAL_MAX_STEPS:
                 raise ValueError("max_steps must be an integer in [1, 2^30), got %r" % (max_steps,))
             T = int(max_steps)
+        E = None
+        if episodes is not None:
+            if isinstance(episodes, bool) or not isinstance(episodes, (int, np.integer)) or not 1 <= int(episodes) <= EVAL_MAX_EPISODES:
+                raise ValueError("episodes must be an integer in [1, %d], got %r" % (EVAL_MAX_EPISODES, episodes))
+            E = int(episodes)
         if torch.device(environment.device) != self.device:
             raise ValueError("environment is on %s, the robot on %s" % (environment.device, self.device))
         n = environment.num_envs
+        if E is not None and E * n >= EVAL_MAX_ROWS:
+            raise ValueError("episodes x num_envs must lie below 2^31, got %d x %d" % (E, n))
         agent = self.td3_agent
         agent.prepare_forward(n)
         dev = self.device
-        success = torch.zeros(n, dtype=torch.bool, device=dev)
-        steps = torch.zeros(n, dtype=torch.int32, device=dev)
-        best = torch.full((n,), float("inf"), dtype=torch.float64, device=dev)
-        traj = torch.empty((T, 2, n), dtype=torch.float32, device=dev) if record else None
+        lead = () if E is None else (E,)
+        success = torch.zeros(lead + (n,), dtype=torch.bool, device=dev)
+        steps = torch.zeros(lead + (n,), dtype=torch.int32, device=dev)
+        best = torch.full(lead + (n,), float("inf"), dtype=torch.float64, device=dev)
+        traj = torch.empty(lead + (T, 2, n), dtype=torch.float32, device=dev) if record else None
+        starts = None if E is None else torch.empty((E, 2, n), dtype=torch.float32, device=dev)
         if n > 0:
             if self.eval_kernel and agent._f16_ok(n):
                 if self._eval_work is None:
                     self._eval_work = torch.zeros(1, dtype=torch.int32, device=dev)
-                _lib.check(_lib.lib().rtd3_eval_run_f16(
-                    environment._handle, agent.hidden, agent.layers, _lib.ptr(agent.params), _lib.ptr(agent.params_h), _lib.ptr(environment._goal),
-                    _lib.ptr(environment._state[0]), _lib.ptr(environment._state[1]), _lib.ptr(success), _lib.ptr(steps), _lib.ptr(best),
-                    _lib.ptr(traj), 1 if record else 0, n, T, _lib.ptr(self._eval_work), _lib.stream_ptr(dev)), "eval_run_f16")
+                if E is None:
+                    _lib.check(_lib.lib().rtd3_eval_run_f16(
+                        environment._handle, agent.hidden, agent.layers, _lib.ptr(agent.params), _lib.ptr(agent.params_h), _lib.ptr(environment._goal),
+                        _lib.ptr(environment._state[0]), _lib.ptr(environment._state[1]), _lib.ptr(success), _lib.ptr(steps), _lib.ptr(best),
+                        _lib.ptr(traj), 1 if record else 0, n, T, _lib.ptr(self._eval_work), _lib.stream_ptr(dev)), "eval_run_f16")
+                else:
+                    environment._episode_starts(starts)
+                    _lib.check(_lib.lib().rtd3_eval_run_f16_episodes(
+                        environment._handle, agent.hidden, agent.layers, _lib.ptr(agent.params), _lib.ptr(agent.params_h), _lib.ptr(environment._goal),
+                        _lib.ptr(starts), E, _lib.ptr(environment._state[0]), _lib.ptr(environment._state[1]), _lib.ptr(success), _lib.ptr(steps),
+                        _lib.ptr(best), _lib.ptr(traj), 1 if record else 0, n, T, _lib.ptr(self._eval_work), _lib.stream_ptr(dev)), "eval_run_f16_episodes")
             else:
-                self._evaluate_steps(environment, T, traj, success, steps, best)
+                self._evaluate_steps(environment, T, traj, success, steps, best, starts)
         environment._state_np = None
         out = {"success": success, "steps": steps, "best_distance": best}
+        if E is not None:
+            out["start"] = starts.permute(0, 2, 1)
         if record:
-            out["trajectory"] = traj.permute(0, 2, 1)
+            out["trajectory"] = traj.transpose(-1, -2)
         return out
 
-    def _evaluate_steps(self, environment, T, traj, success, steps, best):
+    def _evaluate_steps(self, environment, T, traj, success, steps, best, starts=None):
         """The per-step evaluation: the test steps in blocks of S, each block one replay of a captured graph of S (forward,
         `rtd3_eval_step`) pairs.  Envs that have stopped are left alone by the kernel, so the last block may run past T; S is
-        chosen so that it runs fewer extra forwards than there are blocks."""
+        chosen so that it runs fewer extra forwards than there are blocks.  With `starts` (`[E,2,N]`, E episodes) the rows are
+        the E x N (episode, env) pairs, stepped by `rtd3_eval_step_episodes` on a copy of the start planes drawn here."""
         agent, n, dev = self.td3_agent, environment.num_envs, self.device
+        E = None if starts is None else starts.shape[0]
+        rows = n if E is None else E * n
         blocks = -(-T // EVAL_BLOCK_STEPS)
         S = -(-T // blocks)
         p = lambda t: None if t is None else t.data_ptr()
         fwd = p(agent.params_h) if agent._f16_ok(n) else (p(agent.params_u) if agent._tc_ok(n) else p(agent.params_t))
-        sig = (environment._handle.value, n, S, T, agent.precision, p(agent.params), fwd, environment._map_config(), p(environment._state),
+        sig = (environment._handle.value, n, E, S, T, agent.precision, p(agent.params), fwd, environment._map_config(), p(environment._state),
                p(environment._goal), p(traj))
         st = self._eval_graphs.get(sig)
         if st is None:
             if len(self._eval_graphs) >= EVAL_GRAPHS_KEPT:
                 self._eval_graphs.pop(next(iter(self._eval_graphs)))
-            st = {"base": torch.zeros((n, 2), dtype=torch.float32, device=dev), "success": torch.zeros(n, dtype=torch.uint8, device=dev),
-                  "steps": torch.zeros(n, dtype=torch.int32, device=dev), "best": torch.zeros(n, dtype=torch.float64, device=dev)}
+            st = {"base": torch.zeros((rows, 2), dtype=torch.float32, device=dev), "success": torch.zeros(rows, dtype=torch.uint8, device=dev),
+                  "steps": torch.zeros(rows, dtype=torch.int32, device=dev), "best": torch.zeros(rows, dtype=torch.float64, device=dev)}
             L, x, y = _lib.lib(), environment._state[0], environment._state[1]
+            if E is not None:
+                st["xs"] = torch.zeros((E, 2, n), dtype=torch.float32, device=dev)
 
             def step():
-                residual = agent.forward(NET_ACTOR, st["base"])
-                _lib.check(L.rtd3_eval_step(environment._handle, _lib.ptr(environment._goal), _lib.ptr(x), _lib.ptr(y), _lib.ptr(residual),
-                                            _lib.ptr(st["base"]), _lib.ptr(st["success"]), _lib.ptr(st["steps"]), _lib.ptr(st["best"]),
-                                            _lib.ptr(traj), 0 if traj is None else 1, n, T, _lib.stream_ptr(dev)), "eval_step")
+                residual = agent.forward(NET_ACTOR, st["base"], select=n)
+                if E is None:
+                    _lib.check(L.rtd3_eval_step(environment._handle, _lib.ptr(environment._goal), _lib.ptr(x), _lib.ptr(y), _lib.ptr(residual),
+                                                _lib.ptr(st["base"]), _lib.ptr(st["success"]), _lib.ptr(st["steps"]), _lib.ptr(st["best"]),
+                                                _lib.ptr(traj), 0 if traj is None else 1, n, T, _lib.stream_ptr(dev)), "eval_step")
+                else:
+                    _lib.check(L.rtd3_eval_step_episodes(environment._handle, _lib.ptr(environment._goal), E, _lib.ptr(st["xs"]), _lib.ptr(residual),
+                                                         _lib.ptr(st["base"]), _lib.ptr(st["success"]), _lib.ptr(st["steps"]), _lib.ptr(st["best"]),
+                                                         _lib.ptr(traj), 0 if traj is None else 1, n, T, _lib.stream_ptr(dev)), "eval_step_episodes")
             graph = torch.cuda.CUDAGraph()
             before = _lib.launch_count()
             with _lib.capture(graph):
@@ -364,16 +403,22 @@ class Robot:
         st["success"].zero_()
         st["steps"].zero_()
         st["best"].fill_(float("inf"))
-        _lib.check(_lib.lib().rtd3_robot_baseline(_lib.ptr(environment._state[0]), _lib.ptr(environment._state[1]), _lib.ptr(environment._goal),
-                                                  _lib.ptr(st["base"]), n, _lib.stream_ptr(dev)), "robot_baseline")
+        if E is None:
+            _lib.check(_lib.lib().rtd3_robot_baseline(_lib.ptr(environment._state[0]), _lib.ptr(environment._state[1]), _lib.ptr(environment._goal),
+                                                      _lib.ptr(st["base"]), n, _lib.stream_ptr(dev)), "robot_baseline")
+        else:
+            environment._episode_starts(starts, st["base"])
+            st["xs"].copy_(starts)
         for b in range(blocks):
             st["graph"].replay()
             _lib.lib().rtd3_launch_count_add(st["launches"])
             if EVAL_CHECK_BLOCKS and b + 1 < blocks and not bool(((st["steps"] < T) & (st["success"] == 0)).any()):
                 break
-        success.copy_(st["success"])
-        steps.copy_(st["steps"])
-        best.copy_(st["best"])
+        success.view(-1).copy_(st["success"])
+        steps.view(-1).copy_(st["steps"])
+        best.view(-1).copy_(st["best"])
+        if E is not None:
+            environment._state.copy_(st["xs"][E - 1])
 
     # ---- robot.py:645-675 ------------------------------------------------------------------------------------------
     def process_transition(self, state, action, next_state, money_remaining, push=True, types=None):

@@ -8,6 +8,13 @@ environment reset outside); the median is reported, with milliseconds per evalua
 steps the envs actually took, the sum of `steps`).  The card's name, power limit and SM clocks are read in the same run.
 
     python tools/eval_perf.py --out profiles/r7_policy_eval.json
+
+`--episodes E1,E2,...`: the multi-episode form instead.  Per point, one call `evaluate(env, episodes=E)` against the loop it
+replaces, E x (env.reset() + evaluate(env)), alternating inside each window and timed with CUDA events around the whole call
+or loop (the resets included in both).  Grid: `--sizes` (default 4 096, 16 384, 65 536) x E x zero / homing actor, for the same
+two actors.
+
+    python tools/eval_perf.py --episodes 1,16 --out profiles/r8_eval_episodes.json
 """
 import argparse
 import json
@@ -70,19 +77,79 @@ def timed(fn):
     return a.elapsed_time(b), work
 
 
+SHAPES = {"f16_2x256": (256, 2, "f16"), "fp32_3x200": (200, 3, "fp32")}
+
+
+def median_point(paths, times, work, **key):
+    pt = dict(key, paths={})
+    for name in paths:
+        med = statistics.median(times[name])
+        pt["paths"][name] = {"ms_median": med, "ms_all": times[name], "env_steps": work[name], "env_steps_per_s": work[name] / (med * 1e-3)}
+    print(json.dumps(key), {k: round(v["ms_median"], 3) for k, v in pt["paths"].items()}, flush=True)
+    return pt
+
+
+def episodes_main(args, maps, res):
+    """One call with E episodes against E x (reset + evaluate), per (actor shape, n, actor, E)."""
+    T = args.steps
+    res["episodes"] = [int(e) for e in args.episodes.split(",")]
+    for shape, (hidden, layers, precision) in SHAPES.items():
+        for n in [int(s) for s in args.sizes.split(",")]:
+            env = rt.Environment(num_envs=n, seed=5, maps=maps)
+            torch.manual_seed(1)
+            robot = rt.Robot(env.goal_state, hidden=hidden, layers=layers, seed=3)
+            robot.td3_agent.precision = precision
+            for actor in ("zero", "homing"):
+                set_actor(robot, actor)
+                for E in res["episodes"]:
+                    def one_call():
+                        return robot.evaluate(env, max_steps=T, episodes=E)["steps"]
+
+                    def loop():
+                        steps = []
+                        for _ in range(E):
+                            env.reset()
+                            steps.append(robot.evaluate(env, max_steps=T)["steps"])
+                        return torch.stack(steps)
+                    paths = {"one_call": one_call, "loop": loop}
+                    times = {k: [] for k in paths}
+                    work = {}
+                    for fn in paths.values():                         # warm-up: captures, module loads
+                        fn()
+                    torch.cuda.synchronize()
+                    for _ in range(args.windows):
+                        for name, fn in paths.items():
+                            torch.cuda.synchronize()
+                            ms, w = timed(fn)
+                            times[name].append(ms)
+                            work[name] = int(w.long().sum())
+                    res["points"].append(median_point(paths, times, work, shape=shape, n=n, actor=actor, E=E,
+                                                      persistent=bool(robot.td3_agent._f16_ok(n))))
+            del robot, env
+            torch.cuda.empty_cache()
+
+
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r7_policy_eval.json"))
-    ap.add_argument("--sizes", default="4096,8192,65536,262144")
+    ap.add_argument("--out", default=None)
+    ap.add_argument("--sizes", default=None)
     ap.add_argument("--windows", type=int, default=5)
     ap.add_argument("--steps", type=int, default=1000)
     ap.add_argument("--python-loop-max", type=int, default=1 << 30, help="largest n for which the Python loop is timed")
+    ap.add_argument("--episodes", default=None, help="comma-separated E: time evaluate(episodes=E) against the reset + evaluate loop")
     args = ap.parse_args()
     assert torch.cuda.is_available(), "needs the GPU"
+    if args.out is None:
+        args.out = os.path.join(ROOT, "profiles", "r8_eval_episodes.json" if args.episodes else "r7_policy_eval.json")
+    if args.sizes is None:
+        args.sizes = "4096,16384,65536" if args.episodes else "4096,8192,65536,262144"
     T = args.steps
     speed, angle = rt.synthetic_maps(0)
     maps = (speed, (angle * 0.05).astype(np.float32))                # at most 18 degrees of turn: the homing actor reaches goals
     res = {"card": card(), "T": T, "windows": args.windows, "maps": "synthetic_maps(0), angle x 0.05", "points": []}
+    if args.episodes:
+        episodes_main(args, maps, res)
+        return finish(args, res)
     for shape in ("f16_2x256", "fp32_3x200"):
         hidden, layers, precision = (256, 2, "f16") if shape == "f16_2x256" else (200, 3, "fp32")
         for n in [int(s) for s in args.sizes.split(",")]:
@@ -129,6 +196,10 @@ def main():
                       {k: round(v["ms_median"], 3) for k, v in pt["paths"].items()}, flush=True)
             del robot, env
             torch.cuda.empty_cache()
+    finish(args, res)
+
+
+def finish(args, res):
     res["card_after"] = card()
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
     with open(args.out, "w") as f:
