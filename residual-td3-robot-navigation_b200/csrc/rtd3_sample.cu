@@ -256,6 +256,7 @@ sample_swaps_pipelined_kernel(rtd3_mt_bank b, int64_t stream_id, int32_t n, int3
   __shared__ MaybeRec mb[2][NW][32];
   __shared__ __align__(8) uint64_t full[kRing], empty[kRing];
   __shared__ volatile int s_done, s_last;
+  __shared__ int s_gen_stop;                          // s_done as the generator's thread 0 read it before the generator barrier
   const int tid = threadIdx.x;
   for (int k = tid; k < RTD3_MT_N; k += NC + 256) mt[k] = b.mt[(int64_t)k * b.n + stream_id];
   const int pos0 = b.pos[stream_id];
@@ -272,10 +273,16 @@ sample_swaps_pipelined_kernel(rtd3_mt_bank b, int64_t stream_id, int32_t n, int3
     constexpr int N = RTD3_MT_N, M = 397;
     for (int blk = 0;; ++blk) {
       const int slot = blk % kRing;
-      if (blk >= kRing && t == 0)                        // one thread polls (the others wait at the barrier, off the issue slots)
-        while (!mbar_try_wait(&empty[slot], (uint32_t)((blk / kRing - 1) & 1)) && !s_done) __nanosleep(64);
+      if (t == 0) {
+        if (blk >= kRing)                                // one thread polls (the others wait at the barrier, off the issue slots)
+          while (!mbar_try_wait(&empty[slot], (uint32_t)((blk / kRing - 1) & 1)) && !s_done) __nanosleep(64);
+        // the consumers may set s_done at any time: one read decides for all 256 threads, or some warps could leave the loop
+        // while the others wait for them at the next generator barrier.  Thread 0 writes s_gen_stop again only after the barrier
+        // that ends this block, which every thread reaches after its read.
+        s_gen_stop = s_done;
+      }
       bar_named(2, 256);
-      if (s_done) break;
+      if (s_gen_stop) break;
       if (blk > 0) {
         const int lo[3] = {0, N - M, 2 * (N - M)}, hi[3] = {N - M, 2 * (N - M), N};
 #pragma unroll
