@@ -349,6 +349,14 @@ int32_t rtd3_robot_process_demonstration(const rtd3_mt_bank* bank, const double*
                                          float* rp_a, float* rp_r, float* rp_s2, float* rp_notdone, int64_t capacity, uint64_t* rp_total,
                                          void* stream);
 
+/* The per-env search grids of rtd3_robot_process_demonstration rebuilt on their own from the sets (a restored checkpoint stores
+ * `sets` and `set_count` only): for each of the n envs a counting sort of sets[i][0 .. set_count[i]) into sorted [n][cap][2]
+ * float64 by the cell of its 25 x 25 grid, with the cell start offsets in cells [n][RTD3_ENV_DEMO_CELLS + 1].  cells is
+ * deterministic; the order of the states within a cell is not (the nearest-state search takes a min of exact float64 values, so
+ * no result depends on it).  The caller guarantees set_count[i] <= cap.  One launch of n CTAs; n == 0 launches nothing. */
+int32_t rtd3_robot_demo_grids(const double* sets, const int32_t* set_count, int64_t cap, int64_t n, double* sorted, int32_t* cells,
+                              void* stream);
+
 /* Candidate lists for the nearest-demonstration term of compute_reward (robot.py:753: cdist(...).min() over ALL demonstration
  * states).  For every 1 x 1 cell of the world: the states that can be the nearest one for some point of the cell - a state is
  * dropped when another state is closer at all four corners of the cell (then it is closer everywhere in it); tested against the

@@ -153,6 +153,7 @@ _SIGNATURES = {
     "rtd3_robot_process_demonstration": (c_int32, [POINTER(MtBankStruct), _P, _P, _P, _P, c_int32, _P, _P, _P, _P, c_int64, c_int32, c_int32,
                                                    c_double, _P, _P, _P, _P, _P, c_int64, _P, _P]),
     "rtd3_robot_next_action_type": (c_int32, [_P] * 10 + [c_int64, _P]),
+    "rtd3_robot_demo_grids": (c_int32, [_P, _P, c_int64, c_int64, _P, _P, _P]),
 }
 
 _lib = None

@@ -352,4 +352,15 @@ int32_t rtd3_robot_process_demonstration(const rtd3_mt_bank* bank, const double*
   return 0;
 }
 
+int32_t rtd3_robot_demo_grids(const double* sets, const int32_t* set_count, int64_t cap, int64_t n, double* sorted, int32_t* cells,
+                              void* stream) {
+  RTD3_CHECK_ARG(sets && set_count && sorted && cells, "null argument");
+  RTD3_CHECK_ARG(cap >= 1, "cap must be >= 1");
+  RTD3_CHECK_ARG(n >= 0 && n < (1ll << 31), "n must lie in [0, 2^31)");
+  if (n == 0) return 0;
+  demo_grid_build_kernel<<<(int)n, 256, 0, (cudaStream_t)stream>>>(sets, set_count, cap, sorted, cells);
+  RTD3_LAUNCHED();
+  return 0;
+}
+
 }  // extern "C"

@@ -217,6 +217,19 @@ class Environment:
         except Exception:
             pass
 
+    # ---- checkpoint (checkpoint.py) ----------------------------------------------------------------------------------
+    def state_dict(self):
+        """The whole state of this Environment as CPU tensors and plain values (checkpoint.py; synchronises the device)."""
+        from . import checkpoint
+        return checkpoint.env_state(self)
+
+    def load_state_dict(self, sd):
+        """Load `sd` (from `state_dict` of a Environment of the same configuration) in place; every check runs before anything is
+        written (ValueError).  With numpy's global stream, numpy's global state is restored too."""
+        from . import checkpoint
+        checkpoint.load_state(self, sd)
+        return self
+
     # ---- RNG plumbing -------------------------------------------------------------------------------
     def _rng_in(self):
         if self._numpy_global:

@@ -160,6 +160,19 @@ class ReplayBuffer:
         if self._numpy_global:
             self._bank.sync_to_numpy()
 
+    # ---- checkpoint (checkpoint.py) ----------------------------------------------------------------------------------
+    def state_dict(self):
+        """The whole state of this ReplayBuffer as CPU tensors and plain values (checkpoint.py; synchronises the device)."""
+        from . import checkpoint
+        return checkpoint.replay_state(self)
+
+    def load_state_dict(self, sd):
+        """Load `sd` (from `state_dict` of a ReplayBuffer of the same configuration) in place; every check runs before anything is
+        written (ValueError).  With numpy's global stream, numpy's global state is restored too."""
+        from . import checkpoint
+        checkpoint.load_state(self, sd)
+        return self
+
     def gather(self, idx):
         B = idx.numel()
         idx = idx.to(device=self.device, dtype=torch.int32).contiguous()
@@ -467,6 +480,31 @@ class TD3:
                 self._handle = None
         except Exception:
             pass
+
+    # ---- checkpoint (checkpoint.py) ----------------------------------------------------------------------------------
+    def state_dict(self):
+        """The whole state of this TD3 as CPU tensors and plain values (checkpoint.py; synchronises the device)."""
+        from . import checkpoint
+        return checkpoint.td3_state(self)
+
+    def load_state_dict(self, sd):
+        """Load `sd` (from `state_dict` of a TD3 of the same configuration) in place; every check runs before anything is
+        written (ValueError).  With numpy's global stream, numpy's global state is restored too."""
+        from . import checkpoint
+        checkpoint.load_state(self, sd)
+        return self
+
+    def export_networks(self):
+        """The six networks (online and target) as `nn.Module` state dicts keyed by the reference's attribute names (robot.py:232-234):
+        {"actor_network": {"layer_1.weight": ..., "output_layer.bias": ...}, ...}, CPU float32.  Loads into modules whose `nn.Linear`
+        layers carry the names of robot.py:145-148."""
+        from . import checkpoint
+        return checkpoint.export_networks(self)
+
+    def import_networks(self, d):
+        """Inverse of `export_networks` (bit-exact round trip); checks everything before writing (ValueError)."""
+        from . import checkpoint
+        checkpoint.import_networks(self, d)
 
     # ---- arena access ---------------------------------------------------------------------------------
     def flat(self, net):

@@ -132,6 +132,19 @@ class Robot:
         self._eval_graphs = {}
         self._eval_work = None
 
+    # ---- checkpoint (checkpoint.py) ----------------------------------------------------------------------------------
+    def state_dict(self):
+        """The whole state of this Robot as CPU tensors and plain values (checkpoint.py; synchronises the device)."""
+        from . import checkpoint
+        return checkpoint.robot_state(self)
+
+    def load_state_dict(self, sd):
+        """Load `sd` (from `state_dict` of a Robot of the same configuration) in place; every check runs before anything is
+        written (ValueError).  With numpy's global stream, numpy's global state is restored too."""
+        from . import checkpoint
+        checkpoint.load_state(self, sd)
+        return self
+
     # ---- reference attributes (single-env views of the device state) --------------------------------------------
     def _scalar(self, t):
         return t[0].item()

@@ -104,6 +104,19 @@ class DriverLoop:
         if self.verbose:
             print(msg)
 
+    # ---- checkpoint (checkpoint.py) ----------------------------------------------------------------------------------
+    def state_dict(self):
+        """The whole state of this DriverLoop as CPU tensors and plain values (checkpoint.py; synchronises the device)."""
+        from . import checkpoint
+        return checkpoint.loop_state(self)
+
+    def load_state_dict(self, sd):
+        """Load `sd` (from `state_dict` of a DriverLoop of the same configuration) in place; every check runs before anything is
+        written (ValueError).  With numpy's global stream, numpy's global state is restored too."""
+        from . import checkpoint
+        checkpoint.load_state(self, sd)
+        return self
+
     def calculate_remaining_money(self):
         c = constants
         cpu_time_bought = self.ticks * self.tick_seconds
@@ -247,6 +260,19 @@ class BatchedTrainer:
             self.test_success = torch.zeros(self.n, dtype=torch.uint8, device=dev)
             self.penalty = torch.zeros(self.n, dtype=torch.uint8, device=dev)
             self.test_timeout_ticks = max(1, int(round(constants.TEST_TIMEOUT / self.tick_seconds))) if self.tick_seconds > 0 else 1000
+
+    # ---- checkpoint (checkpoint.py) ----------------------------------------------------------------------------------
+    def state_dict(self):
+        """The whole state of this BatchedTrainer as CPU tensors and plain values (checkpoint.py; synchronises the device)."""
+        from . import checkpoint
+        return checkpoint.trainer_state(self)
+
+    def load_state_dict(self, sd):
+        """Load `sd` (from `state_dict` of a BatchedTrainer of the same configuration) in place; every check runs before anything is
+        written (ValueError).  With numpy's global stream, numpy's global state is restored too."""
+        from . import checkpoint
+        checkpoint.load_state(self, sd)
+        return self
 
     def money_remaining(self, tick_charge=None):
         """calculate_remaining_money (robot-learning.py:45-50) per env, float64 `[N]`; the wall-clock term is ticks x tick_charge
