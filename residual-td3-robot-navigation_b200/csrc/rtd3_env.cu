@@ -471,18 +471,26 @@ env_rollout_tma_kernel(int64_t n, float* __restrict__ x, float* __restrict__ y, 
   }
 }
 
-// ---- T-step rollout, warp-pair variant: chain warp + helper warp per 32 envs -------------------------------------------
+// ---- T-step rollout, warp-pair variant: chain warps + helper warp per 32 envs ------------------------------------------
 // At 4096 envs every SM gets one warp, and that warp's issue slots - not memory - bound the TMA kernel above (31
 // instr/step, of which only 13 are the state recurrence; ncu r1: 42 % fixed-latency waits).  Here the recurrence runs
-// alone on the CHAIN warp (per step: one LDS.64 of the pre-clipped action, the chain, two STS of the new state); a
+// alone on the CHAIN warps (per step: one LDS.64 of the pre-clipped action, the chain, two STS of the new state); a
 // HELPER warp on another scheduler of the same SM waits for the TMA action tiles, clips them (or flags the chunk for the
-// careful NaN path), re-arms the loads and issues the trajectory tile stores.  The two meet on mbarriers over
-// double-buffered shared-memory tiles.  The table is the halo table (see kHalo), so that on a map that fits, the chain
-// of a step is FFMA, FFMA -> FADD.RZ -> IMAD, IMAD -> LDS.64: the clip, the action load and the trajectory stores are
+// careful NaN path), re-arms the loads and issues the trajectory tile stores.  They meet on mbarriers over
+// double-buffered shared-memory tiles of 32 envs.  The table is the halo table (see kHalo), so that on a map that fits, the
+// chain of a step is FFMA, FFMA -> FADD.RZ -> IMAD, IMAD -> LDS.64: the clip, the action load and the trajectory stores are
 // issued while the table load is in flight.
+// A chain warp steps kChainLanes envs of the tile, one per lane, and its other lanes idle: the table gather of a step reads
+// one 8-byte cell per active lane from unrelated places, and the bank conflicts of that gather sit on the dependent chain of
+// every step (tools/lds_chain/lds_chain.cu on a B200: 34.4 cycles per dependent gather at 32 lanes, 28.3 at 16, 24.1 without
+// conflicts).  A chain warp issues the same instructions per step whatever its width, and the SM's other schedulers are idle
+// at these batch sizes.  16 lanes rather than 8: at 8 the helper shares a scheduler with a chain warp, and with two tiles per
+// CTA (8 192 envs) the step got slower than with 32 lanes (DESIGN.md).
 constexpr int kPairU = 32;        // steps per tile of the pair kernel
-constexpr int kPairStages = 4;    // action tiles in flight (128 steps of lead, as kDeep x kU), one pair per CTA
-constexpr int kPairStages2 = 3;   // two pairs per CTA: 4 stages do not fit next to the halo table
+constexpr int kPairStages = 4;    // action tiles in flight (128 steps of lead, as kDeep x kU), one tile per CTA
+constexpr int kPairStages2 = 3;   // two tiles per CTA: 4 stages do not fit next to the halo table
+constexpr int kChainLanes = 16;     // envs per chain warp
+constexpr int pair_warps(int lanes) { return 32 / lanes + 1; }   // warps per 32-env tile: the chain warps, then the helper
 struct PairSmem {
   static constexpr int kBars = 16;   // full[8] | prepped[2] | consumed[2] | outfull[2] | outfree[2]
 };
@@ -538,8 +546,8 @@ __device__ __forceinline__ void stamp(uint32_t slot, int phase) {
 // the map index are read after the wait.  traj_host: the trajectory is host memory, so the helper waits for its last store to
 // complete before exiting; for device memory the completion of the grid covers it, and the helper only waits for the store to
 // have read its shared-memory tile.
-template <bool kTraj, int kStages, int kUp, bool kBank = false>
-__global__ void __launch_bounds__(256)
+template <bool kTraj, int kStages, int kUp, int kLanes, bool kBank = false>
+__global__ void __launch_bounds__(2 * pair_warps(kLanes) * 32)
 env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __grid_constant__ CUtensorMap tm_act,
                         const __grid_constant__ CUtensorMap tm_traj, int64_t n, int64_t T, MapBank bank, int traj_host) {
   extern __shared__ __align__(128) unsigned char smem_raw[];
@@ -548,27 +556,31 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
   launch_dependents();
   constexpr int kU = kUp;                            // steps per action / trajectory tile of this kernel (shadows the file-wide kU)
   constexpr int kTileFloats = kU * 2 * 32;
+  constexpr int kChains = 32 / kLanes;               // chain warps per tile
+  static_assert(kLanes * kChains == 32, "the chain warps of a tile cover its 32 envs");
   float2* s_table = reinterpret_cast<float2*>(smem_raw);
   uint64_t* bar = reinterpret_cast<uint64_t*>(smem_raw + kHaloBytes);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, npairs = blockDim.x >> 6;
-  const int pair = warp >> 1;
-  const bool is_chain = (warp & 1) == 0;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + kHaloBytes + 16) + pair * PairSmem::kBars;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, ntiles = blockDim.x / (pair_warps(kLanes) * 32);
+  const int tile = warp / pair_warps(kLanes);
+  const int cw = warp % pair_warps(kLanes);          // chain warp cw of the tile, or the helper (cw == kChains)
+  const bool is_chain = cw < kChains;
+  uint64_t* bars = reinterpret_cast<uint64_t*>(smem_raw + kHaloBytes + 16) + tile * PairSmem::kBars;
   uint64_t* full = bars, *prepped = bars + 8, *consumed = bars + 10, *outfull = bars + 12, *outfree = bars + 14;
-  // per pair: kStages raw tiles | 2 prepped tiles (float2 per step and env = 2 tiles' worth each... [kU][32] float2 = 4 KB) | 2 out tiles
-  float* tiles = reinterpret_cast<float*>(smem_raw + ((kHaloBytes + 16 + npairs * PairSmem::kBars * 8 + 127) & ~127u));
-  float* my = tiles + (size_t)pair * (kStages + 4) * kTileFloats;
+  // per tile: kStages raw tiles | 2 prepped tiles (float2 per step and env = 2 tiles' worth each... [kU][32] float2 = 4 KB) | 2 out tiles
+  float* tiles = reinterpret_cast<float*>(smem_raw + ((kHaloBytes + 16 + ntiles * PairSmem::kBars * 8 + 127) & ~127u));
+  float* my = tiles + (size_t)tile * (kStages + 4) * kTileFloats;
   float* raw = my;                                   // [kStages][kU*2][32]
   float2* prep = reinterpret_cast<float2*>(my + kStages * kTileFloats);                 // [2][kU][32]
   float* outt = my + (kStages + 2) * kTileFloats;    // [2][kU*2][32]
-  __shared__ int s_flag[4][2];                       // careful flag per pair and prepped buffer
-  if (lane == 0 && is_chain) {
+  __shared__ int s_flag[2][2];                       // careful flag per tile and prepped buffer
+  // consumed / outfull count one arrival per env of the tile: the active lanes of its chain warps
+  if (lane == 0 && !is_chain) {
 #pragma unroll
     for (int s = 0; s < kStages; ++s) mbar_init(full + s, 1);
     for (int b = 0; b < 2; ++b) { mbar_init(prepped + b, 32); mbar_init(consumed + b, 32); mbar_init(outfull + b, 32); mbar_init(outfree + b, 1); }
     fence_mbar_init();
   }
-  const int64_t i0 = ((int64_t)blockIdx.x * npairs + pair) * 32;
+  const int64_t i0 = ((int64_t)blockIdx.x * ntiles + tile) * 32;
   const int64_t chunks = (T + kU - 1) / kU;
   if (lane == 0 && !is_chain) {
     prefetch_tensormap(&tm_act);
@@ -576,6 +588,7 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
     if (i0 < n)
       for (int s = 0; s < kStages && s < chunks; ++s) tma_prefetch_l2_2d(&tm_act, (int)i0, s * (2 * kU));
   }
+  const int col = cw * kLanes + lane;                // a chain lane's env within the tile (lane < kLanes)
   int staged = 0;
   BankLanes bl{};
   const auto stage = [&] {   // contains the __syncthreads that publishes the barrier inits
@@ -585,9 +598,9 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
   grid_dep_wait();
   RTD3_STAMP(threadIdx.x == 0, kStampWaited);
   if constexpr (kBank) {
-    staged = bank.map<kBank>((int64_t)blockIdx.x * npairs * 32);   // the CTA stages the halo table of its first env's map
-    const int64_t env = ((int64_t)blockIdx.x * npairs + pair) * 32 + lane;
-    bl = bank_lanes(bank, staged, env, env < n);
+    staged = bank.map<kBank>((int64_t)blockIdx.x * ntiles * 32);   // the CTA stages the halo table of its first env's map
+    const int64_t env = i0 + col;                    // mixed: over the active lanes of this chain warp
+    bl = bank_lanes(bank, staged, env, is_chain && lane < kLanes && env < n);
     stage();
   }
 
@@ -623,7 +636,7 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
       for (int u = 0; u < kU; ++u)
         tp[u * 32] = careful ? make_float2(ax[u], ay[u])
                              : make_float2(fminf(fmaxf(ax[u], -kMaxAction), kMaxAction), fminf(fmaxf(ay[u], -kMaxAction), kMaxAction));
-      if (lane == 0) s_flag[pair][b] = careful ? 1 : 0;
+      if (lane == 0) s_flag[tile][b] = careful ? 1 : 0;
       __syncwarp();
       issue_load(c + kStages);                                       // raw stage s is in registers / prepped now
       mbar_arrive(prepped + b);
@@ -658,23 +671,24 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
     return;
   }
 
-  // ================================= chain warp =================================
-  const int64_t i = i0 + lane;
+  // ================================= chain warps =================================
+  if (lane >= kLanes) return;
+  const int64_t i = i0 + col;
   const bool live = i < n;
   const bool fits = __ldg(bank.fits + staged) != 0;  // lands while the table is staging
   float sx = live ? fminf(fmaxf(x[i], 0.0f), 99.99999f) : 0.0f;
   float sy = live ? fminf(fmaxf(y[i], 0.0f), 99.99999f) : 0.0f;
   const uint32_t addr_bias = smem_u32(s_table) - 0x4B000000u * (kHaloRowBytes + 8u);
   mbar_wait(bar, 0);
-  RTD3_STAMP(lane == 0, kStampTable);
+  RTD3_STAMP(col == 0, kStampTable);
   for (int64_t c = 0; c < chunks; ++c) {
     const int b = (int)(c & 1);
     mbar_wait(prepped + b, (uint32_t)((c >> 1) & 1));
-    RTD3_STAMP(lane == 0 && c == 0, kStampChain0);
+    RTD3_STAMP(col == 0 && c == 0, kStampChain0);
     if (kTraj && c >= 2) mbar_wait(outfree + b, (uint32_t)(((c >> 1) - 1) & 1));   // out tile b has been stored (chunk c-2)
-    const bool careful = s_flag[pair][b] != 0;
-    const uint32_t tp = smem_u32(prep + b * (kU * 32) + lane);
-    const uint32_t tout = smem_u32(outt + b * kTileFloats + lane);
+    const bool careful = s_flag[tile][b] != 0;
+    const uint32_t tp = smem_u32(prep + b * (kU * 32) + col);
+    const uint32_t tout = smem_u32(outt + b * kTileFloats + col);
     auto store_state = [&](int u) {                  // the state after step u into the trajectory tile
       asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u) * 128u), "f"(sx) : "memory");
       asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u + 1) * 128u), "f"(sy) : "memory");
@@ -727,9 +741,9 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
     mbar_arrive(consumed + b);
     if (kTraj) mbar_arrive(outfull + b);
   }
-  RTD3_STAMP(lane == 0, kStampChainEnd);
+  RTD3_STAMP(col == 0, kStampChainEnd);
   if (live) { x[i] = sx; y[i] = sy; }
-  RTD3_STAMP(lane == 0, kStampChainExit);
+  RTD3_STAMP(col == 0, kStampChainExit);
 }
 
 // ---- seeded init / reset on per-env legacy MT19937 streams ------------------------------------
@@ -871,13 +885,13 @@ static const TmaKernel kTmaKernels[2][2][2] = {
      {env_rollout_tma_kernel<true, kShallow>, env_rollout_tma_kernel<true, kDeep>}},
     {{env_rollout_tma_kernel<false, kShallow, true>, env_rollout_tma_kernel<false, kDeep, true>},
      {env_rollout_tma_kernel<true, kShallow, true>, env_rollout_tma_kernel<true, kDeep, true>}}};
-// pair kernel, [bank][traj][two pairs per CTA]
-using PairKernel = decltype(&env_rollout_pair_kernel<false, kPairStages, kPairU>);
+// pair kernel, [bank][traj][two tiles per CTA]
+using PairKernel = decltype(&env_rollout_pair_kernel<false, kPairStages, kPairU, kChainLanes>);
 static const PairKernel kPairKernels[2][2][2] = {
-    {{env_rollout_pair_kernel<false, kPairStages, kPairU>, env_rollout_pair_kernel<false, kPairStages2, kPairU>},
-     {env_rollout_pair_kernel<true, kPairStages, kPairU>, env_rollout_pair_kernel<true, kPairStages2, kPairU>}},
-    {{env_rollout_pair_kernel<false, kPairStages, kPairU, true>, env_rollout_pair_kernel<false, kPairStages2, kPairU, true>},
-     {env_rollout_pair_kernel<true, kPairStages, kPairU, true>, env_rollout_pair_kernel<true, kPairStages2, kPairU, true>}}};
+    {{env_rollout_pair_kernel<false, kPairStages, kPairU, kChainLanes>, env_rollout_pair_kernel<false, kPairStages2, kPairU, kChainLanes>},
+     {env_rollout_pair_kernel<true, kPairStages, kPairU, kChainLanes>, env_rollout_pair_kernel<true, kPairStages2, kPairU, kChainLanes>}},
+    {{env_rollout_pair_kernel<false, kPairStages, kPairU, kChainLanes, true>, env_rollout_pair_kernel<false, kPairStages2, kPairU, kChainLanes, true>},
+     {env_rollout_pair_kernel<true, kPairStages, kPairU, kChainLanes, true>, env_rollout_pair_kernel<true, kPairStages2, kPairU, kChainLanes, true>}}};
 
 // A rollout launch; with `overlap` it may start while the stream's previous kernel drains (programmatic dependent launch, see
 // env_rollout_pair_kernel).
@@ -1132,12 +1146,13 @@ int32_t rtd3::env_rollout(rtd3_env* h, float* x, float* y, const float* actions,
       make_plane_map(&tm_traj, traj ? traj : actions, n, T, tile_steps) == 0) {
     const int64_t warps_total = ceil_div(n, 32);
     if (pair) {
-      // one chain warp + one helper warp per 32 envs, up to 2 pairs per CTA
-      const int ppc = (int)std::max<int64_t>(1, std::min<int64_t>(2, ceil_div(warps_total, (int64_t)h->num_sms)));
-      const int pstages = ppc == 1 ? kPairStages : kPairStages2;
-      const int psmem = ((kHaloBytes + 16 + ppc * PairSmem::kBars * 8 + 127) & ~127) + ppc * (pstages + 4) * (kPairU * 2 * 32) * 4;
-      const PairKernel kern = kPairKernels[with_bank][with_traj][ppc == 2];
-      RTD3_CUDA(launch_rollout(kern, (int)ceil_div(warps_total, ppc), ppc * 64, psmem, st, overlap, x, y, tm_act, tm_traj, n, T, bank, th));
+      // chain warps + one helper warp per 32-env tile, up to 2 tiles per CTA
+      const int tpc = (int)std::max<int64_t>(1, std::min<int64_t>(2, ceil_div(warps_total, (int64_t)h->num_sms)));
+      const int pstages = tpc == 1 ? kPairStages : kPairStages2;
+      const int psmem = ((kHaloBytes + 16 + tpc * PairSmem::kBars * 8 + 127) & ~127) + tpc * (pstages + 4) * (kPairU * 2 * 32) * 4;
+      const PairKernel kern = kPairKernels[with_bank][with_traj][tpc == 2];
+      RTD3_CUDA(launch_rollout(kern, (int)ceil_div(warps_total, tpc), tpc * pair_warps(kChainLanes) * 32, psmem, st, overlap, x, y, tm_act,
+                               tm_traj, n, T, bank, th));
     } else {
       // one warp per 32 envs; few warps per CTA while the batch cannot fill the SMs, 8 once it can
       const int wpc = deep ? (int)std::max<int64_t>(1, std::min<int64_t>(8, ceil_div(warps_total, (int64_t)h->num_sms))) : 8;
