@@ -21,7 +21,9 @@ Measured on a B200 (1000 W power limit), worst |x - x64| / M over the cases of t
   controls (fp32), smallest distance from the kernel's gradient: 9.3e-7 (one `done` flipped, H = 200, L = 3, B = 2368)
 TAU_FP32 = 2^-21 sits between the two: far below the 2^-15 that fp32 summation-error arithmetic allows, because the magnitude sums
 M are loose by the networks' cancellation.  TF32 operands resolve only the actor-through-critic-2 control (2.4e-2); max instead of min
-(1.1e-2) and the unclipped noise (1.5e-4) are within TF32's error at B = 8192.
+(1.1e-2) and the unclipped noise (1.5e-4) are within TF32's error at B = 8192.  tests/test_tc_exact_gpu.py closes that gap: on dyadic
+vectors where nothing rounds (oracle/exact_grid.py) the TF32 critic step, actor step and update epoch must equal the float64 reference
+bit for bit, and tests/test_exact_grid.py checks that every one of these controls changes that reference.
 
 Optimiser: the Adam / Polyak kernel, element for element against oracle/td3_oracle.py's adam_step / soft_update (pinned to
 torch.optim.Adam), with lr a Python float as in torch, and the Adam step of the fused, cooperative and TF32 update paths against the
