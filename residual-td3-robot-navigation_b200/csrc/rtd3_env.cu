@@ -3,6 +3,7 @@
 #include <cuda.h>
 
 #include <memory>
+#include <type_traits>
 #include <utility>
 
 #include "rtd3_common.cuh"
@@ -641,6 +642,12 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
       issue_load(c + kStages);                                       // raw stage s is in registers / prepped now
       mbar_arrive(prepped + b);
       RTD3_STAMP(lane == 0 && c == 0, kStampPrepped0);
+      // Out tile b is freed before the store of chunk c-1 is issued: the chain warp's wait for it at the start of chunk c then
+      // depends only on the store of chunk c-2 (issued a chunk earlier), not on its own arrival at the end of chunk c-1.
+      if (kTraj && c >= 2 && lane == 0) {
+        bulk_wait_read<0>();                                         // the store of chunk c-2 has read its tile ...
+        mbar_arrive(outfree + b);                                    // ... which is the tile chunk c will write
+      }
       if (kTraj && c >= 1) {                                         // trajectory tile of the previous chunk
         const int pb = (int)((c - 1) & 1);
         mbar_wait(outfull + pb, (uint32_t)(((c - 1) >> 1) & 1));
@@ -648,8 +655,6 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
         if (lane == 0) {
           tma_store_2d(&tm_traj, (int)i0, (int)((c - 1) * (2 * kU)), outt + pb * kTileFloats);
           bulk_commit();
-          bulk_wait_read<1>();                                       // the store of chunk c-2 has read its tile ...
-          if (c >= 2) mbar_arrive(outfree + (int)(c & 1));           // ... which is the tile chunk c will write
         }
         __syncwarp();
       }
@@ -681,38 +686,87 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
   const uint32_t addr_bias = smem_u32(s_table) - 0x4B000000u * (kHaloRowBytes + 8u);
   mbar_wait(bar, 0);
   RTD3_STAMP(col == 0, kStampTable);
+  // Between two fast chunks nothing waits on the chain: the next chunk's barriers and careful flag are probed a few steps before
+  // the end of a chunk (ready, next_careful), and its first table address is the one the last step computed (carried).
+  constexpr int kProbeStep = kU - 4;
+  constexpr uint32_t kPrepBytes = kU * 32 * sizeof(float2), kOutBytes = kTileFloats * sizeof(float);
+  const uint32_t tp0 = smem_u32(prep + col), tout0 = smem_u32(outt + col);
+  uint32_t addr = 0;
+  bool carried = false, ready = false;
+  int next_careful = 0;
   for (int64_t c = 0; c < chunks; ++c) {
-    const int b = (int)(c & 1);
-    mbar_wait(prepped + b, (uint32_t)((c >> 1) & 1));
+    int b = (int)(c & 1);
+    int careful = next_careful;
+    if (!ready) {
+      mbar_wait(prepped + b, (uint32_t)((c >> 1) & 1));
+      if (kTraj && c >= 2) mbar_wait(outfree + b, (uint32_t)(((c >> 1) - 1) & 1));   // out tile b has been stored (chunk c-2)
+      careful = s_flag[tile][b];
+    }
     RTD3_STAMP(col == 0 && c == 0, kStampChain0);
-    if (kTraj && c >= 2) mbar_wait(outfree + b, (uint32_t)(((c >> 1) - 1) & 1));   // out tile b has been stored (chunk c-2)
-    const bool careful = s_flag[tile][b] != 0;
-    const uint32_t tp = smem_u32(prep + b * (kU * 32) + col);
-    const uint32_t tout = smem_u32(outt + b * kTileFloats + col);
+    ready = false;
+    uint32_t tp = tp0 + b * kPrepBytes, tout = tout0 + b * kOutBytes;
     auto store_state = [&](int u) {                  // the state after step u into the trajectory tile
       asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u) * 128u), "f"(sx) : "memory");
       asm volatile("st.shared.f32 [%0], %1;" ::"r"(tout + (2 * u + 1) * 128u), "f"(sy) : "memory");
     };
-    if (!careful && fits && !(kBank && bl.mixed)) {
-      // Step 0 is addressed from the state (which may be in [99, 100) after NaN actions) and step 1 from its clipped
-      // successor; every later step from the unclipped successor of the step before.  The previous step's trajectory
-      // stores follow the table load in program order: issued before it, ptxas put them between the address IMAD and the
-      // load (a store may not move past a load that could alias it).  The next step's action is loaded one step ahead.
+    // Chunk c+1's prepped tile (and out tile) without blocking; a step later its careful flag, which is only used when both
+    // tests passed.  No branches on the chain: at c+1 == 1 the out-tile test passes (the phase before a barrier's first one
+    // counts as complete, as with mbar_wait), and at c+1 == chunks the loop ends whatever they return.
+    auto probe_next = [&] {
+      const uint32_t cn = (uint32_t)c + 1u;
+      ready = mbar_test(prepped + (b ^ 1), (cn >> 1) & 1u);
+      if (kTraj) ready &= mbar_test(outfree + (b ^ 1), ((cn >> 1) - 1u) & 1u);
+    };
+    auto probed_go_on = [&] { return ready && next_careful == 0 && c + 1 < chunks; };
+    // Step 0 of a chunk is addressed from the state (which may be in [99, 100) after NaN actions) and step 1 from its clipped
+    // successor, unless the chunk before ran this path too: its last step started from a clipped state, so the carried address
+    // of its unclipped successor is as good as any inside a chunk.  Every later step is addressed from the unclipped successor
+    // of the step before.  The previous step's trajectory stores follow the table load in program order: issued before it,
+    // ptxas put them between the address IMAD and the load (a store may not move past a load that could alias it).  The next
+    // step's action is loaded one step ahead.
+    //
+    // A carried run stays in this loop from chunk to chunk while the probes find the next chunk ready and fast: the last step
+    // already loads the next chunk's first action, and the previous chunk's consumed / outfull arrivals go after the next
+    // chunk's first table load, so the boundary adds two stores, the loop bookkeeping and one branch to the chain.
+    auto fast_chunks = [&](auto from_carry) {
       float2 a = lds_f2(tp);
-      uint32_t addr = halo_addr_state(addr_bias, sx, sy);
+      if (!from_carry) addr = halo_addr_state(addr_bias, sx, sy);
+      bool pending = false;                          // chunk c-1 of this run still owes its arrivals
+      while (true) {
+        const uint32_t tp_next = tp0 + (b ^ 1) * kPrepBytes;
 #pragma unroll
-      for (int u = 0; u < kU; ++u) {
-        const float2 cs = lds_f2(addr);
-        if (kTraj && u > 0) store_state(u - 1);
-        const float2 an = u + 1 < kU ? lds_f2(tp + (u + 1) * 256u) : a;
-        const float nx = fmaf(a.x, cs.x, fmaf(-a.y, cs.y, sx));
-        const float ny = fmaf(a.x, cs.y, fmaf(a.y, cs.x, sy));
-        sx = fminf(fmaxf(nx, 0.0f), kClipHi);
-        sy = fminf(fmaxf(ny, 0.0f), kClipHi);
-        addr = u == 0 ? halo_addr(addr_bias, sx, sy) : halo_addr(addr_bias, nx, ny);
-        a = an;
+        for (int u = 0; u < kU; ++u) {
+          const float2 cs = lds_f2(addr);
+          if (u == 0 && pending) {
+            mbar_arrive(consumed + (b ^ 1));
+            if (kTraj) mbar_arrive(outfull + (b ^ 1));
+          }
+          if (kTraj && u > 0) store_state(u - 1);
+          if (u == kProbeStep) probe_next();
+          if (u == kProbeStep + 1) next_careful = s_flag[tile][b ^ 1];
+          const float2 an = u + 1 < kU ? lds_f2(tp + (u + 1) * 256u) : from_carry ? lds_f2(tp_next) : a;
+          const float nx = fmaf(a.x, cs.x, fmaf(-a.y, cs.y, sx));
+          const float ny = fmaf(a.x, cs.y, fmaf(a.y, cs.x, sy));
+          sx = fminf(fmaxf(nx, 0.0f), kClipHi);
+          sy = fminf(fmaxf(ny, 0.0f), kClipHi);
+          addr = !from_carry && u == 0 ? halo_addr(addr_bias, sx, sy) : halo_addr(addr_bias, nx, ny);
+          a = an;
+        }
+        if (kTraj) store_state(kU - 1);
+        if (!from_carry || !probed_go_on()) break;
+        ++c;
+        b ^= 1;
+        tp = tp_next;
+        tout = tout0 + b * kOutBytes;
+        ready = false;
+        pending = true;
       }
-      if (kTraj) store_state(kU - 1);
+    };
+    const bool fast = !careful && fits && !(kBank && bl.mixed);
+    if (fast && carried) {
+      fast_chunks(std::true_type{});
+    } else if (fast) {
+      fast_chunks(std::false_type{});
     } else if (kBank && bl.mixed) {
       // lanes on different maps: each steps from its own map's plain table, addressed from the state as below (a loop of its
       // own for the same reason as in env_rollout_tma_kernel)
@@ -738,6 +792,7 @@ env_rollout_pair_kernel(float* __restrict__ x, float* __restrict__ y, const __gr
         if (kTraj) store_state(u);
       }
     }
+    carried = fast;
     mbar_arrive(consumed + b);
     if (kTraj) mbar_arrive(outfull + b);
   }
