@@ -478,27 +478,13 @@ int32_t rtd3_td3_target_noise(uint64_t seed, uint64_t counter, float* out, int64
  * Polyak updates.  Everything is issued on `stream` without synchronising (capturable in one CUDA graph). */
 int32_t rtd3_td3_update(rtd3_td3* h, const rtd3_td3_update_args* args, void* stream);
 
-/* The same update as ONE persistent cooperative kernel (csrc/rtd3_coop.cu) - the small-batch learner: one CTA per SM stays
- * resident for all `epochs`, every hidden-layer product is tiled over all SMs, the layers of the chain are separated by grid-wide
- * barriers instead of kernel launches, Adam / Polyak and (world > 1, peer memory only: args->p2p) the gradient all-reduce are stages
- * of the same kernel.  fp32 (FFMA), layers >= 2, batch <= 4096; same arithmetic as the step kernels up to summation order
- * (losses / Q-values within the 1e-3 parity bar).  args->scratch, params_uv, comm and tf32 are not used.
- * coop_scratch: rtd3_td3_coop_scratch_floats(batch) floats, 16 B aligned, ZERO-initialised once by the caller (its first words are
- * the grid barrier) and then left to the kernel. */
-int32_t rtd3_td3_coop_supported(const rtd3_td3* h, int32_t batch);
-int64_t rtd3_td3_coop_scratch_floats(const rtd3_td3* h, int32_t batch);
-int32_t rtd3_td3_update_coop(rtd3_td3* h, const rtd3_td3_update_args* args, float* coop_scratch, void* stream);
-/* Development aid: DEVICE buffer of 256 int64 that the following cooperative updates stamp with %globaltimer at every stage boundary
- * of their last epoch (block 0: arrival at the grid barrier, release from it); NULL switches it off. */
-int32_t rtd3_debug_coop_prof(long long* device_buf);
-
 /* Small-batch step kernels on thread-block clusters (csrc/rtd3_cluster.cu; the default of rtd3_td3_critic_step / rtd3_td3_actor_step /
  * rtd3_td3_update for fp32 batches that are ONE wave of clusters: 8 rows per cluster, 33 clusters on a B200 = up to 264 rows): 1 if the step of `batch` rows runs on that path, and how many of its 4-CTA clusters the
  * device can hold at once (cudaOccupancyMaxActiveClusters of the critic kernel; negative: CUDA error). */
 int32_t rtd3_td3_cluster_supported(const rtd3_td3* h, int32_t batch);
 int32_t rtd3_td3_cluster_occupancy(const rtd3_td3* h, int32_t batch);
 /* Development / test aid: 0 = the step entry points use the row-tile kernels, 2 = the cluster kernels wherever their plan fits (the
- * default); returns the previous mode (1 = a shape forced through RTD3_CLUSTER=R,CS).  Not thread-safe against running launches. */
+ * default); returns the previous mode.  Not thread-safe against running launches. */
 int32_t rtd3_debug_cluster_mode(int32_t mode);
 /* Development: stage stamps (%globaltimer, ns) of the last weight-gradient launch that exchanged its tiles with the peers
  * (rtd3_td3_update at world > 1 over peer memory, RTD3_P2P_PROF=1): out_host [256 blocks][2 threads][8 stages] uint64.  Returns 1 if

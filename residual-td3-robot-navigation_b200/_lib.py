@@ -127,10 +127,6 @@ _SIGNATURES = {
     "rtd3_comm_rank": (c_int32, [_P]),
     "rtd3_allreduce_grads": (c_int32, [_P, _P, c_int64, _P]),
     "rtd3_td3_update": (c_int32, [_P, POINTER(Td3UpdateArgs), _P]),
-    "rtd3_td3_coop_supported": (c_int32, [_P, c_int32]),
-    "rtd3_td3_coop_scratch_floats": (c_int64, [_P, c_int32]),
-    "rtd3_td3_update_coop": (c_int32, [_P, POINTER(Td3UpdateArgs), _P, _P]),
-    "rtd3_debug_coop_prof": (c_int32, [_P]),
     "rtd3_td3_cluster_supported": (c_int32, [_P, c_int32]),
     "rtd3_td3_cluster_occupancy": (c_int32, [_P, c_int32]),
     "rtd3_debug_cluster_prof": (c_int32, [_P, _P]),

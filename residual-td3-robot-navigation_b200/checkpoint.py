@@ -33,7 +33,7 @@ NOT_SAVED = {
             "params_u": "rebuilt: tensor-core operand copies (rtd3_tc_sync_weights)",
             "params_h": "rebuilt: fp16 weight copies (rtd3_tc_sync_weights_f16)",
             "grads": "scratch: written by every step before it is read", "_scratch": "row scratch", "_scratch_retired": "row scratch",
-            "_graphs": "captured update graphs and their buffers", "_coop_scratch": "cooperative-kernel scratch",
+            "_graphs": "captured update graphs and their buffers",
             "_grads_sum": "peer-memory exchange: process-local", "_p2p": "peer-memory receive areas, flags and seq: process-local"},
     "Environment": {"_speed_dev": "stored under this name unless map_seeds rebuild the bank", "_angle_dev": "as _speed_dev",
                     "_cem": "planner scratch", "_pipe_buf": "host-rollout staging"},

@@ -17,8 +17,6 @@
 // copies (an issue costs ~100 cycles per bulk copy, 16 per tile).  The per-row layer inputs / pre-activation gradients go to the same
 // row scratch as before; wgrad_kernel (+ fused Adam) consumes them.
 #include <algorithm>
-#include <cstdlib>
-#include <type_traits>
 
 #include "rtd3_common.cuh"
 #include "rtd3_mlp.cuh"
@@ -795,82 +793,48 @@ td3_actor_cluster_kernel(Arena ar, const float* __restrict__ params, const float
 using namespace rtd3;
 
 namespace {
-// RTD3_CLUSTER environment variable: 0 = never; "R,CS" forces rows per cluster and cluster size (development); unset: see cluster_shape
-int g_mode = -1, g_force_r = 0, g_force_cs = 0;
-void read_mode() {
-  if (g_mode >= 0) return;
-  const char* e = getenv("RTD3_CLUSTER");
-  g_mode = 2;
-  if (e) {
-    int r = 0, cs = 0;
-    if (sscanf(e, "%d,%d", &r, &cs) == 2 && (r == 8 || r == 16) && (cs == 4 || cs == 8)) { g_force_r = r; g_force_cs = cs; g_mode = 1; }
-    else g_mode = atoi(e) ? 2 : 0;
-  }
-}
-struct ClShape { int R, CS; };
+int g_mode = 2;   // rtd3_debug_cluster_mode: 0 = never, 2 = wherever the plan fits and the batch is one wave of clusters
 // clusters of 4 with 8 rows: 32 clusters for the benchmark batch of 256 (the device holds 33 of them at once, but only 15 clusters
 // of 8); larger batches run in several waves (16 rows per cluster do not fit the shared memory next to two 64 KB weight tiles)
-ClShape cluster_shape(int batch) {
-  read_mode();
-  if (g_mode == 1) return ClShape{g_force_r, g_force_cs};
-  (void)batch;
-  return ClShape{8, 4};
-}
+constexpr int kClR = 8, kClCS = 4;
 long long* g_prof[2] = {nullptr, nullptr};   // development: stamp buffers of the critic / actor kernels (rtd3_debug_cluster_prof)
-
-template <typename F>
-int32_t dispatch(const ClShape& s, F&& f) {
-  if (s.R == 8 && s.CS == 4) return f(std::integral_constant<int, 8>{}, std::integral_constant<int, 4>{});
-  if (s.R == 16 && s.CS == 4) return f(std::integral_constant<int, 16>{}, std::integral_constant<int, 4>{});
-  if (s.R == 8 && s.CS == 8) return f(std::integral_constant<int, 8>{}, std::integral_constant<int, 8>{});
-  return f(std::integral_constant<int, 16>{}, std::integral_constant<int, 8>{});
-}
 }  // namespace
 
 // The cluster kernels win while the batch is ONE wave of clusters (B = 256: 32 of the 33 clusters a B200 holds; 47.9 against 77.5 us
 // per epoch); from the second wave on the row-tile kernels are faster again (B = 512: 88.4 against 83.9, B = 1024: 171.8 against
 // 120.7 us per epoch), so larger batches keep them.
 bool rtd3::cluster_path_ok(const rtd3_td3* h, int batch) {
-  read_mode();
   if (g_mode == 0) return false;
-  const ClShape s = cluster_shape(batch);
   const int H = h->ar.critic.hid, L = h->ar.critic.layers;
   if (H % 4 != 0 || H < 4) return false;
-  if (make_plan(s.R, s.CS, H, L, 5, L).bytes > kClSmemLimit || make_plan(s.R, s.CS, H, L, 2, 2 * L).bytes > kClSmemLimit) return false;
-  if (g_mode == 2 && ceil_div(batch, s.R) > h->cluster_cap) return false;
-  return true;
+  if (make_plan(kClR, kClCS, H, L, 5, L).bytes > kClSmemLimit || make_plan(kClR, kClCS, H, L, 2, 2 * L).bytes > kClSmemLimit) return false;
+  return ceil_div(batch, kClR) <= h->cluster_cap;
 }
 
 int32_t rtd3::critic_cluster_launch(rtd3_td3* h, const float* params, const float* params_t, float* scratch, const ReplayView& rp, const int32_t* idx,
                                     const float* noise, int32_t batch, const Td3Hyper& hp, float* loss2, float* q_out, float* y_out, int32_t* steps,
                                     double* beta_pows, cudaStream_t st) {
-  const ClShape s = cluster_shape(batch);
   const int H = h->ar.critic.hid, L = h->ar.critic.layers;
-  const ClPlan p = make_plan(s.R, s.CS, H, L, 5, L);
-  const int grid = (int)ceil_div(batch, s.R) * s.CS;
-  return dispatch(s, [&](auto r, auto cs) -> int32_t {
-    auto* fn = td3_critic_cluster_kernel<decltype(r)::value, decltype(cs)::value>;
-    RTD3_CUDA(ensure_dyn_smem((const void*)fn, p.bytes));
-    fn<<<grid, kClBlock, p.bytes, st>>>(h->ar, params, params_t, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows, p.ns,
-                                        g_prof[0]);
-    RTD3_LAUNCHED();
-    return 0;
-  });
+  const ClPlan p = make_plan(kClR, kClCS, H, L, 5, L);
+  const int grid = (int)ceil_div(batch, kClR) * kClCS;
+  auto* fn = td3_critic_cluster_kernel<kClR, kClCS>;
+  RTD3_CUDA(ensure_dyn_smem((const void*)fn, p.bytes));
+  fn<<<grid, kClBlock, p.bytes, st>>>(h->ar, params, params_t, scratch, rp, idx, noise, batch, hp, loss2, q_out, y_out, steps, beta_pows, p.ns,
+                                      g_prof[0]);
+  RTD3_LAUNCHED();
+  return 0;
 }
 
 int32_t rtd3::actor_cluster_launch(rtd3_td3* h, const float* params, const float* params_t, float* scratch, const ReplayView& rp, const int32_t* idx,
                                    int32_t batch, float* loss1, int32_t* steps, double* beta_pows, cudaStream_t st) {
-  const ClShape s = cluster_shape(batch);
   const int H = h->ar.critic.hid, L = h->ar.critic.layers;
-  const ClPlan p = make_plan(s.R, s.CS, H, L, 2, 2 * L);
-  const int grid = (int)ceil_div(batch, s.R) * s.CS;
-  return dispatch(s, [&](auto r, auto cs) -> int32_t {
-    auto* fn = td3_actor_cluster_kernel<decltype(r)::value, decltype(cs)::value>;
-    RTD3_CUDA(ensure_dyn_smem((const void*)fn, p.bytes));
-    fn<<<grid, kClBlock, p.bytes, st>>>(h->ar, params, params_t, scratch, rp, idx, batch, loss1, steps, beta_pows, p.ns, g_prof[1]);
-    RTD3_LAUNCHED();
-    return 0;
-  });
+  const ClPlan p = make_plan(kClR, kClCS, H, L, 2, 2 * L);
+  const int grid = (int)ceil_div(batch, kClR) * kClCS;
+  auto* fn = td3_actor_cluster_kernel<kClR, kClCS>;
+  RTD3_CUDA(ensure_dyn_smem((const void*)fn, p.bytes));
+  fn<<<grid, kClBlock, p.bytes, st>>>(h->ar, params, params_t, scratch, rp, idx, batch, loss1, steps, beta_pows, p.ns, g_prof[1]);
+  RTD3_LAUNCHED();
+  return 0;
 }
 
 extern "C" {
@@ -879,31 +843,27 @@ int32_t rtd3_td3_cluster_supported(const rtd3_td3* h, int32_t batch) { return (h
 
 int32_t rtd3_td3_cluster_occupancy(const rtd3_td3* h, int32_t batch) {
   if (!h || batch <= 0) return -1;
-  const ClShape s = cluster_shape(batch);
   const int H = h->ar.critic.hid, L = h->ar.critic.layers;
-  const ClPlan p = make_plan(s.R, s.CS, H, L, 5, L);
-  if (H % 4 != 0 || H < 4 || p.bytes > kClSmemLimit || make_plan(s.R, s.CS, H, L, 2, 2 * L).bytes > kClSmemLimit) return 0;   // no plan: no clusters
-  return dispatch(s, [&](auto r, auto cs) -> int32_t {
-    auto* fn = td3_critic_cluster_kernel<decltype(r)::value, decltype(cs)::value>;
-    if (ensure_dyn_smem((const void*)fn, p.bytes) != cudaSuccess) { (void)cudaGetLastError(); return -2; }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(ceil_div(batch, s.R) * s.CS), 1, 1);
-    cfg.blockDim = dim3(kClBlock, 1, 1);
-    cfg.dynamicSmemBytes = p.bytes;
-    cudaLaunchAttribute attr;
-    attr.id = cudaLaunchAttributeClusterDimension;
-    attr.val.clusterDim.x = (unsigned)s.CS; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
-    cfg.attrs = &attr;
-    cfg.numAttrs = 1;
-    int n = 0;
-    const cudaError_t e = cudaOccupancyMaxActiveClusters(&n, fn, &cfg);
-    if (e != cudaSuccess) { (void)cudaGetLastError(); rtd3::set_error("cudaOccupancyMaxActiveClusters: %s", cudaGetErrorString(e)); return -3; }
-    return n;
-  });
+  const ClPlan p = make_plan(kClR, kClCS, H, L, 5, L);
+  if (H % 4 != 0 || H < 4 || p.bytes > kClSmemLimit || make_plan(kClR, kClCS, H, L, 2, 2 * L).bytes > kClSmemLimit) return 0;   // no plan: no clusters
+  auto* fn = td3_critic_cluster_kernel<kClR, kClCS>;
+  if (ensure_dyn_smem((const void*)fn, p.bytes) != cudaSuccess) { (void)cudaGetLastError(); return -2; }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)(ceil_div(batch, kClR) * kClCS), 1, 1);
+  cfg.blockDim = dim3(kClBlock, 1, 1);
+  cfg.dynamicSmemBytes = p.bytes;
+  cudaLaunchAttribute attr;
+  attr.id = cudaLaunchAttributeClusterDimension;
+  attr.val.clusterDim.x = (unsigned)kClCS; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
+  cfg.attrs = &attr;
+  cfg.numAttrs = 1;
+  int n = 0;
+  const cudaError_t e = cudaOccupancyMaxActiveClusters(&n, fn, &cfg);
+  if (e != cudaSuccess) { (void)cudaGetLastError(); rtd3::set_error("cudaOccupancyMaxActiveClusters: %s", cudaGetErrorString(e)); return -3; }
+  return n;
 }
 
 int32_t rtd3_debug_cluster_mode(int32_t mode) {
-  read_mode();
   const int prev = g_mode;
   if (mode == 0 || mode == 2) g_mode = mode;
   return prev;

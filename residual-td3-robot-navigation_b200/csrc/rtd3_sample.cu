@@ -10,9 +10,8 @@
 //      (lane L's decision depends only on lanes < L, so the fixed point is the sequential answer).
 //   2. nothing else: the B outputs do not need the permutation.  Output p is found by walking the swap list
 //      BACKWARDS from position p (pos==i -> j_i, pos==j_i -> i), independently per output and per sample.
-// Kernel A (1 CTA) writes the swap lists J[s][i]; kernel B (one CTA per sample) back-traces the B outputs.
-#include <cstdlib>
-
+// Kernel A (sample_swaps_pipelined_kernel, one CTA) writes the swap lists J[s][i]; kernel B (sample_trace_kernel, one CTA per sample)
+// back-traces the B outputs.
 #include "rtd3_common.cuh"
 #include "rtd3_mt.cuh"
 
@@ -23,194 +22,37 @@ __device__ __forceinline__ uint32_t mt_twist(uint32_t cur, uint32_t nxt, uint32_
   return far ^ (y >> 1) ^ ((y & 1u) ? 0x9908b0dfu : 0u);
 }
 
-// mt19937_gen by one warp, in place, 32 words at a time: read, __syncwarp, write.  The three ranges differ only in
-// where word kk+397 (mod 624) comes from; word 623 pairs with the NEW word 0, as in the reference implementation.
-__device__ void mt_regenerate_warp(uint32_t* mt, int lane) {
-  constexpr int N = RTD3_MT_N, M = 397;
-  for (int base = 0; base < N; base += 32) {
-    const int kk = base + lane;
-    uint32_t v = 0;
-    if (kk < N) {
-      const uint32_t cur = mt[kk];
-      const uint32_t nxt = mt[kk + 1 < N ? kk + 1 : 0];      // kk = 623 reads word 0, already regenerated
-      const uint32_t far = mt[kk + M < N ? kk + M : kk + M - N];
-      v = mt_twist(cur, nxt, far);
-    }
-    __syncwarp();
-    if (kk < N) mt[kk] = v;
-    __syncwarp();
-  }
-}
-
-// Kernel A: swap lists.  J[s*n + i] = j_i for i = 1..n-1 (entry 0 unused).  One CTA of 256 threads.
-//
-// A round takes up to 256 consecutive raw draws, thread t owning draw t.  With i swaps still to draw, thread t's bound
-// (i minus the number of accepted draws before it) lies in [i - t, i].  If the mask is the same at both ends the draw is
-// classified without knowing the exact bound: v <= i - t  -> accepted whatever happened before ("sure"),
-// v > i -> rejected, in between -> "maybe" (a band of at most t values out of >= 2^k, ~1 % of the draws).  Threads whose
-// range crosses a power of two are maybes too; the round is sized (32..256) so that there are at most 32 of those.  One
-// block scan ranks the sure draws; thread 0 then resolves the few maybes in order with their exact bounds, and a second
-// pass adds the accepted maybes into every thread's rank.  The round ends early at the draw that completes a sample.
-// (Round 2 tried 1024-draw rounds over a ring of four generator states, so that no round stops at the end of a 624-word block:
-// 14.1 ms per 150 draws against 13.3 here, and 16.0 with the round sized to keep ~32 draws undecided - the number of undecided
-// draws grows with the square of the round, and they are resolved by ONE warp; the serial resolver, not the round count, is the
-// floor.  A third variant decided the undecided draws block-parallel from their bound intervals [i - S - m, i - S] (the serial
-// resolver then runs only when a value falls inside its own window, ~never) with rounds of 2^(lvl-2) draws: bit-exact as well, and
-// 18.2 ms - a 1024-thread round costs ~3 us against ~1.5 us for a 256-thread round and the low mask levels force small rounds
-// either way.  gpurun_out/r2 sampler logs, git history (57e703c, the commit before this text); the version below is the fastest.)
-#ifndef RTD3_SAMPLE_THREADS
-#define RTD3_SAMPLE_THREADS 256
-#endif
-constexpr int kSampleThreads = RTD3_SAMPLE_THREADS;
-constexpr int kSampleWarps = kSampleThreads / 32;
-
-__device__ __forceinline__ void mt_regenerate_block(uint32_t* mt, uint32_t* raw, int t) {
-  constexpr int N = RTD3_MT_N, M = 397;
-  const int lo[3] = {0, N - M, 2 * (N - M)}, hi[3] = {N - M, 2 * (N - M), N};
-#pragma unroll
-  for (int ph = 0; ph < 3; ++ph) {               // every range reads only words finished by earlier ranges (or still old)
-    // a range is at most 227 words: with fewer threads each one handles several, all read before any is written
-    uint32_t v[4];
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      const int kk = lo[ph] + t + q * kSampleThreads;
-      v[q] = (kk < hi[ph]) ? mt_twist(mt[kk], mt[kk + 1 < N ? kk + 1 : 0], mt[kk + M < N ? kk + M : kk + M - N]) : 0u;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int q = 0; q < 4; ++q) {
-      const int kk = lo[ph] + t + q * kSampleThreads;
-      if (kk < hi[ph]) mt[kk] = v[q];
-    }
-    __syncthreads();
-  }
-  for (int k = t; k < N; k += kSampleThreads) raw[k] = mt_temper(mt[k]);
-  __syncthreads();
-}
-
-__global__ void __launch_bounds__(kSampleThreads)
-sample_swaps_kernel(rtd3_mt_bank b, int64_t stream_id, int32_t n, int32_t count, int32_t* __restrict__ J) {
-  __shared__ uint32_t mt[RTD3_MT_N], raw[RTD3_MT_N];
-  __shared__ int w_sure[2][8], w_maybe[2][8], w_macc[2][8];
-  __shared__ int m_S[kSampleThreads], m_acc[kSampleThreads];
-  __shared__ uint32_t m_raw[kSampleThreads];
-  __shared__ int s_last[2], s_macc_total[2];
-  int par = 0;                                       // round parity: control words alternate between two buffers
-  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
-  const uint32_t lt = (1u << lane) - 1u;
-  for (int k = t; k < RTD3_MT_N; k += kSampleThreads) {
-    mt[k] = b.mt[(int64_t)k * b.n + stream_id];
-    raw[k] = mt_temper(mt[k]);
-  }
-  int pos = b.pos[stream_id];
-  if (t == 0) { s_last[0] = -1; s_macc_total[0] = 0; }
-  __syncthreads();
-
-  for (int s = 0; s < count; ++s) {
-    int32_t* Js = J + (int64_t)s * n;
-    int i = n - 1;                                  // swaps still to draw: indices i, i-1, ..., 1 (same value in every thread)
-    while (i >= 1) {
-      if (pos >= RTD3_MT_N) {
-        mt_regenerate_block(mt, raw, t);
-        pos = 0;
-      }
-      // round size: stay on one mask level while the distance to the next power of two allows rounds of >= 32 draws
-      const int lvl = 31 - __clz(i);                // mask(i) = 2^(lvl+1) - 1
-      const int gap = i - (1 << lvl);               // bounds down to i - gap keep mask(i)
-      const int gmax = kSampleThreads;
-      const int g = min(min(max(gap + 1, 32), gmax), RTD3_MT_N - pos);
-      const bool active = t < g;
-      const uint32_t rw = active ? raw[pos + t] : 0u;
-      const int lo = i - t;                          // bound if every earlier draw of the round was accepted
-      const bool uniform = lo >= 1 && __clz(lo) == __clz(i);
-      const uint32_t v_hi = rw & (0xffffffffu >> __clz(i));
-      const bool sure = active && uniform && (int)v_hi <= lo;
-      const bool maybe = active && !sure && lo < i && ((uniform && (int)v_hi <= i) || (!uniform && i - t < i));
-      const uint32_t bs = __ballot_sync(0xffffffffu, sure), bm = __ballot_sync(0xffffffffu, maybe);
-      if (lane == 0) { w_sure[par][warp] = __popc(bs); w_maybe[par][warp] = __popc(bm); }
-      if (t == 0) { s_last[par ^ 1] = -1; s_macc_total[par ^ 1] = 0; }   // next round's words (nobody reads them now)
-      __syncthreads();
-      int S = __popc(bs & lt), mpos = __popc(bm & lt), total_sure = 0, total_maybe = 0;
-#pragma unroll
-      for (int w = 0; w < kSampleWarps; ++w) {
-        if (w < warp) { S += w_sure[par][w]; mpos += w_maybe[par][w]; }
-        total_sure += w_sure[par][w];
-        total_maybe += w_maybe[par][w];
-      }
-      int rank = S;
-      bool accepted = sure;
-      uint32_t v = v_hi;
-      if (total_maybe > 0) {                         // block-uniform branch
-        if (maybe) { m_S[mpos] = S; m_raw[mpos] = rw; }   // compacted in stream order
-        __syncthreads();
-        if (warp == 0) {
-          // the undecided draws, 32 at a time: bound_q = i - (sure draws before q) - (accepted undecided draws before q);
-          // the last term is resolved by iterating the ballot to its fixed point (lane L depends only on lanes < L)
-          int extra = 0;
-          for (int q0 = 0; q0 < total_maybe; q0 += 32) {
-            const int q = q0 + lane;
-            const bool on = q < total_maybe;
-            const int Sq = on ? m_S[q] : 0;
-            const uint32_t rq = on ? m_raw[q] : 0u;
-            uint32_t acc = 0u, prev;
-            do {
-              prev = acc;
-              const int bound = i - Sq - extra - __popc(prev & lt);
-              const bool a = on && bound >= 1 && (int)(rq & (0xffffffffu >> __clz(max(bound, 1)))) <= bound;
-              acc = __ballot_sync(0xffffffffu, a);
-            } while (acc != prev);
-            if (on) m_acc[q] = (acc >> lane) & 1;
-            extra += __popc(acc);
-          }
-          if (lane == 0) s_macc_total[par] = extra;
-        }
-        __syncthreads();
-        const bool macc = maybe && m_acc[mpos] != 0;
-        const uint32_t ba = __ballot_sync(0xffffffffu, macc);
-        if (lane == 0) w_macc[par][warp] = __popc(ba);
-        __syncthreads();
-        int before = __popc(ba & lt);
-#pragma unroll
-        for (int w = 0; w < kSampleWarps; ++w)
-          if (w < warp) before += w_macc[par][w];
-        rank = S + before;
-        if (maybe) {
-          accepted = macc;
-          v = rw & (0xffffffffu >> __clz(max(i - rank, 1)));
-        }
-      }
-      const int my_i = i - rank;
-      const bool valid = accepted && my_i >= 1;
-      if (valid) {
-        Js[my_i] = (int32_t)v;
-        if (my_i == 1) s_last[par] = t;              // the draw that completes this sample
-      }
-      __syncthreads();
-      const int total_acc = total_sure + s_macc_total[par];
-      const int last = s_last[par];
-      par ^= 1;
-      if (total_acc >= i) { pos += last + 1; i = 0; }
-      else { pos += g; i -= total_acc; }
-    }
-  }
-  for (int k = t; k < RTD3_MT_N; k += kSampleThreads) b.mt[(int64_t)k * b.n + stream_id] = mt[k];
-  if (t == 0) b.pos[stream_id] = pos;
-}
-
-// ---- Kernel A, pipelined form (the default) -------------------------------------------------------------------------------------------
-// The same classification, restructured around what made a round cost ~1.3 us (10 000 rounds per 150 samples of 10 000):
-//  * the generator runs in its OWN warps (threads 256..511): they twist and temper block after block into a ring of four 624-word
-//    blocks (full / empty mbarriers), so a round never stops at the end of a block and never waits for a twist;
+// ---- Kernel A: swap lists.  J[s*n + i] = j_i for i = 1..n-1 (entry 0 unused) --------------------------------------------------------
+// A round takes up to 32 NW consecutive raw draws, consumer thread t owning draw t.  With i swaps still to draw, thread t's bound
+// (i minus the number of accepted draws before it) lies in [i - t, i].  If the mask is the same at both ends the draw is classified
+// without knowing the exact bound: v <= i - t  -> accepted whatever happened before ("sure"), v > i -> rejected, in between ->
+// undecided (a band of at most t values out of >= 2^k, ~1 % of the draws); threads whose range crosses a power of two are undecided
+// too.  The sure draws are ranked by ballot counts, the undecided ones resolved in stream order with their exact bounds, and the round
+// ends early at the draw that completes a sample.
+// A first, block-per-round form of this kernel (256 threads that also twisted the generator whenever a 624-word block ran out, and
+// compacted the undecided draws for ONE resolver warp between block barriers) took 13.3 ms per 150 draws of 10 000 rows: ~1.3 us per
+// round, 10 000 rounds.  This kernel is the same classification restructured around what made a round cost that much (8.75 ms):
+//  * the generator runs in its OWN warps (threads 32 NW .. 32 NW + 255): they twist and temper block after block into a ring of six
+//    624-word blocks (full / empty mbarriers), so a round never stops at the end of a block and never waits for a twist;
 //  * ONE block barrier per round: before it, every warp publishes its count of sure draws and its undecided draws (value + sure
 //    draws before it inside the warp); after it, EVERY warp resolves the undecided draws of the round with the ballot fixed point -
 //    redundantly - instead of compaction, a resolver warp and three more barriers (a per-thread serial walk over them was tried
 //    first: 2 000 of a round's 2 900 cycles);
 //  * smaller rounds only at the lowest mask levels, where the undecided band is wide.
-// Also tried, both bit-exact and both slower or equal: (a) ONE consumer warp with eight consecutive draws per lane, every prefix from
-// per-slot ballots, rounds cut at the mask level, no block barrier at all - 27 ms: ~600 dependent instructions per lane and round on a
-// single warp run at 4-6 cycles each, where eight warps with one draw per lane and one barrier need 1 650 cycles; (b) undecided draws
-// that decide themselves from their exact interval [i - S - M, i - S] plus a second barrier for the counts, the walk only for a
-// truly undecided draw - 8.9 ms against 8.75: the walk was not what a round waits for.
+// Also tried, all bit-exact and all slower or equal:
+//  (a) ONE consumer warp with eight consecutive draws per lane, every prefix from per-slot ballots, rounds cut at the mask level, no
+//      block barrier at all - 27 ms: ~600 dependent instructions per lane and round on a single warp run at 4-6 cycles each, where
+//      eight warps with one draw per lane and one barrier need 1 650 cycles;
+//  (b) undecided draws that decide themselves from their exact interval [i - S - M, i - S] plus a second barrier for the counts, the
+//      walk only for a truly undecided draw - 8.9 ms against 8.75: the walk was not what a round waits for;
+//  (c) 16 consumer warps (512-draw rounds) - 12.2 ms against 8.75;
+//  (d) in the block-per-round form, 1024-draw rounds over a ring of four generator states, so that no round stops at the end of a
+//      624-word block: 14.1 ms against 13.3, and 16.0 with the round sized to keep ~32 draws undecided - the number of undecided
+//      draws grows with the square of the round, and they were resolved by ONE warp; the serial resolver, not the round count, was
+//      the floor.  And undecided draws decided block-parallel from their bound intervals [i - S - m, i - S] (the serial resolver then
+//      ran only when a value fell inside its own window, ~never) with rounds of 2^(lvl-2) draws: 18.2 ms - a 1024-thread round costs
+//      ~3 us against ~1.5 us for a 256-thread round and the low mask levels force small rounds either way.
+// The block-per-round kernel and the 16-warp instantiation are in the tree at 8344fb3, the variants of (d) at 57e703c.
 // The state written back is the un-tempered ring block the stream ended in.
 constexpr int kRing = 6;
 constexpr int kRingWords = kRing * RTD3_MT_N;
@@ -480,11 +322,7 @@ extern "C" int32_t rtd3_sample_indices_mt19937(const rtd3_mt_bank* bank, int64_t
   RTD3_CHECK_ARG(scratch, "scratch (count * n int32) is required");
   RTD3_CUDA(ensure_dyn_smem((const void*)sample_trace_kernel, 56000 * 4));
   cudaStream_t st = (cudaStream_t)stream;
-  static const bool legacy = getenv("RTD3_SAMPLER_LEGACY") != nullptr;      // development: the block-per-round form above
-  static const bool wide = getenv("RTD3_SAMPLER_WIDE") != nullptr;          // 512-draw rounds: measured slower (12.2 against 8.75 ms)
-  if (legacy) sample_swaps_kernel<<<1, kSampleThreads, 0, st>>>(*bank, stream_id, n, count, scratch);
-  else if (wide) sample_swaps_pipelined_kernel<16><<<1, 16 * 32 + 256, 0, st>>>(*bank, stream_id, n, count, scratch);
-  else sample_swaps_pipelined_kernel<8><<<1, 8 * 32 + 256, 0, st>>>(*bank, stream_id, n, count, scratch);
+  sample_swaps_pipelined_kernel<8><<<1, 8 * 32 + 256, 0, st>>>(*bank, stream_id, n, count, scratch);
   RTD3_LAUNCHED();
   const size_t smem = (size_t)((n + 3) & ~3) * 4;
   sample_trace_kernel<<<count, 256, smem, st>>>(scratch, n, batch, out);

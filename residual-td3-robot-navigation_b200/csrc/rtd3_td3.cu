@@ -687,9 +687,7 @@ using namespace rtd3;
 
 // Rows per CTA: few rows while the batch cannot fill the SMs (latency-bound), more rows once it can (every CTA
 // re-streams all weights from L2, so larger tiles cut that traffic).
-static int g_tile_override = -1;   // development hook (RTD3_TILE environment variable): force a row-tile index
 static inline int pick_tile(int64_t B, int num_sms) {
-  if (g_tile_override >= 0) return g_tile_override;
   if (B <= 2 * (int64_t)num_sms) return 0;
   if (B <= 4 * (int64_t)num_sms) return 1;
   if (B <= 16 * (int64_t)num_sms) return 2;
@@ -814,7 +812,6 @@ int32_t rtd3_td3_create(rtd3_td3** out, int32_t device, int32_t hidden, int32_t 
     RTD3_CUDA(set_smem(kActorKernels[i], h->smem_actor[i]));
     RTD3_CUDA(set_smem(kFwdKernels[i], h->smem_fwd[i]));
   }
-  if (const char* e = getenv("RTD3_TILE")) g_tile_override = atoi(e);
   h->cluster_cap = std::max(0, rtd3_td3_cluster_occupancy(h, 256));     // (queried here, never inside a stream capture)
   RTD3_CUDA(cudaSetDevice(prev));
   if (!g_p2p_prof && getenv("RTD3_P2P_PROF") && atoi(getenv("RTD3_P2P_PROF")) == 1) {      // development: stage stamps of the fused exchange

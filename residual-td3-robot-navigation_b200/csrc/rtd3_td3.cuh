@@ -258,7 +258,7 @@ struct rtd3_td3 {
   int cluster_cap;      // clusters of the cluster step kernels the device holds at once (set by rtd3_td3_create; 0: path unavailable)
 };
 
-// the optimiser state of an update call (rtd3_td3_update, rtd3_td3_update_coop)
+// the optimiser state of an update call (rtd3_td3_update)
 inline rtd3::AdamState adam_state(const rtd3_td3* h, const rtd3_td3_update_args* a) {
   return rtd3::AdamState{h->ar, a->params, a->params_t, a->params_uv, a->adam_m, a->adam_v, a->beta_pows, {a->lr_actor, a->lr_critic}, a->tau};
 }

@@ -365,13 +365,6 @@ class TD3:
         self._graphs = {}
         self._p2p = None
         self._comm = None
-        # "steps": the per-step kernels of rtd3_td3.cu behind rtd3_td3_update (the default: the faster form today);
-        # "coop": ONE persistent cooperative kernel per update (csrc/rtd3_coop.cu: layers tiled over all SMs, grid barriers between
-        # them, optimiser and peer-memory all-reduce inside) whenever it applies - fp32, layers >= 2, batch <= 4096, single GPU or
-        # the peer-memory collective.  Parity-green, but its ~12 grid barriers (2.5 us each) and latency-bound small stages make an
-        # epoch 140 us against 79 us at B = 256 (profiles/r2_coop_stage_profile.md): opt-in until that is fixed.
-        self.update_kernel = "steps"
-        self._coop_scratch = {}
         # target-policy smoothing noise (robot.py:338, torch.randn_like - unseeded in the reference): generated inside the critic
         # kernels from Philox4x32-10 keyed (noise_seed, device step counter, batch row) unless a noise tensor is injected
         self.noise_seed = 0x7d3
@@ -728,9 +721,6 @@ class TD3:
         critic kernels (Philox, keyed by the device step counter, which the call advances)."""
         B = idx.shape[1]
         tc = self._tc_learner_ok(B)
-        coop = self._coop_ok(B)
-        if coop:
-            self._u_stale = True                                     # the cooperative kernel keeps params / params_t only
         keep_uv = self.params_u is not None and not self._u_stale
         if tc and not keep_uv:
             raise RuntimeError("tensor-core operand copies are stale: call _sync_chunk_major() first")
@@ -752,24 +742,12 @@ class TD3:
         a.comm = self._comm if (self.world > 1 and self._p2p is None) else None
         if self.world > 1 and self._p2p is not None:
             a.p2p = ctypes.pointer(self._p2p["struct"])
-        if coop:
-            _lib.check(_lib.lib().rtd3_td3_update_coop(self._handle, ctypes.byref(a), _lib.ptr(self._coop_buffer(B)), _lib.stream_ptr(self.device)),
-                       "td3_update_coop")
-            return
         _lib.check(_lib.lib().rtd3_td3_update(self._handle, ctypes.byref(a), _lib.stream_ptr(self.device)), "td3_update")
 
     def _coop_ok(self, B):
-        return (self.update_kernel == "coop" and not self._tc_learner_ok(B) and (self.world == 1 or self._p2p is not None)
-                and bool(_lib.lib().rtd3_td3_coop_supported(self._handle, B)))
-
-    def _coop_buffer(self, B):
-        """Activation scratch + grid-barrier words of the cooperative kernel for batch B: zero-initialised once, then owned by the
-        kernel (captured graphs hold its address: never freed while the learner lives)."""
-        buf = self._coop_scratch.get(B)
-        if buf is None:
-            n = int(_lib.lib().rtd3_td3_coop_scratch_floats(self._handle, B))
-            buf = self._coop_scratch[B] = torch.zeros((n,), dtype=torch.float32, device=self.device)
-        return buf
+        # The cooperative single-kernel update was removed (slower than the step kernels at every measured batch,
+        # profiles/r2_coop_stage_profile.md); bench.py still asks this to label its TD3 rows.
+        return False
 
     def td3_update(self, replay_buffer, noise=None, idx=None, use_graph=True):
         """robot.py:258-285: `num_epochs` critic steps, an actor step + the three Polyak updates every
@@ -803,7 +781,7 @@ class TD3:
     def _update_state(self, replay_buffer, E, B, delay, injected_noise=False):
         """Persistent buffers (and, once captured, the CUDA graph) of an E-epoch block for this replay buffer / batch size."""
         n_actor = len([e for e in range(E) if e % delay == 0])
-        key = (id(replay_buffer), E, B, delay, self.precision, self._tc_learner_ok(B), bool(injected_noise), self._coop_ok(B))
+        key = (id(replay_buffer), E, B, delay, self.precision, self._tc_learner_ok(B), bool(injected_noise))
         st = self._graphs.get(key)
         if st is None:
             st = {"idx": torch.zeros((E + n_actor, B), dtype=torch.int32, device=self.device),
@@ -811,8 +789,6 @@ class TD3:
                   "closs": torch.zeros((E, 2), dtype=torch.float32, device=self.device),
                   "aloss": torch.zeros((max(1, n_actor),), dtype=torch.float32, device=self.device), "graph": None, "launches": 0}
             self._row_scratch(B)
-            if self._coop_ok(B):
-                self._coop_buffer(B)                                 # allocated (and zeroed) outside of the graph capture
             self._graphs[key] = st
         return st
 

@@ -262,7 +262,7 @@ def snapshot(robot, tr=None):
     out = _tensors(robot, "robot.", {}, skip=("_eval_graphs", "_eval_work"))
     _tensors(robot.memory, "memory.", out)
     _tensors(robot._bank, "bank.", out)
-    _tensors(robot.td3_agent, "td3.", out, skip=("params_t", "params_u", "params_h", "_graphs", "_scratch", "_coop_scratch"))
+    _tensors(robot.td3_agent, "td3.", out, skip=("params_t", "params_u", "params_h", "_graphs", "_scratch"))
     if tr is not None:
         _tensors(tr, "trainer.", out, skip=("_graph", "_graph_k"))
     out["counts"] = (robot.num_updates, len(robot.memory), tr.ticks if tr is not None else 0)

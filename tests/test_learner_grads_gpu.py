@@ -7,7 +7,7 @@ of zero), with duplicate rows and rows with `done` set.  Q-values, targets and c
 actor loss is checked against tau * mean |Q|_abs.
   - The raw fp32 step kernels (`_critic_step(apply=False)`, `_actor_step`) at every dispatch boundary: the cluster kernels, the row
     tiles R = 2 / 4 / 8 / 16 (boundaries at 2, 4 and 16 times the SM count) and the weight-gradient batch split above 512 rows.
-  - The production update paths (fused optimiser at B <= 512, unfused above, the cooperative kernel, TF32), with and without the
+  - The production update paths (fused optimiser at B <= 512, unfused above, TF32), with and without the
     CUDA graph.  They expose no gradients, but one epoch from a fresh agent leaves adam_m = RN(0.1f * g), so g = adam_m / 0.1f to one
     ulp.  The actor step of an update reads critic 1 after the critics' Adam step, so its reference uses the final critic 1.
   - Controls: every fp32 case also checks that the bar REJECTS a subtly wrong reference (a dropped row, one `done` flipped, max
@@ -16,7 +16,7 @@ actor loss is checked against tau * mean |Q|_abs.
 Measured on a B200 (1000 W power limit), worst |x - x64| / M over the cases of this file:
   fp32 step kernels, gradients: cluster 1.5e-7 (the 4-wide net; 1.5e-8 at H >= 64), R=2 1.5e-7 (same), R=4 6.5e-9,
     R=4 with the batch split 1.5e-8, R=8 split 3.9e-8, R=16 split 1.6e-8; Q 7.5e-8, y 3.7e-8, critic loss 2.1e-8, actor loss 7e-9
-  update paths, gradients from adam_m: fused 7.6e-9, unfused 8.4e-9, cooperative 1.8e-8, TF32 3.3e-3 (H = 256, B = 8192; 1.5e-4 at
+  update paths, gradients from adam_m: fused 7.6e-9, unfused 8.4e-9, TF32 3.3e-3 (H = 256, B = 8192; 1.5e-4 at
     H = 128, B = 1041)
   controls (fp32), smallest distance from the kernel's gradient: 9.3e-7 (one `done` flipped, H = 200, L = 3, B = 2368)
 TAU_FP32 = 2^-21 sits between the two: far below the 2^-15 that fp32 summation-error arithmetic allows, because the magnitude sums
@@ -26,7 +26,7 @@ vectors where nothing rounds (oracle/exact_grid.py) the TF32 critic step, actor 
 bit for bit, and tests/test_exact_grid.py checks that every one of these controls changes that reference.
 
 Optimiser: the Adam / Polyak kernel, element for element against oracle/td3_oracle.py's adam_step / soft_update (pinned to
-torch.optim.Adam), with lr a Python float as in torch, and the Adam step of the fused, cooperative and TF32 update paths against the
+torch.optim.Adam), with lr a Python float as in torch, and the Adam step of the fused and TF32 update paths against the
 same formula on the device's own moments; the kernels that rebuild the derived weight copies from the whole arena against their layouts.
 """
 import numpy as np
@@ -201,16 +201,13 @@ def test_step_kernel_gradients_vs_float64(pkg, case):
 
 # ---------------------------------------------------------------------------------------------------- (b) the update paths
 UPDATE_CASES = [
-    ("fused", 256, 2, 256), ("fused", 200, 3, 100), ("unfused", 256, 2, 600), ("unfused", 200, 3, 1041), ("coop", 256, 2, 256),
-    ("coop", 200, 3, 100), ("tf32", 128, 2, 1041), ("tf32", 256, 2, 8192),
+    ("fused", 256, 2, 256), ("fused", 200, 3, 100), ("unfused", 256, 2, 600), ("unfused", 200, 3, 1041), ("tf32", 128, 2, 1041),
+    ("tf32", 256, 2, 8192),
 ]
 
 
 def _update_agent(pkg, nets, H, L, B, path):
     agent = make_agent(pkg, nets, H, L, B, num_epochs=1)
-    if path == "coop":
-        agent.update_kernel = "coop"
-        assert agent._coop_ok(B)
     if path == "tf32":
         agent.precision = "tf32"
         assert agent._tc_learner_ok(B)
@@ -370,12 +367,12 @@ def test_adam_polyak_kernel_bit_exact_vs_oracle(pkg, lr):
             ("params_v", t, int((uv[total:total + n_online] != puv[total:total + n_online]).sum()))
 
 
-ADAM_PATHS = [("fused", 256, 2, 256), ("coop", 256, 2, 256), ("tf32", 128, 2, 1041)]
+ADAM_PATHS = [("fused", 256, 2, 256), ("tf32", 128, 2, 1041)]
 
 
 @pytest.mark.parametrize("path,H,L,B", ADAM_PATHS, ids=[c[0] for c in ADAM_PATHS])
 def test_update_path_adam_step_bit_exact(pkg, path, H, L, B):
-    """The Adam step inside the fused, cooperative and TF32 updates, from the device's own state: p_t == p_{t-1} +
+    """The Adam step inside the fused and TF32 updates, from the device's own state: p_t == p_{t-1} +
     (float32(-lr / bc1_t) * m_t) / (sqrt(v_t) / float32(sqrt(bc2_t)) + 1e-8f) bit for bit, at t = 4 and 5 with lr = 1e-5 (steps at which
     a step size formed from a float32 lr is one ulp off).  A third of the online parameters are set to 0 before the step, so the
     step is not absorbed."""

@@ -5,30 +5,19 @@ call the indices `[count, B]` equal `count` calls of `choice(n, B, replace=False
 equal `get_state()`: the kernel writes the stream back as an untempered block plus numpy's position convention, and a stream
 that ends on the last word of a block takes its own branch there (position 624 in the block before).  Covered: n up to the
 56 000-row limit, full permutations, the 150 draws of an update, start positions 0, 1, 623, 624, samples that end on the last
-and on the first word of a block, a multi-stream bank through the C ABI, numpy's global stream (cached Gaussian included),
-and the two development variants of the kernel.
+and on the first word of a block, a multi-stream bank through the C ABI and numpy's global stream (cached Gaussian included).
 
 Philox sampler (`rtd3_sample_indices_philox`, `ReplayBuffer.sampler = "philox"`): out[4t + k] = (r_k * n) >> 32 with
 r = Philox4x32-10((c lo, c hi, 0, 0), (seed lo, seed hi)), c = offset + t, restated on uint64 and pinned to oracle/philox.py;
 the host advances the offset by ceil(count * B / 4) per call.
-
-Run as a script (`python tests/test_sampler_exact_gpu.py legacy|wide`) it runs a reduced set of the exact-sampler cases in a
-process of its own, with the kernel variant that RTD3_SAMPLER_LEGACY / RTD3_SAMPLER_WIDE select (read once per process).
 """
 import math
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-if ROOT not in sys.path:
-    sys.path.insert(0, ROOT)
-
-from oracle import philox  # noqa: E402
+from oracle import philox
 
 pytestmark = pytest.mark.gpu
 MT_N = 624
@@ -389,45 +378,3 @@ def test_philox_td3_update_draws_once(pkg):
     assert len(used) == 1 and np.array_equal(used[0].cpu().numpy(), philox_indices(77, off0, n, B, count))
     assert np.array_equal(rb.sample_indices(5, 1).cpu().numpy(), philox_indices(77, off1, n, 5, 1))
 
-
-# ------------------------------------------------------------------------------------------------ development variants
-VARIANTS = {"legacy": ("RTD3_SAMPLER_LEGACY", "sample_swaps_kernel"), "wide": ("RTD3_SAMPLER_WIDE", "sample_swaps_pipelined_kernel<16>")}
-
-
-def run_variant_cases(pkg, variant):
-    """A reduced set of the cases above, in a process where the library chose `variant`; checks that its kernel ran."""
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        check_start(pkg, 97, 5, 624)
-        torch.cuda.synchronize()
-    names = [e.key for e in prof.key_averages()]
-    assert any(VARIANTS[variant][1] in k for k in names), names
-    for n in (2, 16385, MAX_N):
-        check_sizes(pkg, n, 1)
-    check_update_count(pkg, 10000, 100)
-    for pos in (0, 1, 623, 624):
-        check_start(pkg, 10000, 100, pos)
-    check_block_end(pkg, 100, 7, 3, MT_N)
-    check_block_end(pkg, 10000, 100, 2, MT_N)
-    check_block_end(pkg, 100, 7, 3, 1)
-    check_block_end_inside(pkg, 100, 7)
-    check_n1_unchanged(pkg)
-
-
-@pytest.mark.parametrize("variant", sorted(VARIANTS))
-def test_development_variants(variant):
-    env = dict(os.environ)
-    for var, _ in VARIANTS.values():
-        env.pop(var, None)
-    env[VARIANTS[variant][0]] = "1"
-    flags = [f for f, on in (("-s", sys.flags.no_user_site), ("-E", sys.flags.ignore_environment)) if on]   # start as this one did
-    res = subprocess.run([sys.executable, *flags, os.path.abspath(__file__), variant], env=env, cwd=ROOT, capture_output=True,
-                         text=True, timeout=900)
-    assert res.returncode == 0, res.stdout[-4000:] + res.stderr[-4000:]
-    assert "variant %s ok" % variant in res.stdout
-
-
-if __name__ == "__main__":
-    import importlib
-    run_variant_cases(importlib.import_module("rtd3_b200"), sys.argv[1])
-    print("variant %s ok" % sys.argv[1])

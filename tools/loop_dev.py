@@ -1,5 +1,5 @@
 """Deviation profile of the whole reference run (tests/test_loop_gpu.py::test_whole_driver_loop_vs_reference): max |state - reference|
-per number of completed TD3 updates, for the learner path selected by the environment (RTD3_CLUSTER=0: row-tile kernels)."""
+per number of completed TD3 updates."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch, rtd3_b200 as pkg
