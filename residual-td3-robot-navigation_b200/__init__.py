@@ -9,8 +9,8 @@ from .rng import MtBank  # noqa: F401
 from .learner import ReplayBuffer, Residual_Actor_Network, Residual_Critic_Network, TD3  # noqa: F401
 from .robot import Robot  # noqa: F401
 from .trainer import BatchedTrainer, DriverLoop, shard_range  # noqa: F401
-from .checkpoint import load_checkpoint, save_checkpoint  # noqa: F401
+from .checkpoint import PendingCheckpoint, load_checkpoint, save_checkpoint  # noqa: F401
 
 __all__ = ["Environment", "MtBank", "synthetic_maps", "perlin_maps_device", "constants", "configuration", "ReplayBuffer",
            "Residual_Actor_Network", "Residual_Critic_Network", "TD3", "Robot", "BatchedTrainer", "DriverLoop", "shard_range",
-           "save_checkpoint", "load_checkpoint"]
+           "save_checkpoint", "PendingCheckpoint", "load_checkpoint"]

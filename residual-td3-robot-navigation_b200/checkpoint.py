@@ -9,13 +9,22 @@ contains.  Loading goes into an existing object of the same configuration: every
 then tensors are copied in place, so CUDA graphs the objects have captured stay valid.  What is not stored - data derived from the
 stored state and rebuilt on load, scratch and process-local state - is listed per class in NOT_SAVED.
 
+Each `*_state(obj, take)` is the one definition of what is stored: it runs the guards, synchronises, reads the host values and
+applies `take` to every stored tensor.  A synchronous save takes CPU copies (`_host`).  A background save
+(`save_checkpoint(..., background=True)`) collects the live tensors (`_live`), stages them in device memory with stream-ordered
+copies (`_stage`) and returns; a writer thread copies the staging to pinned host memory on a side stream (`_pinned`), frees it and
+writes the file.
+
 RNG state is part of the run: every MT19937 bank, the Philox offsets and counters, and - for objects that draw from numpy's global
 stream (a single env or robot without a seed) - numpy's global state, which `load_state_dict` RESTORES (a process-wide side effect,
 as the reference draws everything from that stream).  With `noise="randn"` the trainer saves and restores torch's CUDA generator.
 """
+import atexit
 import json
 import os
 import tempfile
+import threading
+import weakref
 
 import numpy as np
 import torch
@@ -73,8 +82,36 @@ def _host(t):
     return t.detach().cpu() if t.is_cuda else t.detach().clone()
 
 
-def _tensors(obj, names):
-    return {k: _host(_get(obj, k)) for k in names}
+def _live(t):
+    """The tensor itself: a background save collects the state with this `take`, then stages the tensors (`_stage`)."""
+    return None if t is None else t.detach()
+
+
+def _stage(t):
+    """A copy of a tensor on its own device: stream-ordered on the current stream for a device tensor."""
+    return t.clone()
+
+
+def _pinned(t):
+    """A pinned host copy of a device tensor, enqueued on the current stream (a background save's writer thread)."""
+    if not t.is_cuda:
+        return t
+    return torch.empty_like(t, device="cpu", pin_memory=True).copy_(t, non_blocking=True)
+
+
+def _map(sd, fn):
+    """`sd` with `fn` applied to every tensor in it."""
+    if isinstance(sd, torch.Tensor):
+        return fn(sd)
+    if isinstance(sd, dict):
+        return {k: _map(v, fn) for k, v in sd.items()}
+    if isinstance(sd, (list, tuple)):
+        return type(sd)(_map(v, fn) for v in sd)
+    return sd
+
+
+def _tensors(obj, names, take=_host):
+    return {k: take(_get(obj, k)) for k in names}
 
 
 def _check_tensor(t, dtype, shape, what):
@@ -148,14 +185,14 @@ def _quiescent(device):
 
 
 # ---------------------------------------------------------------------------------------------------------------- ReplayBuffer
-def replay_state(rb):
+def replay_state(rb, take=_host):
     if rb._in_session:
         raise RuntimeError("cannot save a ReplayBuffer inside an open sampling session")
     _quiescent(rb.device)
     host = {"sampler": rb.sampler, "philox_seed": rb._philox_seed, "philox_offset": rb._philox_offset,
             "numpy": _numpy_state() if rb._numpy_global else None}
     return {"meta": {"class": "ReplayBuffer", "version": FORMAT_VERSION, "capacity": rb.capacity, "numpy_global": rb._numpy_global},
-            "tensors": _tensors(rb, _REPLAY), "host": host}
+            "tensors": _tensors(rb, _REPLAY, take), "host": host}
 
 
 def replay_plan(rb, sd):
@@ -177,12 +214,12 @@ def replay_plan(rb, sd):
 
 
 # ---------------------------------------------------------------------------------------------------------------- TD3
-def td3_state(td3):
+def td3_state(td3, take=_host):
     _quiescent(td3.device)
     rank, world = _rank_world(td3)
-    last = None if td3.last_losses is None else [_host(x) for x in td3.last_losses]
+    last = None if td3.last_losses is None else [take(x) for x in td3.last_losses]
     return {"meta": {"class": "TD3", "version": FORMAT_VERSION, "hidden": td3.hidden, "layers": td3.layers, "rank": rank, "world": world},
-            "tensors": _tensors(td3, _TD3),
+            "tensors": _tensors(td3, _TD3, take),
             "host": {"noise_steps": td3._noise_steps, "noise_seed": td3.noise_seed, "last_losses": last}}
 
 
@@ -252,11 +289,11 @@ def import_networks(td3, d):
 
 
 # ---------------------------------------------------------------------------------------------------------------- Environment
-def env_state(env):
+def env_state(env, take=_host):
     _quiescent(env.device)
     names = _ENV + (("_map_seeds",) if env._map_seeds is not None else ("_speed_dev", "_angle_dev"))
-    t = _tensors(env, names)
-    t["_map_index"] = _host(env._map_index)
+    t = _tensors(env, names, take)
+    t["_map_index"] = take(env._map_index)
     host = {"numpy": _numpy_state() if env._numpy_global else None,
             "state_np": None if env._state_np is None else torch.from_numpy(np.array(env._state_np, dtype=np.float64))}
     return {"meta": {"class": "Environment", "version": FORMAT_VERSION, "num_envs": env.num_envs, "num_maps": env.num_maps,
@@ -309,15 +346,15 @@ def env_plan(env, sd):
 
 
 # ---------------------------------------------------------------------------------------------------------------- Robot
-def robot_state(robot):
+def robot_state(robot, take=_host):
     _quiescent(robot.device)
-    t = _tensors(robot, _ROBOT)
+    t = _tensors(robot, _ROBOT, take)
     d = robot._env_demo
     env_demo = None
     if d is not None:
         k = int(d["count"].max()) if robot.num_envs else 0
-        t["_env_demo.sets"] = d["sets"][:, :k].cpu()
-        t["_env_demo.count"] = d["count"].cpu()
+        t["_env_demo.sets"] = take(d["sets"][:, :k])
+        t["_env_demo.count"] = take(d["count"])
         env_demo = {"cap": int(d["cap"]), "demos": int(d["demos"])}
     arr = lambda rows: None if not rows else torch.from_numpy(np.asarray([np.asarray(r, dtype=np.float64) for r in rows], dtype=np.float64))
     snap = None
@@ -329,7 +366,7 @@ def robot_state(robot):
             "snap": snap, "numpy": _numpy_state() if robot._numpy_global else None}
     return {"meta": {"class": "Robot", "version": FORMAT_VERSION, "num_envs": robot.num_envs, "batched": robot.batched,
                      "numpy_global": robot._numpy_global},
-            "tensors": t, "host": host, "memory": replay_state(robot.memory), "td3_agent": td3_state(robot.td3_agent)}
+            "tensors": t, "host": host, "memory": replay_state(robot.memory, take), "td3_agent": td3_state(robot.td3_agent, take)}
 
 
 def robot_plan(robot, sd):
@@ -411,7 +448,7 @@ def _load_env_demo(robot, ed, t):
 
 
 # ---------------------------------------------------------------------------------------------------------------- BatchedTrainer
-def trainer_state(tr):
+def trainer_state(tr, take=_host):
     _quiescent(tr.device)
     rank, world = _rank_world(tr.robot.td3_agent)
     names = _TRAINER + (_SCHEDULER if tr.scheduler else ())
@@ -419,7 +456,7 @@ def trainer_state(tr):
             "cuda_rng": torch.cuda.get_rng_state(tr.device) if tr.noise == "randn" else None}
     return {"meta": {"class": "BatchedTrainer", "version": FORMAT_VERSION, "num_envs": tr.n, "noise": tr.noise, "scheduler": tr.scheduler,
                      "rank": rank, "world": world},
-            "tensors": _tensors(tr, names), "host": host, "env": env_state(tr.env), "robot": robot_state(tr.robot)}
+            "tensors": _tensors(tr, names, take), "host": host, "env": env_state(tr.env, take), "robot": robot_state(tr.robot, take)}
 
 
 def trainer_plan(tr, sd):
@@ -445,11 +482,11 @@ def trainer_plan(tr, sd):
 
 
 # ---------------------------------------------------------------------------------------------------------------- DriverLoop
-def loop_state(loop):
+def loop_state(loop, take=_host):
     host = {k: float(v) if isinstance(v, float) else v for k, v in ((k, getattr(loop, k)) for k in _LOOP_HOST)}   # numpy floats -> float
     host["state"] = torch.from_numpy(np.array(loop.state))
     return {"meta": {"class": "DriverLoop", "version": FORMAT_VERSION, "num_envs": loop.environment.num_envs},
-            "tensors": {}, "host": host, "env": env_state(loop.environment), "robot": robot_state(loop.robot)}
+            "tensors": {}, "host": host, "env": env_state(loop.environment, take), "robot": robot_state(loop.robot, take)}
 
 
 def loop_plan(loop, sd):
@@ -539,32 +576,24 @@ def _read(path):
     return payload
 
 
-def save_checkpoint(path, obj):
-    """Save `obj` (any of the six classes, with everything it contains) to `path`; returns `path`.
-
-    Single process: one file, written atomically.  Data parallel (the learner has a process group of world > 1): collective, `path`
-    is a directory; every rank writes `rank{r}.pt` (its env shard, robot, replay shard and learner copy), then rank 0 writes
-    `manifest.json` (world, format version, per-rank num_envs).  The manifest is removed before the rank files are written, so a
-    directory whose save was interrupted does not load."""
-    name, save, _ = _kind(obj)
-    sd = save(obj)
-    payload = {"meta": _summary(obj), "state": sd}
-    td3 = _learner(obj)
-    rank, world = _rank_world(td3) if td3 is not None else (0, 1)
-    if world == 1:
-        _atomic_save(payload, path)
-        return path
+def _clear_manifest(pg, rank, path):
+    """Data parallel, before the rank files are written (collective): rank 0 removes the manifest, so a directory whose save is
+    interrupted does not load."""
     import torch.distributed as dist
-    pg = td3.process_group
     manifest = os.path.join(path, "manifest.json")
     if rank == 0:
         os.makedirs(path, exist_ok=True)
         if os.path.exists(manifest):
             os.unlink(manifest)
     dist.barrier(group=pg)
-    _atomic_save(payload, os.path.join(path, "rank%d.pt" % rank))
+
+
+def _write_manifest(pg, rank, world, path, name, num_envs):
+    """Data parallel, once every rank file is written (collective): rank 0 writes the manifest."""
+    import torch.distributed as dist
+    manifest = os.path.join(path, "manifest.json")
     sizes = [None] * world
-    dist.all_gather_object(sizes, payload["meta"]["num_envs"], group=pg)
+    dist.all_gather_object(sizes, num_envs, group=pg)
     if rank == 0:
         tmp = manifest + ".tmp"
         with open(tmp, "w") as f:
@@ -573,7 +602,140 @@ def save_checkpoint(path, obj):
             os.fsync(f.fileno())
         os.replace(tmp, manifest)
     dist.barrier(group=pg)
+
+
+def save_checkpoint(path, obj, background=False):
+    """Save `obj` (any of the six classes, with everything it contains) to `path`; returns `path`.
+
+    Single process: one file, written atomically.  Data parallel (the learner has a process group of world > 1): collective, `path`
+    is a directory; every rank writes `rank{r}.pt` (its env shard, robot, replay shard and learner copy), then rank 0 writes
+    `manifest.json` (world, format version, per-rank num_envs).  The manifest is removed before the rank files are written, so a
+    directory whose save was interrupted does not load.
+
+    `background=True` returns a `PendingCheckpoint` as soon as the state is snapshot into device memory: the device->host copies
+    and the file write run in a writer thread while training continues.  The file is the one a synchronous save at the call would
+    write.  Device memory for the stored state is needed twice until the writer has copied it out (RuntimeError, nothing done,
+    when `torch.cuda.mem_get_info` reports less free); a second background save of the same object first waits for the first's
+    writer.  Data parallel, the call and `PendingCheckpoint.wait()` are collective; the writers never use the process group."""
+    name, save, _ = _kind(obj)
+    if background:
+        return _save_background(path, obj, name, save)
+    sd = save(obj)
+    payload = {"meta": _summary(obj), "state": sd}
+    td3 = _learner(obj)
+    rank, world = _rank_world(td3) if td3 is not None else (0, 1)
+    if world == 1:
+        _atomic_save(payload, path)
+        return path
+    pg = td3.process_group
+    _clear_manifest(pg, rank, path)
+    _atomic_save(payload, os.path.join(path, "rank%d.pt" % rank))
+    _write_manifest(pg, rank, world, path, name, payload["meta"]["num_envs"])
     return path
+
+
+# ---------------------------------------------------------------------------------------------------------------- background saves
+_PENDING = weakref.WeakKeyDictionary()          # object -> its latest background save
+_WRITERS = []                                   # writer threads not yet seen finished
+
+
+@atexit.register
+def _join_writers():
+    """A process that exits with a background save pending still finishes the file."""
+    for t in list(_WRITERS):
+        t.join()
+
+
+class PendingCheckpoint:
+    """A checkpoint being written in the background, returned by `save_checkpoint(path, obj, background=True)`.
+
+    `done()` tells whether this process's writer thread has finished.  `wait()` returns `path` once the file is complete, or
+    re-raises the writer's exception (the file at `path` is then as it was).  Data parallel, `wait()` is collective: every rank joins
+    its writer, then rank 0 writes the manifest if every rank wrote its file; if any rank failed there is no manifest and every
+    rank raises."""
+
+    def __init__(self, path, file, staged, meta, device, event, finish):
+        self.path = path
+        self._finish, self._error, self._waited = finish, None, False
+        self._thread = threading.Thread(target=self._drain, args=(file, staged, meta, device, event), name="rtd3-checkpoint-writer")
+        _WRITERS[:] = [t for t in _WRITERS if t.is_alive()] + [self._thread]
+        self._thread.start()
+
+    def _drain(self, file, staged, meta, device, event):
+        """The writer thread: device->host copies on a side stream once the snapshot is complete, the staging freed, then the file."""
+        try:
+            with torch.cuda.device(device):
+                side = torch.cuda.Stream(device)
+                side.wait_event(event)
+                try:
+                    with torch.cuda.stream(side):
+                        state = _map(staged[0], _pinned)
+                finally:
+                    side.synchronize()
+                    staged.clear()                      # the last reference to the device staging
+            _atomic_save({"meta": meta, "state": state}, file)
+        except BaseException as e:                      # noqa: B036 - handed to wait()
+            self._error = e
+
+    def done(self):
+        return not self._thread.is_alive()
+
+    def wait(self):
+        if not self._waited:
+            self._thread.join()
+            if self._finish is not None:
+                self._error = self._finish(self._error)
+            self._waited = True
+        if self._error is not None:
+            raise self._error
+        return self.path
+
+
+def _save_background(path, obj, name, save):
+    """The call of a background save: the synchronous save's guards and host reads, a size check, then device->device copies of
+    every stored tensor on the current stream and an event the writer thread waits on."""
+    prev = _PENDING.get(obj)
+    if prev is not None:
+        prev._thread.join()                             # at most one staging copy of an object's state
+    live = save(obj, _live)                             # refuses a capture or an open session, synchronises, reads host values
+    meta = _summary(obj)
+    leaves = []
+    _map(live, leaves.append)
+    cuda = [t for t in leaves if t.is_cuda]
+    device = cuda[0].device
+    need = sum(t.numel() * t.element_size() for t in cuda)
+    free = torch.cuda.mem_get_info(device)[0]
+    td3 = _learner(obj)
+    rank, world = _rank_world(td3) if td3 is not None else (0, 1)
+    fits = need <= free
+    if world > 1:                                       # every rank goes on, or none does
+        import torch.distributed as dist
+        flag = torch.tensor([int(fits)], dtype=torch.int32, device=td3.device)
+        dist.all_reduce(flag, op=dist.ReduceOp.MIN, group=td3.process_group)
+        if fits and not int(flag.item()):
+            raise RuntimeError("background checkpoint: another rank lacks the device memory for its snapshot")
+    if not fits:
+        raise RuntimeError("background checkpoint: the snapshot needs %.2f GB of device memory, %.2f GB are free; save with "
+                           "background=False" % (need / 1e9, free / 1e9))
+    file, finish = path, None
+    if world > 1:
+        pg = td3.process_group
+        _clear_manifest(pg, rank, path)
+        file = os.path.join(path, "rank%d.pt" % rank)
+
+        def finish(error):
+            import torch.distributed as dist
+            ok = torch.tensor([0 if error else 1], dtype=torch.int32, device=td3.device)
+            dist.all_reduce(ok, op=dist.ReduceOp.MIN, group=pg)
+            if not int(ok.item()):
+                return error or RuntimeError("%s: another rank failed to write its checkpoint file" % path)
+            _write_manifest(pg, rank, world, path, name, meta["num_envs"])
+            return None
+    staged = [_map(live, _stage)]
+    event = torch.cuda.Event()
+    event.record(torch.cuda.current_stream(device))
+    pending = _PENDING[obj] = PendingCheckpoint(path, file, staged, meta, device, event, finish)
+    return pending
 
 
 def load_checkpoint(path, obj):
